@@ -24,6 +24,7 @@ round 1's Poisson surrogate (iid gaps, uniform nodes; SURVEY.md section 8d).  Ev
   python bench.py [--gpus N] [--steps K] [--warmup W]           (torchrun launches N > 1)
   python bench.py --impl reference ...                          (CPU oracle arm, all host threads)
   python bench.py --config {2,3,5} ...                          (the other BASELINE configs as their own line)
+  python bench.py --dump-outputs DIR ...                        (also write the last timed step's outputs as DIR/<name>.npy)
 """
 import argparse
 import ctypes
@@ -50,6 +51,7 @@ BYTES_EXTRA_WLEN, BYTES_EXTRA_POFF = 2.0, 4.0     # implementation extras, state
 BYTES_PER_ADJ_PAIR = 10.0                         # cached adjacency structure: u16 event index + f64 lag per (child event, window predecessor);
                                                   # 18 B with the LogitNormal payload (u16 + logit + Jacobian) -- the form the library reports is used
 SEED = 20261018
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much
 
 
 def parse():
@@ -69,7 +71,14 @@ def parse():
     ap.add_argument("--cpu-adj-sample", type=float, default=1e5, help="events of the CPU-baseline sample of the adjacency sweep")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config table (cfg2 / cfg3 / cfg5 shape) of the default N = 1 run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (its log-likelihood and the sample of its Gibbs sweep) as DIR/<name>.npy in float64, "
+                         "to compare two builds output for output (config 4, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "ours" or args.config != 4):
+        ap.error("--dump-outputs is implemented for the headline workload (--config 4, --impl ours)")
     args.events_given = args.events is not None
     if args.events is None:
         args.events = 1e8
@@ -463,6 +472,8 @@ def run_ours(args, rank, world, local_rank):
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
     total_ms = float(tmax.item())
     value = n_total * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_step_outputs(ctx, K, ll_last))
 
     # ---- full-size checks (size-independent properties on the whole timed stream; outside the timed region):
     #      the two independent log-likelihood algorithms agree (window sweep over the time-sorted stream vs the active buckets of the
@@ -665,6 +676,32 @@ def run_ours(args, rank, world, local_rank):
     if world > 1:
         lib.nhp_comm_destroy(ctx.h)
         dist.destroy_process_group()
+
+
+def last_step_outputs(ctx, K, ll):
+    """What a caller of the timed step receives: its log-likelihood and the sample its Gibbs sweep leaves in the context
+    (nhp_cont_params_get, nhp_cont_network_get), matrices as X[parent, child]."""
+    from nhp_b200.core import _ptr
+    l0, W, A, mu, tau = np.empty(K), np.empty(K * K), np.empty(K * K), np.empty(K * K), np.empty(K * K)
+    ctx.check(ctx.lib.nhp_cont_params_get(ctx.h, _ptr(l0), _ptr(W), _ptr(A), _ptr(mu), _ptr(tau)))
+    rho = ctypes.c_double()
+    ctx.check(ctx.lib.nhp_cont_network_get(ctx.h, ctypes.byref(rho)))
+    unf = lambda v: v.reshape(K, K).T
+    return {"loglik": np.array([ll]), "rho": np.array([rho.value]), "lambda0": l0, "W": unf(W), "A": unf(A), "mu": unf(mu), "tau": unf(tau)}
+
+
+def dump_outputs(out_dir, arrays):
+    """out_dir/<name>.npy in float64, DUMP_BYTES at most in all: past that budget an array larger than its even share is written as
+    its entries at a fixed, seeded set of flat positions (in ascending order), the same positions in every run of the same shape."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    budget = DUMP_BYTES - 1024 * len(arrays)  # room for the .npy headers
+    share = budget // (8 * len(arrays))
+    sample = sum(a.nbytes for a in arrays.values()) > budget
+    for name, a in arrays.items():
+        if sample and a.size > share:
+            a = a.ravel()[np.sort(np.random.default_rng(SEED).choice(a.size, share, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def parity_check(args, ctx, params, h_t, h_c):
