@@ -1227,11 +1227,18 @@ template <int KIND, int PRE> __global__ void __launch_bounds__(ADJ_THREADS, 1) k
     if (tid == 0) { a.partials[2 * (size_t)blockIdx.x] = total; a.partials[2 * (size_t)blockIdx.x + 1] = 0.0; }
 }
 
-// Log-likelihood through the cached structure when it exists for this handle, covers every column and the horizon, and the
-// network is sparse enough that streaming its active buckets beats the window sweep.  Returns 1 when it does not apply.
+// The structure of a handle was built for one model: its payload is read as lags by an Exponential kernel and as the LogitNormal
+// terms of its build-time dtmax by the 18-byte kernels, so it serves only a model of the same impulse kind (and dtmax, for that payload).
+static bool adj_payload_fits(const nhp_ctx *ctx, const nhp_events *ev) {
+    return ev->adj_impulse == ctx->kind && (ev->adj_kind != 1 || ev->adj_D == ctx->dtmax);
+}
+
+// Log-likelihood through the cached structure when it exists for this handle and model, covers every column and the horizon, and
+// the network is sparse enough that streaming its active buckets beats the window sweep.  Returns 1 when it does not apply.
 int nhp_cont_try_adj_loglik(nhp_ctx *ctx, nhp_events *ev, SweepArgs &sa, int *grid_out, int cb, int cs) {  // structure of the columns c % cs == cb: their share
     { const char *e = getenv("NHP_ADJ_LOGLIK"); if (e && atoi(e) == 0) return 1; }
     if (!ctx->has_A || !ev->d_adj_i || ev->adj_cb != cb || ev->adj_cs != cs || ev->n_halo != 0 || ev->adj_cluster < 0 || sa.lam0ev) return 1;
+    if (!adj_payload_fits(ctx, ev)) return 1;
     if (!(ctx->density <= 0.25) || !(ev->adj_horizon >= sa.horizon) || sa.jmin > 0) return 1;
     if (ctx->kind == NHP_EXPONENTIAL && ev->adj_horizon != sa.horizon && !(sa.horizon < ctx->dtmax)) return 1;  // only a cut-off horizon may be exceeded
     const int64_t K = ctx->K;
@@ -1494,6 +1501,7 @@ static int adj_build_structure(nhp_ctx *ctx, nhp_events *ev, double horizon, int
     if (flag & 128) return fail(nhp_fail(ctx, NHP_ERR_CUDA, "adjacency sampler: structure build disagrees with its own count (internal error)"));
     ev->adj_total = tot; ev->adj_pairs = pairs; ev->adj_nv = nv; ev->adj_horizon = horizon; ev->adj_cb = cb; ev->adj_cs = cs;
     ev->adj_chunk_cap = chunk_cap; ev->adj_chunk_max = chunk_max; ev->adj_cluster = cluster; ev->adj_kind = pre ? 1 : 0;
+    ev->adj_impulse = ctx->kind; ev->adj_D = ctx->dtmax;
     ctx->adj_info[7] = bms;
     return NHP_OK;
 #undef ADJ_B
@@ -1624,7 +1632,7 @@ static int adj_run(nhp_ctx *ctx, nhp_events *ev, const double *d_rho, double rho
     // predecessors whose (tiny) contributions are simply included.  With a parameter-dependent horizon (Exponential cut-off,
     // which moves with every conjugate draw) it is built with a 25 % margin so that a chain does not rebuild it every sweep.
     const bool moving = ctx->kind == NHP_EXPONENTIAL && horizon < ctx->dtmax;
-    const bool have_cache = cached && ev->d_adj_i && ev->adj_cb == (int)col_begin && ev->adj_cs == (int)col_stride && ev->adj_chunk_cap == chunk_cap &&
+    const bool have_cache = cached && ev->d_adj_i && adj_payload_fits(ctx, ev) && ev->adj_cb == (int)col_begin && ev->adj_cs == (int)col_stride && ev->adj_chunk_cap == chunk_cap &&
                             (moving ? (ev->adj_horizon >= horizon && ev->adj_horizon <= 2.0 * horizon) : ev->adj_horizon == horizon);
     if (cached && !have_cache) {
         if (moving) horizon = std::min(ctx->dtmax, 1.25 * horizon);

@@ -336,7 +336,7 @@ void nhp_events_free_adjacency(nhp_ctx *ctx, nhp_events *ev, cudaStream_t s) {
     for (void *b : blocks) if (b) cudaFreeAsync(b, s);
     ev->d_adj_vstart = ev->d_adj_vnode = ev->d_adj_boff = nullptr; ev->d_adj_vbase = nullptr; ev->d_adj_i = nullptr;
     ev->d_adj_dt = ev->d_adj_q = ev->d_adj_lam = nullptr;
-    ev->adj_horizon = -1.0; ev->adj_total = 0; ev->adj_nv = 0;
+    ev->adj_horizon = -1.0; ev->adj_impulse = -1; ev->adj_D = 0.0; ev->adj_total = 0; ev->adj_nv = 0;
 }
 
 extern "C" int nhp_events_free(nhp_ctx *ctx, nhp_events *ev) {

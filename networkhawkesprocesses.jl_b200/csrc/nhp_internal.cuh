@@ -87,8 +87,12 @@ struct nhp_events {
     int64_t n_items = 0;
     // cached structure of the adjacency sampler (cont_adjacency.cu): every (child event, window predecessor) pair, grouped by
     // virtual column = (child column, time chunk of at most adj_chunk_cap of the column's events) and bucketed by parent node,
-    // stably ordered (event, window position) inside a bucket; depends on the data and the look-back horizon only
+    // stably ordered (event, window position) inside a bucket.  The pairs depend on the data and the look-back horizon; the
+    // payload also on the impulse kind it was built for (lags, or LogitNormal terms of the build-time dtmax), so a model of another
+    // kind, or a LogitNormal model of another dtmax, must not read it
     double adj_horizon = -1.0;       // horizon the structure was built with
+    int adj_impulse = -1;            // impulse kind (NHP_EXPONENTIAL / NHP_LOGITNORMAL) it was built for
+    double adj_D = 0.0;              // dtmax it was built for (the LogitNormal payload holds logit(dt / D), 1 / (dt (D - dt)))
     int adj_cb = 0, adj_cs = 1;      // column partition it was built for
     int adj_chunk_cap = 0;           // chunk capacity (child events) it was built with
     int adj_chunk_max = 0;           // largest chunk actually present (sizes the sweep's shared memory)
