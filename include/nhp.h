@@ -90,8 +90,10 @@ int nhp_cont_params_set(nhp_ctx *ctx, int kind, int64_t K, const double *lambda0
  * log-likelihood, intensity and parent sweeps of the context use lambda0_k(t_i) as the baseline rate of event i (parent weights:
  * "baseline last", parents.jl:25-46) and sum_k integrate(lambda0_k) (trapezoid, baselines.jl:336) as the baseline compensator; an
  * event or query time outside [x[0], x[n_grid-1]] is an error (the reference throws a DomainError).  n_grid = 0 returns to the
- * homogeneous lambda0; nhp_cont_params_set also does (re-apply the curves after it).  The adjacency sampler and the analytic
- * gradient take a homogeneous baseline (NHP_ERR_UNSUPPORTED otherwise). */
+ * homogeneous lambda0; nhp_cont_params_set also does (re-apply the curves after it).  The adjacency sampler and the structure
+ * log-likelihood of a network process read lambda0_k(t_i) as well (the sampler returns NHP_ERR_NUMERIC, before changing anything,
+ * when a curve is zero at an event of a column it sweeps); the analytic gradient takes a homogeneous baseline (NHP_ERR_UNSUPPORTED
+ * otherwise).  While the curves are set, the Exponential cut-off horizon measures the omitted tail against their smallest value. */
 int nhp_cont_baseline_grid(nhp_ctx *ctx, int64_t n_grid, const double *x, const double *values);
 /* The likelihood of the elliptical-slice update of the curves (baselines.jl:214-254: resample!(::LogGaussianCoxProcess) =
  * split_extract + loglikelihood per node), for all K nodes at once and for CANDIDATE curves `values` on grid `x`:
@@ -238,7 +240,8 @@ int nhp_comm_allgather_adjacency(nhp_ctx *ctx);
 int nhp_comm_allgather_events(nhp_ctx *ctx, nhp_events *ev_shard, nhp_events **out);
 /* hyper as for nhp_cont_resample_params; net_alpha > 0: BernoulliNetworkModel with rho ~ Beta(net_alpha, net_beta) prior
  * (networks.jl:45-54, 72-78), else link probability 1 (DenseNetworkModel).  ev_full (the unsharded stream, replicated on
- * every rank) is only used by network processes; pass ev_shard itself on a single GPU. */
+ * every rank) is only used by network processes; pass ev_shard itself on a single GPU.  A network process with grid baseline
+ * curves (nhp_cont_baseline_grid) is refused with NHP_ERR_UNSUPPORTED before anything changes: the curves are not drawn here. */
 int nhp_cont_gibbs_sweep(nhp_ctx *ctx, nhp_events *ev_shard, nhp_events *ev_full, uint64_t seed, uint64_t counter, double duration,
                          const double *hyper, int n_hyper, double net_alpha, double net_beta);
 /* Device pointer + length (in doubles) of a statistics buffer, for hosts that run their own collectives. */

@@ -231,6 +231,10 @@ extern "C" int nhp_cont_gibbs_sweep(nhp_ctx *ctx, nhp_events *ev_shard, nhp_even
                                     const double *hyper, int n_hyper, double net_alpha, double net_beta) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
     NHP_CHECK(ctx, ev_shard != nullptr, NHP_ERR_INVALID, "nhp_cont_gibbs_sweep: events handle is NULL");
+    // the draws here are the conjugate ones; the curves of a LogGaussianCoxProcess baseline move with the host's elliptical slice
+    // sampler (resample_on_device_), so a network process with curves is refused before anything changes
+    NHP_CHECK(ctx, !(ctx->cont_set && ctx->has_A && ctx->bgrid_n > 0), NHP_ERR_UNSUPPORTED,
+              "nhp_cont_gibbs_sweep: a network process with a grid baseline takes the elliptical-slice update of its curves on the host");
     for (int i = 0; i < 8; i++) ctx->sweep_info[i] = 0.0;
     NHP_TRY(nhp_cont_resample_parents(ctx, ev_shard, seed, counter, nullptr, nullptr, nullptr));
     ctx->sweep_info[0] = ctx->last_ms;  // parent sweep + fused statistics

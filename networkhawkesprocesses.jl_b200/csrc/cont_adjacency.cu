@@ -3,11 +3,13 @@
 // The reference evaluates, for every (p, c), two full passes over all N events (2 K^2 N work).  The
 // conditional it samples from only depends on the child events on c whose window holds an event of
 // node p:  with G_i[p] = W[p,c] sum_{j in win(i), c_j = p} h_pc(t_i - t_j)  and
-// lambda_i = lambda0_c + sum_p A[p,c] G_i[p],
+// lambda_i = lambda0_c(t_i) + sum_p A[p,c] G_i[p]  (lambda0_c(t_i) = lambda0_c for a homogeneous baseline),
 //     ll1 - ll0 = -W[p,c] n_p + sum_{i on c, G_i[p] > 0} [ log(lambda_i^{-p} + G_i[p]) - log(lambda_i^{-p}) ]
 //                 + log rho - log(1 - rho),          A[p,c] ~ Bernoulli(exp(ll1 - logsumexp(ll0, ll1))),
 // p = 1..K sequentially inside a column, columns independent (the reference's Threads.@threads axis).
-// Same conditional distribution, O(N w) work per sweep instead of O(K^2 N).
+// Same conditional distribution, O(N w) work per sweep instead of O(K^2 N).  The baseline integral cancels in ll1 - ll0: a grid
+// baseline (LogGaussianCoxProcess) only changes the intensities a column starts from (the per-event rates in by-node order) and the
+// lower bound lambda0min_c = min over the column's events of lambda0_c(t_i) that the certification and the ON-bucket floor use.
 //
 // Cached form (default; k_adj_build + k_adj_sweep).  WHICH (child event, window predecessor) pairs exist, and their
 // lags, depends on the data and the look-back horizon only, so the pairs are bucketed once per events handle:
@@ -23,7 +25,7 @@
 // current lambda, every CTA's partial sums travel through distributed shared memory to all CTAs of the cluster (one cluster
 // barrier per batch), each CTA then takes the same decisions in order and accepts them as far as they can be CERTIFIED: a
 // flip moves every intensity by at most its bucket's largest contribution, which bounds a later sum S from both sides,
-// S / (1 + on / lambda0) <= S' <= S (1 + off / lambda0); a decision whose margin exceeds its side's bound is the decision of
+// S / (1 + on / lambda0min_c) <= S' <= S (1 + off / lambda0min_c); a decision whose margin exceeds its side's bound is the decision of
 // the sequential sweep (see the decision block of k_adj_sweep).  The batch is cut at the first bucket that cannot be
 // certified and restarts there; the accepted flips are applied (S follows the observed restart rate, down to 1, the plain
 // sequential sweep).  The result is exactly that of the sequential sweep.  The log terms are
@@ -45,6 +47,7 @@ struct AdjArgs {
     const double *Mn;        // [K] events per node
     int K; const void *table_w;  // table without the adjacency factor
     const double *lambda0; const double *W; double *A;  // A: [K*K] parent-major as passed, updated in place
+    const double *lam0bn, *lam0min;  // grid baseline: per-event rates in by-node order, per-node minima (NULL: lambda0)
     const double *rho; const double *u; uint64_t seed, counter;
     double D, horizon, duration;
     int64_t cap;             // scratch entries per CTA
@@ -82,7 +85,7 @@ template <int KIND> __global__ void __launch_bounds__(256) k_adjacency(const Adj
     for (int c = a.col_begin + blockIdx.x * a.col_stride; c < a.K; c += gridDim.x * a.col_stride) {
         const int e0 = a.node_ptr[c], e1 = a.node_ptr[c + 1];
         const E *col = reinterpret_cast<const E *>(a.table_w) + (size_t)c * a.K;
-        const double lam0 = a.lambda0[c];
+        const double lam0 = a.lam0min ? a.lam0min[c] : a.lambda0[c];  // lower bound of every event's baseline rate
         // ---- A1: bucket sizes
         for (int k = threadIdx.x; k <= a.K; k += blockDim.x) s_off[k] = 0;
         __syncthreads();
@@ -120,7 +123,7 @@ template <int KIND> __global__ void __launch_bounds__(256) k_adjacency(const Adj
                 s += a.A[p + (int64_t)a.K * c] * v;
             }
             s = warp_sum(s);
-            if (lane == 0) { lam[e - e0] = lam0 + s; gacc[e - e0] = 0.0; }
+            if (lane == 0) { lam[e - e0] = (a.lam0bn ? a.lam0bn[e] : lam0) + s; gacc[e - e0] = 0.0; }
         }
         __syncthreads();
         // ---- B: K sequential Bernoulli steps
@@ -143,7 +146,7 @@ template <int KIND> __global__ void __launch_bounds__(256) k_adjacency(const Adj
                     if (v > 0.0) {
                         const int ii = ent_i[e];
                         const double g = gacc[ii], l = lam[ii];
-                        const double base = a_old != 0.0 ? fmax(l - g, lam0) : l;  // the other parents' share is at least lambda0
+                        const double base = a_old != 0.0 ? fmax(l - g, lam0) : l;  // the intensity without this parent is at least lambda0min_c
                         const double term = log((base + g) / base);
                         part += (v == g) ? term : term * (v / g);
                     }
@@ -487,6 +490,7 @@ struct AdjSweepArgs {
     const int *node_ptr;
     int K; const void *table_w;
     const double *lambda0; double *A;   // A: [K*K] parent-major, device, updated in place
+    const double *lam0bn, *lam0min;     // grid baseline: per-event rates in by-node order, per-node minima (NULL: lambda0)
     const double4 *dec;    // [K*K] per link: W Mn[p], logit(rho), u, logit(u)  (k_adj_prep)
     double D;
     const int *vstart; const int64_t *vbase; const int *boff; const unsigned short *ent_i; const double *ent_x;   // PRE: ent_x holds (logit, Jacobian) pairs
@@ -822,7 +826,9 @@ template <int KIND, int PRE, bool CL> __global__ void __launch_bounds__(ADJ_THRE
         const int g_lo = CL ? (int)crank : 0, g_hi = CL ? (int)crank + 1 : G;
         const bool resident = CL || G == 1;
         const E *col = reinterpret_cast<const E *>(a.table_w) + (size_t)c * K;
-        const double lam0 = a.lambda0[c];
+        // lower bound of every intensity of the column without a parent's share: one value per column, so that the CTAs of a
+        // cluster certify alike
+        const double lam0 = a.lam0min ? a.lam0min[c] : a.lambda0[c];
         double *lamg = a.lam + e0;
         double *Acol = a.A + (size_t)K * c;
         __syncthreads();
@@ -840,10 +846,11 @@ template <int KIND, int PRE, bool CL> __global__ void __launch_bounds__(ADJ_THRE
             for (int e = tid; e < brow; e += ADJ_THREADS) s_bo[e] = __ldg(bo_res + e);
             bo_res = s_bo;  // visible behind the barrier that follows the intensities' initialisation
         }
-        // ---- current intensities: lambda0 + the links that are on
+        // ---- current intensities: the baseline rates + the links that are on
         for (int g = g_lo; g < g_hi; g++) {
             const int len = max(0, min(csz, ne - g * csz));
-            for (int e = tid; e < len; e += ADJ_THREADS) lam_s[e] = lam0;
+            if (a.lam0bn) for (int e = tid; e < len; e += ADJ_THREADS) lam_s[e] = __ldg(a.lam0bn + e0 + (size_t)g * csz + e);
+            else for (int e = tid; e < len; e += ADJ_THREADS) lam_s[e] = lam0;
             __syncthreads();
             const int *bo = resident ? bo_res : a.boff + (int64_t)(v0 + g) * brow;
             const int64_t vb = a.vbase[v0 + g];
@@ -1023,7 +1030,8 @@ template <int KIND, int PRE, bool CL> __global__ void __launch_bounds__(ADJ_THRE
                 const unsigned flipmask = __ballot_sync(0xffffffffu, have && new_on != old_on);
                 // Certified speculation.  The sums of this batch were taken with the intensities as they stood at its start.  A flip of
                 // bucket j moves the intensity of every event by at most gmax_j: up when the link goes on, down when it goes off.  A term
-                // of a later bucket is f(b) = log(1 + g / b) with b >= lambda0 its intensity without that bucket's parent, and for r >= 1
+                // of a later bucket is f(b) = log(1 + g / b) with b >= lambda0 its intensity without that bucket's parent (lambda0: the
+                // column's smallest baseline rate lambda0min_c for a grid baseline, the same in every CTA of a cluster), and for r >= 1
                 // log(1 + r x) <= r log(1 + x) (Bernoulli), so with b' the intensity after the flips
                 //   b' <  b:  f(b') <= (b / b') f(b) <= (1 + off / lambda0) f(b),      off = sum of gmax over the accepted flips that went off
                 //   b' >= b:  f(b') >= (b / b') f(b) >= f(b) / (1 + on / lambda0),     on  = ... that went on
@@ -1133,6 +1141,7 @@ template <int KIND, int PRE, bool CL> __global__ void __launch_bounds__(ADJ_THRE
 // a fixed order.  The compensator comes from the per-node counts as in the window sweeps.
 struct AdjLoglikArgs {
     const int *node_ptr; int K; const void *table; const double *lambda0; const uint32_t *abits; int words; double D;
+    const double *lam0bn;  // grid baseline: per-event rates in by-node order (NULL: lambda0)
     const int *vstart, *vnode; const int64_t *vbase; const int *boff; const unsigned short *ent_i; const double *ent_x;
     int nv, chunk_max; double *partials; int *flag;
     int cap;   // links whose section bounds are staged in shared memory per round (0: read from global memory)
@@ -1154,8 +1163,9 @@ template <int KIND, int PRE> __global__ void __launch_bounds__(ADJ_THREADS, 1) k
         const int ne = a.node_ptr[c + 1] - a.node_ptr[c], csz = adj_chunk_size(ne, G);
         const int len = max(0, min(csz, ne - g * csz));
         const double lam0 = a.lambda0[c];
+        const double *rate = a.lam0bn ? a.lam0bn + a.node_ptr[c] + (size_t)g * csz : nullptr;  // the chunk's baseline rates
         __syncthreads();
-        for (int e = tid; e < len; e += ADJ_THREADS) lam_s[e] = lam0;
+        for (int e = tid; e < len; e += ADJ_THREADS) lam_s[e] = rate ? __ldg(rate + e) : lam0;
         if (warp == 0) {  // the column's active parents, in order
             int non = 0;
             const uint32_t *row = a.abits + (size_t)c * a.words;
@@ -1237,7 +1247,7 @@ static bool adj_payload_fits(const nhp_ctx *ctx, const nhp_events *ev) {
 // the network is sparse enough that streaming its active buckets beats the window sweep.  Returns 1 when it does not apply.
 int nhp_cont_try_adj_loglik(nhp_ctx *ctx, nhp_events *ev, SweepArgs &sa, int *grid_out, int cb, int cs) {  // structure of the columns c % cs == cb: their share
     { const char *e = getenv("NHP_ADJ_LOGLIK"); if (e && atoi(e) == 0) return 1; }
-    if (!ctx->has_A || !ev->d_adj_i || ev->adj_cb != cb || ev->adj_cs != cs || ev->n_halo != 0 || ev->adj_cluster < 0 || sa.lam0ev) return 1;
+    if (!ctx->has_A || !ev->d_adj_i || ev->adj_cb != cb || ev->adj_cs != cs || ev->n_halo != 0 || ev->adj_cluster < 0) return 1;
     if (!adj_payload_fits(ctx, ev)) return 1;
     if (!(ctx->density <= 0.25) || !(ev->adj_horizon >= sa.horizon) || sa.jmin > 0) return 1;
     if (ctx->kind == NHP_EXPONENTIAL && ev->adj_horizon != sa.horizon && !(sa.horizon < ctx->dtmax)) return 1;  // only a cut-off horizon may be exceeded
@@ -1252,6 +1262,8 @@ int nhp_cont_try_adj_loglik(nhp_ctx *ctx, nhp_events *ev, SweepArgs &sa, int *gr
     { const char *e = getenv("NHP_ADJ_LL_STAGE"); if (e && atoi(e) == 0) a.cap = 0; }
     if (smem + 3 * (size_t)a.cap * sizeof(int) > (size_t)ctx->smem_optin - 4096) a.cap = 0;
     smem += 3 * (size_t)a.cap * sizeof(int);
+    const double *lam0min = nullptr;  // (the sums of logs need the rates only)
+    NHP_TRY(nhp_cont_event_baseline_bynode(ctx, ev, &a.lam0bn, &lam0min));
     NHP_CUDA(ctx, fast_tables_upload(ctx->stream));
     const int grid = (int)std::min<int64_t>(ev->adj_nv, ctx->sm_count);
     if (ctx->kind == NHP_EXPONENTIAL) {
@@ -1510,7 +1522,7 @@ static int adj_build_structure(nhp_ctx *ctx, nhp_events *ev, double horizon, int
 
 // the uncached sweep: per-call scratch, re-bucketing inside the kernel
 static int adj_run_uncached(nhp_ctx *ctx, nhp_events *ev, double horizon, const double *d_rho, const double *d_u, uint64_t seed, uint64_t counter,
-                            double *d_A, int cb, int cs) {
+                            double *d_A, int cb, int cs, const double *lam0bn, const double *lam0min) {
     const int64_t K = ctx->K, n = ev->n;
     cudaStream_t s = ctx->stream;
     unsigned long long *d_cc = nullptr;
@@ -1554,6 +1566,7 @@ static int adj_run_uncached(nhp_ctx *ctx, nhp_events *ev, double horizon, const 
     AdjArgs a;
     a.t = ev->d_t; a.c = ev->d_c; a.n = n; a.order = ev->d_order; a.node_ptr = ev->d_node_ptr; a.Mn = ev->d_Mn; a.K = (int)K; a.table_w = ctx->d_adj_tw;
     a.lambda0 = ctx->d_lambda0; a.W = ctx->d_W; a.A = d_A; a.rho = d_rho; a.u = d_u; a.seed = seed; a.counter = counter;
+    a.lam0bn = lam0bn; a.lam0min = lam0min;
     a.D = ctx->dtmax; a.horizon = horizon; a.duration = ev->duration; a.flag = ctx->d_flag; a.col_begin = cb; a.col_stride = cs;
     a.cap = cap; a.ent_i = d_ent_i; a.ent_v = d_ent_v; a.lam = d_lam; a.gacc = d_gacc; a.max_col = mc;
     const size_t smem = (size_t)(2 * K + 2) * sizeof(int);
@@ -1608,7 +1621,6 @@ static int adj_run(nhp_ctx *ctx, nhp_events *ev, const double *d_rho, double rho
     NHP_CHECK(ctx, ev != nullptr && ev->K == ctx->K, NHP_ERR_INVALID, "adjacency sampler: bad events handle");
     NHP_CHECK(ctx, ev->n_halo == 0 && ev->index_base == 0, NHP_ERR_UNSUPPORTED,
               "the adjacency sampler works on unsharded data (multi-GPU partitions the columns, not the time axis)");
-    NHP_CHECK(ctx, ctx->bgrid_n == 0, NHP_ERR_UNSUPPORTED, "the adjacency sampler takes a homogeneous baseline (grid baselines serve the log-likelihood, intensity and parent sweeps)");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     NHP_CUDA(ctx, fast_tables_upload(ctx->stream));
     NHP_TRY(adj_ensure_ctx(ctx));
@@ -1623,6 +1635,14 @@ static int adj_run(nhp_ctx *ctx, nhp_events *ev, const double *d_rho, double rho
     AdjPhaseTimer tr(s);
     NHP_TRY(nhp_events_build_node_index(ctx, ev));
     tr.lap("node index");
+    // grid baseline: the per-event rates of the columns in by-node order and their minima.  A zero rate at an event of a swept column
+    // leaves the conditional undefined (the reference's logsumexp(-Inf, -Inf)): refused before anything changes
+    const double *lam0bn = nullptr, *lam0min = nullptr;
+    NHP_TRY(nhp_cont_event_baseline_bynode(ctx, ev, &lam0bn, &lam0min));
+    if (lam0min)
+        for (int64_t c = col_begin; c < K; c += col_stride)
+            NHP_CHECK(ctx, ev->lam0min[(size_t)c] > 0.0, NHP_ERR_NUMERIC, "adjacency sampler: the baseline of node %lld is zero at one of its events", (long long)(c + 1));
+    tr.lap("baseline rates");
     double horizon = adj_horizon_value(ctx, n);
     const char *envc = getenv("NHP_ADJ_CACHE");
     bool cached = !(envc && atoi(envc) == 0);
@@ -1644,6 +1664,7 @@ static int adj_run(nhp_ctx *ctx, nhp_events *ev, const double *d_rho, double rho
     if (cached) {
         AdjSweepArgs w;
         w.node_ptr = ev->d_node_ptr; w.K = (int)K; w.table_w = ctx->d_adj_tw; w.lambda0 = ctx->d_lambda0; w.A = d_A;
+        w.lam0bn = lam0bn; w.lam0min = lam0min;
         k_adj_prep<<<kb, 256, 0, s>>>((int)K, ctx->d_W, ev->d_Mn, d_rho, rho_scalar, d_u, seed, counter, ctx->d_adj_dec);
         NHP_LAUNCHED(ctx);
         w.dec = ctx->d_adj_dec; w.D = ctx->dtmax;
@@ -1685,7 +1706,7 @@ static int adj_run(nhp_ctx *ctx, nhp_events *ev, const double *d_rho, double rho
             NHP_CUDA(ctx, cudaStreamSynchronize(s));
             rho_dev = ctx->d_adj_rho;
         }
-        NHP_TRY(adj_run_uncached(ctx, ev, horizon, rho_dev, d_u, seed, counter, d_A, (int)col_begin, (int)col_stride));
+        NHP_TRY(adj_run_uncached(ctx, ev, horizon, rho_dev, d_u, seed, counter, d_A, (int)col_begin, (int)col_stride, lam0bn, lam0min));
     }
     int flag = 0;
     unsigned long long st[4] = {0, 0, 0, 0};

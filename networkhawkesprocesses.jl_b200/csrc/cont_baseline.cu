@@ -90,6 +90,7 @@ extern "C" int nhp_cont_baseline_grid(nhp_ctx *ctx, int64_t n_grid, const double
     for (int64_t k = 0; k < K; k++) tot += trapezoid(x, values + k * n_grid, n_grid);  // integrated_intensity(p::LogGaussianCoxProcess, duration), baselines.jl:336
     for (int64_t e = 0; e < K * n_grid; e++) mn = std::min(mn, values[e]);
     ctx->baseline_integral = tot;
+    ctx->bgrid_min = mn;
     ctx->lambda0_min = mn;  // the Exponential cut-off horizon measures the omitted tail against the smallest baseline rate
     return NHP_OK;
 }
@@ -112,6 +113,55 @@ int nhp_cont_event_baseline(nhp_ctx *ctx, nhp_events *ev, const double **lam0ev)
     }
     ev->lam0ev_version = ctx->bgrid_version;
     *lam0ev = ev->d_lam0ev;
+    return NHP_OK;
+}
+
+// one CTA per node: its events' rates in the by-node order, and their minimum
+__global__ void k_event_baseline_bynode(const double *__restrict__ lam0ev, const int *__restrict__ order, const int *__restrict__ node_ptr, int K,
+                                        double *__restrict__ bynode, double *__restrict__ colmin) {
+    __shared__ double s_min[32];
+    for (int c = blockIdx.x; c < K; c += gridDim.x) {
+        double m = INFINITY;
+        for (int e = node_ptr[c] + threadIdx.x; e < node_ptr[c + 1]; e += blockDim.x) {
+            const double v = lam0ev[order[e]];
+            bynode[e] = v;
+            m = fmin(m, v);
+        }
+        for (int d = 16; d > 0; d >>= 1) m = fmin(m, __shfl_xor_sync(0xffffffffu, m, d));
+        if ((threadIdx.x & 31) == 0) s_min[threadIdx.x >> 5] = m;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            for (int w = 1; w < (int)(blockDim.x >> 5); w++) m = fmin(m, s_min[w]);
+            colmin[c] = m;
+        }
+        __syncthreads();
+    }
+}
+
+// The adjacency sampler's view of the curves: the per-event rates in the by-node order of the handle (a column chunk's initial
+// intensities are one contiguous read) and their minimum per node, the lower bound of every intensity of the column without any
+// parent's share (certification bound and floor of the sweep).  Rebuilt with the per-event rates, for the same curve version.
+int nhp_cont_event_baseline_bynode(nhp_ctx *ctx, nhp_events *ev, const double **lam0bn, const double **lam0min) {
+    *lam0bn = *lam0min = nullptr;
+    if (ctx->bgrid_n == 0) return NHP_OK;
+    const double *lam0ev = nullptr;
+    NHP_TRY(nhp_cont_event_baseline(ctx, ev, &lam0ev));
+    if (!(ev->d_lam0bn && ev->lam0bn_version == ctx->bgrid_version)) {
+        NHP_TRY(nhp_events_build_node_index(ctx, ev));
+        cudaStream_t s = ctx->stream;
+        const int64_t K = ev->K, own = ev->n - ev->n_halo;
+        if (!ev->d_lam0bn) NHP_CUDA(ctx, cudaMallocAsync(&ev->d_lam0bn, (size_t)std::max<int64_t>(own, 1) * sizeof(double), s));
+        if (!ev->d_lam0min) NHP_CUDA(ctx, cudaMallocAsync(&ev->d_lam0min, (size_t)K * sizeof(double), s));
+        k_event_baseline_bynode<<<(unsigned)std::min<int64_t>(K, (int64_t)ctx->sm_count * 8), 256, 0, s>>>(lam0ev, ev->d_order, ev->d_node_ptr, (int)K, ev->d_lam0bn,
+                                                                                                         ev->d_lam0min);
+        NHP_LAUNCHED(ctx);
+        ev->lam0min.resize((size_t)K);
+        NHP_CUDA(ctx, cudaMemcpyAsync(ev->lam0min.data(), ev->d_lam0min, (size_t)K * sizeof(double), cudaMemcpyDeviceToHost, s));
+        NHP_CUDA(ctx, cudaStreamSynchronize(s));
+        ev->lam0bn_version = ctx->bgrid_version;
+    }
+    *lam0bn = ev->d_lam0bn;
+    *lam0min = ev->d_lam0min;
     return NHP_OK;
 }
 

@@ -156,7 +156,8 @@ int nhp_cont_params_refresh(nhp_ctx *ctx) {
     NHP_CUDA(ctx, cudaMemcpyAsync(h, scratch, sizeof(h), cudaMemcpyDeviceToHost, s));
     NHP_TRY(nhp_cont_derive_tables(ctx));
     NHP_CUDA(ctx, cudaStreamSynchronize(s));
-    ctx->lambda0_min = h[0]; ctx->lambda0_sum = h[1]; ctx->theta_min = h[2]; ctx->wt_max = h[3];
+    ctx->lambda0_min = ctx->bgrid_n > 0 ? ctx->bgrid_min : h[0];  // curves on the device: the cut-off horizon keeps their minimum
+    ctx->lambda0_sum = h[1]; ctx->theta_min = h[2]; ctx->wt_max = h[3];
     ctx->density = h[4] / (double)(K * K);
     ctx->theta_min_all = h[5]; ctx->wt_max_all = h[6];
     ctx->a_sum = ctx->has_A ? h[7] : (double)(K * K);

@@ -355,7 +355,7 @@ extern "C" int nhp_events_free(nhp_ctx *ctx, nhp_events *ev) {
     }
     {
         cudaStream_t as = ctx ? ctx->stream : nullptr;
-        void *blocks[] = {ev->d_order, ev->d_node_ptr, ev->d_item_node, ev->d_item_e0, ev->d_lam0ev};
+        void *blocks[] = {ev->d_order, ev->d_node_ptr, ev->d_item_node, ev->d_item_e0, ev->d_lam0ev, ev->d_lam0bn, ev->d_lam0min};
         for (void *b : blocks) if (b) cudaFreeAsync(b, as);
     }
     nhp_events_free_adjacency(ctx, ev, ctx ? ctx->stream : nullptr);

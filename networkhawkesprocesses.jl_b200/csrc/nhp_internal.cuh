@@ -84,6 +84,11 @@ struct nhp_events {
     int *d_order = nullptr, *d_node_ptr = nullptr, *d_item_node = nullptr, *d_item_e0 = nullptr;
     double *d_lam0ev = nullptr;     // [n] baseline rate at every event for the context's grid baseline (version below), built on first use
     uint64_t lam0ev_version = 0;
+    // the same rates in the by-node order (d_order) and their minimum per node, for the adjacency sampler (same curve version rule)
+    double *d_lam0bn = nullptr;     // [n - n_halo] lam0ev[order[e]]
+    double *d_lam0min = nullptr;    // [K] min over the node's own events (+Inf for a node without events)
+    std::vector<double> lam0min;    // host copy of d_lam0min
+    uint64_t lam0bn_version = 0;
     int64_t n_items = 0;
     // cached structure of the adjacency sampler (cont_adjacency.cu): every (child event, window predecessor) pair, grouped by
     // virtual column = (child column, time chunk of at most adj_chunk_cap of the column's events) and bucketed by parent node,
@@ -155,6 +160,7 @@ struct nhp_ctx {
     double *d_bgrid_x = nullptr, *d_bgrid_v = nullptr;  // [bgrid_n] grid, [K][bgrid_n] values
     int64_t bgrid_n = 0; uint64_t bgrid_version = 0;     // 0 points: homogeneous lambda0
     double baseline_integral = 0.0;                      // sum_k integrate(lambda0_k) over the grid (trapezoid)
+    double bgrid_min = 0.0;                              // smallest curve value: lambda0_min while the grid is active
     double *d_W = nullptr, *d_A = nullptr, *d_p1 = nullptr, *d_p2 = nullptr; // raw [K*K] parent-major as passed
     void *d_table = nullptr;      // EntryLN/EntryEX [K*K] child-major
     double *d_rowsum = nullptr;   // [K] sum_c [A]W[p,c]
@@ -297,6 +303,7 @@ int nhp_cont_run_loglik(nhp_ctx *ctx, nhp_events *ev, int recursive);
 double nhp_cont_horizon_value(const nhp_ctx *ctx, int64_t n_total, int recursive);
 int nhp_events_build_node_index(nhp_ctx *ctx, nhp_events *ev);  // d_order / d_node_ptr (cont_child.cu)
 int nhp_cont_event_baseline(nhp_ctx *ctx, nhp_events *ev, const double **lam0ev);  // cont_baseline.cu: NULL for a homogeneous baseline
+int nhp_cont_event_baseline_bynode(nhp_ctx *ctx, nhp_events *ev, const double **lam0bn, const double **lam0min);  // the same in by-node order + per-node minima
 double nhp_cont_baseline_term(const nhp_ctx *ctx, const nhp_events *ev);             // sum(integrated_intensity(baseline, duration)) of the log-likelihood
 struct SweepArgs;
 int nhp_cont_try_adj_loglik(nhp_ctx *ctx, nhp_events *ev, SweepArgs &sa, int *grid_out, int cb = 0, int cs = 1);  // cont_adjacency.cu: 1 = does not apply

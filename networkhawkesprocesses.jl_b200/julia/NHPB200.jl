@@ -310,7 +310,11 @@ function loglikelihood(process::LogGaussianCoxProcess, data::FusedParents, y::Ma
 end
 
 # optional: the whole `resample!(process, data)` (continuous.jl:202-208 / 350-358) in one call that never leaves the device
+# A LogGaussianCoxProcess baseline is not supported here: the device's draws are the conjugate ones, and its curves move with the
+# elliptical-slice update of `resample!`, which the device serves through the sweeps above.
 function resample_on_device!(process::ContinuousHawkesProcess, data)
+    process.baseline isa LogGaussianCoxProcess &&
+        throw(ArgumentError("resample_on_device!: a LogGaussianCoxProcess baseline takes resample! (elliptical-slice update of the curves)"))
     ev = device_events(process, data)
     push_params!(process)
     SWEEP[] += 1
@@ -343,6 +347,8 @@ end
 # `mcmc!` (inference.jl:49-70) with the chain and its sample trace on the device: the parameters go up once, every sweep is one
 # nhp_cont_gibbs_sweep (which appends its sample to the device-side trace, adjacency bit-packed), one read at the end.
 function mcmc_on_device!(process::ContinuousHawkesProcess, data; nsteps=1000)
+    process.baseline isa LogGaussianCoxProcess &&
+        throw(ArgumentError("mcmc_on_device!: a LogGaussianCoxProcess baseline takes mcmc! (the device trace would hold curves that never move)"))
     ev = device_events(process, data)
     push_params!(process)
     b, w, imp = process.baseline, process.weights, process.impulses

@@ -571,9 +571,11 @@ class MarkovChainMonteCarlo:  # inference.jl:22-31
 def _hyper(process):
     """Hyper-parameters in the order nhp_cont_resample_params expects."""
     b, w, imp = process.baseline, process.weights, process.impulses
+    # a LogGaussianCoxProcess baseline has no Gamma prior: the homogeneous draw these two feed is not used while the curves are on the device
+    a0, b0 = (1.0, 1.0) if isinstance(b, LogGaussianCoxProcess) else (b.alpha0, b.beta0)
     if imp.kind == NHP_EXPONENTIAL:
-        return _f64([b.alpha0, b.beta0, w.kappa, w.nu, imp.alpha, imp.beta])
-    return _f64([b.alpha0, b.beta0, w.kappa, w.nu, imp.mumu, imp.kappamu, imp.alpha0, imp.beta0])
+        return _f64([a0, b0, w.kappa, w.nu, imp.alpha, imp.beta])
+    return _f64([a0, b0, w.kappa, w.nu, imp.mumu, imp.kappamu, imp.alpha0, imp.beta0])
 
 
 def pull_params_(process, ctx=None):
@@ -587,7 +589,8 @@ def pull_params_(process, ctx=None):
     unf = lambda v: v.reshape(K, K).T.copy()
     if A is not None:
         process.adjacency_matrix = unf(A)
-    process.baseline.lam = lam
+    if not isinstance(process.baseline, LogGaussianCoxProcess):  # the host holds the curves (the device's lambda0 stands in for them)
+        process.baseline.lam = lam
     process.weights.W = unf(W)
     if process.impulses.kind == NHP_EXPONENTIAL:
         process.impulses.theta = unf(p1)
@@ -601,7 +604,11 @@ def resample_on_device_(process, data, rng=None, seed=0, counter=0, push=True, p
     baseline / weights / impulses (nhp_cont_resample_params), and for a network process the adjacency sweep on the
     device-resident matrix (nhp_cont_resample_adjacency_dev) and the Beta draw of rho (nhp_cont_resample_network), with
     every table rebuilt in place.  `push=False` continues from the parameters already on the device (a chain);
-    `pull=False` leaves the host objects untouched.  `rng` is unused (kept for the signature of `resample_`)."""
+    `pull=False` leaves the host objects untouched.
+    A LogGaussianCoxProcess baseline takes its elliptical-slice update (with `rng`, or a generator seeded by (seed, counter)) from the
+    device-resident parents after the conjugate draws, and its new curves go to the device before the adjacency sweep.  Weights and
+    impulses are then drawn before the curves; given the parents they do not depend on them, so the sweep samples the same
+    conditionals."""
     ctx = process._ctx()
     d, tmp = process._data(data)
     try:
@@ -613,6 +620,11 @@ def resample_on_device_(process, data, rng=None, seed=0, counter=0, push=True, p
         _resample_parents(ctx, d, seed, counter, None, False)
         hy = _hyper(process)
         ctx.check(ctx.lib.nhp_cont_resample_params(ctx.h, d.h, int(seed), int(counter), float(d.duration), _ptr(hy), hy.size, 1))
+        b = process.baseline
+        if isinstance(b, LogGaussianCoxProcess):
+            b.resample_(ctx, d, rng if rng is not None else np.random.default_rng([int(seed), int(counter)]))
+            # after the slice update: the new curves invalidate the parent assignment it reads
+            ctx.check(ctx.lib.nhp_cont_baseline_grid(ctx.h, b.x.size, _ptr(_f64(b.x)), _ptr(_f64(b.lam_grid.ravel()))))
         if net:
             bern = isinstance(process.network, BernoulliNetworkModel)
             ctx.check(ctx.lib.nhp_cont_resample_adjacency_dev(ctx.h, d.h, -1.0 if bern else 1.0, int(seed), int(counter + (1 << 40)), 0, 1, 1))
@@ -631,6 +643,8 @@ def mcmc_device_(process, data, nsteps=1000, seed=0):
     nhp_cont_gibbs_sweep (which appends its sample to the trace: device-to-device, adjacency bit-packed), and the trace comes back
     in one read at the end.  Returns MarkovChainMonteCarlo with the samples in the order of `params(process)`
     ([rho;] lambda0; theta | mu, tau; W [; vec(A)], continuous.jl:116-119, 325-333); the process holds the last sample."""
+    if isinstance(process.baseline, LogGaussianCoxProcess):  # the device's draws would leave the curves where they are
+        raise ValueError("mcmc_device_: a LogGaussianCoxProcess baseline takes its elliptical-slice update on the host: use mcmc_(device_draws=True)")
     ctx = process._ctx()
     d, tmp = process._data(data)
     t0 = time.time()
