@@ -194,7 +194,8 @@ template <int KIND> __global__ void __launch_bounds__(256) k_adjacency(const Adj
 constexpr int ADJ_CHUNK_MAX = 26624;   // child events per chunk: 208 KB of shared-memory intensities
 constexpr int ADJ_THREADS = 1024;      // sweep CTA: one per SM (512 threads with 128 registers each measured 8 % slower: 45.3 vs 41.9 ms)
 constexpr int ADJ_VW = 32;             // bucket slots of a batch: one per warp (a CTA with fewer warps takes several slots per warp, one after the other)
-constexpr int ADJ_SMAX = 32;           // largest speculative batch (buckets per batch); the size follows the observed flip rate, down to 1
+constexpr int ADJ_SMAX_LOG2 = 5;
+constexpr int ADJ_SMAX = 1 << ADJ_SMAX_LOG2;  // largest speculative batch (buckets per batch); the size follows the observed flip rate, down to 1
 constexpr int ADJ_INIT_PF = 8;       // links ahead whose buckets are prefetched to L2 while a column's intensities are built up
 constexpr int ADJ_CLUSTER_MAX = 8;     // portable cluster size limit
 
@@ -499,9 +500,8 @@ struct AdjSweepArgs {
     int *flag, *next; unsigned long long *stat;
     int col_begin, col_stride, ncols;
     const int *corder;     // [ncols] owned columns, most child events first (NULL: col_begin + i col_stride)
-    int s0, lmax;   // first batch size; log2 of the largest
+    int s0;         // first batch size
     int bo_smem;    // 1: the bucket offsets of the resident chunk are kept in shared memory behind the adjacency bits ((2 K + 1) ints)
-    int cert;       // 1: one-sided certification bounds (default); 0: the symmetric bound with the lambda0 / 2 cut (NHP_ADJ_CERT=0)
 };
 
 // thread-block cluster primitives (distributed shared memory of the CTAs that share a column)
@@ -1040,45 +1040,25 @@ template <int KIND, int PRE, bool CL> __global__ void __launch_bounds__(ADJ_THRE
                 // A decision whose margin |delta - logit(u)| exceeds its side's bound (plus rounding slack) is the decision the sequential
                 // sweep takes; the batch is accepted up to the first bucket that cannot be certified, and restarts there.
                 // on / off = exclusive prefix sums over the flips (warp scan: the same values in every CTA of the cluster).
+                // (The first version used one symmetric bound, 4 S cum / lambda0 from the derivative, valid only while cum <= lambda0 / 2,
+                // so every larger flip ended its batch; DESIGN.md §3.3.)
                 const bool flip = (flipmask >> lane) & 1u;
-                int stop_;
-                if (a.cert) {
-                    double inc_on = (flip && new_on) ? gmax : 0.0, inc_off = (flip && !new_on) ? gmax : 0.0;
+                double inc_on = (flip && new_on) ? gmax : 0.0, inc_off = (flip && !new_on) ? gmax : 0.0;
 #pragma unroll
-                    for (int d = 1; d < 32; d <<= 1) {
-                        const double t1 = __shfl_up_sync(0xffffffffu, inc_on, d), t0 = __shfl_up_sync(0xffffffffu, inc_off, d);
-                        if (lane >= d) { inc_on += t1; inc_off += t0; }
-                    }
-                    double cum_on = __shfl_up_sync(0xffffffffu, inc_on, 1), cum_off = __shfl_up_sync(0xffffffffu, inc_off, 1);
-                    if (lane == 0) { cum_on = 0.0; cum_off = 0.0; }
-                    const double slack = 1e-7 + 1e-10 * fabs(delta);
-                    const double S_ = fabs(sum);
-                    // (1.0000001: the scan's own rounding, so that the bound stays an upper bound)
-                    const double shift = new_on ? S_ * (cum_on / (lam0 + cum_on)) : S_ * (cum_off / lam0);
-                    const bool uncertified = have && (cum_on > 0.0 || cum_off > 0.0) && !(margin > 1.0000001 * shift + slack);
-                    const unsigned um = __ballot_sync(0xffffffffu, uncertified);
-                    stop_ = Sc;
-                    if (um) stop_ = min(stop_, __ffs(um) - 1);
-                } else {
-                    // (the first version: symmetric bound 4 S cum / lambda0 from the derivative, valid while cum <= lambda0 / 2; a flip whose
-                    // change is larger ends the batch behind itself)
-                    double inc = flip ? gmax : 0.0;
-#pragma unroll
-                    for (int d = 1; d < 32; d <<= 1) {
-                        const double t = __shfl_up_sync(0xffffffffu, inc, d);
-                        if (lane >= d) inc += t;
-                    }
-                    double cum = __shfl_up_sync(0xffffffffu, inc, 1);
-                    if (lane == 0) cum = 0.0;
-                    const double slack = 1e-7 + 1e-10 * fabs(delta);
-                    const bool uncertified = have && cum > 0.0 && !(margin > fabs(sum) * cum * (4.0 / lam0) + slack);
-                    const bool toobig = flip && !(gmax <= 0.5 * lam0);
-                    const unsigned um = __ballot_sync(0xffffffffu, uncertified), bm = __ballot_sync(0xffffffffu, toobig);
-                    stop_ = Sc;
-                    if (um) stop_ = min(stop_, __ffs(um) - 1);
-                    if (bm) stop_ = min(stop_, __ffs(bm));
+                for (int d = 1; d < 32; d <<= 1) {
+                    const double t1 = __shfl_up_sync(0xffffffffu, inc_on, d), t0 = __shfl_up_sync(0xffffffffu, inc_off, d);
+                    if (lane >= d) { inc_on += t1; inc_off += t0; }
                 }
-                stop = stop_;
+                double cum_on = __shfl_up_sync(0xffffffffu, inc_on, 1), cum_off = __shfl_up_sync(0xffffffffu, inc_off, 1);
+                if (lane == 0) { cum_on = 0.0; cum_off = 0.0; }
+                const double slack = 1e-7 + 1e-10 * fabs(delta);
+                const double S_ = fabs(sum);
+                // (1.0000001: the scan's own rounding, so that the bound stays an upper bound)
+                const double shift = new_on ? S_ * (cum_on / (lam0 + cum_on)) : S_ * (cum_off / lam0);
+                const bool uncertified = have && (cum_on > 0.0 || cum_off > 0.0) && !(margin > 1.0000001 * shift + slack);
+                const unsigned um = __ballot_sync(0xffffffffu, uncertified);
+                stop = Sc;
+                if (um) stop = min(stop, __ffs(um) - 1);
                 fm = stop >= 32 ? flipmask : (flipmask & ((1u << stop) - 1u));
                 onm = __ballot_sync(0xffffffffu, new_on);
                 // warp 0 records the accepted flips; the others see the new bits behind the barrier of the first flip's application
@@ -1120,7 +1100,7 @@ template <int KIND, int PRE, bool CL> __global__ void __launch_bounds__(ADJ_THRE
             fw_steps = 0.9f * fw_steps + (float)stop; fw_flips = 0.9f * fw_flips + (stop < Sc ? 1.f : 0.f);  // "flip" = a batch cut short
             {
                 const float target = 2.f * rsqrtf(fw_flips / fw_steps + 1e-3f);
-                const int l2 = min(a.lmax, max(0, __float2int_rn(__log2f(target))));
+                const int l2 = min(ADJ_SMAX_LOG2, max(0, __float2int_rn(__log2f(target))));
                 S = 1 << l2;
             }
         }
@@ -1282,11 +1262,6 @@ int nhp_cont_try_adj_loglik(nhp_ctx *ctx, nhp_events *ev, SweepArgs &sa, int *gr
     return NHP_OK;
 }
 
-__global__ void k_iota(int *v, int64_t n) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) v[i] = (int)i;
-}
-
 // table without the adjacency factor (the sampler needs W h for both values of A[p,c])
 __global__ void k_table_noA_ln(int K, const double *__restrict__ W, const double *__restrict__ mu, const double *__restrict__ tau, double D, EntryLN *__restrict__ table) {
     int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1434,8 +1409,7 @@ static int adj_build_structure(nhp_ctx *ctx, nhp_events *ev, double horizon, int
     { const char *e = getenv("NHP_ADJ_PRE"); if (e) pre = pre && atoi(e) != 0; }
     const size_t need = (size_t)tot * (pre ? 18 : 10) + fixed;
     // build kernel: [2K+1] section offsets + 2 K CTA-wide cursors (singles, runs); one CTA of 32 warps per SM
-    int nw = 32;
-    { const char *e = getenv("NHP_ADJ_BUILD_NW"); if (e && atoi(e) >= 1 && atoi(e) <= 32) nw = atoi(e); }
+    constexpr int nw = 32;
     const bool fits = (size_t)(4 * K + 1) * sizeof(int) + 2048 <= (size_t)ctx->smem_optin;
     // the packed predecessor record holds 20 bits of node and 22 bits of same-node distances: longer windows take the uncached sweep
     if ((double)need > 0.75 * (double)free_b || !fits || K > (1 << ADJ_NODE_BITS) || max_win >= (int)ADJ_LINK_SAT) return drop(1);
@@ -1676,11 +1650,6 @@ static int adj_run(nhp_ctx *ctx, nhp_events *ev, const double *d_rho, double rho
         w.ncols = (int)((K - col_begin + col_stride - 1) / col_stride);
         w.s0 = ADJ_SMAX;
         { const char *e = getenv("NHP_ADJ_S0"); if (e && atoi(e) >= 1 && atoi(e) <= 32 && (atoi(e) & (atoi(e) - 1)) == 0) w.s0 = atoi(e); }
-        w.lmax = 5;
-        w.cert = 1;
-        { const char *e = getenv("NHP_ADJ_CERT"); if (e) w.cert = atoi(e) != 0; }
-        { const char *e = getenv("NHP_ADJ_LMAX"); if (e && atoi(e) >= 0 && atoi(e) <= 5) w.lmax = atoi(e); }
-        if (w.s0 > (1 << w.lmax)) w.s0 = 1 << w.lmax;
         size_t smem = (size_t)w.chunk_max * sizeof(double) + (size_t)((K + 31) / 32) * sizeof(unsigned) + 16;
         {   // room for the resident chunk's bucket offsets?  (the kernel's static shared memory: 12.1 KB, see -Xptxas -v)
             const size_t bo_bytes = (size_t)(((K + 31) / 32 + 3) & ~3) * sizeof(unsigned) - (size_t)((K + 31) / 32) * sizeof(unsigned) + (size_t)(2 * K + 1) * sizeof(int);

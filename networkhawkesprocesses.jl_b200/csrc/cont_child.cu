@@ -205,8 +205,7 @@ int nhp_cont_try_child(nhp_ctx *ctx, nhp_events *ev, SweepArgs &a, int mode, int
     // per SM; give those CTAs more warps (the per-event window reads are cold DRAM: latency is hidden by warps in flight)
     const size_t col_bytes = (size_t)K * esz;
     const int fit = (int)std::max<size_t>(1, ((size_t)ctx->smem_optin - 8192) / std::max<size_t>(col_bytes, 1));
-    int block = fit >= 8 ? 256 : (fit >= 4 ? 512 : 1024);
-    { const char *eb = getenv("NHP_CHILD_BLOCK"); if (eb && (atoi(eb) == 256 || atoi(eb) == 512 || atoi(eb) == 1024)) block = atoi(eb); }
+    const int block = fit >= 8 ? 256 : (fit >= 4 ? 512 : 1024);
     const size_t smem = col_bytes + (mode == 2 ? (size_t)CR * block * sizeof(double) : 0);
     if (smem > (size_t)ctx->smem_optin - 8192 || own == 0) return 1;
     // worthwhile when the table no longer sits comfortably in L2 and every column is amortised over enough pairs

@@ -355,8 +355,6 @@ static LaunchPlan make_plan(nhp_ctx *ctx, const nhp_events *ev) {
     int64_t own = ev->n - ev->n_halo;
     p.te = 256;
     if (p.G == 32 && own < 200000) p.te = 64;
-    const char *env = getenv("NHP_TE");
-    if (env) { int v = atoi(env); if (v >= 64 && v % 64 == 0 && v <= 4096) p.te = v; }
     p.tiles = (own + p.te - 1) / p.te;
     int64_t need = ((ev->max_win + p.te + 8) + 3) & ~(int64_t)3;
     int64_t limit = ((int64_t)ctx->smem_optin - 1024 - 16) / 12;

@@ -575,82 +575,7 @@ static int disc_ready(nhp_ctx *ctx, nhp_disc *dd, const char *who) {
 
 // ---------------------------------------------------------------------------------------
 // intensity / log-likelihood: lambda[t,c] = lambda0_c dt + sum_k convT[t,k] bumpM[k,c]   (discrete.jl:115-129)
-// FP64 register-tiled GEMM, 128 x 64 output tile per CTA, 8 x 4 per thread, fused Poisson epilogue.
-// ---------------------------------------------------------------------------------------
-constexpr int GBM = 128, GBN = 64, GBK = 16;
-
-template <bool LOGLIK>
-__global__ void __launch_bounds__(256) k_disc_gemm(const double *__restrict__ convT, const double *__restrict__ bumpM, const double *__restrict__ lambda0,
-                                                   double dt, int N, int NB, int64_t T, int64_t t_first, const int *__restrict__ data,
-                                                   double *__restrict__ lam_out, double *__restrict__ partials) {
-    __shared__ double As[GBK][GBM + 4];
-    __shared__ double Bs[GBK][GBN];
-    __shared__ double red[8];
-    const int tx = threadIdx.x % 16, ty = threadIdx.x / 16;  // tx -> 4 columns, ty -> 8 rows
-    const int64_t t0 = t_first + (int64_t)blockIdx.x * GBM;
-    const int c0 = blockIdx.y * GBN;
-    double acc[8][4];
-#pragma unroll
-    for (int i = 0; i < 8; i++)
-#pragma unroll
-        for (int j = 0; j < 4; j++) acc[i][j] = 0.0;
-    for (int k0 = 0; k0 < NB; k0 += GBK) {
-        // A tile: 128 rows x 16 k (row-major source, k contiguous)
-        for (int e = threadIdx.x; e < GBM * GBK; e += 256) {
-            int r = e / GBK, kk = e % GBK;
-            int64_t t = t0 + r;
-            As[kk][r] = (t < T && k0 + kk < NB) ? __ldg(convT + t * NB + k0 + kk) : 0.0;
-        }
-        for (int e = threadIdx.x; e < GBK * GBN; e += 256) {
-            int kk = e / GBN, cc = e % GBN;
-            Bs[kk][cc] = (k0 + kk < NB && c0 + cc < N) ? __ldg(bumpM + (int64_t)(k0 + kk) * N + c0 + cc) : 0.0;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int kk = 0; kk < GBK; kk++) {
-            double a[8], b[4];
-#pragma unroll
-            for (int i = 0; i < 8; i++) a[i] = As[kk][ty + 16 * i];
-#pragma unroll
-            for (int j = 0; j < 4; j++) b[j] = Bs[kk][tx + 16 * j];
-#pragma unroll
-            for (int i = 0; i < 8; i++)
-#pragma unroll
-                for (int j = 0; j < 4; j++) acc[i][j] = fma(a[i], b[j], acc[i][j]);
-        }
-        __syncthreads();
-    }
-    double part = 0.0;
-#pragma unroll
-    for (int i = 0; i < 8; i++) {
-        int64_t t = t0 + ty + 16 * i;
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            int c = c0 + tx + 16 * j;
-            if (t < T && c < N) {
-                double lam = lambda0[c] * dt + acc[i][j];
-                if (LOGLIK) {
-                    int sct = data[t * N + c];
-                    // log pdf(Poisson(lam), s) = xlogy(s, lam) - lam - loggamma(s + 1)   (discrete.jl:98)
-                    part += (sct ? (double)sct * log(lam) : 0.0) - lam - lgamma((double)sct + 1.0);
-                } else lam_out[t + T * (int64_t)c] = lam;
-            }
-        }
-    }
-    if (LOGLIK) {
-        part = warp_sum_d(part);
-        if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = part;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            double s = 0.0;
-            for (int w = 0; w < 8; w++) s += red[w];
-            partials[(size_t)blockIdx.y * gridDim.x + blockIdx.x] = s;
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------
-// FP64 tensor-core variant of the same contraction: mma.sync.aligned.m8n8k4.f64 (SASS DMMA.8x8x4; tcgen05
+// FP64 tensor-core contraction with a fused Poisson epilogue: mma.sync.aligned.m8n8k4.f64 (SASS DMMA.8x8x4; tcgen05
 // has no FP64 kind).  CTA tile 128 rows x 8*NT columns, warp tile 16 x 8*NT (2 x NT accumulator tiles),
 // k staged 16 at a time through shared memory with pitches chosen so every fragment load is conflict-free.
 // Measured DMMA peak on B200: 36.7 TFLOP/s (nhp_bench_fp64 which=3) vs 33.8 TFLOP/s for DFMA, at 1/8 of
@@ -785,18 +710,19 @@ static int pick_nt(int64_t N) {
     return best;
 }
 
+// returns the grid: one CTA (and one log-likelihood partial) per DBM x 8 pick_nt(N) tile
 template <bool LOGLIK>
-static void launch_dmma(nhp_ctx *ctx, nhp_disc *dd, int64_t t_first, int64_t rows, double *lam_out, double *partials, dim3 *grid_out) {
+static dim3 launch_dmma(nhp_ctx *ctx, nhp_disc *dd, int64_t t_first, int64_t rows, double *lam_out, double *partials) {
     const int64_t N = dd->N, NB = N * dd->B;
     const int nt = pick_nt(N);
     dim3 grid((unsigned)((N + 8 * nt - 1) / (8 * nt)), (unsigned)((rows + DBM - 1) / DBM));
-    *grid_out = grid;
 #define NHP_DMMA_CASE(NTV) { constexpr size_t smem = (size_t)(2 * DBM * DLDA + 2 * DBK * (8 * NTV + 4)) * sizeof(double); \
         cudaFuncSetAttribute(k_disc_dmma<NTV, LOGLIK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         k_disc_dmma<NTV, LOGLIK><<<grid, 256, smem, ctx->stream>>>(dd->d_conv, ctx->dd_bump, ctx->dd_lambda0, ctx->ddt, (int)N, (int)NB, dd->T, t_first, dd->d_data, lam_out, partials); }
     switch (nt) { case 4: NHP_DMMA_CASE(4) break; case 5: NHP_DMMA_CASE(5) break; default: NHP_DMMA_CASE(6) break; }
 #undef NHP_DMMA_CASE
     NHP_LAUNCHED(ctx);
+    return grid;
 }
 
 __global__ void k_sum_partials(const double *__restrict__ partials, int64_t n, double *__restrict__ out) {
@@ -812,16 +738,11 @@ __global__ void k_sum_partials(const double *__restrict__ partials, int64_t n, d
 extern "C" int nhp_disc_intensity(nhp_ctx *ctx, nhp_disc *dd, double *lam) {
     NHP_TRY(disc_ready(ctx, dd, "nhp_disc_intensity"));
     NHP_CHECK(ctx, lam != nullptr, NHP_ERR_INVALID, "nhp_disc_intensity: lam is NULL");
-    const int64_t N = dd->N, NB = N * dd->B, T = dd->T;
+    const int64_t N = dd->N, T = dd->T;
     void *scratch;
     NHP_TRY(nhp_scratch(ctx, (size_t)T * N * sizeof(double), &scratch));
-    dim3 grid((unsigned)((T + GBM - 1) / GBM), (unsigned)((N + GBN - 1) / GBN));
     NHP_TRY(nhp_timer_begin(ctx));
-    const char *env = getenv("NHP_DISC_DMMA");
-    if (env && atoi(env) == 0) {
-        k_disc_gemm<false><<<grid, 256, 0, ctx->stream>>>(dd->d_conv, ctx->dd_bump, ctx->dd_lambda0, ctx->ddt, (int)N, (int)NB, T, 0, dd->d_data, (double *)scratch, nullptr);
-        NHP_LAUNCHED(ctx);
-    } else launch_dmma<false>(ctx, dd, 0, T, (double *)scratch, nullptr, &grid);
+    launch_dmma<false>(ctx, dd, 0, T, (double *)scratch, nullptr);
     DCUDA(ctx, cudaGetLastError());
     NHP_TRY(nhp_timer_end(ctx));
     DCUDA(ctx, cudaMemcpyAsync(lam, scratch, (size_t)T * N * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
@@ -832,16 +753,12 @@ extern "C" int nhp_disc_intensity(nhp_ctx *ctx, nhp_disc *dd, double *lam) {
 extern "C" int nhp_disc_loglik(nhp_ctx *ctx, nhp_disc *dd, double *ll) {
     NHP_TRY(disc_ready(ctx, dd, "nhp_disc_loglik"));
     NHP_CHECK(ctx, ll != nullptr, NHP_ERR_INVALID, "nhp_disc_loglik: ll is NULL");
-    const int64_t N = dd->N, NB = N * dd->B, T = dd->T, own = T - dd->t_halo;
-    dim3 grid((unsigned)((own + GBM - 1) / GBM), (unsigned)((N + GBN - 1) / GBN));
-    double *partials;
-    NHP_TRY(nhp_partials(ctx, (int64_t)((own + 63) / 64 + 2) * ((N + 31) / 32 + 2) + 1, &partials));
+    const int64_t N = dd->N, T = dd->T, own = T - dd->t_halo;
+    const int64_t bn = 8 * pick_nt(N);
+    double *partials;  // [0]: the sum; [1..]: one per CTA of launch_dmma
+    NHP_TRY(nhp_partials(ctx, (own + DBM - 1) / DBM * ((N + bn - 1) / bn) + 1, &partials));
     NHP_TRY(nhp_timer_begin(ctx));
-    const char *env = getenv("NHP_DISC_DMMA");
-    if (env && atoi(env) == 0) {
-        k_disc_gemm<true><<<grid, 256, 0, ctx->stream>>>(dd->d_conv, ctx->dd_bump, ctx->dd_lambda0, ctx->ddt, (int)N, (int)NB, T, dd->t_halo, dd->d_data, nullptr, partials + 1);
-        NHP_LAUNCHED(ctx);
-    } else launch_dmma<true>(ctx, dd, dd->t_halo, own, nullptr, partials + 1, &grid);
+    const dim3 grid = launch_dmma<true>(ctx, dd, dd->t_halo, own, nullptr, partials + 1);
     k_sum_partials<<<1, 1024, 0, ctx->stream>>>(partials + 1, (int64_t)grid.x * grid.y, partials);
     NHP_LAUNCHED(ctx);
     DCUDA(ctx, cudaGetLastError());

@@ -50,7 +50,7 @@ def test_chunked_speculative_sweep_matches_oracle(monkeypatch, kind, K, n, rate,
 def test_flips_larger_than_the_baseline_rate_are_certified_one_sidedly(monkeypatch, chunk):
     """lambda0 far below a single pair's contribution: every accepted flip moves intensities by more than lambda0 / 2, the case the
     first certification rule could only handle by ending the batch.  The one-sided bounds (S / (1 + on / lambda0) <= S' <= S (1 + off / lambda0))
-    must still give exactly the sequential sweep, with no more batches than the old rule (NHP_ADJ_CERT=0), which must agree as well."""
+    must still give exactly the sequential sweep (tests/test_certification_bound.py checks the bound itself)."""
     if chunk is not None:
         monkeypatch.setenv("NHP_ADJ_CHUNK", str(chunk))
     K, n, rho = 70, 9000, 0.5
@@ -62,19 +62,14 @@ def test_flips_larger_than_the_baseline_rate_are_certified_one_sidedly(monkeypat
     proc = nhp.ContinuousNetworkHawkesProcess(nhp.HomogeneousProcess(lam0), nhp.LogitNormalImpulseResponse(mu, tau, 1.0), nhp.DenseWeightModel(W), A0.copy(),
                                               nhp.BernoulliNetworkModel(rho, K))
     om = orc.Cont(1, lam0, W, mu, tau, A=A0, dtmax=1.0)
-    batches = {}
-    for cert in ("1", "0"):
-        monkeypatch.setenv("NHP_ADJ_CERT", cert)
-        bad = flips = 0
-        for rep in range(2):
-            u = np.random.default_rng(500 + rep).random((K, K))
-            A_gpu, A_ref = run_both(proc, om, (t, nodes, T), rho, u, A0)
-            bad += int(np.count_nonzero(A_gpu != A_ref))
-            flips += int(np.count_nonzero(A_ref != A0))
-        assert bad == 0
-        assert flips > 10 * K  # the sweep really flips many links per column
-        batches[cert] = nhp.adjacency_info()["batches"]
-    assert batches["1"] <= batches["0"]
+    bad = flips = 0
+    for rep in range(2):
+        u = np.random.default_rng(500 + rep).random((K, K))
+        A_gpu, A_ref = run_both(proc, om, (t, nodes, T), rho, u, A0)
+        bad += int(np.count_nonzero(A_gpu != A_ref))
+        flips += int(np.count_nonzero(A_ref != A0))
+    assert bad == 0
+    assert flips > 10 * K  # the sweep really flips many links per column
 
 
 @pytest.mark.parametrize("chunk,cluster", [(None, None), (64, None), (64, "0")])

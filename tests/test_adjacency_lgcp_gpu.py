@@ -1,6 +1,6 @@
 """The adjacency sampler and the structure log-likelihood of network processes with LogGaussianCoxProcess baselines
 (csrc/cont_adjacency.cu, csrc/cont_baseline.cu; continuous.jl:444-519 with total_intensity reading lambda0_c(t_i)).  The decisions
-given u must be those of the sequential sweep of tests/grid_reference.py, for every form of the sweep and both certification rules."""
+given u must be those of the sequential sweep of tests/grid_reference.py, for every form of the sweep."""
 import ctypes
 
 import numpy as np
@@ -51,7 +51,6 @@ def run_both(proc, ref, data, rho, u, A0, **kw):
     return A_gpu, A_ref
 
 
-@pytest.mark.parametrize("cert", ["1", "0"])
 @pytest.mark.parametrize("kind,dtmax,env", [
     ("ln", 1.0, {}),                                              # 18-byte LogitNormal payload
     ("ln", 1.0, {"NHP_ADJ_PRE": "0"}),                            # lag payload
@@ -60,11 +59,17 @@ def run_both(proc, ref, data, rho, u, A0, **kw):
     ("ln", 1.0, {"NHP_ADJ_CACHE": "0"}),                          # uncached fallback
     ("exp", 1.0, {}),
     ("exp", np.inf, {}),                                          # cut-off horizon from the curves' minimum
+    ("exp", 1.0, {"NHP_ADJ_CHUNK": "64"}),
+    ("exp", 1.0, {"NHP_ADJ_CHUNK": "7", "NHP_ADJ_CLUSTER": "0"}),
+    ("exp", 1.0, {"NHP_ADJ_CACHE": "0"}),
+    ("exp", np.inf, {"NHP_ADJ_CHUNK": "64"}),
+    ("ln", 1.0, {"NHP_ADJ_PRE": "0", "NHP_ADJ_CHUNK": "64"}),     # lag payload across a cluster
+    ("ln", 1.0, {"NHP_ADJ_S0": "1"}),                             # batches grow from one bucket with the observed flip rate
+    ("ln", 1.0, {"NHP_ADJ_S0": "4", "NHP_ADJ_CHUNK": "64"}),
 ])
-def test_sweep_with_curves_matches_reference(monkeypatch, kind, dtmax, env, cert):
+def test_sweep_with_curves_matches_reference(monkeypatch, kind, dtmax, env):
     for k, v in env.items():
         monkeypatch.setenv(k, v)
-    monkeypatch.setenv("NHP_ADJ_CERT", cert)
     K, rho = 13, 0.4
     n, rate = (1500, 20.0) if dtmax == np.inf else (4000, 60.0)
     t, nodes, T = synth.poisson_stream(n, K, rate, 31)
@@ -89,8 +94,7 @@ def test_sweep_with_curves_matches_reference(monkeypatch, kind, dtmax, env, cert
 @pytest.mark.parametrize("chunk", [None, 64])
 def test_deep_dips_below_the_flips_restart_but_stay_exact(monkeypatch, chunk):
     """Curves that fall to 1e-3 of their mean inside every column, with single contributions far above that minimum: the
-    certification bound (taken from the column minimum) is loose, batches restart, and the decisions are still the sequential ones,
-    under both rules."""
+    certification bound (taken from the column minimum) is loose, batches restart, and the decisions are still the sequential ones."""
     if chunk is not None:
         monkeypatch.setenv("NHP_ADJ_CHUNK", str(chunk))
     K, n, rho = 60, 9000, 0.5
@@ -100,14 +104,12 @@ def test_deep_dips_below_the_flips_restart_but_stay_exact(monkeypatch, chunk):
     A0 = proc.adjacency_matrix.copy()
     rates = np.array([np.interp(t[nodes == c + 1], x, lam[c]).min() for c in range(K)])
     assert np.median(rates) < 2e-3  # the columns do see the dips
-    for cert in ("1", "0"):
-        monkeypatch.setenv("NHP_ADJ_CERT", cert)
-        u = np.random.default_rng(80).random((K, K))
-        A_gpu, A_ref = run_both(proc, ref, (t, nodes, T), rho, u, A0)
-        assert int(np.count_nonzero(A_gpu != A_ref)) == 0
-        assert int(np.count_nonzero(A_ref != A0)) > 5 * K
-        info = nhp.adjacency_info()
-        assert info["batches"] > 0 and info["recomputed_steps"] > 0
+    u = np.random.default_rng(80).random((K, K))
+    A_gpu, A_ref = run_both(proc, ref, (t, nodes, T), rho, u, A0)
+    assert int(np.count_nonzero(A_gpu != A_ref)) == 0
+    assert int(np.count_nonzero(A_ref != A0)) > 5 * K
+    info = nhp.adjacency_info()
+    assert info["batches"] > 0 and info["recomputed_steps"] > 0
 
 
 def test_column_partition_and_config4_shape():

@@ -57,7 +57,5 @@ for w in ("1", "0"):
     os.environ["NHP_DISC_WARP"] = w
     D.resample_parents(proc, dd, seed=1)
     D.vb_statistics(proc, dd, np.ones(N), np.full((N, N, B), 0.1))
-os.environ["NHP_DISC_DMMA"] = "0"
-print(D.loglikelihood(proc, dd))
 D.resample_adjacency_matrix_(proc, dd, seed=2)
 print("all kernels ran")
