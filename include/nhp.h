@@ -101,6 +101,23 @@ int nhp_cont_baseline_grid(nhp_ctx *ctx, int64_t n_grid, const double *x, const 
  * The parent assignment is the device-resident one of the last nhp_cont_resample_parents on `ev` (split_extract never
  * materialises).  Time shards return additive shares. */
 int nhp_cont_baseline_loglik(nhp_ctx *ctx, nhp_events *ev, int64_t n_grid, const double *x, const double *values, double *ll);
+/* The GP prior of the log-curves (baselines.jl:187-212): log lambda0_k = m + y_k, y_k ~ N(0, L L^T) on the grid.  L[g + n_grid*h]
+ * is the lower-triangular Cholesky factor, column-major (its strictly upper triangle is ignored); n_grid must be that of the current
+ * curves and at most 4096, L finite with a positive diagonal (NHP_ERR_INVALID otherwise).  nhp_cont_params_set, nhp_cont_baseline_grid
+ * with n_grid = 0 and a grid of another size drop the prior.  With curves and a prior, nhp_cont_gibbs_sweep updates the curves. */
+int nhp_cont_baseline_prior(nhp_ctx *ctx, int64_t n_grid, const double *L, double m);
+/* resample!(process::LogGaussianCoxProcess, data, parents) (baselines.jl:214-326) for all K nodes on the device: one elliptical-slice
+ * update per node [Murray, Adams & MacKay 2010] with the likelihood of nhp_cont_baseline_loglik, from the parents of the last parent
+ * sweep on `ev` (a rank's time shard: the per-node sums are all-reduced, every rank reaches the same curves).  Random numbers:
+ * z == NULL && u == NULL: Philox keyed by (seed; node, draw, counter); otherwise both are host arrays, z[g + n_grid*k] standard
+ * normals (the prior draw is L z) and u[j + 101*k] uniforms, j = 0 the slice height, j = 1 + a the angle of attempt a (attempt 0:
+ * theta = 2 pi u; after a rejection the bracket side theta is on shrinks to theta and theta = lo + u (hi - lo)).  attempts[K] (may be
+ * NULL) receives the candidates each node evaluated.  NHP_ERR_STATE without curves, prior or parent assignment; NHP_ERR_NUMERIC for
+ * a curve value <= 0 or when a node reaches 100 attempts (baselines.jl:316).  The curves change only when every node accepted; the
+ * new ones invalidate the parent assignment, as nhp_cont_baseline_grid does. */
+int nhp_cont_resample_baseline(nhp_ctx *ctx, nhp_events *ev, uint64_t seed, uint64_t counter, const double *z, const double *u, int64_t *attempts);
+/* The current curves in the layout of nhp_cont_baseline_grid (values[g + n_grid*k]). */
+int nhp_cont_baseline_get(nhp_ctx *ctx, double *values);
 
 /* Look-back horizon the sweeps use for the current parameters: dtmax for LogitNormal; for
  * Exponential min(dtmax, H) where H is the cut-off beyond which the omitted tail of any event's
@@ -205,12 +222,15 @@ int nhp_cont_params_get(nhp_ctx *ctx, double *lambda0, double *W, double *A, dou
  * parameters as they are, the adjacency matrix bit-packed: K^2 / 8 bytes); _push appends the context's current parameters
  * (device-to-device on the context's stream, no host synchronisation) -- nhp_cont_gibbs_sweep does it by itself while a trace is
  * open; _read copies samples [first, first + count) to the host, one sample after the other in the layouts of
- * nhp_cont_params_get (rho[count], lambda0[count*K], W | A | p1 | p2 [count*K*K]; any pointer may be NULL). */
+ * nhp_cont_params_get (rho[count], lambda0[count*K], W | A | p1 | p2 [count*K*K]; any pointer may be NULL).  A trace begun while the
+ * context holds curves and their prior also keeps the K x n_grid curves of every sample (_read_curves: values[g + n_grid*(k + K*j)]
+ * for sample first + j; NHP_ERR_STATE for a trace without curves); _push then refuses a grid of another size. */
 int nhp_cont_trace_begin(nhp_ctx *ctx, int64_t capacity);
 int nhp_cont_trace_push(nhp_ctx *ctx);
 int nhp_cont_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity);
 int nhp_cont_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *rho, double *lambda0, double *W, double *A, double *p1, double *p2);
 int nhp_cont_trace_free(nhp_ctx *ctx);
+int nhp_cont_trace_read_curves(nhp_ctx *ctx, int64_t first, int64_t count, double *values);
 
 /* ---- multi-GPU (one process and one context per GPU; NCCL over NVLink, loaded with dlopen) ---------------------
  * SURVEY.md section 8e.  Time shards (nhp_events_upload with n_halo / index_base) carry the log-likelihood, the parent
@@ -240,8 +260,10 @@ int nhp_comm_allgather_adjacency(nhp_ctx *ctx);
 int nhp_comm_allgather_events(nhp_ctx *ctx, nhp_events *ev_shard, nhp_events **out);
 /* hyper as for nhp_cont_resample_params; net_alpha > 0: BernoulliNetworkModel with rho ~ Beta(net_alpha, net_beta) prior
  * (networks.jl:45-54, 72-78), else link probability 1 (DenseNetworkModel).  ev_full (the unsharded stream, replicated on
- * every rank) is only used by network processes; pass ev_shard itself on a single GPU.  A network process with grid baseline
- * curves (nhp_cont_baseline_grid) is refused with NHP_ERR_UNSUPPORTED before anything changes: the curves are not drawn here. */
+ * every rank) is only used by network processes; pass ev_shard itself on a single GPU.  With grid baseline curves and their prior
+ * (nhp_cont_baseline_prior) the sweep runs nhp_cont_resample_baseline(seed, counter) after the conjugate draws and before the
+ * adjacency sweep.  A network process with curves but no prior is refused with NHP_ERR_UNSUPPORTED before anything changes; a
+ * standard process with curves but no prior keeps its curves. */
 int nhp_cont_gibbs_sweep(nhp_ctx *ctx, nhp_events *ev_shard, nhp_events *ev_full, uint64_t seed, uint64_t counter, double duration,
                          const double *hyper, int n_hyper, double net_alpha, double net_beta);
 /* Device pointer + length (in doubles) of a statistics buffer, for hosts that run their own collectives. */

@@ -24,8 +24,11 @@ int nhp_test_fastmath(nhp_ctx *ctx, int which, const double *x, int64_t n, doubl
  * virtual columns, sweep kernel ms, structure build ms]. */
 int nhp_cont_adjacency_info(const nhp_ctx *ctx, double *out8);
 /* Last nhp_cont_gibbs_sweep of this context: out8 = [parent sweep ms, second pass + conjugate draws + table rebuild ms,
- * adjacency sweep kernel ms, 0...]. */
+ * adjacency sweep kernel ms, slice update of the curves ms, its rounds, 0...]. */
 int nhp_cont_sweep_info(const nhp_ctx *ctx, double *out8);
+/* Last nhp_cont_resample_baseline of this context: out4 = [list build ms (draws, prior draw, baseline-event records, work items),
+ * rounds + commit ms, rounds, work items]. */
+int nhp_cont_slice_info(const nhp_ctx *ctx, double *out4);
 /* Keep / bring back a device-side copy of the continuous parameters (lambda0, W, A, p1, p2) and rebuild the tables:
  * bench.py rewinds a chain to the workload's parameters between timed steps without a host round trip. */
 int nhp_cont_params_save(nhp_ctx *ctx);

@@ -127,6 +127,13 @@ extern "C" int nhp_comm_allreduce_stats(nhp_ctx *ctx, int phase) {
     return NHP_OK;
 }
 
+// all-reduce (sum) of a device vector, in place on the context's stream (the per-node sums of the curves' slice update)
+int nhp_comm_allreduce_dev(nhp_ctx *ctx, double *buf, int64_t n) {
+    if (!ctx->comm || ctx->nranks == 1) return NHP_OK;
+    NHP_NCCL(ctx, g_nccl.AllReduce(buf, buf, (size_t)n, ncclFloat64, ncclSum, (ncclComm_t)ctx->comm, ctx->stream));
+    return NHP_OK;
+}
+
 // all-reduce (sum) of a small host vector (log-likelihood shares, gradient norms, ...): staged through the device
 extern "C" int nhp_comm_allreduce_host(nhp_ctx *ctx, double *inout, int64_t n) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
@@ -225,16 +232,18 @@ extern "C" int nhp_comm_allgather_events(nhp_ctx *ctx, nhp_events *ev_shard, nhp
 
 // One whole Gibbs sweep of `resample!` (continuous.jl:202-208 / 350-358) on the device, for 1..N GPUs with one call
 // sequence: parent sweep + fused statistics on this rank's time shard, all-reduce, second pass, all-reduce, conjugate draws
-// (identical on every rank), and for a network process the adjacency sweep over this rank's columns of the replicated
+// (identical on every rank), with curves and their prior the elliptical-slice update of the curves (per-node sums all-reduced,
+// identical decisions on every rank), and for a network process the adjacency sweep over this rank's columns of the replicated
 // stream `ev_full`, the all-gather of the columns, the table rebuild and the Beta draw of rho.
 extern "C" int nhp_cont_gibbs_sweep(nhp_ctx *ctx, nhp_events *ev_shard, nhp_events *ev_full, uint64_t seed, uint64_t counter, double duration,
                                     const double *hyper, int n_hyper, double net_alpha, double net_beta) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
     NHP_CHECK(ctx, ev_shard != nullptr, NHP_ERR_INVALID, "nhp_cont_gibbs_sweep: events handle is NULL");
-    // the draws here are the conjugate ones; the curves of a LogGaussianCoxProcess baseline move with the host's elliptical slice
-    // sampler (resample_on_device_), so a network process with curves is refused before anything changes
-    NHP_CHECK(ctx, !(ctx->cont_set && ctx->has_A && ctx->bgrid_n > 0), NHP_ERR_UNSUPPORTED,
-              "nhp_cont_gibbs_sweep: a network process with a grid baseline takes the elliptical-slice update of its curves on the host");
+    // curves with a prior (nhp_cont_baseline_prior) take their elliptical-slice update here; without a prior they move with the
+    // host's slice sampler (resample_on_device_), so a network process with curves and no prior is refused before anything changes
+    const bool curves = ctx->cont_set && ctx->bgrid_n > 0, prior = curves && ctx->bprior_n == ctx->bgrid_n;
+    NHP_CHECK(ctx, !(ctx->cont_set && ctx->has_A && curves && !prior), NHP_ERR_UNSUPPORTED,
+              "nhp_cont_gibbs_sweep: a network process with a grid baseline takes the elliptical-slice update of its curves on the host (or set their prior: nhp_cont_baseline_prior)");
     for (int i = 0; i < 8; i++) ctx->sweep_info[i] = 0.0;
     NHP_TRY(nhp_cont_resample_parents(ctx, ev_shard, seed, counter, nullptr, nullptr, nullptr));
     ctx->sweep_info[0] = ctx->last_ms;  // parent sweep + fused statistics
@@ -243,6 +252,11 @@ extern "C" int nhp_cont_gibbs_sweep(nhp_ctx *ctx, nhp_events *ev_shard, nhp_even
     NHP_TRY(nhp_comm_allreduce_stats(ctx, 1));
     NHP_TRY(nhp_cont_resample_params(ctx, ev_shard, seed, counter, duration, hyper, n_hyper, 0));
     ctx->sweep_info[1] = ctx->last_ms;  // (all-reduces, second pass,) conjugate draws + table rebuild: everything since the parent sweep
+    if (prior) {
+        NHP_TRY(nhp_cont_resample_baseline(ctx, ev_shard, seed, counter, nullptr, nullptr, nullptr));
+        ctx->sweep_info[3] = ctx->last_ms;  // slice update of the curves: list build + rounds + commit
+        ctx->sweep_info[4] = ctx->slice_info[2];  // its rounds
+    }
     if (ctx->has_A) {
         NHP_CHECK(ctx, ev_full != nullptr, NHP_ERR_INVALID, "nhp_cont_gibbs_sweep: a network process needs the unsharded stream for the adjacency sweep");
         const double rho = net_alpha > 0.0 ? -1.0 : 1.0;  // Bernoulli network: the context's rho; otherwise a dense network (link probability 1)

@@ -71,11 +71,13 @@ extern "C" int nhp_cont_baseline_grid(nhp_ctx *ctx, int64_t n_grid, const double
         NHP_CUDA(ctx, cudaStreamSynchronize(s));
         cudaFree(ctx->d_bgrid_x); cudaFree(ctx->d_bgrid_v);
         ctx->d_bgrid_x = ctx->d_bgrid_v = nullptr; ctx->bgrid_n = 0; ctx->baseline_integral = 0.0;
+        ctx->bprior_n = 0;
         return NHP_OK;
     }
     const int64_t K = ctx->K;
     NHP_TRY(check_grid(ctx, n_grid, x, values, K, "nhp_cont_baseline_grid"));
     if (ctx->bgrid_n != n_grid) {
+        ctx->bprior_n = 0;  // a prior of another grid size does not apply
         NHP_CUDA(ctx, cudaStreamSynchronize(s));
         cudaFree(ctx->d_bgrid_x); cudaFree(ctx->d_bgrid_v);
         ctx->d_bgrid_x = ctx->d_bgrid_v = nullptr; ctx->bgrid_n = 0;

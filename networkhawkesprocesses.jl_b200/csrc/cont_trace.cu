@@ -31,8 +31,8 @@ extern "C" int nhp_cont_trace_free(nhp_ctx *ctx) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
-    cudaFree(ctx->d_trace); cudaFree(ctx->d_trace_bits);
-    ctx->d_trace = nullptr; ctx->d_trace_bits = nullptr; ctx->trace_cap = ctx->trace_len = 0;
+    cudaFree(ctx->d_trace); cudaFree(ctx->d_trace_bits); cudaFree(ctx->d_trace_curves);
+    ctx->d_trace = nullptr; ctx->d_trace_bits = nullptr; ctx->d_trace_curves = nullptr; ctx->trace_cap = ctx->trace_len = 0; ctx->trace_G = 0;
     return NHP_OK;
 }
 
@@ -43,12 +43,17 @@ extern "C" int nhp_cont_trace_begin(nhp_ctx *ctx, int64_t capacity) {
     NHP_TRY(nhp_cont_trace_free(ctx));
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t sd = trace_slot_doubles(ctx), sw = trace_slot_words(ctx);
+    // curves with a prior move with the sweep (nhp_cont_gibbs_sweep): every slot also keeps them
+    const int64_t G = ctx->bgrid_n > 0 && ctx->bprior_n == ctx->bgrid_n ? ctx->bgrid_n : 0;
+    const size_t sc = (size_t)(ctx->K * G);
     if (cudaMalloc(&ctx->d_trace, (size_t)capacity * sd * sizeof(double)) != cudaSuccess ||
-        (sw && cudaMalloc(&ctx->d_trace_bits, (size_t)capacity * sw * sizeof(uint32_t)) != cudaSuccess)) {
+        (sw && cudaMalloc(&ctx->d_trace_bits, (size_t)capacity * sw * sizeof(uint32_t)) != cudaSuccess) ||
+        (sc && cudaMalloc(&ctx->d_trace_curves, (size_t)capacity * sc * sizeof(double)) != cudaSuccess)) {
         cudaGetLastError();
-        cudaFree(ctx->d_trace); ctx->d_trace = nullptr;
-        return nhp_fail(ctx, NHP_ERR_CUDA, "nhp_cont_trace_begin: cannot allocate %lld slots of %.1f MB", (long long)capacity, 1e-6 * (double)(sd * 8 + sw * 4));
+        cudaFree(ctx->d_trace); cudaFree(ctx->d_trace_bits); ctx->d_trace = nullptr; ctx->d_trace_bits = nullptr;
+        return nhp_fail(ctx, NHP_ERR_CUDA, "nhp_cont_trace_begin: cannot allocate %lld slots of %.1f MB", (long long)capacity, 1e-6 * (double)(sd * 8 + sw * 4 + sc * 8));
     }
+    ctx->trace_G = G;
     ctx->trace_cap = capacity; ctx->trace_len = 0; ctx->trace_K = ctx->K; ctx->trace_kind = ctx->kind; ctx->trace_has_A = ctx->has_A;
     return NHP_OK;
 }
@@ -60,6 +65,8 @@ extern "C" int nhp_cont_trace_push(nhp_ctx *ctx) {
     NHP_CHECK(ctx, ctx->cont_set && ctx->trace_K == ctx->K && ctx->trace_kind == ctx->kind && ctx->trace_has_A == ctx->has_A, NHP_ERR_STATE,
               "nhp_cont_trace_push: the model changed since nhp_cont_trace_begin");
     NHP_CHECK(ctx, ctx->trace_len < ctx->trace_cap, NHP_ERR_STATE, "nhp_cont_trace_push: the trace is full (%lld slots)", (long long)ctx->trace_cap);
+    NHP_CHECK(ctx, ctx->trace_G == 0 || ctx->bgrid_n == ctx->trace_G, NHP_ERR_STATE, "nhp_cont_trace_push: the curves' grid changed since nhp_cont_trace_begin (%lld -> %lld points)",
+              (long long)ctx->trace_G, (long long)ctx->bgrid_n);
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t K = (size_t)ctx->K, KK = K * K, sd = trace_slot_doubles(ctx), sw = trace_slot_words(ctx);
     cudaStream_t s = ctx->stream;
@@ -70,6 +77,10 @@ extern "C" int nhp_cont_trace_push(nhp_ctx *ctx) {
     NHP_CUDA(ctx, cudaMemcpyAsync(slot + 1 + K, ctx->d_W, KK * sizeof(double), cudaMemcpyDeviceToDevice, s));
     NHP_CUDA(ctx, cudaMemcpyAsync(slot + 1 + K + KK, ctx->d_p1, KK * sizeof(double), cudaMemcpyDeviceToDevice, s));
     if (ctx->kind == NHP_LOGITNORMAL) NHP_CUDA(ctx, cudaMemcpyAsync(slot + 1 + K + 2 * KK, ctx->d_p2, KK * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    if (ctx->trace_G > 0) {
+        const size_t sc = K * (size_t)ctx->trace_G;
+        NHP_CUDA(ctx, cudaMemcpyAsync(ctx->d_trace_curves + (size_t)ctx->trace_len * sc, ctx->d_bgrid_v, sc * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    }
     if (sw) {
         const int64_t warps = (int64_t)sw;
         k_trace_pack_bits<<<(unsigned)((warps + 7) / 8), 256, 0, s>>>(ctx->d_A, (int64_t)KK, ctx->d_trace_bits + (size_t)ctx->trace_len * sw);
@@ -116,5 +127,20 @@ extern "C" int nhp_cont_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, d
         }
     }
     NHP_CUDA(ctx, cudaStreamSynchronize(s));
+    return NHP_OK;
+}
+
+// the curves of samples [first, first + count): values[g + G (k + K j)] is curve point g of node k in sample first + j
+extern "C" int nhp_cont_trace_read_curves(nhp_ctx *ctx, int64_t first, int64_t count, double *values) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    NHP_CHECK(ctx, ctx->trace_G > 0, NHP_ERR_STATE, "nhp_cont_trace_read_curves: the trace holds no curves (begin it with curves and their prior set)");
+    NHP_CHECK(ctx, first >= 0 && count >= 0 && first + count <= ctx->trace_len, NHP_ERR_INVALID, "nhp_cont_trace_read_curves: samples [%lld, %lld) outside the %lld stored",
+              (long long)first, (long long)(first + count), (long long)ctx->trace_len);
+    if (count == 0) return NHP_OK;
+    NHP_CHECK(ctx, values != nullptr, NHP_ERR_INVALID, "nhp_cont_trace_read_curves: NULL argument");
+    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t sc = (size_t)ctx->trace_K * (size_t)ctx->trace_G;
+    NHP_CUDA(ctx, cudaMemcpyAsync(values, ctx->d_trace_curves + (size_t)first * sc, (size_t)count * sc * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return NHP_OK;
 }

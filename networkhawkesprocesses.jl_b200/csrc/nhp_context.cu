@@ -84,7 +84,7 @@ extern "C" int nhp_destroy(nhp_ctx *ctx) {
     cudaFree(ctx->d_partials); cudaFree(ctx->d_scratch); cudaFree(ctx->d_flag); cudaFree(ctx->d_winstat);
     cudaFree(ctx->dd_lambda0); cudaFree(ctx->dd_W); cudaFree(ctx->dd_A); cudaFree(ctx->dd_theta); cudaFree(ctx->dd_bump);
     cudaFree(ctx->dd_klist); cudaFree(ctx->dd_kptr); cudaFree(ctx->dd_btc); cudaFree(ctx->dd_counts);
-    cudaFree(ctx->d_bgrid_x); cudaFree(ctx->d_bgrid_v);
+    cudaFree(ctx->d_bgrid_x); cudaFree(ctx->d_bgrid_v); cudaFree(ctx->d_bprior_L); cudaFree(ctx->d_slice);
     cudaFree(ctx->d_adj_ctl); cudaFree(ctx->d_adj_stat);
     cudaEventDestroy(ctx->ev0); cudaEventDestroy(ctx->ev1);
     cudaStreamDestroy(ctx->own_stream);
@@ -355,7 +355,8 @@ extern "C" int nhp_events_free(nhp_ctx *ctx, nhp_events *ev) {
     }
     {
         cudaStream_t as = ctx ? ctx->stream : nullptr;
-        void *blocks[] = {ev->d_order, ev->d_node_ptr, ev->d_item_node, ev->d_item_e0, ev->d_lam0ev, ev->d_lam0bn, ev->d_lam0min};
+        void *blocks[] = {ev->d_order, ev->d_node_ptr, ev->d_item_node, ev->d_item_e0, ev->d_lam0ev, ev->d_lam0bn, ev->d_lam0min,
+                          ev->d_sl_g, ev->d_sl_item, ev->d_sl_t, ev->d_sl_part};
         for (void *b : blocks) if (b) cudaFreeAsync(b, as);
     }
     nhp_events_free_adjacency(ctx, ev, ctx ? ctx->stream : nullptr);
@@ -441,6 +442,7 @@ extern "C" int nhp_cont_params_set(nhp_ctx *ctx, int kind, int64_t K, const doub
     NHP_CHECK(ctx, kind == NHP_EXPONENTIAL || p2 != nullptr, NHP_ERR_INVALID, "nhp_cont_params_set: LogitNormal needs tau (p2)");
     NHP_CHECK(ctx, dtmax > 0.0, NHP_ERR_INVALID, "nhp_cont_params_set: dtmax must be positive");
     if (ctx->bgrid_n > 0) { ctx->bgrid_n = 0; ctx->bgrid_version++; }  // a new parameter set starts from its homogeneous lambda0; curves are re-applied with nhp_cont_baseline_grid
+    ctx->bprior_n = 0;  // and their prior with nhp_cont_baseline_prior
     NHP_CHECK(ctx, kind == NHP_EXPONENTIAL || std::isfinite(dtmax), NHP_ERR_INVALID, "nhp_cont_params_set: LogitNormal needs a finite dtmax");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     const int64_t KK = K * K;

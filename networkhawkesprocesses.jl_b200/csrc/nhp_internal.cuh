@@ -90,6 +90,9 @@ struct nhp_events {
     std::vector<double> lam0min;    // host copy of d_lam0min
     uint64_t lam0bn_version = 0;
     int64_t n_items = 0;
+    // elliptical-slice update of the curves (cont_slice.cu): baseline-event records in by-node order, work items, partial sums
+    int *d_sl_g = nullptr, *d_sl_item = nullptr;
+    double *d_sl_t = nullptr, *d_sl_part = nullptr;
     // cached structure of the adjacency sampler (cont_adjacency.cu): every (child event, window predecessor) pair, grouped by
     // virtual column = (child column, time chunk of at most adj_chunk_cap of the column's events) and bucketed by parent node,
     // stably ordered (event, window position) inside a bucket.  The pairs depend on the data and the look-back horizon; the
@@ -161,6 +164,10 @@ struct nhp_ctx {
     int64_t bgrid_n = 0; uint64_t bgrid_version = 0;     // 0 points: homogeneous lambda0
     double baseline_integral = 0.0;                      // sum_k integrate(lambda0_k) over the grid (trapezoid)
     double bgrid_min = 0.0;                              // smallest curve value: lambda0_min while the grid is active
+    // GP prior of the log-curves, log lambda0_k = m + y_k, y_k ~ N(0, L L^T) (nhp_cont_baseline_prior; cont_slice.cu): [bprior_n^2] L
+    double *d_bprior_L = nullptr; int64_t bprior_n = 0, bprior_cap = 0; double bprior_m = 0.0;  // 0 points: no prior
+    void *d_slice = nullptr; size_t slice_cap = 0;       // work buffers of the elliptical-slice update
+    double slice_info[4] = {0};                          // last update: list build ms, rounds + commit ms, rounds, work items
     double *d_W = nullptr, *d_A = nullptr, *d_p1 = nullptr, *d_p2 = nullptr; // raw [K*K] parent-major as passed
     void *d_table = nullptr;      // EntryLN/EntryEX [K*K] child-major
     double *d_rowsum = nullptr;   // [K] sum_c [A]W[p,c]
@@ -179,7 +186,8 @@ struct nhp_ctx {
     // device-side sample trace (cont_trace.cu): [trace_cap] slots of (rho, lambda0, W, p1 [, p2]) + bit-packed adjacency matrices
     double *d_trace = nullptr; uint32_t *d_trace_bits = nullptr;
     int64_t trace_cap = 0, trace_len = 0, trace_K = 0; int trace_kind = 0; bool trace_has_A = false;
-    double sweep_info[8] = {0};   // last nhp_cont_gibbs_sweep: ms of the parent sweep, of (second pass + draws + tables), of the adjacency kernel
+    double *d_trace_curves = nullptr; int64_t trace_G = 0;  // [trace_cap][K][trace_G] curves, for a trace begun with curves and a prior
+    double sweep_info[8] = {0};   // last nhp_cont_gibbs_sweep: ms of the parent sweep, of (second pass + draws + tables), of the adjacency kernel, of the curves' slice update, its rounds
     double adj_info[8] = {0};     // last adjacency sweep: steps, batches, flips, recomputed steps, entries, chunks, kernel ms, build ms
 
     // ---- statistics

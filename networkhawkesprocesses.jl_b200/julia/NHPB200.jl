@@ -29,6 +29,7 @@ import NetworkHawkesProcesses: loglikelihood, intensity, rand, resample_parents,
     ExponentialImpulseResponse, LogitNormalImpulseResponse, DiscreteGaussianImpulseResponse,
     BernoulliNetworkModel, link_probability, ndims, basis, fillna!, variational_log_expectation
 using Distributions: Gamma, Dirichlet
+using LinearAlgebra: cholesky, Symmetric
 
 const LIB = Ref{String}("libnhp")
 const CTX = Ref{Ptr{Cvoid}}(C_NULL)
@@ -309,18 +310,48 @@ function loglikelihood(process::LogGaussianCoxProcess, data::FusedParents, y::Ma
     return ll
 end
 
+# The elliptical-slice update of the curves on the device (nhp_cont_resample_baseline): the GP prior goes up as cholesky(Σ).L and m
+# (nhp_cont_baseline_prior; push_params! drops it, so it follows every push), the curves come back with nhp_cont_baseline_get.
+function push_baseline_prior!(b::LogGaussianCoxProcess)
+    L = Matrix{Float64}(cholesky(Symmetric(Matrix{Float64}(b.Σ))).L)   # column-major: L[g + n_grid*h]
+    check(ccall((:nhp_cont_baseline_prior, LIB[]), Cint, (Ptr{Cvoid}, Int64, Ptr{Float64}, Float64), CTX[], length(b.x), L, Float64(b.m)))
+end
+function pull_baseline!(b::LogGaussianCoxProcess)
+    vals = Matrix{Float64}(undef, length(b.x), length(b.λ))             # [grid, node]
+    check(ccall((:nhp_cont_baseline_get, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Float64}), CTX[], vals))
+    b.λ = [vals[:, k] for k in axes(vals, 2)]
+    return nothing
+end
+# resample!(process::LogGaussianCoxProcess, data, parents) for the parents of the last parent sweep on `data`, without a host round
+# trip per attempt; Philox keyed by (seed, counter).  Returns the candidates each node evaluated.
+function resample_baseline_on_device!(process::ContinuousHawkesProcess, data; seed::UInt64=Base.rand(UInt64), counter::UInt64=UInt64(0))
+    b = process.baseline
+    ev = device_events(process, data)
+    push_baseline_prior!(b)
+    attempts = Vector{Int64}(undef, length(b.λ))
+    check(ccall((:nhp_cont_resample_baseline, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, UInt64, UInt64, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}),
+        CTX[], ev.h, seed, counter, C_NULL, C_NULL, attempts))
+    pull_baseline!(b)
+    return attempts
+end
+gibbs_hyper(b, w, imp) = begin
+    a0, b0 = b isa LogGaussianCoxProcess ? (1.0, 1.0) : (b.α0, b.β0)   # the curves replace the homogeneous draw these feed
+    imp isa ExponentialImpulseResponse ? Float64[a0, b0, w.κ, w.ν, imp.α, imp.β] : Float64[a0, b0, w.κ, w.ν, imp.μμ, imp.κμ, imp.α0, imp.β0]
+end
+
 # optional: the whole `resample!(process, data)` (continuous.jl:202-208 / 350-358) in one call that never leaves the device
-# A LogGaussianCoxProcess baseline is not supported here: the device's draws are the conjugate ones, and its curves move with the
-# elliptical-slice update of `resample!`, which the device serves through the sweeps above.
-function resample_on_device!(process::ContinuousHawkesProcess, data)
-    process.baseline isa LogGaussianCoxProcess &&
-        throw(ArgumentError("resample_on_device!: a LogGaussianCoxProcess baseline takes resample! (elliptical-slice update of the curves)"))
+# A LogGaussianCoxProcess baseline needs `baseline_on_device=true`: the sweep then runs the elliptical-slice update of the curves
+# on the device after the conjugate draws (nhp_cont_gibbs_sweep with the prior set).
+function resample_on_device!(process::ContinuousHawkesProcess, data; baseline_on_device::Bool=false)
+    lgcp = process.baseline isa LogGaussianCoxProcess
+    lgcp && !baseline_on_device &&
+        throw(ArgumentError("resample_on_device!: a LogGaussianCoxProcess baseline takes resample! (elliptical-slice update of the curves on the host) unless baseline_on_device=true"))
     ev = device_events(process, data)
     push_params!(process)
+    lgcp && push_baseline_prior!(process.baseline)
     SWEEP[] += 1
     b, w, imp = process.baseline, process.weights, process.impulses
-    hyper = imp isa ExponentialImpulseResponse ? Float64[b.α0, b.β0, w.κ, w.ν, imp.α, imp.β] :
-                                                  Float64[b.α0, b.β0, w.κ, w.ν, imp.μμ, imp.κμ, imp.α0, imp.β0]
+    hyper = gibbs_hyper(b, w, imp)
     net = process isa ContinuousNetworkHawkesProcess
     bern = net && process.network isa BernoulliNetworkModel
     bern && check(ccall((:nhp_cont_network_set, LIB[]), Cint, (Ptr{Cvoid}, Float64), CTX[], Float64(process.network.ρ)))
@@ -333,7 +364,7 @@ function resample_on_device!(process::ContinuousHawkesProcess, data)
     q1 = Matrix{Float64}(undef, K, K); q2 = Matrix{Float64}(undef, K, K)
     check(ccall((:nhp_cont_params_get, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
         CTX[], λ, W, net ? A : C_NULL, q1, imp isa ExponentialImpulseResponse ? C_NULL : q2))
-    b.λ = λ; w.W = W
+    lgcp ? pull_baseline!(b) : (b.λ = λ); w.W = W
     if imp isa ExponentialImpulseResponse; imp.θ = q1 else imp.μ = q1; imp.τ = q2 end
     net && (process.adjacency_matrix .= A)
     if bern
@@ -345,15 +376,17 @@ function resample_on_device!(process::ContinuousHawkesProcess, data)
 end
 
 # `mcmc!` (inference.jl:49-70) with the chain and its sample trace on the device: the parameters go up once, every sweep is one
-# nhp_cont_gibbs_sweep (which appends its sample to the device-side trace, adjacency bit-packed), one read at the end.
-function mcmc_on_device!(process::ContinuousHawkesProcess, data; nsteps=1000)
-    process.baseline isa LogGaussianCoxProcess &&
-        throw(ArgumentError("mcmc_on_device!: a LogGaussianCoxProcess baseline takes mcmc! (the device trace would hold curves that never move)"))
+# nhp_cont_gibbs_sweep (which appends its sample to the device-side trace, adjacency bit-packed), one read at the end.  A
+# LogGaussianCoxProcess baseline needs `baseline_on_device=true`: the trace then also keeps the curves of every sample.
+function mcmc_on_device!(process::ContinuousHawkesProcess, data; nsteps=1000, baseline_on_device::Bool=false)
+    lgcp = process.baseline isa LogGaussianCoxProcess
+    lgcp && !baseline_on_device &&
+        throw(ArgumentError("mcmc_on_device!: a LogGaussianCoxProcess baseline takes mcmc! (elliptical-slice update of the curves on the host) unless baseline_on_device=true"))
     ev = device_events(process, data)
     push_params!(process)
+    lgcp && push_baseline_prior!(process.baseline)
     b, w, imp = process.baseline, process.weights, process.impulses
-    hyper = imp isa ExponentialImpulseResponse ? Float64[b.α0, b.β0, w.κ, w.ν, imp.α, imp.β] :
-                                                  Float64[b.α0, b.β0, w.κ, w.ν, imp.μμ, imp.κμ, imp.α0, imp.β0]
+    hyper = gibbs_hyper(b, w, imp)
     net = process isa ContinuousNetworkHawkesProcess
     bern = net && process.network isa BernoulliNetworkModel
     bern && check(ccall((:nhp_cont_network_set, LIB[]), Cint, (Ptr{Cvoid}, Float64), CTX[], Float64(process.network.ρ)))
@@ -372,13 +405,19 @@ function mcmc_on_device!(process::ContinuousHawkesProcess, data; nsteps=1000)
     check(ccall((:nhp_cont_trace_read, LIB[]), Cint,
         (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
         CTX[], 0, nsteps, ρ, λ, W, net ? A : C_NULL, q1, ln ? q2 : C_NULL))
+    if lgcp   # curves[g, k, sample]: they take the baseline's place in the samples
+        G = length(b.x)
+        C = Array{Float64}(undef, G, K, nsteps)
+        check(ccall((:nhp_cont_trace_read_curves, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}), CTX[], 0, nsteps, C))
+    end
     check(ccall((:nhp_cont_trace_free, LIB[]), Cint, (Ptr{Cvoid},), CTX[]))
     samples = Vector{Vector{Float64}}(undef, nsteps)
     for k in 1:nsteps   # the order of params(process): continuous.jl:116-119 / 325-333
         impv = ln ? [vec(q1[:, :, k]); vec(q2[:, :, k])] : vec(q1[:, :, k])
-        samples[k] = net ? [bern ? [ρ[k]] : Float64[]; λ[:, k]; vec(W[:, :, k]); impv; vec(A[:, :, k])] : [λ[:, k]; impv; vec(W[:, :, k])]
+        base = lgcp ? vec(C[:, :, k]) : λ[:, k]
+        samples[k] = net ? [bern ? [ρ[k]] : Float64[]; base; vec(W[:, :, k]); impv; vec(A[:, :, k])] : [base; impv; vec(W[:, :, k])]
     end
-    b.λ = λ[:, end]; w.W = W[:, :, end]
+    lgcp ? (b.λ = [C[:, j, end] for j in 1:K]) : (b.λ = λ[:, end]); w.W = W[:, :, end]
     if ln; imp.μ = q1[:, :, end]; imp.τ = q2[:, :, end] else imp.θ = q1[:, :, end] end
     net && (process.adjacency_matrix .= A[:, :, end])
     bern && (process.network.ρ = ρ[end])

@@ -69,11 +69,16 @@ PROTOTYPES = {
     "nhp_cont_loglik_dist": (c_int, [c_void_p, c_void_p, c_void_p, c_int, POINTER(c_double)]),
     "nhp_cont_baseline_grid": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     "nhp_cont_baseline_loglik": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "nhp_cont_baseline_prior": (c_int, [c_void_p, c_int64, c_void_p, c_double]),
+    "nhp_cont_resample_baseline": (c_int, [c_void_p, c_void_p, c_uint64, c_uint64, c_void_p, c_void_p, c_void_p]),
+    "nhp_cont_baseline_get": (c_int, [c_void_p, c_void_p]),
+    "nhp_cont_slice_info": (c_int, [c_void_p, c_double_p]),
     "nhp_cont_trace_begin": (c_int, [c_void_p, c_int64]),
     "nhp_cont_trace_push": (c_int, [c_void_p]),
     "nhp_cont_trace_count": (c_int, [c_void_p, POINTER(c_int64), POINTER(c_int64)]),
     "nhp_cont_trace_read": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "nhp_cont_trace_free": (c_int, [c_void_p]),
+    "nhp_cont_trace_read_curves": (c_int, [c_void_p, c_int64, c_int64, c_void_p]),
     "nhp_comm_allgather_adjacency": (c_int, [c_void_p]),
     "nhp_comm_allgather_events": (c_int, [c_void_p, c_void_p, ctypes.POINTER(c_void_p)]),
     "nhp_cont_gibbs_sweep": (c_int, [c_void_p, c_void_p, c_void_p, c_uint64, c_uint64, c_double, c_void_p, c_int, c_double, c_double]),

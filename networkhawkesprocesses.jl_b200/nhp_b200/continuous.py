@@ -63,7 +63,7 @@ class LogGaussianCoxProcess:
     """baselines.jl:187-336: lambda_k(t) = exp(m + y_k(t)), y_k ~ GP(0, SquaredExponentialKernel(sigma, eta)) on the grid `x`, linearly
     interpolated in between (utils/interpolation.jl).  `lam[k, g]` are the curve values at the grid points.  On the device the curves
     live inside the sweeps (nhp_cont_baseline_grid); the elliptical-slice update evaluates its likelihood for all nodes at once from the
-    device-resident parent assignment (nhp_cont_baseline_loglik)."""
+    device-resident parent assignment (nhp_cont_baseline_loglik), or runs on the device as a whole (resample_device_)."""
 
     def __init__(self, x, lam, m=0.0, sigma=1.0, eta=1.0):
         self.x = np.array(x, dtype=np.float64).reshape(-1)
@@ -135,6 +135,35 @@ class LogGaussianCoxProcess:
             raise RuntimeError("Elliptical slice sampling reached maximum attempts.")  # baselines.jl:316
         self.lam_grid = np.exp(self.m + ynew)
         return self.lam_grid.copy()
+
+    def push_prior(self, ctx):
+        """Send the GP prior of the log-curves to the device (nhp_cont_baseline_prior): the Cholesky factor of Sigma and m.  The
+        context must hold the curves; setting them again with another grid size, or new parameters, drops the prior."""
+        ctx.check(ctx.lib.nhp_cont_baseline_prior(ctx.h, self.x.size, _ptr(_f64(self._chol.ravel(order="F"))), self.m))
+
+    def pull_(self, ctx):
+        """Read the device's curves into `lam_grid` (nhp_cont_baseline_get)."""
+        v = np.empty(self.lam_grid.size)
+        ctx.check(ctx.lib.nhp_cont_baseline_get(ctx.h, _ptr(v)))
+        self.lam_grid = v.reshape(self.lam_grid.shape)
+        return self.lam_grid
+
+    def resample_device_(self, ctx, d, seed=0, counter=0, z=None, u=None):
+        """The update of `resample_` on the device (nhp_cont_resample_baseline), from the parents of the last parent sweep on `d`,
+        which must hold the current curves.  Random numbers: Philox keyed by (seed, counter), or the explicit `z[k, g]` standard
+        normals and `u[k, j]` uniforms (j = 0 slice height, j = 1 + a angle of attempt a; 101 per node) in the order `resample_`
+        consumes them.  Returns the new curves; `last_attempts` holds the candidates each node evaluated."""
+        K, G = self.lam_grid.shape
+        self.push_prior(ctx)
+        zz = uu = None
+        if z is not None or u is not None:
+            zz, uu = _f64(z).reshape(-1), _f64(u).reshape(-1)
+            if zz.size != K * G or uu.size != K * 101:
+                raise ValueError("z must hold K x len(x) normals and u K x 101 uniforms")
+        att = np.zeros(K, dtype=np.int64)
+        ctx.check(ctx.lib.nhp_cont_resample_baseline(ctx.h, d.h, int(seed), int(counter), _ptr(zz), _ptr(uu), _ptr(att)))
+        self.last_attempts = att
+        return self.pull_(ctx).copy()
 
 
 class ExponentialImpulseResponse:
@@ -599,7 +628,7 @@ def pull_params_(process, ctx=None):
     return process.params()
 
 
-def resample_on_device_(process, data, rng=None, seed=0, counter=0, push=True, pull=True):
+def resample_on_device_(process, data, rng=None, seed=0, counter=0, push=True, pull=True, baseline_on_device=False):
     """One Gibbs sweep that never leaves the GPU: parent sweep + fused statistics, second pass, the conjugate draws of
     baseline / weights / impulses (nhp_cont_resample_params), and for a network process the adjacency sweep on the
     device-resident matrix (nhp_cont_resample_adjacency_dev) and the Beta draw of rho (nhp_cont_resample_network), with
@@ -608,7 +637,8 @@ def resample_on_device_(process, data, rng=None, seed=0, counter=0, push=True, p
     A LogGaussianCoxProcess baseline takes its elliptical-slice update (with `rng`, or a generator seeded by (seed, counter)) from the
     device-resident parents after the conjugate draws, and its new curves go to the device before the adjacency sweep.  Weights and
     impulses are then drawn before the curves; given the parents they do not depend on them, so the sweep samples the same
-    conditionals."""
+    conditionals.  `baseline_on_device=True` runs that update on the device instead (nhp_cont_resample_baseline, Philox keyed by
+    (seed, counter)): the curves do not cross PCIe unless `pull`."""
     ctx = process._ctx()
     d, tmp = process._data(data)
     try:
@@ -621,7 +651,12 @@ def resample_on_device_(process, data, rng=None, seed=0, counter=0, push=True, p
         hy = _hyper(process)
         ctx.check(ctx.lib.nhp_cont_resample_params(ctx.h, d.h, int(seed), int(counter), float(d.duration), _ptr(hy), hy.size, 1))
         b = process.baseline
-        if isinstance(b, LogGaussianCoxProcess):
+        if isinstance(b, LogGaussianCoxProcess) and baseline_on_device:
+            b.push_prior(ctx)
+            ctx.check(ctx.lib.nhp_cont_resample_baseline(ctx.h, d.h, int(seed), int(counter), None, None, None))
+            if pull:
+                b.pull_(ctx)
+        elif isinstance(b, LogGaussianCoxProcess):
             b.resample_(ctx, d, rng if rng is not None else np.random.default_rng([int(seed), int(counter)]))
             # after the slice update: the new curves invalidate the parent assignment it reads
             ctx.check(ctx.lib.nhp_cont_baseline_grid(ctx.h, b.x.size, _ptr(_f64(b.x)), _ptr(_f64(b.lam_grid.ravel()))))
@@ -638,13 +673,17 @@ def resample_on_device_(process, data, rng=None, seed=0, counter=0, push=True, p
             d.free()
 
 
-def mcmc_device_(process, data, nsteps=1000, seed=0):
+def mcmc_device_(process, data, nsteps=1000, seed=0, baseline_on_device=False):
     """`mcmc!` (inference.jl:49-70) with the chain AND its sample trace on the device: parameters go up once, every sweep is one
     nhp_cont_gibbs_sweep (which appends its sample to the trace: device-to-device, adjacency bit-packed), and the trace comes back
     in one read at the end.  Returns MarkovChainMonteCarlo with the samples in the order of `params(process)`
-    ([rho;] lambda0; theta | mu, tau; W [; vec(A)], continuous.jl:116-119, 325-333); the process holds the last sample."""
-    if isinstance(process.baseline, LogGaussianCoxProcess):  # the device's draws would leave the curves where they are
-        raise ValueError("mcmc_device_: a LogGaussianCoxProcess baseline takes its elliptical-slice update on the host: use mcmc_(device_draws=True)")
+    ([rho;] lambda0; theta | mu, tau; W [; vec(A)], continuous.jl:116-119, 325-333); the process holds the last sample.
+    A LogGaussianCoxProcess baseline needs `baseline_on_device=True`: its prior goes up with the parameters, every sweep runs the
+    elliptical-slice update of the curves on the device, and the samples hold `lam_grid.ravel()` in the baseline's place."""
+    lgcp = isinstance(process.baseline, LogGaussianCoxProcess)
+    if lgcp and not baseline_on_device:  # the device's draws would leave the curves where they are
+        raise ValueError("mcmc_device_: a LogGaussianCoxProcess baseline takes its elliptical-slice update on the host unless "
+                         "baseline_on_device=True: pass it, or use mcmc_(device_draws=True)")
     ctx = process._ctx()
     d, tmp = process._data(data)
     t0 = time.time()
@@ -653,6 +692,8 @@ def mcmc_device_(process, data, nsteps=1000, seed=0):
         net = process.adjacency_matrix is not None
         bern = net and isinstance(process.network, BernoulliNetworkModel)
         process._push(ctx)
+        if lgcp:
+            process.baseline.push_prior(ctx)
         if bern:
             ctx.check(ctx.lib.nhp_cont_network_set(ctx.h, float(process.network.rho)))
         ctx.check(ctx.lib.nhp_cont_trace_begin(ctx.h, int(nsteps)))
@@ -665,6 +706,10 @@ def mcmc_device_(process, data, nsteps=1000, seed=0):
         p2 = np.empty((nsteps, K * K)) if ln else None
         A = np.empty((nsteps, K * K)) if net else None
         ctx.check(ctx.lib.nhp_cont_trace_read(ctx.h, 0, int(nsteps), _ptr(rho), _ptr(l0), _ptr(W), _ptr(A), _ptr(p1), _ptr(p2)))
+        if lgcp:  # the curves take the baseline's place in the samples
+            l0 = np.empty((nsteps, process.baseline.lam_grid.size))
+            ctx.check(ctx.lib.nhp_cont_trace_read_curves(ctx.h, 0, int(nsteps), _ptr(l0)))
+            process.baseline.lam_grid = l0[-1].reshape(process.baseline.lam_grid.shape).copy()
         ctx.check(ctx.lib.nhp_cont_trace_free(ctx.h))
         pull_params_(process, ctx)
         if bern:
@@ -696,10 +741,11 @@ def adjacency_info(ctx=None):
     return d
 
 
-def mcmc_(process, data, nsteps=1000, log_freq=100, verbose=False, seed=0, device_draws=False, store_every=1):
+def mcmc_(process, data, nsteps=1000, log_freq=100, verbose=False, seed=0, device_draws=False, store_every=1, baseline_on_device=False):
     """`mcmc!` (inference.jl:49-70): data is uploaded once and stays on the device.  `device_draws=True` keeps the whole
     sweep on the GPU (resample_on_device_): parameters are pushed once and pulled every `store_every` sweeps (and at the
-    end), so neither the K^2 statistics nor the K^2 parameters cross PCIe in between."""
+    end), so neither the K^2 statistics nor the K^2 parameters cross PCIe in between.  With it, `baseline_on_device=True` also
+    runs the elliptical-slice update of LogGaussianCoxProcess curves on the device."""
     rng = np.random.default_rng(seed)
     d = process.upload(data)
     t0 = time.time()
@@ -707,7 +753,7 @@ def mcmc_(process, data, nsteps=1000, log_freq=100, verbose=False, seed=0, devic
     for step in range(nsteps):
         if device_draws:
             keep = (step + 1) % store_every == 0 or step == nsteps - 1
-            x = resample_on_device_(process, d, rng, seed=seed, counter=step, push=(step == 0), pull=keep)
+            x = resample_on_device_(process, d, rng, seed=seed, counter=step, push=(step == 0), pull=keep, baseline_on_device=baseline_on_device)
             if keep:
                 samples.append(x)
         else:

@@ -9,6 +9,9 @@ libnhp) and the result is compared with the single-GPU computation of the same t
   * parent sweep + statistics: all-reduced counts == unsharded counts exactly (same Philox uniforms: keyed by the global event index)
   * adjacency sweep: column partition + nhp_comm_allgather_adjacency == full sweep, identical matrix
   * nhp_cont_gibbs_sweep: the composite call leaves identical parameters on every rank (checked through an all-reduce of a checksum)
+  * LogGaussianCoxProcess curves with a prior: nhp_cont_resample_baseline on the time shards (per-node sums all-reduced) == the update
+    of the unsharded stream on a context without communicator, 1e-12 with identical attempt counts; then three composite sweeps
+    leave identical curves on every rank
   * discrete time shards with an L-bin halo: log-likelihood and Gibbs counts summed over ranks == unsharded
 Prints one JSON line on rank 0; exit code 1 on any mismatch."""
 import ctypes
@@ -130,6 +133,40 @@ def main():
     res["composite_param_spread"] = float(np.max(np.abs(tot / world - chk) / np.maximum(1.0, np.abs(chk))))
     res["composite_links"] = int(Ad.sum())
     ok &= res["composite_param_spread"] < 1e-12 and np.all(np.isfinite(chk))
+
+    # ---------------- LGCP network with a prior: the slice update of the curves on the time shards
+    G = 41
+    rg = np.random.default_rng(8)
+    xg = np.linspace(0.0, T, G)
+    cv = lam0[:, None] * (1.0 + 0.3 * np.sin(2 * np.pi * rg.uniform(1.0, 4.0, (K, 1)) * xg[None, :] / T + rg.uniform(0, 2 * np.pi, (K, 1))))
+    zs, us = rg.standard_normal(K * G), rg.random(K * 101)
+
+    def lgcp_update(c, ev):
+        lg = nhp.ContinuousNetworkHawkesProcess(nhp.LogGaussianCoxProcess(xg, cv, m=float(np.log(lam0.mean())), eta=T / 10.0),
+                                                nhp.LogitNormalImpulseResponse(mu, tau, 1.0), nhp.DenseWeightModel(W), A, nhp.BernoulliNetworkModel(rho, K))
+        lg.ctx = c
+        lg._push(c)
+        c.check(c.lib.nhp_cont_resample_parents(c.h, ev.h, 41, 2, None, None, None))
+        lg.baseline.resample_device_(c, ev, z=zs, u=us)
+        return lg, lg.baseline.lam_grid.copy(), lg.baseline.last_attempts.copy()
+
+    single = nhp.Context(local)
+    full1 = ContinuousData(single, t, nodes, T, K)
+    _, cur_ref, att_ref = lgcp_update(single, full1)
+    full1.free()
+    lg, cur, att = lgcp_update(ctx, shard)
+    res["lgcp_curves_max_rel_err"] = float(np.max(np.abs(cur - cur_ref) / cur_ref))
+    res["lgcp_attempt_mismatches"] = int(np.count_nonzero(att != att_ref))
+    res["lgcp_attempts_max"] = int(att.max())
+    ok &= res["lgcp_curves_max_rel_err"] < 1e-12 and res["lgcp_attempt_mismatches"] == 0
+    ctx.check(lib.nhp_cont_network_set(ctx.h, rho))
+    for sweep in range(3):
+        ctx.check(lib.nhp_cont_gibbs_sweep(ctx.h, shard.h, full.h, 32, sweep, float(T), _ptr(hyper), hyper.size, 1.0, 1.0))
+    cur = lg.baseline.pull_(ctx).ravel()
+    tot = cur.copy()
+    ctx.check(lib.nhp_comm_allreduce_host(ctx.h, _ptr(tot), tot.size))
+    res["lgcp_composite_curve_spread"] = float(np.max(np.abs(tot / world - cur) / cur))
+    ok &= res["lgcp_composite_curve_spread"] < 1e-12
 
     # ---------------- intensity(process, data, times): the query times are sharded, the stream is replicated, no exchange but the gather
     proc._push(ctx)
