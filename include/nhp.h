@@ -305,8 +305,8 @@ int nhp_disc_gibbs_counts(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t co
  * nhp_disc_gibbs_counts left there (its `counts` argument may be NULL):  lambda0[c] ~ Gamma(alpha0 + counts[c,0], 1/(beta0 + T dt))
  * (baselines.jl:413-419, intended form), W[p,c] ~ Gamma(kappa + sum_b counts[c,p,b], 1/(nu + Mn[p])) (weights.jl:59-64),
  * theta[p,c,:] ~ Dirichlet(gamma + counts[c,p,:]) (impulses.jl:337-353).  Mn[N] = events per node; hyper = [alpha0, beta0, kappa, nu,
- * gamma]; Philox keyed (seed, element, counter).  The new parameters replace the context's (every derived table is rebuilt) and are
- * returned in the layouts of nhp_disc_params_set.  Parity with the reference is distributional. */
+ * gamma]; Philox keyed (seed, element, counter).  The new parameters replace the context's (every derived table is rebuilt on the
+ * device) and are returned in the layouts of nhp_disc_params_set.  Parity with the reference is distributional. */
 int nhp_disc_resample_params(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t counter, const double *Mn, const double *hyper, int n_hyper,
                              double *lambda0, double *W, double *theta);
 /* update_parents + the three VB reductions  parents.jl:136-177, baselines.jl:444-452,
@@ -316,6 +316,39 @@ int nhp_disc_vb_stats(nhp_ctx *ctx, nhp_disc *dd, const double *e0, const double
 /* resample_adjacency_matrix!(process, data, convolved)  discrete.jl:426-480 */
 int nhp_disc_resample_adjacency(nhp_ctx *ctx, nhp_disc *dd, const double *rho, uint64_t seed, uint64_t counter, const double *u,
                                 double *A_inout);
+/* Current parameters in the layouts of nhp_disc_params_set; any pointer may be NULL (A: NHP_ERR_STATE for a standard process). */
+int nhp_disc_params_get(nhp_ctx *ctx, double *lambda0, double *W, double *A, double *theta);
+/* Device-resident form for chains (`resample_adjacency_matrix!` of discrete.jl:426-460 without the N^2 matrices crossing PCIe):
+ * the sweep runs in place on the context's adjacency matrix with the scalar link probability `rho` of a BernoulliNetworkModel
+ * (networks.jl:65-68; rho < 0: the value kept by nhp_disc_network_set / nhp_disc_gibbs_sweep) and Philox uniforms keyed
+ * (seed, p + N c, counter), as nhp_disc_resample_adjacency with u = NULL; the derived tables follow the new matrix.  Unsharded
+ * data only (NHP_ERR_UNSUPPORTED for t_halo > 0). */
+int nhp_disc_resample_adjacency_dev(nhp_ctx *ctx, nhp_disc *dd, double rho, uint64_t seed, uint64_t counter);
+/* Link probability of the discrete BernoulliNetworkModel (networks.jl:45-54) kept with the context, apart from the continuous
+ * model's (nhp_cont_network_set). */
+int nhp_disc_network_set(nhp_ctx *ctx, double rho);
+int nhp_disc_network_get(const nhp_ctx *ctx, double *rho);
+/* Device-side sample trace of the discrete `mcmc!` (inference.jl:49-70; the reference pushes params(process) per sweep,
+ * discrete.jl:178-182 / 406-414).  Same semantics as nhp_cont_trace_*: one slot holds (rho, lambda0[N], W[N*N], theta[N*N*B]) and
+ * the adjacency matrix bit-packed; _push appends the context's current discrete parameters and rho (nhp_disc_gibbs_sweep does it
+ * while the trace has room) and refuses a model whose N or B changed, or that gained or lost A, since _begin; _read copies samples
+ * [first, first + count) in the layouts of nhp_disc_params_get, one after the other (any pointer may be NULL).  The discrete trace
+ * is independent of the continuous one. */
+int nhp_disc_trace_begin(nhp_ctx *ctx, int64_t capacity);
+int nhp_disc_trace_push(nhp_ctx *ctx);
+int nhp_disc_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity);
+int nhp_disc_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *rho, double *lambda0, double *W, double *A, double *theta);
+int nhp_disc_trace_free(nhp_ctx *ctx);
+/* One whole Gibbs sweep of the discrete `resample!` (discrete.jl:361-367 / 416-424) on the device, with no N^2-sized host transfer:
+ * parent counts (Philox: seed, uniform index, counter), the conjugate draws of nhp_disc_resample_params from them (Mn = the events
+ * per node kept with the data), and for a network process the in-place adjacency sweep (nhp_disc_resample_adjacency_dev with counter
+ * + 2^40) followed, when net_alpha > 0, by rho ~ Beta(net_alpha + sum(A), net_beta + N^2 - sum(A)) (networks.jl:72-78; otherwise link
+ * probability 1, DenseNetworkModel); then a push to the discrete trace while it has room.  Given the same (seed, counter) and state,
+ * lambda0, W, theta and A equal those of nhp_disc_gibbs_counts + nhp_disc_resample_params + nhp_disc_resample_adjacency.  hyper as
+ * for nhp_disc_resample_params (n_hyper = 5).  Time-sharded data or a communicator of more than one rank: NHP_ERR_UNSUPPORTED,
+ * before anything changes. */
+int nhp_disc_gibbs_sweep(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t counter, const double *hyper, int n_hyper, double net_alpha,
+                         double net_beta);
 
 #ifdef __cplusplus
 }

@@ -269,6 +269,34 @@ extern "C" int nhp_cont_gibbs_sweep(nhp_ctx *ctx, nhp_events *ev_shard, nhp_even
     return NHP_OK;
 }
 
+// One whole Gibbs sweep of the discrete `resample!` (discrete.jl:361-367 / 416-424) on one GPU, in the order and with the Philox keys
+// of discrete.resample_on_device_: parent counts (seed, counter), conjugate draws (seed, counter) with Mn = the events per node kept
+// with the data, table refresh, and for a network process the in-place adjacency sweep (seed, counter + 2^40) and the Beta draw of
+// rho (seed, counter).  Only scalars cross PCIe.
+extern "C" int nhp_disc_gibbs_sweep(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t counter, const double *hyper, int n_hyper, double net_alpha,
+                                    double net_beta) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    NHP_CHECK(ctx, dd != nullptr, NHP_ERR_INVALID, "nhp_disc_gibbs_sweep: data handle is NULL");
+    NHP_CHECK(ctx, dd->t_halo == 0, NHP_ERR_UNSUPPORTED, "nhp_disc_gibbs_sweep works on unsharded data");
+    NHP_CHECK(ctx, !(ctx->comm && ctx->nranks > 1), NHP_ERR_UNSUPPORTED, "nhp_disc_gibbs_sweep runs on one GPU (the context has a communicator of %d ranks)", ctx->nranks);
+    NHP_CHECK(ctx, ctx->disc_set, NHP_ERR_STATE, "nhp_disc_gibbs_sweep: discrete parameters not set (call nhp_disc_params_set)");
+    NHP_CHECK(ctx, dd->d_conv != nullptr, NHP_ERR_STATE, "nhp_disc_gibbs_sweep: call nhp_disc_convolve first");
+    NHP_CHECK(ctx, hyper != nullptr && n_hyper == 5, NHP_ERR_INVALID, "nhp_disc_gibbs_sweep: expected 5 hyper-parameters, got %d", n_hyper);
+    for (int i = 0; i < n_hyper; i++) NHP_CHECK(ctx, std::isfinite(hyper[i]), NHP_ERR_INVALID, "nhp_disc_gibbs_sweep: hyper-parameter %d is not finite", i);
+    const bool bern = ctx->d_has_A && net_alpha > 0.0;
+    NHP_CHECK(ctx, !bern || net_beta > 0.0, NHP_ERR_INVALID, "nhp_disc_gibbs_sweep: net_beta must be positive");
+    NHP_CHECK(ctx, !bern || ctx->dd_rho >= 0.0, NHP_ERR_STATE, "nhp_disc_gibbs_sweep: no link probability kept with the context (nhp_disc_network_set)");
+    NHP_TRY(nhp_disc_gibbs_counts(ctx, dd, seed, counter, nullptr, 0, nullptr));
+    NHP_TRY(nhp_disc_draw_params(ctx, dd, seed, counter, nhp_disc_rowsum(dd), hyper));
+    NHP_TRY(nhp_disc_tables_refresh(ctx));
+    if (ctx->d_has_A) {
+        NHP_TRY(nhp_disc_resample_adjacency_dev(ctx, dd, bern ? -1.0 : 1.0, seed, counter + (1ull << 40)));  // Bernoulli: the context's rho; else dense (1)
+        if (bern) NHP_TRY(nhp_disc_draw_network(ctx, seed, counter, net_alpha, net_beta));
+    }
+    if (ctx->dd_trace_cap > 0 && ctx->dd_trace_len < ctx->dd_trace_cap) NHP_TRY(nhp_disc_trace_push(ctx));  // the sample stays on the device
+    return NHP_OK;
+}
+
 extern "C" int nhp_cont_sweep_info(const nhp_ctx *ctx, double *out8) {
     if (!ctx || !out8) return NHP_ERR_INVALID;
     for (int i = 0; i < 8; i++) out8[i] = ctx->sweep_info[i];

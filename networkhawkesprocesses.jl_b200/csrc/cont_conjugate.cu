@@ -221,10 +221,10 @@ extern "C" int nhp_cont_params_get(nhp_ctx *ctx, double *lambda0, double *W, dou
 }
 
 // rho ~ Beta(alpha + sum(A), beta + K^2 - sum(A))  (networks.jl:72-78) as a ratio of two Gamma draws, on the device so that every
-// rank of a multi-GPU chain draws the same value from the same (seed, counter); out[0] = rho
-__global__ void k_network_draw(uint64_t seed, uint64_t counter, double a, double b, double *out) {
+// rank of a multi-GPU chain draws the same value from the same (seed, counter); out[0] = rho.  Stream ids: 3 continuous, 11 discrete.
+__global__ void k_network_draw(uint64_t seed, uint64_t counter, uint32_t param, double a, double b, double *out) {
     if (threadIdx.x != 0 || blockIdx.x != 0) return;
-    PhiloxStream r(seed, 0u, 3u, counter);
+    PhiloxStream r(seed, 0u, param, counter);
     const double x = r.gamma(a, 1.0), y = r.gamma(b, 1.0);
     out[0] = x / (x + y);
 }
@@ -237,7 +237,7 @@ extern "C" int nhp_cont_resample_network(nhp_ctx *ctx, uint64_t seed, uint64_t c
     double *scratch;
     NHP_TRY(nhp_partials(ctx, 8, &scratch));
     const double KK = (double)ctx->K * (double)ctx->K;
-    k_network_draw<<<1, 32, 0, ctx->stream>>>(seed, counter, alpha + ctx->a_sum, beta + KK - ctx->a_sum, scratch);
+    k_network_draw<<<1, 32, 0, ctx->stream>>>(seed, counter, 3u, alpha + ctx->a_sum, beta + KK - ctx->a_sum, scratch);
     NHP_LAUNCHED(ctx);
     double rho = 0.0;
     NHP_CUDA(ctx, cudaMemcpyAsync(&rho, scratch, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
@@ -333,6 +333,19 @@ __global__ void k_disc_conjugate(const DiscConjArgs a) {
     for (int b = 0; b < a.B; b++) a.theta[e + NN * b] /= tot;
 }
 
+// the draws in place on the context's parameters; d_Mn: events per node on the device.  The derived tables are not refreshed here.
+int nhp_disc_draw_params(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t counter, const double *d_Mn, const double *hyper) {
+    const int64_t N = ctx->dN, NN = N * N;
+    DiscConjArgs a;
+    a.N = (int)N; a.B = (int)ctx->dB; a.seed = seed; a.counter = counter; a.Tdt = (double)(dd->T - dd->t_halo) * ctx->ddt;
+    a.alpha0 = hyper[0]; a.beta0 = hyper[1]; a.kappa = hyper[2]; a.nu = hyper[3]; a.gamma = hyper[4];
+    a.counts = ctx->dd_counts; a.Mn = d_Mn; a.lambda0 = ctx->dd_lambda0; a.W = ctx->dd_W; a.theta = ctx->dd_theta;
+    k_disc_conjugate<<<(unsigned)((NN + 127) / 128), 128, 0, ctx->stream>>>(a);
+    NHP_LAUNCHED(ctx);
+    NHP_CUDA(ctx, cudaGetLastError());
+    return NHP_OK;
+}
+
 extern "C" int nhp_disc_resample_params(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t counter, const double *Mn, const double *hyper, int n_hyper,
                                         double *lambda0, double *W, double *theta) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
@@ -347,27 +360,30 @@ extern "C" int nhp_disc_resample_params(nhp_ctx *ctx, nhp_disc *dd, uint64_t see
     void *scratch = nullptr;
     NHP_TRY(nhp_scratch(ctx, (size_t)N * sizeof(double), &scratch));
     NHP_CUDA(ctx, cudaMemcpyAsync(scratch, Mn, (size_t)N * sizeof(double), cudaMemcpyHostToDevice, s));
-    DiscConjArgs a;
-    a.N = (int)N; a.B = (int)B; a.seed = seed; a.counter = counter; a.Tdt = (double)(dd->T - dd->t_halo) * ctx->ddt;
-    a.alpha0 = hyper[0]; a.beta0 = hyper[1]; a.kappa = hyper[2]; a.nu = hyper[3]; a.gamma = hyper[4];
-    a.counts = ctx->dd_counts; a.Mn = (const double *)scratch; a.lambda0 = ctx->dd_lambda0; a.W = ctx->dd_W; a.theta = ctx->dd_theta;
     NHP_TRY(nhp_timer_begin(ctx));
-    k_disc_conjugate<<<(unsigned)((NN + 127) / 128), 128, 0, s>>>(a);
-    NHP_LAUNCHED(ctx);
-    NHP_CUDA(ctx, cudaGetLastError());
+    NHP_TRY(nhp_disc_draw_params(ctx, dd, seed, counter, (const double *)scratch, hyper));
     NHP_TRY(nhp_timer_end(ctx));
-    // the new parameters go to the host (they are the sample), and the derived tables (bump, sparse parent lists) follow them
+    // the derived tables (bump, sparse parent lists) follow the new parameters on the device; the parameters go to the host (they are the sample)
+    const double ms = ctx->last_ms;
+    NHP_TRY(nhp_disc_tables_refresh(ctx));
+    ctx->last_ms = ms;
     NHP_CUDA(ctx, cudaMemcpyAsync(lambda0, ctx->dd_lambda0, (size_t)N * sizeof(double), cudaMemcpyDeviceToHost, s));
     NHP_CUDA(ctx, cudaMemcpyAsync(W, ctx->dd_W, (size_t)NN * sizeof(double), cudaMemcpyDeviceToHost, s));
     NHP_CUDA(ctx, cudaMemcpyAsync(theta, ctx->dd_theta, (size_t)(NN * B) * sizeof(double), cudaMemcpyDeviceToHost, s));
-    std::vector<double> A;
-    if (ctx->d_has_A) {
-        A.resize((size_t)NN);
-        NHP_CUDA(ctx, cudaMemcpyAsync(A.data(), ctx->dd_A, (size_t)NN * sizeof(double), cudaMemcpyDeviceToHost, s));
-    }
     NHP_CUDA(ctx, cudaStreamSynchronize(s));
-    const double ms = ctx->last_ms;
-    const int rc = nhp_disc_params_set(ctx, N, B, lambda0, W, ctx->d_has_A ? A.data() : nullptr, theta, ctx->ddt);
-    ctx->last_ms = ms;
-    return rc;
+    return NHP_OK;
+}
+
+// rho of the discrete Bernoulli network from the sum of A left by the last table refresh; the value stays with the context
+int nhp_disc_draw_network(nhp_ctx *ctx, uint64_t seed, uint64_t counter, double alpha, double beta) {
+    double *scratch;
+    NHP_TRY(nhp_partials(ctx, 8, &scratch));
+    const double NN = (double)ctx->dN * (double)ctx->dN;
+    k_network_draw<<<1, 32, 0, ctx->stream>>>(seed, counter, 11u, alpha + ctx->dd_a_sum, beta + NN - ctx->dd_a_sum, scratch);
+    NHP_LAUNCHED(ctx);
+    double rho = 0.0;
+    NHP_CUDA(ctx, cudaMemcpyAsync(&rho, scratch, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->dd_rho = rho;
+    return NHP_OK;
 }

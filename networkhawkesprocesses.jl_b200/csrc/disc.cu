@@ -21,6 +21,7 @@ struct DiscExtra {  // hangs off nhp_disc (kept here so the public struct stays 
     double *rowsum = nullptr;   // [N] sum_t data[p,t] over own bins
     double *phi = nullptr;      // [L*B]
     double *csum = nullptr;     // [N*B] sum over own bins of convT[:, k]
+    int max_ne = 0;             // most non-zero bins of one child (grid of the streaming adjacency sweep)
 };
 static DiscExtra *extra_of(nhp_disc *dd) { return reinterpret_cast<DiscExtra *>(dd->d_scan); }
 
@@ -179,6 +180,12 @@ extern "C" int nhp_disc_upload(nhp_ctx *ctx, const int64_t *data, int64_t N, int
     k_prefix_small<<<1, 32, 0, s>>>(ex->child_ptr, (int)N);
     NHP_LAUNCHED(ctx);
     UP_CUDA(cudaGetLastError());
+    {  // the longest column depends on the data only: kept here so that no adjacency sweep synchronises to find it
+        std::vector<int> cp((size_t)N + 1);
+        UP_CUDA(cudaMemcpyAsync(cp.data(), ex->child_ptr, (size_t)(N + 1) * sizeof(int), cudaMemcpyDeviceToHost, s));
+        UP_CUDA(cudaStreamSynchronize(s));
+        for (int64_t c = 0; c < N; c++) ex->max_ne = std::max(ex->max_ne, cp[c + 1] - cp[c]);
+    }
 #undef UP_CUDA
     int rc = fin(NHP_OK);
     if (rc == NHP_OK) *out = dd;
@@ -496,6 +503,124 @@ __global__ void k_compact_bump(int NB, const double *__restrict__ bumpT, const i
     for (int i = kptr[c] + threadIdx.x; i < kptr[c + 1]; i += blockDim.x) btc[i] = bumpT[(int64_t)c * NB + klist[i]];
 }
 
+// Compact per-child lists of the structurally non-zero (parent, basis) entries, k = p*B + b with [A]W[p,c] != 0, built on the
+// device from the resident parameters: a count per child, one scan over the children, then every child writes its list in
+// ascending k.  Only sparse effective weights (<= 50 % non-zero) get lists; dense models keep the full parent scan.
+__global__ void __launch_bounds__(256) k_disc_klist_count(int N, const double *__restrict__ W, const double *__restrict__ A, int *__restrict__ kcnt,
+                                                          double *__restrict__ acol) {
+    __shared__ int s_n[8];
+    __shared__ double s_a[8];
+    const int c = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int n = 0;
+    double a = 0.0;
+    for (int p = threadIdx.x; p < N; p += 256) {
+        const int64_t e = p + (int64_t)N * c;
+        const double av = A ? A[e] : 1.0;
+        n += (A ? av * W[e] : W[e]) != 0.0;
+        a += av;
+    }
+    n = __reduce_add_sync(0xffffffffu, n);
+    a = warp_sum_d(a);
+    if (lane == 0) { s_n[warp] = n; s_a[warp] = a; }
+    __syncthreads();
+    if (threadIdx.x == 0) {  // fixed order: the same sum of A on every call
+        int tn = 0;
+        double ta = 0.0;
+        for (int w = 0; w < 8; w++) { tn += s_n[w]; ta += s_a[w]; }
+        kcnt[c] = tn;
+        acol[c] = ta;
+    }
+}
+// kptr[c] = B * (non-zero entries of the children before c); out = [list length, longest list, non-zero entries, sum of A]
+__global__ void __launch_bounds__(1024) k_disc_klist_scan(int N, int B, const int *__restrict__ kcnt, const double *__restrict__ acol, int *__restrict__ kptr,
+                                                          double *__restrict__ out) {
+    typedef cub::BlockScan<int, 1024> Scan;
+    typedef cub::BlockReduce<double, 1024> Red;
+    __shared__ union { typename Scan::TempStorage scan; typename Red::TempStorage red; } tmp;
+    __shared__ int s_max;
+    if (threadIdx.x == 0) s_max = 0;
+    __syncthreads();
+    int carry = 0;
+    double asum = 0.0;  // thread 0
+    for (int c0 = 0; c0 < N; c0 += 1024) {
+        const int c = c0 + threadIdx.x;
+        const int v = c < N ? kcnt[c] : 0;
+        int excl, tot;
+        Scan(tmp.scan).ExclusiveSum(v, excl, tot);
+        if (c < N) kptr[c] = (carry + excl) * B;
+        carry += tot;
+        if (v) atomicMax(&s_max, v);
+        __syncthreads();
+        const double a = Red(tmp.red).Sum(c < N ? acol[c] : 0.0);
+        if (threadIdx.x == 0) asum += a;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        kptr[N] = carry * B;
+        out[0] = (double)carry * B; out[1] = (double)s_max * B; out[2] = (double)carry; out[3] = asum;
+    }
+}
+__global__ void __launch_bounds__(256) k_disc_klist_fill(int N, int B, const double *__restrict__ W, const double *__restrict__ A, const int *__restrict__ kptr,
+                                                         int *__restrict__ klist) {
+    typedef cub::BlockScan<int, 256> Scan;
+    __shared__ typename Scan::TempStorage tmp;
+    const int c = blockIdx.x;
+    int next = kptr[c];
+    for (int p0 = 0; p0 < N; p0 += 256) {
+        const int p = p0 + threadIdx.x;
+        int f = 0;
+        if (p < N) {
+            const int64_t e = p + (int64_t)N * c;
+            f = (A ? A[e] * W[e] : W[e]) != 0.0;
+        }
+        int r, tot;
+        Scan(tmp).ExclusiveSum(f, r, tot);
+        if (f) for (int b = 0; b < B; b++) klist[next + r * B + b] = p * B + b;
+        next += tot * B;
+        __syncthreads();
+    }
+}
+
+// Everything that follows from the context's lambda0, W, A, theta: the bump table (both layouts), the compact parent lists, the
+// density of the effective weights and the sum of A.  One synchronisation: four scalars come back to the host.
+int nhp_disc_tables_refresh(nhp_ctx *ctx) {
+    cudaStream_t s = ctx->stream;
+    const int64_t N = ctx->dN, B = ctx->dB, NN = N * N, NB = N * B;
+    const double *A = ctx->d_has_A ? ctx->dd_A : nullptr;
+    k_bump<<<(unsigned)((NB * N + 255) / 256), 256, 0, s>>>((int)N, (int)B, ctx->dd_W, A, ctx->dd_theta, ctx->ddt, ctx->dd_bump, ctx->dd_bump + NB * N);
+    NHP_LAUNCHED(ctx);
+    k_disc_klist_count<<<(unsigned)N, 256, 0, s>>>((int)N, ctx->dd_W, A, ctx->dd_kcnt, ctx->dd_ksum + 4);
+    NHP_LAUNCHED(ctx);
+    k_disc_klist_scan<<<1, 1024, 0, s>>>((int)N, (int)B, ctx->dd_kcnt, ctx->dd_ksum + 4, ctx->dd_kptr, ctx->dd_ksum);
+    NHP_LAUNCHED(ctx);
+    DCUDA(ctx, cudaGetLastError());
+    double h[4];
+    DCUDA(ctx, cudaMemcpyAsync(h, ctx->dd_ksum, sizeof(h), cudaMemcpyDeviceToHost, s));
+    DCUDA(ctx, cudaStreamSynchronize(s));
+    ctx->dd_density = h[2] / (double)NN;
+    ctx->dd_a_sum = A ? h[3] : (double)NN;
+    ctx->dd_lists = false;
+    ctx->dd_maxNA = 0;
+    if (h[2] > 0.0 && ctx->dd_density <= 0.5) {
+        const size_t need = (size_t)h[0];
+        if (need > ctx->dd_klist_cap) {
+            cudaFree(ctx->dd_klist); cudaFree(ctx->dd_btc);
+            ctx->dd_klist = nullptr; ctx->dd_btc = nullptr; ctx->dd_klist_cap = 0;
+            DCUDA(ctx, cudaMalloc(&ctx->dd_klist, need * sizeof(int)));
+            DCUDA(ctx, cudaMalloc(&ctx->dd_btc, need * sizeof(double)));
+            ctx->dd_klist_cap = need;
+        }
+        k_disc_klist_fill<<<(unsigned)N, 256, 0, s>>>((int)N, (int)B, ctx->dd_W, A, ctx->dd_kptr, ctx->dd_klist);
+        NHP_LAUNCHED(ctx);
+        k_compact_bump<<<(unsigned)N, 256, 0, s>>>((int)NB, ctx->dd_bump + NB * N, ctx->dd_klist, ctx->dd_kptr, ctx->dd_btc);
+        NHP_LAUNCHED(ctx);
+        DCUDA(ctx, cudaGetLastError());
+        ctx->dd_maxNA = (int64_t)h[1];
+        ctx->dd_lists = true;
+    }
+    return NHP_OK;
+}
+
 extern "C" int nhp_disc_params_set(nhp_ctx *ctx, int64_t N, int64_t B, const double *lambda0, const double *W, const double *A, const double *theta, double dt) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
     NHP_CHECK(ctx, N >= 1 && B >= 1 && lambda0 && W && theta && dt > 0.0, NHP_ERR_INVALID, "nhp_disc_params_set: bad argument");
@@ -506,12 +631,19 @@ extern "C" int nhp_disc_params_set(nhp_ctx *ctx, int64_t N, int64_t B, const dou
     if (ctx->dN != N || ctx->dB != B) {
         DCUDA(ctx, cudaStreamSynchronize(s));
         cudaFree(ctx->dd_lambda0); cudaFree(ctx->dd_W); cudaFree(ctx->dd_A); cudaFree(ctx->dd_theta); cudaFree(ctx->dd_bump);
-        ctx->dd_lambda0 = ctx->dd_W = ctx->dd_A = ctx->dd_theta = ctx->dd_bump = nullptr;
+        cudaFree(ctx->dd_klist); cudaFree(ctx->dd_kptr); cudaFree(ctx->dd_btc); cudaFree(ctx->dd_kcnt); cudaFree(ctx->dd_ksum);
+        ctx->dd_lambda0 = ctx->dd_W = ctx->dd_A = ctx->dd_theta = ctx->dd_bump = ctx->dd_btc = ctx->dd_ksum = nullptr;
+        ctx->dd_klist = ctx->dd_kptr = ctx->dd_kcnt = nullptr;
+        ctx->dd_klist_cap = 0; ctx->dd_lists = false;
+        ctx->dN = ctx->dB = 0;
         DCUDA(ctx, cudaMalloc(&ctx->dd_lambda0, (size_t)N * sizeof(double)));
         DCUDA(ctx, cudaMalloc(&ctx->dd_W, (size_t)NN * sizeof(double)));
         DCUDA(ctx, cudaMalloc(&ctx->dd_A, (size_t)NN * sizeof(double)));
         DCUDA(ctx, cudaMalloc(&ctx->dd_theta, (size_t)(NN * B) * sizeof(double)));
         DCUDA(ctx, cudaMalloc(&ctx->dd_bump, (size_t)(2 * NB * N) * sizeof(double)));
+        DCUDA(ctx, cudaMalloc(&ctx->dd_kptr, (size_t)(N + 1) * sizeof(int)));
+        DCUDA(ctx, cudaMalloc(&ctx->dd_kcnt, (size_t)N * sizeof(int)));
+        DCUDA(ctx, cudaMalloc(&ctx->dd_ksum, (size_t)(4 + N) * sizeof(double)));
         ctx->dN = N; ctx->dB = B;
     }
     ctx->disc_set = false;
@@ -520,47 +652,41 @@ extern "C" int nhp_disc_params_set(nhp_ctx *ctx, int64_t N, int64_t B, const dou
     DCUDA(ctx, cudaMemcpyAsync(ctx->dd_W, W, (size_t)NN * sizeof(double), cudaMemcpyHostToDevice, s));
     if (A) DCUDA(ctx, cudaMemcpyAsync(ctx->dd_A, A, (size_t)NN * sizeof(double), cudaMemcpyHostToDevice, s));
     DCUDA(ctx, cudaMemcpyAsync(ctx->dd_theta, theta, (size_t)(NN * B) * sizeof(double), cudaMemcpyHostToDevice, s));
-    k_bump<<<(unsigned)((NB * N + 255) / 256), 256, 0, s>>>((int)N, (int)B, ctx->dd_W, A ? ctx->dd_A : nullptr, ctx->dd_theta, dt, ctx->dd_bump, ctx->dd_bump + NB * N);
-    NHP_LAUNCHED(ctx);
-    // compact per-child lists of the structurally non-zero (parent, basis) entries: k = p*B + b with [A]W[p,c] != 0.
-    // Built only for sparse effective weights (<= 50 % non-zero); dense models keep the full parent scan.
-    {
-        int64_t nnzw = 0;
-        for (int64_t e = 0; e < NN; e++) nnzw += ((A ? A[e] * W[e] : W[e]) != 0.0);
-        ctx->dd_density = (double)nnzw / (double)NN;
-        ctx->dd_maxNA = 0;
-        cudaFree(ctx->dd_klist); cudaFree(ctx->dd_kptr); cudaFree(ctx->dd_btc);
-        ctx->dd_klist = ctx->dd_kptr = nullptr; ctx->dd_btc = nullptr;
-        if (nnzw > 0 && ctx->dd_density <= 0.5) {
-            std::vector<int> kptr(N + 1, 0), klist;
-            klist.reserve((size_t)(nnzw * B));
-            int64_t maxNA = 0;
-            for (int64_t c = 0; c < N; c++) {
-                kptr[c] = (int)klist.size();
-                for (int64_t pp = 0; pp < N; pp++) {
-                    const double w = A ? A[pp + N * c] * W[pp + N * c] : W[pp + N * c];
-                    if (w != 0.0) for (int64_t b = 0; b < B; b++) klist.push_back((int)(pp * B + b));
-                }
-                maxNA = std::max<int64_t>(maxNA, (int64_t)klist.size() - kptr[c]);
-            }
-            kptr[N] = (int)klist.size();
-            ctx->dd_maxNA = maxNA;
-            DCUDA(ctx, cudaMalloc(&ctx->dd_klist, klist.size() * sizeof(int)));
-            DCUDA(ctx, cudaMalloc(&ctx->dd_kptr, (size_t)(N + 1) * sizeof(int)));
-            DCUDA(ctx, cudaMalloc(&ctx->dd_btc, klist.size() * sizeof(double)));
-            DCUDA(ctx, cudaMemcpyAsync(ctx->dd_kptr, kptr.data(), (size_t)(N + 1) * sizeof(int), cudaMemcpyHostToDevice, s));
-            DCUDA(ctx, cudaMemcpyAsync(ctx->dd_klist, klist.data(), klist.size() * sizeof(int), cudaMemcpyHostToDevice, s));
-            k_compact_bump<<<(unsigned)N, 256, 0, s>>>((int)NB, ctx->dd_bump + NB * N, ctx->dd_klist, ctx->dd_kptr, ctx->dd_btc);
-            NHP_LAUNCHED(ctx);
-            DCUDA(ctx, cudaGetLastError());
-            DCUDA(ctx, cudaStreamSynchronize(s));  // kptr / klist are stack-owned host vectors
-        }
-    }
-    DCUDA(ctx, cudaGetLastError());
-    DCUDA(ctx, cudaStreamSynchronize(s));
+    NHP_TRY(nhp_disc_tables_refresh(ctx));
     ctx->disc_set = true;
     return NHP_OK;
 }
+
+// Current parameters in the layouts of nhp_disc_params_set; any pointer may be NULL
+extern "C" int nhp_disc_params_get(nhp_ctx *ctx, double *lambda0, double *W, double *A, double *theta) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    NHP_CHECK(ctx, ctx->disc_set, NHP_ERR_STATE, "nhp_disc_params_get: discrete parameters not set");
+    NHP_CHECK(ctx, !A || ctx->d_has_A, NHP_ERR_STATE, "nhp_disc_params_get: the process has no adjacency matrix");
+    DCUDA(ctx, cudaSetDevice(ctx->device));
+    const int64_t N = ctx->dN, NN = N * N;
+    cudaStream_t s = ctx->stream;
+    if (lambda0) DCUDA(ctx, cudaMemcpyAsync(lambda0, ctx->dd_lambda0, (size_t)N * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (W) DCUDA(ctx, cudaMemcpyAsync(W, ctx->dd_W, (size_t)NN * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (A) DCUDA(ctx, cudaMemcpyAsync(A, ctx->dd_A, (size_t)NN * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (theta) DCUDA(ctx, cudaMemcpyAsync(theta, ctx->dd_theta, (size_t)(NN * ctx->dB) * sizeof(double), cudaMemcpyDeviceToHost, s));
+    DCUDA(ctx, cudaStreamSynchronize(s));
+    return NHP_OK;
+}
+
+// link probability of the discrete BernoulliNetworkModel (networks.jl:45-54), kept apart from the continuous model's
+extern "C" int nhp_disc_network_set(nhp_ctx *ctx, double rho) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    NHP_CHECK(ctx, rho >= 0.0 && rho <= 1.0, NHP_ERR_INVALID, "BernoulliNetworkModel: link probability must be in [0, 1]");
+    ctx->dd_rho = rho;
+    return NHP_OK;
+}
+extern "C" int nhp_disc_network_get(const nhp_ctx *ctx, double *rho) {
+    if (!ctx || !rho) return NHP_ERR_INVALID;
+    *rho = ctx->dd_rho;
+    return NHP_OK;
+}
+
+const double *nhp_disc_rowsum(nhp_disc *dd) { return extra_of(dd)->rowsum; }
 
 static int disc_ready(nhp_ctx *ctx, nhp_disc *dd, const char *who) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
@@ -1035,7 +1161,7 @@ extern "C" int nhp_disc_gibbs_counts(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, 
     if (ex->nnz > 0) {
         int slabs = pick_slabs(ctx, N, ex->nnz);
         const char *envs = getenv("NHP_DISC_SPARSE");
-        const bool sparse = ctx->dd_klist && ctx->dd_density <= 0.5 && !(envs && atoi(envs) == 0);
+        const bool sparse = ctx->dd_lists && ctx->dd_density <= 0.5 && !(envs && atoi(envs) == 0);
         const int64_t wid = sparse ? ctx->dd_maxNA : NB;
         const size_t wsmem = (size_t)8 * 32 * (((wid + 31) / 32) | 1) * sizeof(double);
         const char *envw = getenv("NHP_DISC_WARP");
@@ -1247,8 +1373,8 @@ extern "C" int nhp_disc_loglik_grad(nhp_ctx *ctx, nhp_disc *dd, double *ll, doub
 // ---------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_disc_adjacency(const double *__restrict__ convT, const double *__restrict__ csum, const double *__restrict__ lambda0,
                                                         const double *__restrict__ W, const double *__restrict__ theta, double dt, double *__restrict__ A,
-                                                        const double *__restrict__ rho, const double *__restrict__ u, uint64_t seed, uint64_t counter, int N, int B,
-                                                        const int *__restrict__ nz_t, const int *__restrict__ nz_s, const int *__restrict__ child_ptr,
+                                                        const double *__restrict__ rho, double rho_s, const double *__restrict__ u, uint64_t seed, uint64_t counter,
+                                                        int N, int B, const int *__restrict__ nz_t, const int *__restrict__ nz_s, const int *__restrict__ child_ptr,
                                                         double *__restrict__ lam_scratch, int *__restrict__ flag) {
     __shared__ double red[8];
     __shared__ double s_anew;
@@ -1286,7 +1412,7 @@ __global__ void __launch_bounds__(256) k_disc_adjacency(const double *__restrict
         }
         double sum = block_sum_256(part, red);
         if (threadIdx.x == 0) {
-            double r = rho[kk];
+            double r = rho ? rho[kk] : rho_s;
             double delta = sum - gsum + (log(r) - log(1.0 - r));
             double p1 = delta >= 0.0 ? 1.0 / (1.0 + exp(-delta)) : exp(delta) / (1.0 + exp(delta));
             if (delta != delta) { atomicOr(flag, 64); p1 = 0.0; }
@@ -1361,8 +1487,8 @@ __global__ void __launch_bounds__(256) k_disc_adj_gather(const double *__restric
 }
 
 __global__ void __launch_bounds__(1024) k_disc_adj_steps(const double *__restrict__ csum, const double *__restrict__ W, const double *__restrict__ theta, double dt,
-                                                         double *__restrict__ A, const double *__restrict__ rho, const double *__restrict__ u, uint64_t seed,
-                                                         uint64_t counter, int N, int B, const int *__restrict__ nz_s, const int *__restrict__ child_ptr,
+                                                         double *__restrict__ A, const double *__restrict__ rho, double rho_s, const double *__restrict__ u,
+                                                         uint64_t seed, uint64_t counter, int N, int B, const int *__restrict__ nz_s, const int *__restrict__ child_ptr,
                                                          double *__restrict__ lam_scratch, const double *__restrict__ g_scratch, int *__restrict__ flag) {
     __shared__ double red[32];
     __shared__ double s_anew;
@@ -1391,7 +1517,7 @@ __global__ void __launch_bounds__(1024) k_disc_adj_steps(const double *__restric
         if (threadIdx.x == 0) {
             double sum = 0.0;
             for (int wv = 0; wv < (int)(blockDim.x >> 5); wv++) sum += red[wv];
-            const double r = rho[kk];
+            const double r = rho ? rho[kk] : rho_s;
             const double delta = sum - gsum + (log(r) - log(1.0 - r));
             double p1 = delta >= 0.0 ? 1.0 / (1.0 + exp(-delta)) : exp(delta) / (1.0 + exp(delta));
             if (delta != delta) { atomicOr(flag, 64); p1 = 0.0; }
@@ -1409,46 +1535,39 @@ __global__ void __launch_bounds__(1024) k_disc_adj_steps(const double *__restric
     }
 }
 
-extern "C" int nhp_disc_resample_adjacency(nhp_ctx *ctx, nhp_disc *dd, const double *rho, uint64_t seed, uint64_t counter, const double *u, double *A_inout) {
-    NHP_TRY(disc_ready(ctx, dd, "nhp_disc_resample_adjacency"));
-    NHP_CHECK(ctx, rho && A_inout, NHP_ERR_INVALID, "nhp_disc_resample_adjacency: NULL rho/A");
-    NHP_CHECK(ctx, dd->t_halo == 0, NHP_ERR_UNSUPPORTED, "nhp_disc_resample_adjacency works on unsharded data");
-    DiscExtra *ex = extra_of(dd);
-    const int64_t N = dd->N, B = dd->B, NN = N * N;
-    cudaStream_t s = ctx->stream;
-    void *scratch;
-    const int64_t nnz1 = std::max<int64_t>(ex->nnz, 1);
-    size_t tot = (size_t)(3 * NN + nnz1) * sizeof(double);
-    // streaming variant: + G[p][e] for every (parent, non-zero bin)
+// The sweep over every column of the device matrix A (in place).  rho: per-entry link probabilities [N*N], or NULL for the scalar
+// rho_s; u: uniforms [N*N] or NULL for Philox (seed, p + N c, counter).  The streaming form needs G[p][e] for every (parent, non-zero
+// bin) next to the bins' intensities in the work buffer: adj_work_doubles tells the caller how much to reserve.
+static bool adj_streaming(nhp_ctx *ctx, const nhp_disc *dd, size_t *work_doubles) {
+    const int64_t N = dd->N, B = dd->B, nnz1 = std::max<int64_t>(extra_of(const_cast<nhp_disc *>(dd))->nnz, 1);
     const size_t g_bytes = (size_t)nnz1 * (size_t)N * sizeof(double), coef_smem = (size_t)(N * B + N * (ADJ_TE + 1)) * sizeof(double);
     size_t free_b = 0, total_b = 0;
     cudaMemGetInfo(&free_b, &total_b);
     const char *envt = getenv("NHP_DISC_ADJ_STREAM");
     const bool stream_variant = !(envt && atoi(envt) == 0) && coef_smem <= (size_t)ctx->smem_optin - 4096 && g_bytes <= free_b / 2 + ctx->scratch_cap;
-    if (stream_variant) tot += g_bytes;
-    NHP_TRY(nhp_scratch(ctx, tot, &scratch));
-    double *d_A = (double *)scratch, *d_rho = d_A + NN, *d_u = d_rho + NN, *d_lam = d_u + NN, *d_G = d_lam + nnz1;
-    DCUDA(ctx, cudaMemcpyAsync(d_A, A_inout, (size_t)NN * sizeof(double), cudaMemcpyHostToDevice, s));
-    DCUDA(ctx, cudaMemcpyAsync(d_rho, rho, (size_t)NN * sizeof(double), cudaMemcpyHostToDevice, s));
-    if (u) DCUDA(ctx, cudaMemcpyAsync(d_u, u, (size_t)NN * sizeof(double), cudaMemcpyHostToDevice, s));
+    *work_doubles = (size_t)nnz1 + (stream_variant ? (size_t)nnz1 * (size_t)N : 0);
+    return stream_variant;
+}
+static int adj_sweep(nhp_ctx *ctx, nhp_disc *dd, bool stream_variant, double *d_A, const double *d_rho, double rho_s, const double *d_u, uint64_t seed,
+                     uint64_t counter, double *work) {
+    DiscExtra *ex = extra_of(dd);
+    const int64_t N = dd->N, B = dd->B, nnz1 = std::max<int64_t>(ex->nnz, 1);
+    cudaStream_t s = ctx->stream;
+    double *d_lam = work, *d_G = work + nnz1;
     DCUDA(ctx, cudaMemsetAsync(ctx->d_flag, 0, sizeof(int), s));
     NHP_TRY(nhp_timer_begin(ctx));
     if (stream_variant) {
-        std::vector<int> cp(N + 1);
-        DCUDA(ctx, cudaMemcpyAsync(cp.data(), ex->child_ptr, (size_t)(N + 1) * sizeof(int), cudaMemcpyDeviceToHost, s));
-        DCUDA(ctx, cudaStreamSynchronize(s));
-        int max_ne = 0;
-        for (int64_t c = 0; c < N; c++) max_ne = std::max(max_ne, cp[c + 1] - cp[c]);
-        if (max_ne > 0) {
+        if (ex->max_ne > 0) {
+            const size_t coef_smem = (size_t)(N * B + N * (ADJ_TE + 1)) * sizeof(double);
             DCUDA(ctx, cudaFuncSetAttribute(k_disc_adj_gather, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coef_smem));
-            dim3 gg((unsigned)N, (unsigned)((max_ne + ADJ_TE - 1) / ADJ_TE));
+            dim3 gg((unsigned)N, (unsigned)((ex->max_ne + ADJ_TE - 1) / ADJ_TE));
             k_disc_adj_gather<<<gg, 256, coef_smem, s>>>(dd->d_conv, ctx->dd_lambda0, ctx->dd_W, ctx->dd_theta, ctx->ddt, d_A, (int)N, (int)B, ex->nz_t, ex->child_ptr, d_lam, d_G);
             NHP_LAUNCHED(ctx);
         }
-        k_disc_adj_steps<<<(unsigned)N, 1024, 0, s>>>(ex->csum, ctx->dd_W, ctx->dd_theta, ctx->ddt, d_A, d_rho, u ? d_u : nullptr, seed, counter, (int)N, (int)B, ex->nz_s,
+        k_disc_adj_steps<<<(unsigned)N, 1024, 0, s>>>(ex->csum, ctx->dd_W, ctx->dd_theta, ctx->ddt, d_A, d_rho, rho_s, d_u, seed, counter, (int)N, (int)B, ex->nz_s,
                                                        ex->child_ptr, d_lam, d_G, ctx->d_flag);
     } else
-    k_disc_adjacency<<<(unsigned)N, 256, 0, s>>>(dd->d_conv, ex->csum, ctx->dd_lambda0, ctx->dd_W, ctx->dd_theta, ctx->ddt, d_A, d_rho, u ? d_u : nullptr, seed, counter,
+    k_disc_adjacency<<<(unsigned)N, 256, 0, s>>>(dd->d_conv, ex->csum, ctx->dd_lambda0, ctx->dd_W, ctx->dd_theta, ctx->ddt, d_A, d_rho, rho_s, d_u, seed, counter,
                                                  (int)N, (int)B, ex->nz_t, ex->nz_s, ex->child_ptr, d_lam, ctx->d_flag);
     NHP_LAUNCHED(ctx);
     DCUDA(ctx, cudaGetLastError());
@@ -1456,19 +1575,51 @@ extern "C" int nhp_disc_resample_adjacency(nhp_ctx *ctx, nhp_disc *dd, const dou
     DCUDA(ctx, cudaMemcpyAsync(&flag, ctx->d_flag, sizeof(int), cudaMemcpyDeviceToHost, s));
     NHP_TRY(nhp_timer_end(ctx));
     NHP_CHECK(ctx, !(flag & 64), NHP_ERR_NUMERIC, "discrete adjacency sampler: NaN log-likelihood difference");
-    DCUDA(ctx, cudaMemcpyAsync(A_inout, d_A, (size_t)NN * sizeof(double), cudaMemcpyDeviceToHost, s));
-    DCUDA(ctx, cudaStreamSynchronize(s));
-    // the new adjacency becomes the context's A
-    if (ctx->d_has_A) {
-        DCUDA(ctx, cudaMemcpyAsync(ctx->dd_A, A_inout, (size_t)NN * sizeof(double), cudaMemcpyHostToDevice, s));
-        int64_t NB = N * B;
-        k_bump<<<(unsigned)((NB * N + 255) / 256), 256, 0, s>>>((int)N, (int)B, ctx->dd_W, ctx->dd_A, ctx->dd_theta, ctx->ddt, ctx->dd_bump, ctx->dd_bump + NB * N);
-        NHP_LAUNCHED(ctx);
-        DCUDA(ctx, cudaStreamSynchronize(s));
-        // the compact non-zero parent lists describe the old adjacency: drop them (dense parent scan until the next nhp_disc_params_set)
-        cudaFree(ctx->dd_klist); cudaFree(ctx->dd_kptr); cudaFree(ctx->dd_btc);
-        ctx->dd_klist = ctx->dd_kptr = nullptr; ctx->dd_btc = nullptr;
-        ctx->dd_maxNA = 0;
-    }
     return NHP_OK;
+}
+
+extern "C" int nhp_disc_resample_adjacency(nhp_ctx *ctx, nhp_disc *dd, const double *rho, uint64_t seed, uint64_t counter, const double *u, double *A_inout) {
+    NHP_TRY(disc_ready(ctx, dd, "nhp_disc_resample_adjacency"));
+    NHP_CHECK(ctx, rho && A_inout, NHP_ERR_INVALID, "nhp_disc_resample_adjacency: NULL rho/A");
+    NHP_CHECK(ctx, dd->t_halo == 0, NHP_ERR_UNSUPPORTED, "nhp_disc_resample_adjacency works on unsharded data");
+    const int64_t NN = dd->N * dd->N;
+    cudaStream_t s = ctx->stream;
+    size_t work = 0;
+    const bool stream_variant = adj_streaming(ctx, dd, &work);
+    void *scratch;
+    NHP_TRY(nhp_scratch(ctx, (size_t)(3 * NN) * sizeof(double) + work * sizeof(double), &scratch));
+    double *d_A = (double *)scratch, *d_rho = d_A + NN, *d_u = d_rho + NN, *d_work = d_u + NN;
+    DCUDA(ctx, cudaMemcpyAsync(d_A, A_inout, (size_t)NN * sizeof(double), cudaMemcpyHostToDevice, s));
+    DCUDA(ctx, cudaMemcpyAsync(d_rho, rho, (size_t)NN * sizeof(double), cudaMemcpyHostToDevice, s));
+    if (u) DCUDA(ctx, cudaMemcpyAsync(d_u, u, (size_t)NN * sizeof(double), cudaMemcpyHostToDevice, s));
+    NHP_TRY(adj_sweep(ctx, dd, stream_variant, d_A, d_rho, 0.0, u ? d_u : nullptr, seed, counter, d_work));
+    DCUDA(ctx, cudaMemcpyAsync(A_inout, d_A, (size_t)NN * sizeof(double), cudaMemcpyDeviceToHost, s));
+    // the new adjacency becomes the context's A, and the derived tables (bump, compact parent lists) follow it
+    if (ctx->d_has_A) {
+        DCUDA(ctx, cudaMemcpyAsync(ctx->dd_A, d_A, (size_t)NN * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        NHP_TRY(nhp_disc_tables_refresh(ctx));
+    }
+    DCUDA(ctx, cudaStreamSynchronize(s));
+    return NHP_OK;
+}
+
+// resample_adjacency_matrix! (discrete.jl:426-460) in place on the context's adjacency matrix, with a scalar link probability
+extern "C" int nhp_disc_resample_adjacency_dev(nhp_ctx *ctx, nhp_disc *dd, double rho, uint64_t seed, uint64_t counter) {
+    NHP_TRY(disc_ready(ctx, dd, "nhp_disc_resample_adjacency_dev"));
+    NHP_CHECK(ctx, dd->t_halo == 0, NHP_ERR_UNSUPPORTED, "nhp_disc_resample_adjacency_dev works on unsharded data");
+    NHP_CHECK(ctx, ctx->d_has_A, NHP_ERR_STATE, "nhp_disc_resample_adjacency_dev: the process has no adjacency matrix");
+    if (rho < 0.0) {
+        NHP_CHECK(ctx, ctx->dd_rho >= 0.0, NHP_ERR_STATE, "nhp_disc_resample_adjacency_dev: no link probability kept with the context (nhp_disc_network_set)");
+        rho = ctx->dd_rho;
+    }
+    NHP_CHECK(ctx, rho <= 1.0, NHP_ERR_INVALID, "BernoulliNetworkModel: link probability must be in [0, 1]");
+    size_t work = 0;
+    const bool stream_variant = adj_streaming(ctx, dd, &work);
+    void *scratch;
+    NHP_TRY(nhp_scratch(ctx, work * sizeof(double), &scratch));
+    const int rc = adj_sweep(ctx, dd, stream_variant, ctx->dd_A, nullptr, rho, nullptr, seed, counter, (double *)scratch);
+    const double ms = ctx->last_ms;
+    NHP_TRY(nhp_disc_tables_refresh(ctx));  // also after a refused decision: the tables follow whatever A now holds
+    ctx->last_ms = ms;
+    return rc;
 }

@@ -79,11 +79,12 @@ extern "C" int nhp_destroy(nhp_ctx *ctx) {
     cudaStreamSynchronize(ctx->stream);
     nhp_comm_destroy(ctx);
     nhp_cont_trace_free(ctx);
+    nhp_disc_trace_free(ctx);
     nhp_big_flush(ctx);
     free_cont(ctx);
     cudaFree(ctx->d_partials); cudaFree(ctx->d_scratch); cudaFree(ctx->d_flag); cudaFree(ctx->d_winstat);
     cudaFree(ctx->dd_lambda0); cudaFree(ctx->dd_W); cudaFree(ctx->dd_A); cudaFree(ctx->dd_theta); cudaFree(ctx->dd_bump);
-    cudaFree(ctx->dd_klist); cudaFree(ctx->dd_kptr); cudaFree(ctx->dd_btc); cudaFree(ctx->dd_counts);
+    cudaFree(ctx->dd_klist); cudaFree(ctx->dd_kptr); cudaFree(ctx->dd_btc); cudaFree(ctx->dd_counts); cudaFree(ctx->dd_kcnt); cudaFree(ctx->dd_ksum);
     cudaFree(ctx->d_bgrid_x); cudaFree(ctx->d_bgrid_v); cudaFree(ctx->d_bprior_L); cudaFree(ctx->d_slice);
     cudaFree(ctx->d_adj_ctl); cudaFree(ctx->d_adj_stat);
     cudaEventDestroy(ctx->ev0); cudaEventDestroy(ctx->ev1);

@@ -221,10 +221,19 @@ struct nhp_ctx {
     double *dd_bump = nullptr;    // [N*B][N] row k=(p*B+b), col c: [A]W theta dt
     int *dd_klist = nullptr, *dd_kptr = nullptr;  // per child: ascending k = p*B+b of the structurally non-zero entries
     double *dd_btc = nullptr;     // bumpT values at dd_klist
+    int *dd_kcnt = nullptr;       // [N] non-zero effective weights per child (table refresh work array)
+    double *dd_ksum = nullptr;    // [4]: list length, longest child list, non-zero effective weights, sum of A (table refresh results)
+    size_t dd_klist_cap = 0;      // entries allocated in dd_klist / dd_btc
+    bool dd_lists = false;        // dd_klist / dd_kptr / dd_btc describe the current parameters (density <= 0.5)
     double dd_density = 1.0;
+    double dd_a_sum = 0.0;        // sum of the discrete adjacency matrix, refreshed with the tables
+    double dd_rho = -1.0;         // link probability of the discrete Bernoulli network (nhp_disc_network_set); the continuous model keeps its own
     double *dd_counts = nullptr;  // [N * (1 + N B)] counts of the last discrete Gibbs parent sweep (counts[c + N k]), kept for the device-side draws
     size_t dd_counts_cap = 0; int64_t dd_counts_N = 0, dd_counts_B = 0;
     int64_t dd_maxNA = 0;
+    // discrete sample trace (cont_trace.cu): [dd_trace_cap] slots of (rho, lambda0, W, theta) + bit-packed adjacency matrices
+    double *dd_trace = nullptr; uint32_t *dd_trace_bits = nullptr;
+    int64_t dd_trace_cap = 0, dd_trace_len = 0, dd_trace_N = 0, dd_trace_B = 0; bool dd_trace_has_A = false;
 };
 
 // launch bookkeeping
@@ -320,3 +329,8 @@ void *nhp_big_alloc(nhp_ctx *ctx, size_t bytes);              // nullptr when th
 void nhp_big_free(nhp_ctx *ctx, void *p, size_t bytes);       // ctx == nullptr: cudaFree
 size_t nhp_big_cached_bytes(const nhp_ctx *ctx);
 void nhp_big_flush(nhp_ctx *ctx);                 // cached structure of the adjacency sampler (nhp_context.cu)
+// discrete chain pieces shared between translation units
+int nhp_disc_tables_refresh(nhp_ctx *ctx);        // disc.cu: bump table, compact parent lists, density, sum of A from the device-resident parameters
+const double *nhp_disc_rowsum(nhp_disc *dd);      // disc.cu: [N] events per node (device)
+int nhp_disc_draw_params(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t counter, const double *d_Mn, const double *hyper);  // cont_conjugate.cu
+int nhp_disc_draw_network(nhp_ctx *ctx, uint64_t seed, uint64_t counter, double alpha, double beta);  // cont_conjugate.cu: ctx->dd_rho ~ Beta

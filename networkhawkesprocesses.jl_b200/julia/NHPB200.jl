@@ -619,4 +619,43 @@ function resample_adjacency_matrix!(process::DiscreteNetworkHawkesProcess, data,
     return copy(process.adjacency_matrix)
 end
 
+# `mcmc!` (inference.jl:49-70) of a discrete process with the chain and its sample trace on the device: the parameters (and ρ of a
+# BernoulliNetworkModel) go up once, every sweep is one nhp_disc_gibbs_sweep (which appends its sample to the discrete trace,
+# adjacency bit-packed), one read at the end.  Samples in the order of params(process): discrete.jl:178-182 / 406-414.
+function mcmc_on_device!(process::DiscreteHawkesProcess, data; nsteps=1000)
+    d = device_counts(data)
+    ensure_convolved!(process, d)
+    push_params!(process)
+    b, w, imp = process.baseline, process.weights, process.impulses
+    hyper = Float64[b.α0, b.β0, w.κ, w.ν, imp.γ]
+    net = process isa DiscreteNetworkHawkesProcess
+    bern = net && process.network isa BernoulliNetworkModel
+    bern && check(ccall((:nhp_disc_network_set, LIB[]), Cint, (Ptr{Cvoid}, Float64), CTX[], Float64(process.network.ρ)))
+    check(ccall((:nhp_disc_trace_begin, LIB[]), Cint, (Ptr{Cvoid}, Int64), CTX[], nsteps))
+    seed = Base.rand(UInt64)
+    start = time()
+    for step in 1:nsteps
+        check(ccall((:nhp_disc_gibbs_sweep, LIB[]), Cint,
+            (Ptr{Cvoid}, Ptr{Cvoid}, UInt64, UInt64, Ptr{Float64}, Cint, Float64, Float64),
+            CTX[], d.h, seed, UInt64(step), hyper, length(hyper),
+            bern ? Float64(process.network.α) : 0.0, bern ? Float64(process.network.β) : 0.0))
+    end
+    N = ndims(process); B = size(imp.θ, 3)
+    ρ = Vector{Float64}(undef, nsteps); λ = Matrix{Float64}(undef, N, nsteps); W = Array{Float64}(undef, N, N, nsteps)
+    θ = Array{Float64}(undef, N, N, B, nsteps); A = Array{Float64}(undef, N, N, nsteps)
+    check(ccall((:nhp_disc_trace_read, LIB[]), Cint,
+        (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+        CTX[], 0, nsteps, ρ, λ, W, net ? A : C_NULL, θ))
+    check(ccall((:nhp_disc_trace_free, LIB[]), Cint, (Ptr{Cvoid},), CTX[]))
+    samples = Vector{Vector{Float64}}(undef, nsteps)
+    for k in 1:nsteps
+        samples[k] = net ? [bern ? [ρ[k]] : Float64[]; λ[:, k]; vec(W[:, :, k]); vec(θ[:, :, :, k]); vec(A[:, :, k])] :
+                           [λ[:, k]; vec(W[:, :, k] .* θ[:, :, :, k])]
+    end
+    b.λ = λ[:, end]; w.W = W[:, :, end]; imp.θ = θ[:, :, :, end]
+    net && (process.adjacency_matrix .= A[:, :, end])
+    bern && (process.network.ρ = ρ[end])
+    return NetworkHawkesProcesses.MarkovChainMonteCarlo(samples, time() - start)
+end
+
 end # module

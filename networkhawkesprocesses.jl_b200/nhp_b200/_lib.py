@@ -98,6 +98,16 @@ PROTOTYPES = {
     "nhp_disc_gibbs_counts": (c_int, [c_void_p, c_void_p, c_uint64, c_uint64, c_void_p, c_int64, c_void_p]),
     "nhp_disc_vb_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "nhp_disc_resample_adjacency": (c_int, [c_void_p, c_void_p, c_void_p, c_uint64, c_uint64, c_void_p, c_void_p]),
+    "nhp_disc_params_get": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "nhp_disc_resample_adjacency_dev": (c_int, [c_void_p, c_void_p, c_double, c_uint64, c_uint64]),
+    "nhp_disc_network_set": (c_int, [c_void_p, c_double]),
+    "nhp_disc_network_get": (c_int, [c_void_p, c_double_p]),
+    "nhp_disc_trace_begin": (c_int, [c_void_p, c_int64]),
+    "nhp_disc_trace_push": (c_int, [c_void_p]),
+    "nhp_disc_trace_count": (c_int, [c_void_p, POINTER(c_int64), POINTER(c_int64)]),
+    "nhp_disc_trace_read": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "nhp_disc_trace_free": (c_int, [c_void_p]),
+    "nhp_disc_gibbs_sweep": (c_int, [c_void_p, c_void_p, c_uint64, c_uint64, c_void_p, c_int, c_double, c_double]),
 }
 
 _lib = None

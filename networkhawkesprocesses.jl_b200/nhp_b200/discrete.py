@@ -4,7 +4,7 @@
   processes   DiscreteStandardHawkesProcess (discrete.jl:161-170), DiscreteNetworkHawkesProcess (discrete.jl:395-402)
   functions   basis, convolve, intensity, loglikelihood, resample_parents (reduced over t: counts[c, k]),
               update_ (one VB step, discrete.jl:369-375), resample_ (one Gibbs sweep, discrete.jl:361-367 / 416-424),
-              resample_adjacency_matrix_, mcmc_, vb_
+              resample_adjacency_matrix_, mcmc_, mcmc_device_ (the chain and its trace on the device), vb_
 `data` is an N x T integer matrix (numpy row = node) as in the reference; arrays indexed theta[p, c, b].
 """
 import ctypes
@@ -306,6 +306,51 @@ def mcmc_(process, data, nsteps=1000, seed=0):
     d = process._ready(data)
     t0 = time.time()
     samples = [resample_(process, d, rng, seed=seed, counter=s) for s in range(nsteps)]
+    from .continuous import MarkovChainMonteCarlo
+    return MarkovChainMonteCarlo(samples, time.time() - t0)
+
+
+def mcmc_device_(process, data, nsteps=1000, seed=0):
+    """`mcmc!` (inference.jl:49-70) with the chain AND its sample trace on the device: the parameters (and rho of a Bernoulli network)
+    go up once, every sweep is one nhp_disc_gibbs_sweep (Philox keyed by (seed, step), as resample_on_device_; it appends its sample
+    to the device-side trace), and the trace comes back in one read at the end.  Returns MarkovChainMonteCarlo with the samples in
+    the order of `params(process)` ([rho;] lambda0; vec(W); vec(theta); vec(A) for a network process, discrete.jl:406-414;
+    lambda0; vec(W .* theta) for a standard one, discrete.jl:178-182); the process holds the last sample."""
+    ctx = process._ctx()
+    d = process._ready(data)
+    t0 = time.time()
+    N, B = d.N, process.impulses.nbasis()
+    net = process.adjacency_matrix is not None
+    bern = net and isinstance(process.network, BernoulliNetworkModel)
+    b, w, imp = process.baseline, process.weights, process.impulses
+    process._push(ctx)
+    if bern:
+        ctx.check(ctx.lib.nhp_disc_network_set(ctx.h, float(process.network.rho)))
+    hy = np.array([b.alpha0, b.beta0, w.kappa, w.nu, imp.gamma], dtype=np.float64)
+    ctx.check(ctx.lib.nhp_disc_trace_begin(ctx.h, int(nsteps)))
+    try:
+        for step in range(nsteps):
+            ctx.check(ctx.lib.nhp_disc_gibbs_sweep(ctx.h, d.h, int(seed), int(step), _ptr(hy), hy.size,
+                                                   float(process.network.alpha) if bern else 0.0, float(process.network.beta) if bern else 0.0))
+        rho, lam, W, th = np.empty(nsteps), np.empty((nsteps, N)), np.empty((nsteps, N * N)), np.empty((nsteps, N * N * B))
+        A = np.empty((nsteps, N * N)) if net else None
+        ctx.check(ctx.lib.nhp_disc_trace_read(ctx.h, 0, int(nsteps), _ptr(rho), _ptr(lam), _ptr(W), _ptr(A), _ptr(th)))
+    finally:
+        ctx.check(ctx.lib.nhp_disc_trace_free(ctx.h))
+    b.lam = lam[-1].copy()
+    w.W = W[-1].reshape(N, N).T.copy()                              # W[p + N c] -> [p, c]
+    imp.theta = th[-1].reshape(B, N, N).transpose(2, 1, 0).copy()   # theta[p + N (c + N b)] -> [p, c, b]
+    if net:
+        process.adjacency_matrix = A[-1].reshape(N, N).T.copy()
+    if bern:
+        process.network.rho = float(rho[-1])
+    samples = []
+    for k in range(nsteps):
+        if net:    # discrete.jl:406-414: [network; baseline; vec(W); vec(theta); vec(A)]
+            parts = ([rho[k:k + 1]] if bern else [process.network.params()]) + [lam[k], W[k], th[k], A[k]]
+        else:      # discrete.jl:178-182: [baseline; vec(W .* theta)]
+            parts = [lam[k], np.tile(W[k], B) * th[k]]
+        samples.append(np.concatenate(parts))
     from .continuous import MarkovChainMonteCarlo
     return MarkovChainMonteCarlo(samples, time.time() - t0)
 
