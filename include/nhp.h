@@ -349,6 +349,27 @@ int nhp_disc_trace_free(nhp_ctx *ctx);
  * before anything changes. */
 int nhp_disc_gibbs_sweep(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t counter, const double *hyper, int n_hyper, double net_alpha,
                          double net_beta);
+/* Mean-field VB of a discrete standard process (`vb!`, inference.jl:153-181) with its state on the device.  The state is the
+ * reference's variational_params vector (discrete.jl:204-209), q = [alphav(N); betav(N); vec(gammav)(N*N*B); vec(kappav)(N*N);
+ * vec(nuv)(N*N)] with gammav[p + N*(c + N*b)], kappav[p + N*c], nuv[p + N*c].  _set validates (every entry of q and hyper finite and
+ * > 0, dt > 0) and keeps q, hyper = [alpha0, beta0, kappa, nu, gamma] and dt with the context (buffers grow with N or B only, and are
+ * freed by nhp_destroy); _get copies q back. */
+int nhp_disc_vb_set(nhp_ctx *ctx, int64_t N, int64_t B, double dt, const double *hyper, int n_hyper, const double *q);
+int nhp_disc_vb_get(nhp_ctx *ctx, double *q);
+/* One `update!(process, data, convolved)` (discrete.jl:369-375) on the device: the exp-expectations from q (digamma on the device),
+ * the statistics of nhp_disc_vb_stats, then in place alphav = alpha0 + alpha_sum, betav = 1/beta0 + T dt (baselines.jl:450 as
+ * written), gammav = gamma + gamma_sum, kappav = kappa + kappa_sum, nuv = nu + events of the parent node; then a push to the VB trace
+ * while it has room.  change (may be NULL) = max_i |q_new[i] - q_old[i]| / q_old[i], the only value that crosses PCIe.  Needs
+ * nhp_disc_convolve.  Refused before anything changes: time-sharded data or a communicator of more than one rank
+ * (NHP_ERR_UNSUPPORTED); no state or no convolution (NHP_ERR_STATE); N or B of the state not those of dd (NHP_ERR_INVALID); an open
+ * VB trace whose slot size is not the state's (NHP_ERR_STATE). */
+int nhp_disc_vb_step(nhp_ctx *ctx, nhp_disc *dd, double *change);
+/* Device-side trace of the VB state, independent of the Gibbs traces: one slot is q (2 N + N*N*(B + 2) doubles, laid out for the
+ * state at _begin); _read copies slots [first, first + count) one after the other. */
+int nhp_disc_vb_trace_begin(nhp_ctx *ctx, int64_t capacity);
+int nhp_disc_vb_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity);
+int nhp_disc_vb_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *q_out);
+int nhp_disc_vb_trace_free(nhp_ctx *ctx);
 
 #ifdef __cplusplus
 }

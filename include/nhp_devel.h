@@ -17,8 +17,8 @@ int64_t nhp_launch_count(const nhp_ctx *ctx);
  * 4 adjacency-bit probes [probes/s] (one shared-memory node id + one shared-memory bit-row word per probe, the
  * inner loop of the sparse sweep's filter with nothing else around it). */
 int nhp_bench_fp64(nhp_ctx *ctx, int which, double *result);
-/* Test hook for the table-driven FP64 log (which = 0) / exp (which = 1) the impulse evaluation uses:
- * out[i] = f(x[i]), host pointers. */
+/* Test hook for the table-driven FP64 log (which = 0) / exp (which = 1) the impulse evaluation uses, and for the digamma of the
+ * VB expectations (which = 2, x > 0): out[i] = f(x[i]), host pointers. */
 int nhp_test_fastmath(nhp_ctx *ctx, int which, const double *x, int64_t n, double *out);
 /* Last adjacency sweep of this context: out8 = [steps taken, batches, flips, recomputed steps, cached pairs,
  * virtual columns, sweep kernel ms, structure build ms]. */

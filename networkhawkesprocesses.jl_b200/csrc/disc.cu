@@ -1223,6 +1223,28 @@ __global__ void k_vb_finish(const double *__restrict__ gammaT, const double *__r
     nu[p + (int64_t)N * c] = rowsum[p];
 }
 
+// responsibilities + reductions of one VB step into zeroed alpha_sum[N] and gammaT[c][p*B+b]: the warp-per-bin kernel when its
+// buffers fit shared memory (and NHP_DISC_WARP is not 0), the block kernel otherwise; nothing to do without non-zero bins
+int nhp_disc_vb_reduce(nhp_ctx *ctx, nhp_disc *dd, const double *e0, const double *ET, double *alpha_sum, double *gammaT) {
+    DiscExtra *ex = extra_of(dd);
+    if (ex->nnz == 0) return NHP_OK;
+    const int64_t N = dd->N, NB = N * dd->B;
+    cudaStream_t s = ctx->stream;
+    const size_t wsmem = (size_t)9 * NB * sizeof(double);
+    const char *envw = getenv("NHP_DISC_WARP");
+    if (wsmem <= (size_t)ctx->smem_optin - 4096 && !(envw && atoi(envw) == 0)) {
+        DCUDA(ctx, cudaFuncSetAttribute(k_disc_vb_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
+        const int tb = pick_time_block(ctx, dd, ex->nnz);
+        const int64_t nblk = (dd->T + tb - 1) / tb;
+        k_disc_vb_warp<<<(unsigned)(N * nblk), 256, wsmem, s>>>(dd->d_conv, ET, e0, (int)N, (int)NB, ex->nz_t, ex->nz_s, ex->child_ptr, tb, alpha_sum, gammaT);
+    } else {
+        const int slabs = pick_slabs(ctx, N, ex->nnz);
+        k_disc_vb<<<(unsigned)(N * slabs), 256, 0, s>>>(dd->d_conv, ET, e0, (int)N, (int)NB, ex->nz_t, ex->nz_s, ex->child_ptr, slabs, alpha_sum, gammaT);
+    }
+    NHP_LAUNCHED(ctx);
+    return NHP_OK;
+}
+
 extern "C" int nhp_disc_vb_stats(nhp_ctx *ctx, nhp_disc *dd, const double *e0, const double *E, double *alpha_sum, double *kappa_sum, double *nu_sum,
                                  double *gamma_sum) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
@@ -1245,19 +1267,7 @@ extern "C" int nhp_disc_vb_stats(nhp_ctx *ctx, nhp_disc *dd, const double *e0, c
     k_transpose_E<<<eb, 256, 0, s>>>(d_E, (int)N, (int)B, d_ET);
     NHP_LAUNCHED(ctx);
     NHP_TRY(nhp_timer_begin(ctx));
-    if (ex->nnz > 0) {
-        int slabs = pick_slabs(ctx, N, ex->nnz);
-        const size_t wsmem = (size_t)9 * NB * sizeof(double);
-        const char *envw = getenv("NHP_DISC_WARP");
-        if (wsmem <= (size_t)ctx->smem_optin - 4096 && !(envw && atoi(envw) == 0)) {
-            DCUDA(ctx, cudaFuncSetAttribute(k_disc_vb_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
-            const int tb = pick_time_block(ctx, dd, ex->nnz);
-            const int64_t nblk = (dd->T + tb - 1) / tb;
-            k_disc_vb_warp<<<(unsigned)(N * nblk), 256, wsmem, s>>>(dd->d_conv, d_ET, d_e0, (int)N, (int)NB, ex->nz_t, ex->nz_s, ex->child_ptr, tb, d_alpha, d_gT);
-        } else
-        k_disc_vb<<<(unsigned)(N * slabs), 256, 0, s>>>(dd->d_conv, d_ET, d_e0, (int)N, (int)NB, ex->nz_t, ex->nz_s, ex->child_ptr, slabs, d_alpha, d_gT);
-        NHP_LAUNCHED(ctx);
-    }
+    NHP_TRY(nhp_disc_vb_reduce(ctx, dd, d_e0, d_ET, d_alpha, d_gT));
     k_vb_finish<<<(unsigned)((N * N + 255) / 256), 256, 0, s>>>(d_gT, ex->rowsum, (int)N, (int)B, d_kappa, d_nu, d_gamma);
     NHP_LAUNCHED(ctx);
     DCUDA(ctx, cudaGetLastError());

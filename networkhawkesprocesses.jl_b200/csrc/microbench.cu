@@ -107,17 +107,17 @@ extern "C" int nhp_bench_fp64(nhp_ctx *ctx, int which, double *result) {
     return NHP_OK;
 }
 
-// test hook: out[i] = fast_log(x[i]) (which = 0) or fast_exp(x[i]) (which = 1); HOST pointers
+// test hook: out[i] = fast_log(x[i]) (which = 0), fast_exp(x[i]) (which = 1) or nhp_digamma(x[i]) (which = 2); HOST pointers
 __global__ void k_fastmath_eval(const double *x, double *out, int64_t n, int which) {
     __shared__ FastTables s_ft;
     fast_tables_load(&s_ft);
     __syncthreads();
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) out[i] = which == 0 ? fast_log(x[i], &s_ft) : fast_exp(x[i], &s_ft);
+    if (i < n) out[i] = which == 0 ? fast_log(x[i], &s_ft) : which == 1 ? fast_exp(x[i], &s_ft) : nhp_digamma(x[i]);
 }
 extern "C" int nhp_test_fastmath(nhp_ctx *ctx, int which, const double *x, int64_t n, double *out) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, x && out && n > 0 && (which == 0 || which == 1), NHP_ERR_INVALID, "nhp_test_fastmath: bad argument");
+    NHP_CHECK(ctx, x && out && n > 0 && which >= 0 && which <= 2, NHP_ERR_INVALID, "nhp_test_fastmath: bad argument");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     NHP_CUDA(ctx, fast_tables_upload(ctx->stream));
     void *scratch;

@@ -80,6 +80,8 @@ extern "C" int nhp_destroy(nhp_ctx *ctx) {
     nhp_comm_destroy(ctx);
     nhp_cont_trace_free(ctx);
     nhp_disc_trace_free(ctx);
+    nhp_disc_vb_trace_free(ctx);
+    cudaFree(ctx->dv_q);
     nhp_big_flush(ctx);
     free_cont(ctx);
     cudaFree(ctx->d_partials); cudaFree(ctx->d_scratch); cudaFree(ctx->d_flag); cudaFree(ctx->d_winstat);

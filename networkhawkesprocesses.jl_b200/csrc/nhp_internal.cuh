@@ -234,6 +234,14 @@ struct nhp_ctx {
     // discrete sample trace (cont_trace.cu): [dd_trace_cap] slots of (rho, lambda0, W, theta) + bit-packed adjacency matrices
     double *dd_trace = nullptr; uint32_t *dd_trace_bits = nullptr;
     int64_t dd_trace_cap = 0, dd_trace_len = 0, dd_trace_N = 0, dd_trace_B = 0; bool dd_trace_has_A = false;
+
+    // ---- discrete mean-field VB (disc_vb.cu): q = [alphav(N); betav(N); gammav(N^2 B); kappav(N^2); nuv(N^2)] and its trace
+    bool dv_set = false;
+    int64_t dv_N = 0, dv_B = 0;
+    double dv_dt = 1.0, dv_hyper[5] = {0};  // alpha0, beta0, kappa, nu, gamma
+    double *dv_q = nullptr; size_t dv_cap = 0;  // doubles allocated
+    double *dv_trace = nullptr;                 // [dv_trace_cap] slots of q for (dv_trace_N, dv_trace_B)
+    int64_t dv_trace_cap = 0, dv_trace_len = 0, dv_trace_N = 0, dv_trace_B = 0;
 };
 
 // launch bookkeeping
@@ -332,5 +340,6 @@ void nhp_big_flush(nhp_ctx *ctx);                 // cached structure of the adj
 // discrete chain pieces shared between translation units
 int nhp_disc_tables_refresh(nhp_ctx *ctx);        // disc.cu: bump table, compact parent lists, density, sum of A from the device-resident parameters
 const double *nhp_disc_rowsum(nhp_disc *dd);      // disc.cu: [N] events per node (device)
+int nhp_disc_vb_reduce(nhp_ctx *ctx, nhp_disc *dd, const double *e0, const double *ET, double *alpha_sum, double *gammaT);  // disc.cu: VB statistics into zeroed sums
 int nhp_disc_draw_params(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t counter, const double *d_Mn, const double *hyper);  // cont_conjugate.cu
 int nhp_disc_draw_network(nhp_ctx *ctx, uint64_t seed, uint64_t counter, double alpha, double beta);  // cont_conjugate.cu: ctx->dd_rho ~ Beta

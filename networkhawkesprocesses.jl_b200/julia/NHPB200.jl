@@ -658,4 +658,37 @@ function mcmc_on_device!(process::DiscreteHawkesProcess, data; nsteps=1000)
     return NetworkHawkesProcesses.MarkovChainMonteCarlo(samples, time() - start)
 end
 
+# `vb!` (inference.jl:153-181) of a discrete standard process with the loop and its trace on the device: variational_params(process)
+# (discrete.jl:204-209) and the hyper-parameters go up once, every step is one nhp_disc_vb_step (`update!`, discrete.jl:369-375, with
+# digamma on the device; it appends the new state to the VB trace), one read at the end.  With `rtol`, the loop stops after the first
+# step whose largest relative change of a variational parameter is <= rtol (this package's criterion: the reference's test is
+# commented out, inference.jl:163-176).  Returns the trace, one variational_params vector per step; the process holds the last one.
+function vb_on_device!(process::DiscreteStandardHawkesProcess, data; max_steps=100, rtol=nothing)
+    d = device_counts(data)
+    ensure_convolved!(process, d)
+    b, w, imp = process.baseline, process.weights, process.impulses
+    N = ndims(process); B = size(imp.θ, 3)
+    q = Vector{Float64}(NetworkHawkesProcesses.variational_params(process))
+    hyper = Float64[b.α0, b.β0, w.κ, w.ν, imp.γ]
+    check(ccall((:nhp_disc_vb_set, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, Float64, Ptr{Float64}, Cint, Ptr{Float64}),
+        CTX[], N, B, process.dt, hyper, length(hyper), q))
+    check(ccall((:nhp_disc_vb_trace_begin, LIB[]), Cint, (Ptr{Cvoid}, Int64), CTX[], max_steps))
+    change = Ref{Float64}(0.0)
+    steps = 0
+    for step in 1:max_steps
+        check(ccall((:nhp_disc_vb_step, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}), CTX[], d.h,
+            rtol === nothing ? C_NULL : change))
+        steps = step
+        rtol !== nothing && change[] <= rtol && break
+    end
+    Q = Matrix{Float64}(undef, length(q), steps)
+    check(ccall((:nhp_disc_vb_trace_read, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}), CTX[], 0, steps, Q))
+    check(ccall((:nhp_disc_vb_trace_free, LIB[]), Cint, (Ptr{Cvoid},), CTX[]))
+    trace = [Q[:, k] for k in 1:steps]
+    last = trace[end]; o = 2N + N * N * B
+    b.αv = last[1:N]; b.βv = last[N+1:2N]
+    imp.γv = reshape(last[2N+1:o], N, N, B); w.κv = reshape(last[o+1:o+N*N], N, N); w.νv = reshape(last[o+N*N+1:end], N, N)
+    return trace
+end
+
 end # module

@@ -4,7 +4,8 @@
   processes   DiscreteStandardHawkesProcess (discrete.jl:161-170), DiscreteNetworkHawkesProcess (discrete.jl:395-402)
   functions   basis, convolve, intensity, loglikelihood, resample_parents (reduced over t: counts[c, k]),
               update_ (one VB step, discrete.jl:369-375), resample_ (one Gibbs sweep, discrete.jl:361-367 / 416-424),
-              resample_adjacency_matrix_, mcmc_, mcmc_device_ (the chain and its trace on the device), vb_
+              resample_adjacency_matrix_, mcmc_, mcmc_device_ (the chain and its trace on the device), vb_, vb_device_ (the VB loop
+              and its trace on the device)
 `data` is an N x T integer matrix (numpy row = node) as in the reference; arrays indexed theta[p, c, b].
 """
 import ctypes
@@ -360,3 +361,58 @@ def vb_(process, data, max_steps=100):
     d = process._ready(data)
     trace = [update_(process, d) for _ in range(max_steps)]
     return trace
+
+
+def set_variational_params_(process, q):
+    """Inverse of `variational_params` (discrete.jl:204-209): q = [alphav; betav; vec(gammav); vec(kappav); vec(nuv)]."""
+    b, w, imp = process.baseline, process.weights, process.impulses
+    N, B = process.ndims(), imp.nbasis()
+    q = np.asarray(q, dtype=np.float64).reshape(-1)
+    if q.size != 2 * N + N * N * (B + 2):
+        raise ValueError(f"variational parameter vector of {q.size} entries; N = {N}, B = {B} needs {2 * N + N * N * (B + 2)}")
+    o = 2 * N + N * N * B
+    b.alphav, b.betav = q[:N].copy(), q[N:2 * N].copy()
+    imp.gammav = q[2 * N:o].reshape(B, N, N).transpose(2, 1, 0).copy()  # gammav[p + N (c + N b)] -> [p, c, b]
+    w.kappav = q[o:o + N * N].reshape(N, N).T.copy()                     # [p + N c] -> [p, c]
+    w.nuv = q[o + N * N:].reshape(N, N).T.copy()
+
+
+def vb_device_(process, data, max_steps=100, rtol=None):
+    """`vb!` (inference.jl:153-181) with the loop and its trace on the device.  The variational parameters (kappav / nuv initialised
+    as update_ does) and the hyper-parameters go up once (nhp_disc_vb_set); each step is one nhp_disc_vb_step, the `update!` of
+    discrete.jl:369-375 with digamma on the device, which appends the new state to the device-side VB trace; the trace comes back
+    in one read.  Without `rtol` it runs max_steps steps, as vb_.  With `rtol` it stops after the first step whose largest relative
+    change of any variational parameter, max_i |q_new[i] - q_old[i]| / q_old[i], is <= rtol: a criterion of this package, since the
+    reference's own convergence test is commented out (inference.jl:163-176).  Returns the list of variational_params vectors, one
+    per step, as vb_; the process holds the last state.  A network process raises ValueError: the reference's update! for it is
+    non-functional (quirk Q10)."""
+    if isinstance(process, DiscreteNetworkHawkesProcess):
+        raise ValueError("vb_device_: the reference's update! of a DiscreteNetworkHawkesProcess is non-functional (quirk Q10); "
+                         "VB runs on DiscreteStandardHawkesProcess")
+    ctx = process._ctx()
+    d = process._ready(data)
+    if max_steps < 1:
+        return []
+    b, w, imp = process.baseline, process.weights, process.impulses
+    if not hasattr(w, "kappav"):
+        w.kappav, w.nuv = np.ones_like(w.W), np.ones_like(w.W)
+    N, B = d.N, imp.nbasis()
+    q = _f64(process.variational_params())
+    if q.size != 2 * N + N * N * (B + 2):
+        raise ValueError("variational parameter shapes do not match the data's number of nodes")
+    hy = np.array([b.alpha0, b.beta0, w.kappa, w.nu, imp.gamma], dtype=np.float64)
+    ctx.check(ctx.lib.nhp_disc_vb_set(ctx.h, N, B, process.dt, _ptr(hy), hy.size, _ptr(q)))
+    ctx.check(ctx.lib.nhp_disc_vb_trace_begin(ctx.h, int(max_steps)))
+    try:
+        change, steps = ctypes.c_double(), 0
+        for _ in range(max_steps):
+            ctx.check(ctx.lib.nhp_disc_vb_step(ctx.h, d.h, None if rtol is None else ctypes.byref(change)))
+            steps += 1
+            if rtol is not None and change.value <= rtol:
+                break
+        out = np.empty((steps, q.size))
+        ctx.check(ctx.lib.nhp_disc_vb_trace_read(ctx.h, 0, steps, _ptr(out)))
+    finally:
+        ctx.check(ctx.lib.nhp_disc_vb_trace_free(ctx.h))
+    set_variational_params_(process, out[-1])
+    return list(out)
