@@ -278,6 +278,20 @@ int nhp_cont_loglik_dev(nhp_ctx *ctx, nhp_events *ev, int recursive);
  * read-only history for the convolution. */
 int nhp_disc_upload(nhp_ctx *ctx, const int64_t *data, int64_t N, int64_t T, int64_t t_halo, nhp_disc **out);
 int nhp_disc_free(nhp_ctx *ctx, nhp_disc *dd);
+/* rand(process::DiscreteHawkesProcess, T)  discrete.jl:20-38: one N x T sample of the discrete process whose parameters the context
+ * holds (nhp_disc_params_set; standard, or network with A), simulated on the device and left there as an unsharded (t_halo = 0),
+ * not yet convolved count handle -- the same handle nhp_disc_upload would make of the sample.  The law is the one nhp_disc_loglik
+ * evaluates: given the earlier bins, data[c, t] ~ Poisson(lambda[t, c]) independently, lambda as nhp_disc_intensity returns it with
+ * phi = nhp_disc_basis(L, B, dt) and no events before bin 0; it is drawn in the cluster representation (baseline events, then
+ * Poisson children per event, generation by generation).  L is the impulse response's nlags.  Philox keyed by `seed`: the sample is a
+ * deterministic function of (parameters, T, L, seed); parity with the reference is distributional.  Refused, with no handle and
+ * nothing left allocated: no discrete parameters (NHP_ERR_STATE); T < 1, N*T >= 2^31, L < 1 or L*B > 4096, a negative or non-finite
+ * lambda0, [A]W or theta, or a sample of more than max_events generated events, dropped children included (NHP_ERR_INVALID).
+ * nhp_disc_download copies every bin of a handle (halo included) to the host as data[n + N*t]; nhp_disc_events_count gives the
+ * events in its own bins. */
+int nhp_disc_rand(nhp_ctx *ctx, int64_t T, int64_t L, uint64_t seed, int64_t max_events, nhp_disc **out);
+int nhp_disc_download(nhp_ctx *ctx, nhp_disc *dd, int64_t *data);
+int64_t nhp_disc_events_count(const nhp_disc *dd);
 /* basis(impulse)  impulses.jl:321-335 -> phi[l + L*b] */
 int nhp_disc_basis(int64_t L, int64_t B, double dt, double *phi);
 /* convolve(process, data)  discrete.jl:146-151; result stays on the device; conv_out (T*N*B,

@@ -104,10 +104,37 @@ extern "C" int nhp_disc_upload(nhp_ctx *ctx, const int64_t *data, int64_t N, int
     NHP_CHECK(ctx, N * T < (int64_t)2147483000, NHP_ERR_INVALID, "nhp_disc_upload: N*T must stay below 2^31 per handle (shard the time axis)");
     DCUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
+    const int64_t total = N * T;
+    int *d_data = nullptr;
+    auto fail = [&](int rc) { cudaStreamSynchronize(s); cudaFree(d_data); return rc; };
+#define IN_CUDA(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) return fail(nhp_fail(ctx, NHP_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e__))); } while (0)
+    void *scratch;
+    NHP_TRY(nhp_scratch(ctx, (size_t)total * sizeof(int64_t), &scratch));
+    IN_CUDA(cudaMalloc(&d_data, (size_t)total * sizeof(int)));
+    IN_CUDA(cudaMemcpyAsync(scratch, data, (size_t)total * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    IN_CUDA(cudaMemsetAsync(ctx->d_flag, 0, sizeof(int), s));
+    unsigned blocks = (unsigned)((total + 255) / 256);
+    k_disc_ingest<<<blocks, 256, 0, s>>>((const int64_t *)scratch, d_data, total, ctx->d_flag);
+    NHP_LAUNCHED(ctx);
+    int flag = 0;
+    IN_CUDA(cudaMemcpyAsync(&flag, ctx->d_flag, sizeof(int), cudaMemcpyDeviceToHost, s));
+    IN_CUDA(cudaStreamSynchronize(s));
+#undef IN_CUDA
+    if (flag & 1) return fail(nhp_fail(ctx, NHP_ERR_INVALID, "nhp_disc_upload: counts must be in [0, 2^31)"));
+    return nhp_disc_from_device(ctx, d_data, N, T, t_halo, out);
+}
+
+// Everything a handle derives from its counts, for a grid already on the device (the upload's, the simulator's): the non-zero own
+// bins in memory order, the running draw index, the per-child CSR, the row sums, total_events and the longest column.  Takes
+// ownership of d_data (freed with the handle, or here on failure).
+int nhp_disc_from_device(nhp_ctx *ctx, int *d_data, int64_t N, int64_t T, int64_t t_halo, nhp_disc **out) {
+    *out = nullptr;
+    cudaStream_t s = ctx->stream;
     const int64_t total = N * T, first = t_halo * N;
     nhp_disc *dd = new nhp_disc();
     DiscExtra *ex = new DiscExtra();
     dd->N = N; dd->T = T; dd->t_halo = t_halo; dd->d_scan = reinterpret_cast<int64_t *>(ex);
+    dd->d_data = d_data;
     unsigned char *d_flags = nullptr; int64_t *d_cnt = nullptr, *d_scan = nullptr, *d_idx = nullptr, *d_nnz = nullptr; void *d_tmp = nullptr;
     int *d_key = nullptr, *d_pos = nullptr, *d_key2 = nullptr, *d_pos2 = nullptr;
     auto fin = [&](int rc) {
@@ -117,14 +144,7 @@ extern "C" int nhp_disc_upload(nhp_ctx *ctx, const int64_t *data, int64_t N, int
         return rc;
     };
 #define UP_CUDA(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) return fin(nhp_fail(ctx, NHP_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e__))); } while (0)
-    void *scratch;
-    { int rc = nhp_scratch(ctx, (size_t)total * sizeof(int64_t), &scratch); if (rc != NHP_OK) return fin(rc); }
-    UP_CUDA(cudaMalloc(&dd->d_data, (size_t)total * sizeof(int)));
-    UP_CUDA(cudaMemcpyAsync(scratch, data, (size_t)total * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-    UP_CUDA(cudaMemsetAsync(ctx->d_flag, 0, sizeof(int), s));
     unsigned blocks = (unsigned)((total + 255) / 256);
-    k_disc_ingest<<<blocks, 256, 0, s>>>((const int64_t *)scratch, dd->d_data, total, ctx->d_flag);
-    NHP_LAUNCHED(ctx);
     // non-zero bins (own bins only) in memory order + the running draw index
     UP_CUDA(cudaMalloc(&d_flags, (size_t)total));
     UP_CUDA(cudaMalloc(&d_cnt, (size_t)total * sizeof(int64_t)));
@@ -143,14 +163,11 @@ extern "C" int nhp_disc_upload(nhp_ctx *ctx, const int64_t *data, int64_t N, int
     UP_CUDA(cub::DeviceSelect::Flagged(d_tmp, tb, iota, d_flags, d_idx, d_nnz, (int)total, s));
     NHP_LAUNCHED(ctx); NHP_LAUNCHED(ctx);
     int64_t h_nnz = 0, h_last[2] = {0, 0};
-    int flag = 0;
     UP_CUDA(cudaMemcpyAsync(&h_nnz, d_nnz, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
     UP_CUDA(cudaMemcpyAsync(&h_last[0], d_scan + total - 1, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
     UP_CUDA(cudaMemcpyAsync(&h_last[1], d_cnt + total - 1, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
-    UP_CUDA(cudaMemcpyAsync(&flag, ctx->d_flag, sizeof(int), cudaMemcpyDeviceToHost, s));
     UP_CUDA(cudaStreamSynchronize(s));
-    if (flag & 1) return fin(nhp_fail(ctx, NHP_ERR_INVALID, "nhp_disc_upload: counts must be in [0, 2^31)"));
-    if (h_nnz >= (int64_t)2147483000) return fin(nhp_fail(ctx, NHP_ERR_INVALID, "nhp_disc_upload: too many non-zero bins"));
+    if (h_nnz >= (int64_t)2147483000) return fin(nhp_fail(ctx, NHP_ERR_INVALID, "nhp_disc: too many non-zero bins"));
     ex->nnz = h_nnz;
     dd->total_events = h_last[0] + h_last[1];
     UP_CUDA(cudaMalloc(&ex->child_ptr, (size_t)(N + 1) * sizeof(int)));

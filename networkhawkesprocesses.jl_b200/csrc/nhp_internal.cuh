@@ -337,6 +337,10 @@ void *nhp_big_alloc(nhp_ctx *ctx, size_t bytes);              // nullptr when th
 void nhp_big_free(nhp_ctx *ctx, void *p, size_t bytes);       // ctx == nullptr: cudaFree
 size_t nhp_big_cached_bytes(const nhp_ctx *ctx);
 void nhp_big_flush(nhp_ctx *ctx);                 // cached structure of the adjacency sampler (nhp_context.cu)
+int nhp_events_from_device(nhp_ctx *ctx, const double *d_t, const int *d_c, int64_t n, double duration, int64_t K, nhp_events **out);  // nhp_context.cu
+// disc.cu: the handle of an int32 count grid d_data[t*N + n] already on the device (non-zero bins, draw scan, per-child CSR, row sums,
+// total_events, longest column); takes ownership of d_data, also on failure
+int nhp_disc_from_device(nhp_ctx *ctx, int *d_data, int64_t N, int64_t T, int64_t t_halo, nhp_disc **out);
 // discrete chain pieces shared between translation units
 int nhp_disc_tables_refresh(nhp_ctx *ctx);        // disc.cu: bump table, compact parent lists, density, sum of A from the device-resident parameters
 const double *nhp_disc_rowsum(nhp_disc *dd);      // disc.cu: [N] events per node (device)

@@ -10,16 +10,8 @@ N, T, B, L = 2, 20000, 3, 4
 theta = rng.dirichlet(np.ones(B), (N, N))
 W = np.array([[0.2, 0.1], [0.1, 0.2]])
 process = D.DiscreteStandardHawkesProcess(D.DiscreteHomogeneousProcess(np.array([0.1, 0.2])), D.DiscreteGaussianImpulseResponse(theta, L), nhp.DenseWeightModel(W))
-# simulate counts (host-side, discrete.jl:20-38)
-phi = process.impulses.basis()
-ir = np.einsum("pcb,lb->pcl", W[:, :, None] * theta, phi)
-data = rng.poisson(process.baseline.lam[:, None] * np.ones((N, T)))
-for t in range(T - 1):
-    for p in np.nonzero(data[:, t])[0]:
-        smax = min(L, T - 1 - t)
-        data[:, t + 1:t + 1 + smax] += rng.poisson(data[p, t] * ir[p][:, :smax])
-d = process.upload(data)
-print("events:", int(data.sum()), " loglikelihood:", D.loglikelihood(process, d))
+d = D.rand_device(process, T, seed=0)  # rand(process, T) (discrete.jl:20-38) on the device; the sample stays there
+print("events:", d.events_count(), " loglikelihood:", D.loglikelihood(process, d))
 D.vb_(process, d, max_steps=50)
 b, w, i = process.baseline, process.weights, process.impulses
 print("E[lambda] =", b.alphav / b.betav, " truth", [0.1, 0.2])        # posterior means as the reference example prints them

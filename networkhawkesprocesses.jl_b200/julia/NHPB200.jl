@@ -480,6 +480,27 @@ function push_params!(process::DiscreteHawkesProcess)
         convert(Array{Float64,3}, process.impulses.θ), process.dt))
 end
 
+# (R) discrete.jl:20-38: the cluster simulator on the device (nhp_disc_rand).  The sample comes back as the reference's
+# Matrix{Int64}, and its live device handle is registered in COUNT_CACHE under that matrix, so a following mcmc!, mcmc_on_device! or
+# vb_on_device! on it uploads nothing.
+function rand(process::DiscreteHawkesProcess, T::Integer)
+    push_params!(process)
+    N = ndims(process); B = size(process.impulses.θ, 3)
+    ϕ = hcat(basis(process.impulses)...)                     # L x B
+    Weff = process isa DiscreteNetworkHawkesProcess ? process.adjacency_matrix .* process.weights.W : process.weights.W
+    e = Weff .* dropdims(sum(process.impulses.θ .* reshape(vec(sum(ϕ, dims=1)) .* process.dt, 1, 1, B), dims=3), dims=3)
+    expected = sum(process.baseline.λ) * process.dt * T / max(0.05, 1 - min(0.95, maximum(sum(e, dims=2))))
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:nhp_disc_rand, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, UInt64, Int64, Ref{Ptr{Cvoid}}),
+        CTX[], T, size(ϕ, 1), Base.rand(UInt64), ceil(Int64, min(2.1e9, 2expected + 10sqrt(expected) + 1000)), h))
+    d = DeviceCounts(h[], N, Int(T), false)
+    finalizer(x -> ccall((:nhp_disc_free, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}), CTX[], x.h), d)
+    data = Matrix{Int64}(undef, N, T)                        # data[n + N*t]
+    check(ccall((:nhp_disc_download, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Int64}), CTX[], d.h, data))
+    COUNT_CACHE[objectid(data)] = CacheEntry{DeviceCounts}(WeakRef(data), fingerprint(data), d)
+    return data
+end
+
 # (E) discrete.jl:115
 function intensity(process::DiscreteHawkesProcess, convolved::DeviceConvolved)
     push_params!(process)

@@ -90,6 +90,9 @@ PROTOTYPES = {
     "nhp_cont_loglik_dev": (c_int, [c_void_p, c_void_p, c_int]),
     "nhp_disc_upload": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, POINTER(c_void_p)]),
     "nhp_disc_free": (c_int, [c_void_p, c_void_p]),
+    "nhp_disc_rand": (c_int, [c_void_p, c_int64, c_int64, c_uint64, c_int64, POINTER(c_void_p)]),
+    "nhp_disc_download": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "nhp_disc_events_count": (c_int64, [c_void_p]),
     "nhp_disc_basis": (c_int, [c_int64, c_int64, c_double, c_void_p]),
     "nhp_disc_convolve": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
     "nhp_disc_params_set": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_double]),

@@ -5,7 +5,7 @@
   functions   basis, convolve, intensity, loglikelihood, resample_parents (reduced over t: counts[c, k]),
               update_ (one VB step, discrete.jl:369-375), resample_ (one Gibbs sweep, discrete.jl:361-367 / 416-424),
               resample_adjacency_matrix_, mcmc_, mcmc_device_ (the chain and its trace on the device), vb_, vb_device_ (the VB loop
-              and its trace on the device)
+              and its trace on the device), rand (host) and rand_device (nhp_disc_rand: the sample stays on the device)
 `data` is an N x T integer matrix (numpy row = node) as in the reference; arrays indexed theta[p, c, b].
 """
 import ctypes
@@ -81,6 +81,25 @@ class DiscreteData:
         self.convolved = False
         self._fin = weakref.finalize(self, ctx.lib.nhp_disc_free, ctx.h, h)
 
+    @classmethod
+    def from_handle(cls, ctx, h, N, T):
+        """Wrap an unsharded count handle the library created on the device (nhp_disc_rand)."""
+        self = cls.__new__(cls)
+        self.ctx, self.h, self.N, self.T = ctx, h, int(N), int(T)
+        self.convolved = False
+        self._fin = weakref.finalize(self, ctx.lib.nhp_disc_free, ctx.h, h)
+        return self
+
+    def download(self):
+        """The N x T int64 count matrix on the host (every bin, halo included)."""
+        flat = np.empty(self.N * self.T, dtype=np.int64)
+        self.ctx.check(self.ctx.lib.nhp_disc_download(self.ctx.h, self.h, _ptr(flat)))
+        return flat.reshape(self.T, self.N).T.copy()  # data[n + N*t] -> [n, t]
+
+    def events_count(self):
+        """Events in the handle's own bins (nhp_disc_events_count)."""
+        return int(self.ctx.lib.nhp_disc_events_count(self.h))
+
     def free(self):
         self._fin()
 
@@ -109,6 +128,11 @@ class DiscreteHawkesProcess:
 
     def upload(self, data):
         return data if isinstance(data, DiscreteData) else DiscreteData(self._ctx(), data)
+
+    def effective_weights(self):
+        """e[p, c] = [A]W[p, c] sum_b theta[p, c, b] sum_l phi_b[l] dt: the expected children on node c of one event on node p."""
+        W = self.weights.W if self.adjacency_matrix is None else self.adjacency_matrix * self.weights.W
+        return W * np.einsum("pcb,b->pc", self.impulses.theta, self.impulses.basis().sum(axis=0) * self.dt)
 
     def _ready(self, data):
         d = self.upload(data)
@@ -416,3 +440,45 @@ def vb_device_(process, data, max_steps=100, rtol=None):
         ctx.check(ctx.lib.nhp_disc_vb_trace_free(ctx.h))
     set_variational_params_(process, out[-1])
     return list(out)
+
+
+# ------------------------------------------------------------------------------------------
+# rand: on the device (nhp_disc_rand) or on the host (discrete.jl:20-38; sequential over bins, kept for small samples and as an
+# independent check of the device one)
+# ------------------------------------------------------------------------------------------
+def rand_device(process, T, seed=0, max_events=None):
+    """`rand(process, T)` simulated on the GPU: an N x T sample with the law `loglikelihood` evaluates, left on the device as
+    DiscreteData (`.download()` gives the N x T int64 matrix).  Deterministic in (parameters, T, nlags, seed)."""
+    ctx = process._ctx()
+    process._push(ctx)
+    N, T = process.ndims(), int(T)
+    if max_events is None:  # stationary mean (I - e^T)^-1 lambda0 dt T with head room
+        e, l0 = process.effective_weights(), process.baseline.lam * process.dt
+        rad = float(np.max(np.sum(e, axis=1))) if N else 0.0
+        mean = float(np.sum(l0)) * T / max(1.0 - min(rad, 0.95), 0.05)
+        if 0 < N <= 2048:  # the exact mean where it is cheap: the row-sum bound misses non-normal e (a chain of strong links)
+            m = np.linalg.solve(np.eye(N) - e.T, l0)
+            if np.all(np.isfinite(m)) and np.all(m >= 0):  # a non-negative solution: spectral radius of e below 1
+                mean = max(mean, float(np.sum(m)) * T)
+        max_events = int(min(2.1e9, 2.0 * mean + 10.0 * np.sqrt(mean) + 1000))
+    h = ctypes.c_void_p()
+    ctx.check(ctx.lib.nhp_disc_rand(ctx.h, T, process.impulses.nlags, int(seed), int(max_events), ctypes.byref(h)))
+    return DiscreteData.from_handle(ctx, h, N, T)
+
+
+def rand(process, T, rng=None):
+    """`rand(process, T)` on the host: bin by bin, data[:, t] ~ Poisson(lambda[t, :]) given the earlier bins, with lambda as `intensity`
+    computes it (lambda0 dt + sum over lags l = 1..L of data[:, t - l] @ ([A]W theta phi[l] dt)).  Returns the N x T int64 matrix."""
+    rng = rng or np.random.default_rng()
+    N, T = process.ndims(), int(T)
+    W = process.weights.W if process.adjacency_matrix is None else process.adjacency_matrix * process.weights.W
+    phi = process.impulses.basis()  # [l, b]
+    L = phi.shape[0]
+    ir = np.einsum("pcb,lb->lpc", W[:, :, None] * process.impulses.theta, phi) * process.dt  # ir[l - 1, p, c]
+    base = process.baseline.lam * process.dt
+    data = np.zeros((N, T), dtype=np.int64)
+    for t in range(T):
+        w = min(L, t)
+        lam = base + np.einsum("pl,lpc->c", data[:, t - w:t][:, ::-1], ir[:w]) if w else base
+        data[:, t] = rng.poisson(lam)
+    return data
