@@ -378,6 +378,17 @@ int nhp_disc_vb_get(nhp_ctx *ctx, double *q);
  * (NHP_ERR_UNSUPPORTED); no state or no convolution (NHP_ERR_STATE); N or B of the state not those of dd (NHP_ERR_INVALID); an open
  * VB trace whose slot size is not the state's (NHP_ERR_STATE). */
 int nhp_disc_vb_step(nhp_ctx *ctx, nhp_disc *dd, double *change);
+/* One step of stochastic variational inference (Hoffman et al. 2013; the reference's `svi!`, inference.jl:183-190, is an empty stub)
+ * on the state of nhp_disc_vb_set, from the window of n_bins bins (t_begin + j) mod T, j = 0 .. n_bins - 1, of the T bins of dd; a
+ * window may wrap around the end, so with t_begin uniform on [0, T) every bin is in it with probability n_bins / T and the scaled
+ * statistics are unbiased.  With s = T / n_bins and the statistics of nhp_disc_vb_stats over the window's bins only (the convolution
+ * still covers the whole series, so the window's responsibilities are exact), the targets are alphav* = alpha0 + s alpha_sum,
+ * betav* = 1/beta0 + T dt (the full-data value, unscaled), gammav* = gamma + s gamma_sum, kappav* = kappa + s kappa_sum, nuv* = nu + s
+ * (events of the parent node in the window), and in place q = (1 - step) q + step q*; then a push to the VB trace while it has room.
+ * t_begin = 0, n_bins = T, step = 1 is the arithmetic of nhp_disc_vb_step.  The kernels visit only the window's non-zero bins.  change
+ * (may be NULL) as for nhp_disc_vb_step.  Refused before anything changes, as nhp_disc_vb_step, and also: a window outside
+ * 0 <= t_begin < T, 1 <= n_bins <= T, or step outside (0, 1] or not finite (NHP_ERR_INVALID). */
+int nhp_disc_svi_step(nhp_ctx *ctx, nhp_disc *dd, int64_t t_begin, int64_t n_bins, double step, double *change);
 /* Device-side trace of the VB state, independent of the Gibbs traces: one slot is q (2 N + N*N*(B + 2) doubles, laid out for the
  * state at _begin); _read copies slots [first, first + count) one after the other. */
 int nhp_disc_vb_trace_begin(nhp_ctx *ctx, int64_t capacity);

@@ -985,13 +985,23 @@ __global__ void __launch_bounds__(256) k_disc_gibbs(const double *__restrict__ c
     }
 }
 
-// VB: Z = e0_c + sum_k convT[t,k] ET[c][k];  alpha_sum[c] += s e0_c / Z;  gamma[c][k] += s convT[t,k] ET[c][k] / Z
+// first index in [lo, hi) of a child's time-sorted non-zero bins with nz_t >= t (hi if none)
+__device__ __forceinline__ int nz_lower_bound(const int *__restrict__ nz_t, int lo, int hi, int t) {
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (nz_t[mid] < t) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+// VB: Z = e0_c + sum_k convT[t,k] ET[c][k];  alpha_sum[c] += s e0_c / Z;  gamma[c][k] += s convT[t,k] ET[c][k] / Z over the bins
+// t_lo <= t < t_hi, the child's share split into `slabs` equal slabs
 __global__ void __launch_bounds__(256) k_disc_vb(const double *__restrict__ convT, const double *__restrict__ ET, const double *__restrict__ e0, int N, int NB,
                                                  const int *__restrict__ nz_t, const int *__restrict__ nz_s, const int *__restrict__ child_ptr, int slabs,
-                                                 double *__restrict__ alpha_sum, double *__restrict__ gammaT /* [c][k] */) {
+                                                 int t_lo, int t_hi, double *__restrict__ alpha_sum, double *__restrict__ gammaT /* [c][k] */) {
     __shared__ double red[8];
     const int c = blockIdx.x / slabs, slab = blockIdx.x % slabs;
-    const int e0i = child_ptr[c], e1 = child_ptr[c + 1];
+    const int e0i = nz_lower_bound(nz_t, child_ptr[c], child_ptr[c + 1], t_lo), e1 = nz_lower_bound(nz_t, e0i, child_ptr[c + 1], t_hi);
     const int per = (e1 - e0i + slabs - 1) / slabs;
     const int b0 = e0i + slab * per, b1 = min(e1, b0 + per);
     const double *et = ET + (int64_t)c * NB;
@@ -1030,14 +1040,7 @@ __global__ void __launch_bounds__(256) k_disc_vb(const double *__restrict__ conv
 // Work decomposition of the warp-per-bin kernels: CTA = (time block, child).  All children of a time block are resident
 // together (blockIdx.x = block * N + child), so the block's conv rows are fetched from HBM once and served from L2 to
 // the other children (the earlier (child, slab) split streamed every row once per child: 63 GB of DRAM reads at
-// config 3 against 9.6 GB of rows).  A child's bins are time-sorted, so its share of a block is a binary search.
-__device__ __forceinline__ int nz_lower_bound(const int *__restrict__ nz_t, int lo, int hi, int t) {
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (nz_t[mid] < t) lo = mid + 1; else hi = mid;
-    }
-    return lo;
-}
+// config 3 against 9.6 GB of rows).  A child's bins are time-sorted, so its share of a block is a binary search (nz_lower_bound).
 
 // Gibbs: the warp stores the NB weights of a bin in its shared-memory buffer, every lane sums a contiguous chunk,
 // a warp scan of the chunk sums gives the cdf at chunk granularity, and the lane owning the target walks its chunk.
@@ -1106,16 +1109,17 @@ __global__ void __launch_bounds__(256) k_disc_gibbs_warp(const double *__restric
     }
 }
 
-// VB: Z and the gamma accumulators per warp; the child's exp-expectation row is shared by the CTA.
+// VB: Z and the gamma accumulators per warp; the child's exp-expectation row is shared by the CTA.  Time block blk covers the bins
+// [t_lo + blk tb, t_lo + (blk + 1) tb) of the range [t_lo, t_hi).
 __global__ void __launch_bounds__(256) k_disc_vb_warp(const double *__restrict__ convT, const double *__restrict__ ET, const double *__restrict__ e0, int N, int NB,
                                                       const int *__restrict__ nz_t, const int *__restrict__ nz_s, const int *__restrict__ child_ptr, int tb,
-                                                      double *__restrict__ alpha_sum, double *__restrict__ gammaT) {
+                                                      int t_lo, int t_hi, double *__restrict__ alpha_sum, double *__restrict__ gammaT) {
     extern __shared__ double s_buf[];  // [NB] ET row | [8][NB] per-warp accumulators
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     double *et = s_buf, *acc = s_buf + NB + (size_t)warp * NB;
     const int c = blockIdx.x % N, blk = blockIdx.x / N;
-    const int ei0 = child_ptr[c], e1 = child_ptr[c + 1];
-    const int b0 = nz_lower_bound(nz_t, ei0, e1, blk * tb), b1 = nz_lower_bound(nz_t, b0, e1, (blk + 1) * tb);
+    const int ei0 = child_ptr[c], e1 = child_ptr[c + 1], lo = t_lo + blk * tb;
+    const int b0 = nz_lower_bound(nz_t, ei0, e1, lo), b1 = nz_lower_bound(nz_t, b0, e1, min(lo + tb, t_hi));
     if (b0 == b1) return;  // block-uniform
     for (int k = threadIdx.x; k < NB; k += 256) et[k] = ET[(int64_t)c * NB + k];
     for (int k = lane; k < NB; k += 32) acc[k] = 0.0;
@@ -1240,24 +1244,59 @@ __global__ void k_vb_finish(const double *__restrict__ gammaT, const double *__r
     nu[p + (int64_t)N * c] = rowsum[p];
 }
 
-// responsibilities + reductions of one VB step into zeroed alpha_sum[N] and gammaT[c][p*B+b]: the warp-per-bin kernel when its
-// buffers fit shared memory (and NHP_DISC_WARP is not 0), the block kernel otherwise; nothing to do without non-zero bins
-int nhp_disc_vb_reduce(nhp_ctx *ctx, nhp_disc *dd, const double *e0, const double *ET, double *alpha_sum, double *gammaT) {
+// responsibilities + reductions of one VB step over the bins t_lo <= t < t_hi into zeroed alpha_sum[N] and gammaT[c][p*B+b] (the
+// sums accumulate, so a range split in two is two calls): the warp-per-bin kernel when its buffers fit shared memory (and
+// NHP_DISC_WARP is not 0), the block kernel otherwise; nothing to do without non-zero bins.  A range shorter than the series takes
+// time blocks short enough that its CTAs fill the SMs once, and the slabs of the share of non-zero bins it expects, so the cost of
+// a window scales with the window.
+int nhp_disc_vb_reduce(nhp_ctx *ctx, nhp_disc *dd, int64_t t_lo, int64_t t_hi, const double *e0, const double *ET, double *alpha_sum, double *gammaT) {
     DiscExtra *ex = extra_of(dd);
-    if (ex->nnz == 0) return NHP_OK;
+    const int64_t n = t_hi - t_lo;
+    if (ex->nnz == 0 || n <= 0) return NHP_OK;
     const int64_t N = dd->N, NB = N * dd->B;
+    const bool window = n < dd->T;
     cudaStream_t s = ctx->stream;
     const size_t wsmem = (size_t)9 * NB * sizeof(double);
     const char *envw = getenv("NHP_DISC_WARP");
     if (wsmem <= (size_t)ctx->smem_optin - 4096 && !(envw && atoi(envw) == 0)) {
         DCUDA(ctx, cudaFuncSetAttribute(k_disc_vb_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
-        const int tb = pick_time_block(ctx, dd, ex->nnz);
-        const int64_t nblk = (dd->T + tb - 1) / tb;
-        k_disc_vb_warp<<<(unsigned)(N * nblk), 256, wsmem, s>>>(dd->d_conv, ET, e0, (int)N, (int)NB, ex->nz_t, ex->nz_s, ex->child_ptr, tb, alpha_sum, gammaT);
+        int tb = pick_time_block(ctx, dd, ex->nnz);
+        if (window) {
+            int per_sm = 1;
+            DCUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_disc_vb_warp, 256, wsmem));
+            const int64_t want = ((int64_t)ctx->sm_count * std::max(per_sm, 1) + N - 1) / N;  // time blocks of one full wave
+            tb = (int)std::min<int64_t>(tb, std::max<int64_t>(32, (n + want - 1) / want));
+        }
+        const int64_t nblk = (n + tb - 1) / tb;
+        k_disc_vb_warp<<<(unsigned)(N * nblk), 256, wsmem, s>>>(dd->d_conv, ET, e0, (int)N, (int)NB, ex->nz_t, ex->nz_s, ex->child_ptr, tb, (int)t_lo, (int)t_hi,
+                                                                 alpha_sum, gammaT);
     } else {
-        const int slabs = pick_slabs(ctx, N, ex->nnz);
-        k_disc_vb<<<(unsigned)(N * slabs), 256, 0, s>>>(dd->d_conv, ET, e0, (int)N, (int)NB, ex->nz_t, ex->nz_s, ex->child_ptr, slabs, alpha_sum, gammaT);
+        const int slabs = pick_slabs(ctx, N, window ? ex->nnz * n / dd->T : ex->nnz);
+        k_disc_vb<<<(unsigned)(N * slabs), 256, 0, s>>>(dd->d_conv, ET, e0, (int)N, (int)NB, ex->nz_t, ex->nz_s, ex->child_ptr, slabs, (int)t_lo, (int)t_hi,
+                                                        alpha_sum, gammaT);
     }
+    NHP_LAUNCHED(ctx);
+    return NHP_OK;
+}
+
+// events[p] += sum of data[p, t] over t_lo <= t < t_hi: one warp per node, a binary search into its time-sorted non-zero bins and a sum
+// of their counts
+__global__ void __launch_bounds__(256) k_disc_range_events(const int *__restrict__ nz_t, const int *__restrict__ nz_s, const int *__restrict__ child_ptr, int N,
+                                                           int t_lo, int t_hi, double *__restrict__ events) {
+    const int p = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (p >= N) return;  // warp-uniform
+    const int b0 = nz_lower_bound(nz_t, child_ptr[p], child_ptr[p + 1], t_lo), b1 = nz_lower_bound(nz_t, b0, child_ptr[p + 1], t_hi);
+    long long sum = 0;
+    for (int e = b0 + lane; e < b1; e += 32) sum += nz_s[e];
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, d);
+    if (lane == 0) events[p] += (double)sum;
+}
+
+int nhp_disc_range_events(nhp_ctx *ctx, nhp_disc *dd, int64_t t_lo, int64_t t_hi, double *events) {
+    DiscExtra *ex = extra_of(dd);
+    if (ex->nnz == 0 || t_hi <= t_lo) return NHP_OK;
+    k_disc_range_events<<<(unsigned)((dd->N + 7) / 8), 256, 0, ctx->stream>>>(ex->nz_t, ex->nz_s, ex->child_ptr, (int)dd->N, (int)t_lo, (int)t_hi, events);
     NHP_LAUNCHED(ctx);
     return NHP_OK;
 }
@@ -1284,7 +1323,7 @@ extern "C" int nhp_disc_vb_stats(nhp_ctx *ctx, nhp_disc *dd, const double *e0, c
     k_transpose_E<<<eb, 256, 0, s>>>(d_E, (int)N, (int)B, d_ET);
     NHP_LAUNCHED(ctx);
     NHP_TRY(nhp_timer_begin(ctx));
-    NHP_TRY(nhp_disc_vb_reduce(ctx, dd, d_e0, d_ET, d_alpha, d_gT));
+    NHP_TRY(nhp_disc_vb_reduce(ctx, dd, 0, dd->T, d_e0, d_ET, d_alpha, d_gT));
     k_vb_finish<<<(unsigned)((N * N + 255) / 256), 256, 0, s>>>(d_gT, ex->rowsum, (int)N, (int)B, d_kappa, d_nu, d_gamma);
     NHP_LAUNCHED(ctx);
     DCUDA(ctx, cudaGetLastError());

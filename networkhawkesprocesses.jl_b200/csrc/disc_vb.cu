@@ -5,7 +5,12 @@
 // One step: k_vb_expect turns q into the exp-expectations e0[c] and ET[c][p*B + b] (the statistics kernels' layout, so there is no
 // transpose), nhp_disc_vb_reduce runs the responsibilities and reductions of nhp_disc_vb_stats, k_vb_update writes the new q in place
 // and reduces the largest relative change.  Only that scalar crosses PCIe.
+//
+// Stochastic VI (Hoffman et al. 2013; the reference's `svi!` is an empty stub) runs the same step on a window of n of the T bins,
+// (t_begin + j) mod T for j < n: the statistics of the window only, scaled by s = T / n, give the target q*, and q moves to
+// (1 - step) q + step q*.  The VB step is the window of all T bins with (s, step) = (1, 1), which is the plain update bit for bit.
 #include "nhp_internal.cuh"
+#include <algorithm>
 #include <cmath>
 
 static size_t vb_q_doubles(int64_t N, int64_t B) { return (size_t)(2 * N) + (size_t)(N * N) * (size_t)(B + 2); }
@@ -29,13 +34,16 @@ __global__ void __launch_bounds__(256) k_vb_expect(const double *__restrict__ q,
 
 __device__ __forceinline__ double rel_change(double nw, double old) { return fabs(nw - old) / old; }
 
-// in place, one thread per (p, c) (+ alphav, betav for e < N):
-//   gammav = gamma + g,  kappav = kappa + sum_b g (b = 0 .. B-1, as k_vb_finish),  nuv = nu + rowsum[p],  alphav = alpha0 + alpha_sum,
-//   betav = betav_new (1/beta0 + T dt, computed on the host);  change = max |new - old| / old over all of q (bit order of non-negative
-//   doubles is their numeric order: an integer atomicMax per warp)
+__device__ __forceinline__ double blend(double old, double target, double step) { return (1.0 - step) * old + step * target; }
+
+// in place, one thread per (p, c) (+ alphav, betav for e < N), the targets
+//   gammav* = gamma + s g,  kappav* = kappa + s sum_b g (b = 0 .. B-1, as k_vb_finish),  nuv* = nu + s events[p],
+//   alphav* = alpha0 + s alpha_sum,  betav* = betav_new (1/beta0 + T dt, computed on the host, unscaled)
+// blended as q = (1 - step) q + step q*;  change = max |new - old| / old over all of q (bit order of non-negative doubles is their
+// numeric order: an integer atomicMax per warp)
 __global__ void __launch_bounds__(256) k_vb_update(double *__restrict__ q, const double *__restrict__ gammaT, const double *__restrict__ alpha_sum,
-                                                   const double *__restrict__ rowsum, int N, int B, double alpha0, double betav_new, double kappa,
-                                                   double nu, double gamma, unsigned long long *__restrict__ change) {
+                                                   const double *__restrict__ events, int N, int B, double alpha0, double betav_new, double kappa,
+                                                   double nu, double gamma, double s, double step, unsigned long long *__restrict__ change) {
     const int64_t NN = (int64_t)N * N;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     double mx = 0.0;
@@ -47,19 +55,19 @@ __global__ void __launch_bounds__(256) k_vb_update(double *__restrict__ q, const
         for (int b = 0; b < B; b++) {
             const double gb = g[b];
             ks += gb;
-            const double nw = gamma + gb;
-            mx = fmax(mx, rel_change(nw, gv[e + NN * b]));
+            const double old = gv[e + NN * b], nw = blend(old, gamma + s * gb, step);
+            mx = fmax(mx, rel_change(nw, old));
             gv[e + NN * b] = nw;
         }
-        const double kn = kappa + ks, nn = nu + rowsum[e % N];
+        const double kn = blend(kv[e], kappa + s * ks, step), nn = blend(nv[e], nu + s * events[e % N], step);
         mx = fmax(mx, fmax(rel_change(kn, kv[e]), rel_change(nn, nv[e])));
         kv[e] = kn;
         nv[e] = nn;
         if (e < N) {
-            const double an = alpha0 + alpha_sum[e];
-            mx = fmax(mx, fmax(rel_change(an, q[e]), rel_change(betav_new, q[N + e])));
+            const double an = blend(q[e], alpha0 + s * alpha_sum[e], step), bn = blend(q[N + e], betav_new, step);
+            mx = fmax(mx, fmax(rel_change(an, q[e]), rel_change(bn, q[N + e])));
             q[e] = an;
-            q[N + e] = betav_new;
+            q[N + e] = bn;
         }
     }
 #pragma unroll
@@ -103,32 +111,47 @@ extern "C" int nhp_disc_vb_get(nhp_ctx *ctx, double *q) {
     return NHP_OK;
 }
 
-extern "C" int nhp_disc_vb_step(nhp_ctx *ctx, nhp_disc *dd, double *change) {
+// One step over the window (t_begin + j) mod T, j < n_bins, blended with `step`; the refusals come before anything changes.  The window
+// of all T bins uses the events per node kept with the data, a shorter one counts them in its ranges.
+static int vb_window_step(nhp_ctx *ctx, nhp_disc *dd, const char *fn, int64_t t_begin, int64_t n_bins, double step, double *change) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, dd != nullptr, NHP_ERR_INVALID, "nhp_disc_vb_step: data handle is NULL");
-    NHP_CHECK(ctx, dd->t_halo == 0, NHP_ERR_UNSUPPORTED, "nhp_disc_vb_step works on unsharded data");
-    NHP_CHECK(ctx, !(ctx->comm && ctx->nranks > 1), NHP_ERR_UNSUPPORTED, "nhp_disc_vb_step runs on one GPU (the context has a communicator of %d ranks)", ctx->nranks);
-    NHP_CHECK(ctx, ctx->dv_set, NHP_ERR_STATE, "nhp_disc_vb_step: no VB state (call nhp_disc_vb_set)");
-    NHP_CHECK(ctx, dd->d_conv != nullptr, NHP_ERR_STATE, "nhp_disc_vb_step: call nhp_disc_convolve first");
-    const int64_t N = ctx->dv_N, B = ctx->dv_B, NN = N * N, NB = N * B;
-    NHP_CHECK(ctx, dd->N == N && dd->B == B, NHP_ERR_INVALID, "nhp_disc_vb_step: the VB state has N=%lld B=%lld, the data N=%lld B=%lld", (long long)N,
+    NHP_CHECK(ctx, dd != nullptr, NHP_ERR_INVALID, "%s: data handle is NULL", fn);
+    NHP_CHECK(ctx, dd->t_halo == 0, NHP_ERR_UNSUPPORTED, "%s works on unsharded data", fn);
+    NHP_CHECK(ctx, !(ctx->comm && ctx->nranks > 1), NHP_ERR_UNSUPPORTED, "%s runs on one GPU (the context has a communicator of %d ranks)", fn, ctx->nranks);
+    NHP_CHECK(ctx, ctx->dv_set, NHP_ERR_STATE, "%s: no VB state (call nhp_disc_vb_set)", fn);
+    NHP_CHECK(ctx, dd->d_conv != nullptr, NHP_ERR_STATE, "%s: call nhp_disc_convolve first", fn);
+    const int64_t N = ctx->dv_N, B = ctx->dv_B, NN = N * N, NB = N * B, T = dd->T;
+    NHP_CHECK(ctx, dd->N == N && dd->B == B, NHP_ERR_INVALID, "%s: the VB state has N=%lld B=%lld, the data N=%lld B=%lld", fn, (long long)N,
               (long long)B, (long long)dd->N, (long long)dd->B);
     NHP_CHECK(ctx, ctx->dv_trace_cap == 0 || (ctx->dv_trace_N == N && ctx->dv_trace_B == B), NHP_ERR_STATE,
-              "nhp_disc_vb_step: the open VB trace was begun for N=%lld B=%lld", (long long)ctx->dv_trace_N, (long long)ctx->dv_trace_B);
+              "%s: the open VB trace was begun for N=%lld B=%lld", fn, (long long)ctx->dv_trace_N, (long long)ctx->dv_trace_B);
+    NHP_CHECK(ctx, t_begin >= 0 && t_begin < T && n_bins >= 1 && n_bins <= T, NHP_ERR_INVALID,
+              "%s: window (t_begin=%lld, n_bins=%lld) outside 0 <= t_begin < T, 1 <= n_bins <= T (T=%lld)", fn, (long long)t_begin, (long long)n_bins, (long long)T);
+    NHP_CHECK(ctx, step > 0.0 && step <= 1.0, NHP_ERR_INVALID, "%s: step=%g outside (0, 1]", fn, step);
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
     void *scratch;
-    // layout: e0[N] | ET[N*NB] | gammaT[N*NB] | alpha_sum[N] | change (the last three zeroed together)
-    NHP_TRY(nhp_scratch(ctx, (size_t)(2 * N + 2 * NB * N + 1) * sizeof(double), &scratch));
-    double *d_e0 = (double *)scratch, *d_ET = d_e0 + N, *d_gT = d_ET + NB * N, *d_alpha = d_gT + NB * N, *d_change = d_alpha + N;
-    NHP_CUDA(ctx, cudaMemsetAsync(d_gT, 0, (size_t)(NB * N + N + 1) * sizeof(double), s));
+    // layout: e0[N] | ET[N*NB] | gammaT[N*NB] | alpha_sum[N] | events[N] | change (the last four zeroed together)
+    NHP_TRY(nhp_scratch(ctx, (size_t)(3 * N + 2 * NB * N + 1) * sizeof(double), &scratch));
+    double *d_e0 = (double *)scratch, *d_ET = d_e0 + N, *d_gT = d_ET + NB * N, *d_alpha = d_gT + NB * N, *d_events = d_alpha + N, *d_change = d_events + N;
+    NHP_CUDA(ctx, cudaMemsetAsync(d_gT, 0, (size_t)(NB * N + 2 * N + 1) * sizeof(double), s));
     const unsigned blocks = (unsigned)((NN + 255) / 256);
     k_vb_expect<<<blocks, 256, 0, s>>>(ctx->dv_q, (int)N, (int)B, d_e0, d_ET);
     NHP_LAUNCHED(ctx);
-    NHP_TRY(nhp_disc_vb_reduce(ctx, dd, d_e0, d_ET, d_alpha, d_gT));
+    // the window as at most two ranges [t_begin, end) and, when it wraps, [0, t_begin + n_bins - T)
+    const int64_t end = std::min(t_begin + n_bins, T), wrap = t_begin + n_bins - end;
+    NHP_TRY(nhp_disc_vb_reduce(ctx, dd, t_begin, end, d_e0, d_ET, d_alpha, d_gT));
+    NHP_TRY(nhp_disc_vb_reduce(ctx, dd, 0, wrap, d_e0, d_ET, d_alpha, d_gT));
+    const double *events = nhp_disc_rowsum(dd);
+    if (n_bins < T) {
+        NHP_TRY(nhp_disc_range_events(ctx, dd, t_begin, end, d_events));
+        NHP_TRY(nhp_disc_range_events(ctx, dd, 0, wrap, d_events));
+        events = d_events;
+    }
     const double *h = ctx->dv_hyper;
-    const double betav = 1.0 / h[1] + (double)dd->T * ctx->dv_dt;  // baselines.jl:450 as written (1 / beta0, not beta0)
-    k_vb_update<<<blocks, 256, 0, s>>>(ctx->dv_q, d_gT, d_alpha, nhp_disc_rowsum(dd), (int)N, (int)B, h[0], betav, h[2], h[3], h[4],
+    const double betav = 1.0 / h[1] + (double)T * ctx->dv_dt;  // baselines.jl:450 as written (1 / beta0, not beta0)
+    const double scale = (double)T / (double)n_bins;
+    k_vb_update<<<blocks, 256, 0, s>>>(ctx->dv_q, d_gT, d_alpha, events, (int)N, (int)B, h[0], betav, h[2], h[3], h[4], scale, step,
                                        (unsigned long long *)d_change);
     NHP_LAUNCHED(ctx);
     NHP_CUDA(ctx, cudaGetLastError());
@@ -142,6 +165,14 @@ extern "C" int nhp_disc_vb_step(nhp_ctx *ctx, nhp_disc *dd, double *change) {
         NHP_CUDA(ctx, cudaStreamSynchronize(s));
     }
     return NHP_OK;
+}
+
+extern "C" int nhp_disc_vb_step(nhp_ctx *ctx, nhp_disc *dd, double *change) {
+    return vb_window_step(ctx, dd, "nhp_disc_vb_step", 0, dd ? dd->T : 1, 1.0, change);
+}
+
+extern "C" int nhp_disc_svi_step(nhp_ctx *ctx, nhp_disc *dd, int64_t t_begin, int64_t n_bins, double step, double *change) {
+    return vb_window_step(ctx, dd, "nhp_disc_svi_step", t_begin, n_bins, step, change);
 }
 
 extern "C" int nhp_disc_vb_trace_free(nhp_ctx *ctx) {

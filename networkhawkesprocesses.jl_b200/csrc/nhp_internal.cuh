@@ -344,6 +344,8 @@ int nhp_disc_from_device(nhp_ctx *ctx, int *d_data, int64_t N, int64_t T, int64_
 // discrete chain pieces shared between translation units
 int nhp_disc_tables_refresh(nhp_ctx *ctx);        // disc.cu: bump table, compact parent lists, density, sum of A from the device-resident parameters
 const double *nhp_disc_rowsum(nhp_disc *dd);      // disc.cu: [N] events per node (device)
-int nhp_disc_vb_reduce(nhp_ctx *ctx, nhp_disc *dd, const double *e0, const double *ET, double *alpha_sum, double *gammaT);  // disc.cu: VB statistics into zeroed sums
+// disc.cu: VB statistics of the bins t_lo <= t < t_hi added into zeroed sums; the events of each node over those bins added into events[N]
+int nhp_disc_vb_reduce(nhp_ctx *ctx, nhp_disc *dd, int64_t t_lo, int64_t t_hi, const double *e0, const double *ET, double *alpha_sum, double *gammaT);
+int nhp_disc_range_events(nhp_ctx *ctx, nhp_disc *dd, int64_t t_lo, int64_t t_hi, double *events);
 int nhp_disc_draw_params(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, uint64_t counter, const double *d_Mn, const double *hyper);  // cont_conjugate.cu
 int nhp_disc_draw_network(nhp_ctx *ctx, uint64_t seed, uint64_t counter, double alpha, double beta);  // cont_conjugate.cu: ctx->dd_rho ~ Beta

@@ -712,4 +712,40 @@ function vb_on_device!(process::DiscreteStandardHawkesProcess, data; max_steps=1
     return trace
 end
 
+# Stochastic variational inference (the reference's `svi!`, inference.jl:183-190, is an empty stub) with the loop and its trace on
+# the device, modelled on vb_on_device!: step s = 1 … nsteps is one nhp_disc_svi_step on the batch_bins bins (t + j) mod T from a
+# t uniform on 0 … T-1 (a window may wrap around the end, which keeps the scaled statistics unbiased), with step size (s + τ0)^(-κ);
+# it moves the state to (1 - step) q + step q*, q* being the VB update from the window's statistics scaled by T / batch_bins.  The
+# windows come from Julia's own RNG, so a run does not reproduce the Python svi_device_ bit for bit.  Returns the trace, one
+# variational_params vector per step; the process holds the last one.
+function svi_on_device!(process::DiscreteStandardHawkesProcess, data; nsteps, batch_bins, τ0=1.0, κ=0.75)
+    T = size(data, 2)
+    1 <= batch_bins <= T || throw(ArgumentError("batch_bins = $batch_bins outside 1 … T = $T"))
+    0.5 < κ <= 1 || throw(ArgumentError("κ = $κ outside (0.5, 1]"))
+    (τ0 >= 0 && isfinite(τ0)) || throw(ArgumentError("τ0 = $τ0 must be finite and >= 0"))
+    nsteps >= 0 || throw(ArgumentError("nsteps = $nsteps is negative"))
+    nsteps == 0 && return Vector{Vector{Float64}}()
+    d = device_counts(data)
+    ensure_convolved!(process, d)
+    b, w, imp = process.baseline, process.weights, process.impulses
+    N = ndims(process); B = size(imp.θ, 3)
+    q = Vector{Float64}(NetworkHawkesProcesses.variational_params(process))
+    hyper = Float64[b.α0, b.β0, w.κ, w.ν, imp.γ]
+    check(ccall((:nhp_disc_vb_set, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, Float64, Ptr{Float64}, Cint, Ptr{Float64}),
+        CTX[], N, B, process.dt, hyper, length(hyper), q))
+    check(ccall((:nhp_disc_vb_trace_begin, LIB[]), Cint, (Ptr{Cvoid}, Int64), CTX[], nsteps))
+    for s in 1:nsteps
+        check(ccall((:nhp_disc_svi_step, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Int64, Int64, Float64, Ptr{Float64}), CTX[], d.h,
+            rand(0:T-1), batch_bins, (s + τ0)^(-κ), C_NULL))
+    end
+    Q = Matrix{Float64}(undef, length(q), nsteps)
+    check(ccall((:nhp_disc_vb_trace_read, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}), CTX[], 0, nsteps, Q))
+    check(ccall((:nhp_disc_vb_trace_free, LIB[]), Cint, (Ptr{Cvoid},), CTX[]))
+    trace = [Q[:, k] for k in 1:nsteps]
+    last = trace[end]; o = 2N + N * N * B
+    b.αv = last[1:N]; b.βv = last[N+1:2N]
+    imp.γv = reshape(last[2N+1:o], N, N, B); w.κv = reshape(last[o+1:o+N*N], N, N); w.νv = reshape(last[o+N*N+1:end], N, N)
+    return trace
+end
+
 end # module

@@ -114,6 +114,7 @@ PROTOTYPES = {
     "nhp_disc_vb_set": (c_int, [c_void_p, c_int64, c_int64, c_double, c_void_p, c_int, c_void_p]),
     "nhp_disc_vb_get": (c_int, [c_void_p, c_void_p]),
     "nhp_disc_vb_step": (c_int, [c_void_p, c_void_p, c_double_p]),
+    "nhp_disc_svi_step": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_double, c_double_p]),
     "nhp_disc_vb_trace_begin": (c_int, [c_void_p, c_int64]),
     "nhp_disc_vb_trace_count": (c_int, [c_void_p, POINTER(c_int64), POINTER(c_int64)]),
     "nhp_disc_vb_trace_read": (c_int, [c_void_p, c_int64, c_int64, c_void_p]),

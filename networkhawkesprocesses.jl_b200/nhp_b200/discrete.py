@@ -5,7 +5,8 @@
   functions   basis, convolve, intensity, loglikelihood, resample_parents (reduced over t: counts[c, k]),
               update_ (one VB step, discrete.jl:369-375), resample_ (one Gibbs sweep, discrete.jl:361-367 / 416-424),
               resample_adjacency_matrix_, mcmc_, mcmc_device_ (the chain and its trace on the device), vb_, vb_device_ (the VB loop
-              and its trace on the device), rand (host) and rand_device (nhp_disc_rand: the sample stays on the device)
+              and its trace on the device), svi_schedule and svi_device_ (stochastic VI over windows of bins, on the device),
+              rand (host) and rand_device (nhp_disc_rand: the sample stays on the device)
 `data` is an N x T integer matrix (numpy row = node) as in the reference; arrays indexed theta[p, c, b].
 """
 import ctypes
@@ -401,22 +402,11 @@ def set_variational_params_(process, q):
     w.nuv = q[o + N * N:].reshape(N, N).T.copy()
 
 
-def vb_device_(process, data, max_steps=100, rtol=None):
-    """`vb!` (inference.jl:153-181) with the loop and its trace on the device.  The variational parameters (kappav / nuv initialised
-    as update_ does) and the hyper-parameters go up once (nhp_disc_vb_set); each step is one nhp_disc_vb_step, the `update!` of
-    discrete.jl:369-375 with digamma on the device, which appends the new state to the device-side VB trace; the trace comes back
-    in one read.  Without `rtol` it runs max_steps steps, as vb_.  With `rtol` it stops after the first step whose largest relative
-    change of any variational parameter, max_i |q_new[i] - q_old[i]| / q_old[i], is <= rtol: a criterion of this package, since the
-    reference's own convergence test is commented out (inference.jl:163-176).  Returns the list of variational_params vectors, one
-    per step, as vb_; the process holds the last state.  A network process raises ValueError: the reference's update! for it is
-    non-functional (quirk Q10)."""
-    if isinstance(process, DiscreteNetworkHawkesProcess):
-        raise ValueError("vb_device_: the reference's update! of a DiscreteNetworkHawkesProcess is non-functional (quirk Q10); "
-                         "VB runs on DiscreteStandardHawkesProcess")
+def _vb_device_run(process, d, nsteps, step):
+    """The device VB loop shared by vb_device_ and svi_device_: the variational parameters (kappav / nuv initialised as update_ does)
+    and the hyper-parameters go up once (nhp_disc_vb_set), the trace is open for nsteps slots, step(ctx, k) runs step k and returns
+    True to stop after it; the trace comes back in one read and the process holds the last state."""
     ctx = process._ctx()
-    d = process._ready(data)
-    if max_steps < 1:
-        return []
     b, w, imp = process.baseline, process.weights, process.impulses
     if not hasattr(w, "kappav"):
         w.kappav, w.nuv = np.ones_like(w.W), np.ones_like(w.W)
@@ -426,13 +416,13 @@ def vb_device_(process, data, max_steps=100, rtol=None):
         raise ValueError("variational parameter shapes do not match the data's number of nodes")
     hy = np.array([b.alpha0, b.beta0, w.kappa, w.nu, imp.gamma], dtype=np.float64)
     ctx.check(ctx.lib.nhp_disc_vb_set(ctx.h, N, B, process.dt, _ptr(hy), hy.size, _ptr(q)))
-    ctx.check(ctx.lib.nhp_disc_vb_trace_begin(ctx.h, int(max_steps)))
+    ctx.check(ctx.lib.nhp_disc_vb_trace_begin(ctx.h, int(nsteps)))
     try:
-        change, steps = ctypes.c_double(), 0
-        for _ in range(max_steps):
-            ctx.check(ctx.lib.nhp_disc_vb_step(ctx.h, d.h, None if rtol is None else ctypes.byref(change)))
+        steps = 0
+        for k in range(nsteps):
+            stop = step(ctx, k)
             steps += 1
-            if rtol is not None and change.value <= rtol:
+            if stop:
                 break
         out = np.empty((steps, q.size))
         ctx.check(ctx.lib.nhp_disc_vb_trace_read(ctx.h, 0, steps, _ptr(out)))
@@ -440,6 +430,84 @@ def vb_device_(process, data, max_steps=100, rtol=None):
         ctx.check(ctx.lib.nhp_disc_vb_trace_free(ctx.h))
     set_variational_params_(process, out[-1])
     return list(out)
+
+
+def _refuse_network(process, name):
+    if isinstance(process, DiscreteNetworkHawkesProcess):
+        raise ValueError(f"{name}: the reference's update! of a DiscreteNetworkHawkesProcess is non-functional (quirk Q10); "
+                         "VB runs on DiscreteStandardHawkesProcess")
+
+
+def vb_device_(process, data, max_steps=100, rtol=None):
+    """`vb!` (inference.jl:153-181) with the loop and its trace on the device.  The variational parameters (kappav / nuv initialised
+    as update_ does) and the hyper-parameters go up once (nhp_disc_vb_set); each step is one nhp_disc_vb_step, the `update!` of
+    discrete.jl:369-375 with digamma on the device, which appends the new state to the device-side VB trace; the trace comes back
+    in one read.  Without `rtol` it runs max_steps steps, as vb_.  With `rtol` it stops after the first step whose largest relative
+    change of any variational parameter, max_i |q_new[i] - q_old[i]| / q_old[i], is <= rtol: a criterion of this package, since the
+    reference's own convergence test is commented out (inference.jl:163-176).  Returns the list of variational_params vectors, one
+    per step, as vb_; the process holds the last state.  A network process raises ValueError: the reference's update! for it is
+    non-functional (quirk Q10)."""
+    _refuse_network(process, "vb_device_")
+    d = process._ready(data)
+    if max_steps < 1:
+        return []
+    change = ctypes.c_double()
+
+    def step(ctx, k):
+        ctx.check(ctx.lib.nhp_disc_vb_step(ctx.h, d.h, None if rtol is None else ctypes.byref(change)))
+        return rtol is not None and change.value <= rtol
+
+    return _vb_device_run(process, d, max_steps, step)
+
+
+def _whole(x, name):
+    if isinstance(x, (bool, np.bool_)) or not float(x).is_integer():
+        raise ValueError(f"{name} must be an integer, got {x!r}")
+    return int(x)
+
+
+def svi_schedule(T, nsteps, batch_bins, tau0=1.0, kappa=0.75, seed=0):
+    """The windows and step sizes of stochastic VI (Hoffman et al. 2013) over T bins: t_begin[k] uniform on [0, T) (an int64 array
+    from np.random.default_rng(seed)) and step[k] = (k + 1 + tau0)^(-kappa) for the steps k = 0 .. nsteps - 1, so the first step is
+    at most 1 and the steps satisfy sum step = inf, sum step^2 < inf.  Window k covers the batch_bins bins (t_begin[k] + j) mod T; it
+    wraps around the end, which keeps every bin's chance of being in it at batch_bins / T.  Checks, with ValueError and before anything
+    else: T >= 1, 1 <= batch_bins <= T, 0.5 < kappa <= 1, tau0 >= 0, nsteps >= 0."""
+    T, nsteps, batch_bins = _whole(T, "T"), _whole(nsteps, "nsteps"), _whole(batch_bins, "batch_bins")
+    if T < 1:
+        raise ValueError(f"svi_schedule: T = {T} bins; need at least one")
+    if not 1 <= batch_bins <= T:
+        raise ValueError(f"svi_schedule: batch_bins = {batch_bins} outside [1, T = {T}]")
+    if not 0.5 < kappa <= 1.0:
+        raise ValueError(f"svi_schedule: kappa = {kappa} outside (0.5, 1]")
+    if not tau0 >= 0.0 or not np.isfinite(tau0):
+        raise ValueError(f"svi_schedule: tau0 = {tau0} must be finite and >= 0")
+    if nsteps < 0:
+        raise ValueError(f"svi_schedule: nsteps = {nsteps} is negative")
+    t_begin = np.random.default_rng(seed).integers(0, T, size=nsteps, dtype=np.int64)
+    step = (np.arange(1, nsteps + 1, dtype=np.float64) + float(tau0)) ** (-float(kappa))
+    return t_begin, step
+
+
+def svi_device_(process, data, nsteps, batch_bins, tau0=1.0, kappa=0.75, seed=0):
+    """Stochastic variational inference (the reference's `svi!`, inference.jl:183-190, is an empty stub) with the loop and its trace
+    on the device, shaped like vb_device_: the state goes up once, step k is one nhp_disc_svi_step on the window (t_begin[k],
+    batch_bins) with step size step[k] of svi_schedule(T, nsteps, batch_bins, tau0, kappa, seed), and the trace comes back in one read.
+    Each step reads only the window's bins and moves q to (1 - step) q + step q*, where q* is the VB update from the window's
+    statistics scaled by T / batch_bins.  Returns the list of variational_params vectors, one per step; the process holds the last
+    state.  Bad schedule arguments and a network process (quirk Q10) raise ValueError before any device call."""
+    T = data.T if isinstance(data, DiscreteData) else np.shape(data)[1]
+    t_begin, steps = svi_schedule(T, nsteps, batch_bins, tau0, kappa, seed)
+    _refuse_network(process, "svi_device_")
+    d = process._ready(data)
+    if nsteps < 1:
+        return []
+    n = int(batch_bins)
+
+    def step(ctx, k):
+        ctx.check(ctx.lib.nhp_disc_svi_step(ctx.h, d.h, int(t_begin[k]), n, float(steps[k]), None))
+        return False
+
+    return _vb_device_run(process, d, nsteps, step)
 
 
 # ------------------------------------------------------------------------------------------
