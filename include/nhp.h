@@ -389,8 +389,31 @@ int nhp_disc_vb_step(nhp_ctx *ctx, nhp_disc *dd, double *change);
  * (may be NULL) as for nhp_disc_vb_step.  Refused before anything changes, as nhp_disc_vb_step, and also: a window outside
  * 0 <= t_begin < T, 1 <= n_bins <= T, or step outside (0, 1] or not finite (NHP_ERR_INVALID). */
 int nhp_disc_svi_step(nhp_ctx *ctx, nhp_disc *dd, int64_t t_begin, int64_t n_bins, double step, double *change);
-/* Device-side trace of the VB state, independent of the Gibbs traces: one slot is q (2 N + N*N*(B + 2) doubles, laid out for the
- * state at _begin); _read copies slots [first, first + count) one after the other. */
+/* Mean-field VB of a discrete network process with a BernoulliNetworkModel (the reference's update! for it, discrete.jl:494-502,
+ * is non-functional, quirk Q10).  A true spike W = A W' gives E[ln W] = -inf whenever q(A=1) < 1, so the model is a Gamma mixture:
+ * A[p,c] ~ Bernoulli(rho), rho ~ Beta(alpha_rho, beta_rho), W | A=1 ~ Gamma(kappa, nu) (the slab), W | A=0 ~ Gamma(kappa0, nu0) (the
+ * spike), lambda0 and theta as for the standard process, W entering the intensity directly.  The state extends the standard layout:
+ * q = [alphav(N); betav(N); gammav(N*N*B); kappav(N*N); nuv(N*N); kappa0v(N*N); nu0v(N*N); pv(N*N); alpharhov; betarhov]
+ * (2 N + N*N*(B + 5) + 2 doubles), with q(W | A=1) = Gamma(kappav, nuv), q(W | A=0) = Gamma(kappa0v, nu0v), pv[p + N*c] = q(A[p,c] = 1),
+ * q(rho) = Beta(alpharhov, betarhov); hyper = [alpha0, beta0, kappa, nu, gamma, kappa0, nu0, alpha_rho, beta_rho] (n_hyper = 9).
+ * _network_set validates (every hyper-parameter and every entry of q finite and > 0, except pv: in [0, 1]; dt > 0; otherwise
+ * NHP_ERR_INVALID and the kept state is as it was) and keeps a state of network kind; nhp_disc_vb_set keeps a standard one, and the
+ * later of the two calls decides the kind.  nhp_disc_vb_get, nhp_disc_vb_step, nhp_disc_svi_step and the VB trace work on either.
+ * On a network state a step over the window (s = T / n_bins; the VB step is s = 1, step = 1) takes the expectations from the old q,
+ * with E[ln W] = pv (psi(kappav) - ln nuv) + (1 - pv) (psi(kappa0v) - ln nu0v), and the statistics of nhp_disc_vb_stats; with
+ * G = s sum_b gamma_sum[p,c,b] and E = s (events of p in the window), the targets are those of the standard step, kappa0v* = kappa0 + G,
+ * nu0v* = nu0 + E, and
+ *   logit pv* = psi(alpharhov) - psi(betarhov) + [lgamma(kappav*) - lgamma(kappa) + kappa ln nu - kappav* ln nuv*]
+ *                                              - [lgamma(kappa0v*) - lgamma(kappa0) + kappa0 ln nu0 - kappa0v* ln nu0v*]
+ * (the log marginal likelihoods of the link's statistics under slab and spike), then with S = sum of pv* (a fixed-order two-stage
+ * sum: the same state and statistics give the same bits) alpharhov* = alpha_rho + S, betarhov* = beta_rho + N*N - S (unscaled: N*N
+ * counts links).  Every entry moves to (1 - step) q + step q* in place; then a push to the VB trace while it has room.  change = the
+ * largest of |new - old| / old over the positive entries and |new - old| over pv.  Refusals as for the standard steps; a step on an
+ * open VB trace begun for the other kind of state is NHP_ERR_STATE. */
+int nhp_disc_vb_network_set(nhp_ctx *ctx, int64_t N, int64_t B, double dt, const double *hyper, int n_hyper, const double *q);
+/* Device-side trace of the VB state, independent of the Gibbs traces: one slot is q (2 N + N*N*(B + 2) doubles for a standard state,
+ * 2 N + N*N*(B + 5) + 2 for a network state, laid out for the state at _begin); _read copies slots [first, first + count) one after
+ * the other. */
 int nhp_disc_vb_trace_begin(nhp_ctx *ctx, int64_t capacity);
 int nhp_disc_vb_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity);
 int nhp_disc_vb_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *q_out);

@@ -9,11 +9,20 @@
 // Stochastic VI (Hoffman et al. 2013; the reference's `svi!` is an empty stub) runs the same step on a window of n of the T bins,
 // (t_begin + j) mod T for j < n: the statistics of the window only, scaled by s = T / n, give the target q*, and q moves to
 // (1 - step) q + step q*.  The VB step is the window of all T bins with (s, step) = (1, 1), which is the plain update bit for bit.
+//
+// A network state (nhp_disc_vb_network_set) fits the Gamma mixture W | A=1 ~ Gamma(kappa, nu), W | A=0 ~ Gamma(kappa0, nu0),
+// A ~ Bernoulli(rho), rho ~ Beta(alpha_rho, beta_rho) with the factors q(W | A=1) = Gamma(kappav, nuv), q(W | A=0) = Gamma(kappa0v,
+// nu0v), q(A=1) = pv, q(rho) = Beta(alpharhov, betarhov) appended to q.  The step reuses nhp_disc_vb_reduce as it is: k_vbn_expect
+// adds the mixture E[ln W] to the expectations, k_vbn_update writes the per-link targets and block sums of the new q(A=1), and
+// k_vbn_finish adds those sums in a fixed order into q(rho).
 #include "nhp_internal.cuh"
 #include <algorithm>
 #include <cmath>
 
 static size_t vb_q_doubles(int64_t N, int64_t B) { return (size_t)(2 * N) + (size_t)(N * N) * (size_t)(B + 2); }
+// the network state: the standard layout, then kappa0v(N^2); nu0v(N^2); pv(N^2); alpharhov; betarhov
+static size_t vbn_q_doubles(int64_t N, int64_t B) { return (size_t)(2 * N) + (size_t)(N * N) * (size_t)(B + 5) + 2; }
+static size_t vb_state_doubles(int64_t N, int64_t B, bool network) { return network ? vbn_q_doubles(N, B) : vb_q_doubles(N, B); }
 
 // one thread per (p, c), e = p + N c: B + 2 digammas; threads e < N also write e0[e]
 //   e0[c]             = exp(psi(alphav[c]) - log betav[c])                                       baselines.jl:454-456
@@ -75,17 +84,136 @@ __global__ void __launch_bounds__(256) k_vb_update(double *__restrict__ q, const
     if ((threadIdx.x & 31) == 0 && mx > 0.0) atomicMax(change, (unsigned long long)__double_as_longlong(mx));
 }
 
-extern "C" int nhp_disc_vb_set(nhp_ctx *ctx, int64_t N, int64_t B, double dt, const double *hyper, int n_hyper, const double *q) {
+// the network state, one thread per link e = p + N c: as k_vb_expect with the mixture
+//   E[ln W[p,c]] = pv (psi(kappav) - log nuv) + (1 - pv) (psi(kappa0v) - log nu0v)
+// in place of psi(kappav) - log nuv; thread 0 also writes lrho = psi(alpharhov) - psi(betarhov), the prior log-odds of a link
+__global__ void __launch_bounds__(256) k_vbn_expect(const double *__restrict__ q, int N, int B, double *__restrict__ e0, double *__restrict__ ET,
+                                                    double *__restrict__ lrho) {
+    const int64_t NN = (int64_t)N * N;
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= NN) return;
+    const double *gv = q + 2 * N, *kv = gv + NN * B, *nv = kv + NN, *k0v = nv + NN, *n0v = k0v + NN, *pv = n0v + NN;
+    if (e < N) e0[e] = exp(nhp_digamma(q[e]) - log(q[N + e]));
+    if (e == 0) *lrho = nhp_digamma(pv[NN]) - nhp_digamma(pv[NN + 1]);
+    const double p = pv[e];
+    const double lw = p * (nhp_digamma(kv[e]) - log(nv[e])) + (1.0 - p) * (nhp_digamma(k0v[e]) - log(n0v[e]));
+    double S = 0.0;
+    for (int b = 0; b < B; b++) S += gv[e + NN * b];
+    const double psiS = nhp_digamma(S);
+    double *out = ET + e * B;
+    for (int b = 0; b < B; b++) out[b] = exp((nhp_digamma(gv[e + NN * b]) - psiS) + lw);
+}
+
+// 1 / (1 + exp(-x)) without overflow for either sign of x
+__device__ __forceinline__ double stable_sigmoid(double x) {
+    if (x >= 0.0) return 1.0 / (1.0 + exp(-x));
+    const double z = exp(x);
+    return z / (1.0 + z);
+}
+
+// the network state in place, one thread per link (+ alphav, betav for e < N); with ks = sum_b g (b = 0 .. B-1) and E = events[p]
+//   gammav* = gamma + s g,  kappav* = kappa + s ks,  nuv* = nu + s E,  kappa0v* = kappa0 + s ks,  nu0v* = nu0 + s E,
+//   alphav* = alpha0 + s alpha_sum,  betav* = betav_new,
+//   pv* = sigmoid(lrho + [lgamma(kappav*) - kappav* log nuv*] - [lgamma(kappa0v*) - kappa0v* log nu0v*] + cprior)
+// where cprior = [kappa log nu - lgamma(kappa)] - [kappa0 log nu0 - lgamma(kappa0)] (the brackets are the log marginal likelihoods of
+// the link's statistics under slab and spike), blended as q = (1 - step) q + step q*.  Each block writes the sum of its pv* to
+// psum[blockIdx.x] (a fixed shuffle tree, then the warps in order); change = max of |new - old| / old over the positive entries and
+// |new - old| over pv, which may be exactly 0 or 1
+__global__ void __launch_bounds__(256) k_vbn_update(double *__restrict__ q, const double *__restrict__ gammaT, const double *__restrict__ alpha_sum,
+                                                    const double *__restrict__ events, const double *__restrict__ lrho, int N, int B, double alpha0,
+                                                    double betav_new, double kappa, double nu, double gamma, double kappa0, double nu0, double cprior,
+                                                    double s, double step, unsigned long long *__restrict__ change, double *__restrict__ psum) {
+    __shared__ double warp_sum[8];
+    const int64_t NN = (int64_t)N * N;
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    double mx = 0.0, pt = 0.0;
+    if (e < NN) {
+        double *gv = q + 2 * N, *kv = gv + NN * B, *nv = kv + NN, *k0v = nv + NN, *n0v = k0v + NN, *pv = n0v + NN;
+        const double *g = gammaT + e * B;
+        double ks = 0.0;
+#pragma unroll 1  // as k_vb_update
+        for (int b = 0; b < B; b++) {
+            const double gb = g[b];
+            ks += gb;
+            const double old = gv[e + NN * b], nw = blend(old, gamma + s * gb, step);
+            mx = fmax(mx, rel_change(nw, old));
+            gv[e + NN * b] = nw;
+        }
+        const double ev = s * events[e % N];
+        const double k1 = kappa + s * ks, n1 = nu + ev, k0 = kappa0 + s * ks, n0 = nu0 + ev;
+        pt = stable_sigmoid(*lrho + (lgamma(k1) - k1 * log(n1)) - (lgamma(k0) - k0 * log(n0)) + cprior);
+        const double kn = blend(kv[e], k1, step), nn = blend(nv[e], n1, step);
+        const double k0n = blend(k0v[e], k0, step), n0n = blend(n0v[e], n0, step), pn = blend(pv[e], pt, step);
+        mx = fmax(mx, fmax(rel_change(kn, kv[e]), rel_change(nn, nv[e])));
+        mx = fmax(mx, fmax(rel_change(k0n, k0v[e]), rel_change(n0n, n0v[e])));
+        mx = fmax(mx, fabs(pn - pv[e]));
+        kv[e] = kn; nv[e] = nn; k0v[e] = k0n; n0v[e] = n0n; pv[e] = pn;
+        if (e < N) {
+            const double an = blend(q[e], alpha0 + s * alpha_sum[e], step), bn = blend(q[N + e], betav_new, step);
+            mx = fmax(mx, fmax(rel_change(an, q[e]), rel_change(bn, q[N + e])));
+            q[e] = an;
+            q[N + e] = bn;
+        }
+    }
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) {
+        mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
+        pt += __shfl_xor_sync(0xffffffffu, pt, d);
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (mx > 0.0) atomicMax(change, (unsigned long long)__double_as_longlong(mx));
+        warp_sum[threadIdx.x >> 5] = pt;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = 0.0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += warp_sum[w];
+        psum[blockIdx.x] = t;
+    }
+}
+
+// one block of 256: S = sum of the nblocks partial sums in a fixed order, then alpharhov* = alpha_rho + S, betarhov* = beta_rho + N^2 - S
+// (N^2 counts links, not data: never scaled), blended, their relative change folded into change
+__global__ void __launch_bounds__(256) k_vbn_finish(double *__restrict__ rho, const double *__restrict__ psum, int nblocks, double alpha_rho,
+                                                    double beta_rho, double links, double step, unsigned long long *__restrict__ change) {
+    __shared__ double sh[256];
+    double a = 0.0;
+    for (int i = threadIdx.x; i < nblocks; i += 256) a += psum[i];
+    sh[threadIdx.x] = a;
+    __syncthreads();
+    for (int w = 128; w > 0; w >>= 1) {
+        if ((int)threadIdx.x < w) sh[threadIdx.x] += sh[threadIdx.x + w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        const double S = sh[0];
+        const double an = blend(rho[0], alpha_rho + S, step), bn = blend(rho[1], (beta_rho + links) - S, step);
+        const double mx = fmax(rel_change(an, rho[0]), rel_change(bn, rho[1]));
+        rho[0] = an;
+        rho[1] = bn;
+        if (mx > 0.0) atomicMax(change, (unsigned long long)__double_as_longlong(mx));
+    }
+}
+
+// the two set calls: every entry of hyper positive and finite; every entry of q positive and finite except, for a network state,
+// pv (finite, in [0, 1]); refused before anything changes
+static int vb_set_state(nhp_ctx *ctx, const char *fn, bool network, int64_t N, int64_t B, double dt, const double *hyper, int n_hyper, const double *q) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, N >= 1 && N <= 32768 && B >= 1, NHP_ERR_INVALID, "nhp_disc_vb_set: bad dimensions N=%lld B=%lld", (long long)N, (long long)B);
-    NHP_CHECK(ctx, hyper != nullptr && q != nullptr, NHP_ERR_INVALID, "nhp_disc_vb_set: NULL argument");
-    NHP_CHECK(ctx, n_hyper == 5, NHP_ERR_INVALID, "nhp_disc_vb_set: expected 5 hyper-parameters, got %d", n_hyper);
-    NHP_CHECK(ctx, dt > 0.0 && std::isfinite(dt), NHP_ERR_INVALID, "nhp_disc_vb_set: dt must be positive and finite");
+    NHP_CHECK(ctx, N >= 1 && N <= 32768 && B >= 1, NHP_ERR_INVALID, "%s: bad dimensions N=%lld B=%lld", fn, (long long)N, (long long)B);
+    NHP_CHECK(ctx, hyper != nullptr && q != nullptr, NHP_ERR_INVALID, "%s: NULL argument", fn);
+    const int want = network ? 9 : 5;
+    NHP_CHECK(ctx, n_hyper == want, NHP_ERR_INVALID, "%s: expected %d hyper-parameters, got %d", fn, want, n_hyper);
+    NHP_CHECK(ctx, dt > 0.0 && std::isfinite(dt), NHP_ERR_INVALID, "%s: dt must be positive and finite", fn);
     for (int i = 0; i < n_hyper; i++)
-        NHP_CHECK(ctx, hyper[i] > 0.0 && std::isfinite(hyper[i]), NHP_ERR_INVALID, "nhp_disc_vb_set: hyper-parameter %d must be positive and finite", i);
-    const size_t n = vb_q_doubles(N, B);
-    for (size_t i = 0; i < n; i++)
-        NHP_CHECK(ctx, q[i] > 0.0 && std::isfinite(q[i]), NHP_ERR_INVALID, "nhp_disc_vb_set: q[%zu] = %g is not positive and finite", i, q[i]);
+        NHP_CHECK(ctx, hyper[i] > 0.0 && std::isfinite(hyper[i]), NHP_ERR_INVALID, "%s: hyper-parameter %d must be positive and finite", fn, i);
+    const size_t n = vb_state_doubles(N, B, network);
+    const size_t p_lo = network ? (size_t)(2 * N) + (size_t)(N * N) * (size_t)(B + 4) : n, p_hi = network ? p_lo + (size_t)(N * N) : n;
+    for (size_t i = 0; i < n; i++) {
+        if (i >= p_lo && i < p_hi)
+            NHP_CHECK(ctx, q[i] >= 0.0 && q[i] <= 1.0, NHP_ERR_INVALID, "%s: q[%zu] = %g is a link probability outside [0, 1]", fn, i, q[i]);
+        else
+            NHP_CHECK(ctx, q[i] > 0.0 && std::isfinite(q[i]), NHP_ERR_INVALID, "%s: q[%zu] = %g is not positive and finite", fn, i, q[i]);
+    }
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     if (ctx->dv_cap < n) {
         NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -95,10 +223,18 @@ extern "C" int nhp_disc_vb_set(nhp_ctx *ctx, int64_t N, int64_t B, double dt, co
     }
     NHP_CUDA(ctx, cudaMemcpyAsync(ctx->dv_q, q, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the caller may reuse q after return
-    ctx->dv_N = N; ctx->dv_B = B; ctx->dv_dt = dt;
-    for (int i = 0; i < 5; i++) ctx->dv_hyper[i] = hyper[i];
+    ctx->dv_N = N; ctx->dv_B = B; ctx->dv_dt = dt; ctx->dv_network = network;
+    for (int i = 0; i < n_hyper; i++) ctx->dv_hyper[i] = hyper[i];
     ctx->dv_set = true;
     return NHP_OK;
+}
+
+extern "C" int nhp_disc_vb_set(nhp_ctx *ctx, int64_t N, int64_t B, double dt, const double *hyper, int n_hyper, const double *q) {
+    return vb_set_state(ctx, "nhp_disc_vb_set", false, N, B, dt, hyper, n_hyper, q);
+}
+
+extern "C" int nhp_disc_vb_network_set(nhp_ctx *ctx, int64_t N, int64_t B, double dt, const double *hyper, int n_hyper, const double *q) {
+    return vb_set_state(ctx, "nhp_disc_vb_network_set", true, N, B, dt, hyper, n_hyper, q);
 }
 
 extern "C" int nhp_disc_vb_get(nhp_ctx *ctx, double *q) {
@@ -106,7 +242,7 @@ extern "C" int nhp_disc_vb_get(nhp_ctx *ctx, double *q) {
     NHP_CHECK(ctx, ctx->dv_set, NHP_ERR_STATE, "nhp_disc_vb_get: no VB state (call nhp_disc_vb_set)");
     NHP_CHECK(ctx, q != nullptr, NHP_ERR_INVALID, "nhp_disc_vb_get: NULL argument");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    NHP_CUDA(ctx, cudaMemcpyAsync(q, ctx->dv_q, vb_q_doubles(ctx->dv_N, ctx->dv_B) * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    NHP_CUDA(ctx, cudaMemcpyAsync(q, ctx->dv_q, vb_state_doubles(ctx->dv_N, ctx->dv_B, ctx->dv_network) * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return NHP_OK;
 }
@@ -125,18 +261,27 @@ static int vb_window_step(nhp_ctx *ctx, nhp_disc *dd, const char *fn, int64_t t_
               (long long)B, (long long)dd->N, (long long)dd->B);
     NHP_CHECK(ctx, ctx->dv_trace_cap == 0 || (ctx->dv_trace_N == N && ctx->dv_trace_B == B), NHP_ERR_STATE,
               "%s: the open VB trace was begun for N=%lld B=%lld", fn, (long long)ctx->dv_trace_N, (long long)ctx->dv_trace_B);
+    NHP_CHECK(ctx, ctx->dv_trace_cap == 0 || ctx->dv_trace_network == ctx->dv_network, NHP_ERR_STATE, "%s: the open VB trace was begun for a %s state",
+              fn, ctx->dv_trace_network ? "network" : "standard");
     NHP_CHECK(ctx, t_begin >= 0 && t_begin < T && n_bins >= 1 && n_bins <= T, NHP_ERR_INVALID,
               "%s: window (t_begin=%lld, n_bins=%lld) outside 0 <= t_begin < T, 1 <= n_bins <= T (T=%lld)", fn, (long long)t_begin, (long long)n_bins, (long long)T);
     NHP_CHECK(ctx, step > 0.0 && step <= 1.0, NHP_ERR_INVALID, "%s: step=%g outside (0, 1]", fn, step);
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
     void *scratch;
-    // layout: e0[N] | ET[N*NB] | gammaT[N*NB] | alpha_sum[N] | events[N] | change (the last four zeroed together)
-    NHP_TRY(nhp_scratch(ctx, (size_t)(3 * N + 2 * NB * N + 1) * sizeof(double), &scratch));
-    double *d_e0 = (double *)scratch, *d_ET = d_e0 + N, *d_gT = d_ET + NB * N, *d_alpha = d_gT + NB * N, *d_events = d_alpha + N, *d_change = d_events + N;
-    NHP_CUDA(ctx, cudaMemsetAsync(d_gT, 0, (size_t)(NB * N + 2 * N + 1) * sizeof(double), s));
+    const bool net = ctx->dv_network;
     const unsigned blocks = (unsigned)((NN + 255) / 256);
-    k_vb_expect<<<blocks, 256, 0, s>>>(ctx->dv_q, (int)N, (int)B, d_e0, d_ET);
+    // layout: e0[N] | ET[N*NB] | gammaT[N*NB] | alpha_sum[N] | events[N] | change (the last four zeroed together), and for a network
+    // state | lrho | psum[blocks]
+    const size_t extra = net ? 1 + (size_t)blocks : 0;
+    NHP_TRY(nhp_scratch(ctx, (size_t)(3 * N + 2 * NB * N + 1 + extra) * sizeof(double), &scratch));
+    double *d_e0 = (double *)scratch, *d_ET = d_e0 + N, *d_gT = d_ET + NB * N, *d_alpha = d_gT + NB * N, *d_events = d_alpha + N, *d_change = d_events + N;
+    double *d_lrho = d_change + 1, *d_psum = d_lrho + 1;
+    NHP_CUDA(ctx, cudaMemsetAsync(d_gT, 0, (size_t)(NB * N + 2 * N + 1) * sizeof(double), s));
+    if (net)
+        k_vbn_expect<<<blocks, 256, 0, s>>>(ctx->dv_q, (int)N, (int)B, d_e0, d_ET, d_lrho);
+    else
+        k_vb_expect<<<blocks, 256, 0, s>>>(ctx->dv_q, (int)N, (int)B, d_e0, d_ET);
     NHP_LAUNCHED(ctx);
     // the window as at most two ranges [t_begin, end) and, when it wraps, [0, t_begin + n_bins - T)
     const int64_t end = std::min(t_begin + n_bins, T), wrap = t_begin + n_bins - end;
@@ -151,12 +296,22 @@ static int vb_window_step(nhp_ctx *ctx, nhp_disc *dd, const char *fn, int64_t t_
     const double *h = ctx->dv_hyper;
     const double betav = 1.0 / h[1] + (double)T * ctx->dv_dt;  // baselines.jl:450 as written (1 / beta0, not beta0)
     const double scale = (double)T / (double)n_bins;
-    k_vb_update<<<blocks, 256, 0, s>>>(ctx->dv_q, d_gT, d_alpha, events, (int)N, (int)B, h[0], betav, h[2], h[3], h[4], scale, step,
+    if (net) {
+        const double cprior = (h[2] * std::log(h[3]) - std::lgamma(h[2])) - (h[5] * std::log(h[6]) - std::lgamma(h[5]));
+        k_vbn_update<<<blocks, 256, 0, s>>>(ctx->dv_q, d_gT, d_alpha, events, d_lrho, (int)N, (int)B, h[0], betav, h[2], h[3], h[4], h[5], h[6],
+                                            cprior, scale, step, (unsigned long long *)d_change, d_psum);
+        NHP_LAUNCHED(ctx);
+        k_vbn_finish<<<1, 256, 0, s>>>(ctx->dv_q + vbn_q_doubles(N, B) - 2, d_psum, (int)blocks, h[7], h[8], (double)NN, step,
                                        (unsigned long long *)d_change);
-    NHP_LAUNCHED(ctx);
+        NHP_LAUNCHED(ctx);
+    } else {
+        k_vb_update<<<blocks, 256, 0, s>>>(ctx->dv_q, d_gT, d_alpha, events, (int)N, (int)B, h[0], betav, h[2], h[3], h[4], scale, step,
+                                           (unsigned long long *)d_change);
+        NHP_LAUNCHED(ctx);
+    }
     NHP_CUDA(ctx, cudaGetLastError());
     if (ctx->dv_trace_cap > 0 && ctx->dv_trace_len < ctx->dv_trace_cap) {  // the state of this step stays on the device
-        const size_t n = vb_q_doubles(N, B);
+        const size_t n = vb_state_doubles(N, B, net);
         NHP_CUDA(ctx, cudaMemcpyAsync(ctx->dv_trace + (size_t)ctx->dv_trace_len * n, ctx->dv_q, n * sizeof(double), cudaMemcpyDeviceToDevice, s));
         ctx->dv_trace_len++;
     }
@@ -190,13 +345,14 @@ extern "C" int nhp_disc_vb_trace_begin(nhp_ctx *ctx, int64_t capacity) {
     NHP_CHECK(ctx, capacity >= 1, NHP_ERR_INVALID, "nhp_disc_vb_trace_begin: capacity must be positive");
     NHP_TRY(nhp_disc_vb_trace_free(ctx));
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = vb_q_doubles(ctx->dv_N, ctx->dv_B);
+    const size_t n = vb_state_doubles(ctx->dv_N, ctx->dv_B, ctx->dv_network);
     if (cudaMalloc(&ctx->dv_trace, (size_t)capacity * n * sizeof(double)) != cudaSuccess) {
         cudaGetLastError();
         ctx->dv_trace = nullptr;
         return nhp_fail(ctx, NHP_ERR_CUDA, "nhp_disc_vb_trace_begin: cannot allocate %lld slots of %.2f MB", (long long)capacity, 1e-6 * (double)(n * 8));
     }
     ctx->dv_trace_cap = capacity; ctx->dv_trace_len = 0; ctx->dv_trace_N = ctx->dv_N; ctx->dv_trace_B = ctx->dv_B;
+    ctx->dv_trace_network = ctx->dv_network;
     return NHP_OK;
 }
 
@@ -214,7 +370,7 @@ extern "C" int nhp_disc_vb_trace_read(nhp_ctx *ctx, int64_t first, int64_t count
     if (count == 0) return NHP_OK;
     NHP_CHECK(ctx, q_out != nullptr, NHP_ERR_INVALID, "nhp_disc_vb_trace_read: NULL argument");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = vb_q_doubles(ctx->dv_trace_N, ctx->dv_trace_B);
+    const size_t n = vb_state_doubles(ctx->dv_trace_N, ctx->dv_trace_B, ctx->dv_trace_network);
     NHP_CUDA(ctx, cudaMemcpyAsync(q_out, ctx->dv_trace + (size_t)first * n, (size_t)count * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return NHP_OK;

@@ -235,13 +235,14 @@ struct nhp_ctx {
     double *dd_trace = nullptr; uint32_t *dd_trace_bits = nullptr;
     int64_t dd_trace_cap = 0, dd_trace_len = 0, dd_trace_N = 0, dd_trace_B = 0; bool dd_trace_has_A = false;
 
-    // ---- discrete mean-field VB (disc_vb.cu): q = [alphav(N); betav(N); gammav(N^2 B); kappav(N^2); nuv(N^2)] and its trace
-    bool dv_set = false;
+    // ---- discrete mean-field VB (disc_vb.cu): q = [alphav(N); betav(N); gammav(N^2 B); kappav(N^2); nuv(N^2)] and its trace; a
+    // network state (dv_network) appends [kappa0v(N^2); nu0v(N^2); pv(N^2); alpharhov; betarhov]
+    bool dv_set = false, dv_network = false;
     int64_t dv_N = 0, dv_B = 0;
-    double dv_dt = 1.0, dv_hyper[5] = {0};  // alpha0, beta0, kappa, nu, gamma
+    double dv_dt = 1.0, dv_hyper[9] = {0};  // alpha0, beta0, kappa, nu, gamma (+ kappa0, nu0, alpha_rho, beta_rho for a network state)
     double *dv_q = nullptr; size_t dv_cap = 0;  // doubles allocated
-    double *dv_trace = nullptr;                 // [dv_trace_cap] slots of q for (dv_trace_N, dv_trace_B)
-    int64_t dv_trace_cap = 0, dv_trace_len = 0, dv_trace_N = 0, dv_trace_B = 0;
+    double *dv_trace = nullptr;                 // [dv_trace_cap] slots of q for (dv_trace_N, dv_trace_B, dv_trace_network)
+    int64_t dv_trace_cap = 0, dv_trace_len = 0, dv_trace_N = 0, dv_trace_B = 0; bool dv_trace_network = false;
 };
 
 // launch bookkeeping

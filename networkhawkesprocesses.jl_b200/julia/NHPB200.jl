@@ -748,4 +748,68 @@ function svi_on_device!(process::DiscreteStandardHawkesProcess, data; nsteps, ba
     return trace
 end
 
+# VB and SVI of a discrete network process with a BernoulliNetworkModel (the reference's update! for it, discrete.jl:494-502, is
+# non-functional, quirk Q10) on the device: the Gamma-mixture model of nhp_disc_vb_network_set (W | A=1 ~ Gamma(κ, ν), W | A=0 ~
+# Gamma(κ0, ν0), A ~ Bernoulli(ρ), ρ ~ Beta(α, β) of the network model).  The state is variational_params(process) followed by
+# [vec(κ0v); vec(ν0v); vec(pv); αρv; βρv]; the reference's structs have no fields for those factors, so they are kept per process in
+# NETWORK_VB and a later call resumes from them (first call: κ0v = κ0, ν0v = ν0, pv = ρ, q(ρ) = Beta(α, β)).  The methods return the
+# trace, one state vector per step, and set the fields the standard methods set.
+const NETWORK_VB = IdDict{Any,Vector{Float64}}()
+
+function network_vb_run!(process::DiscreteNetworkHawkesProcess, data, nsteps, κ0, ν0, step!)
+    (κ0 > 0 && isfinite(κ0) && ν0 > 0 && isfinite(ν0)) || throw(ArgumentError("κ0 = $κ0, ν0 = $ν0 must be positive and finite"))
+    net = process.network
+    net isa NetworkHawkesProcesses.BernoulliNetworkModel || throw(ArgumentError("network VB needs a BernoulliNetworkModel"))
+    d = device_counts(data)
+    ensure_convolved!(process, d)
+    b, w, imp = process.baseline, process.weights, process.impulses
+    N = ndims(process); B = size(imp.θ, 3)
+    extra = get(NETWORK_VB, process, vcat(fill(κ0, N * N), fill(ν0, N * N), fill(net.ρ, N * N), [net.α, net.β]))
+    q = vcat(b.αv, b.βv, vec(imp.γv), vec(w.κv), vec(w.νv), extra)
+    hyper = Float64[b.α0, b.β0, w.κ, w.ν, imp.γ, κ0, ν0, net.α, net.β]
+    check(ccall((:nhp_disc_vb_network_set, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, Float64, Ptr{Float64}, Cint, Ptr{Float64}),
+        CTX[], N, B, process.dt, hyper, length(hyper), q))
+    check(ccall((:nhp_disc_vb_trace_begin, LIB[]), Cint, (Ptr{Cvoid}, Int64), CTX[], nsteps))
+    steps = 0
+    for s in 1:nsteps
+        steps = s
+        step!(d, s) && break
+    end
+    Q = Matrix{Float64}(undef, length(q), steps)
+    check(ccall((:nhp_disc_vb_trace_read, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}), CTX[], 0, steps, Q))
+    check(ccall((:nhp_disc_vb_trace_free, LIB[]), Cint, (Ptr{Cvoid},), CTX[]))
+    trace = [Q[:, k] for k in 1:steps]
+    last = trace[end]; o = 2N + N * N * B
+    b.αv = last[1:N]; b.βv = last[N+1:2N]
+    imp.γv = reshape(last[2N+1:o], N, N, B); w.κv = reshape(last[o+1:o+N*N], N, N); w.νv = reshape(last[o+N*N+1:o+2N*N], N, N)
+    NETWORK_VB[process] = last[o+2N*N+1:end]
+    return trace
+end
+
+# `vb!` of a network process: every step is one nhp_disc_vb_step on the network state; `rtol` stops after the first step whose change
+# (relative over the positive entries, absolute over pv) is <= rtol.
+function vb_on_device!(process::DiscreteNetworkHawkesProcess, data; max_steps=100, rtol=nothing, κ0=0.1, ν0=10.0)
+    change = Ref{Float64}(0.0)
+    network_vb_run!(process, data, max_steps, κ0, ν0, (d, s) -> begin
+        check(ccall((:nhp_disc_vb_step, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}), CTX[], d.h,
+            rtol === nothing ? C_NULL : change))
+        rtol !== nothing && change[] <= rtol
+    end)
+end
+
+# `svi!` of a network process: the windows and step sizes of svi_on_device!, each step one nhp_disc_svi_step on the network state.
+function svi_on_device!(process::DiscreteNetworkHawkesProcess, data; nsteps, batch_bins, τ0=1.0, κ=0.75, κ0=0.1, ν0=10.0)
+    T = size(data, 2)
+    1 <= batch_bins <= T || throw(ArgumentError("batch_bins = $batch_bins outside 1 … T = $T"))
+    0.5 < κ <= 1 || throw(ArgumentError("κ = $κ outside (0.5, 1]"))
+    (τ0 >= 0 && isfinite(τ0)) || throw(ArgumentError("τ0 = $τ0 must be finite and >= 0"))
+    nsteps >= 0 || throw(ArgumentError("nsteps = $nsteps is negative"))
+    nsteps == 0 && return Vector{Vector{Float64}}()
+    network_vb_run!(process, data, nsteps, κ0, ν0, (d, s) -> begin
+        check(ccall((:nhp_disc_svi_step, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Int64, Int64, Float64, Ptr{Float64}), CTX[], d.h,
+            rand(0:T-1), batch_bins, (s + τ0)^(-κ), C_NULL))
+        false
+    end)
+end
+
 end # module

@@ -113,6 +113,7 @@ PROTOTYPES = {
     "nhp_disc_gibbs_sweep": (c_int, [c_void_p, c_void_p, c_uint64, c_uint64, c_void_p, c_int, c_double, c_double]),
     "nhp_disc_vb_set": (c_int, [c_void_p, c_int64, c_int64, c_double, c_void_p, c_int, c_void_p]),
     "nhp_disc_vb_get": (c_int, [c_void_p, c_void_p]),
+    "nhp_disc_vb_network_set": (c_int, [c_void_p, c_int64, c_int64, c_double, c_void_p, c_int, c_void_p]),
     "nhp_disc_vb_step": (c_int, [c_void_p, c_void_p, c_double_p]),
     "nhp_disc_svi_step": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_double, c_double_p]),
     "nhp_disc_vb_trace_begin": (c_int, [c_void_p, c_int64]),

@@ -6,6 +6,8 @@
               update_ (one VB step, discrete.jl:369-375), resample_ (one Gibbs sweep, discrete.jl:361-367 / 416-424),
               resample_adjacency_matrix_, mcmc_, mcmc_device_ (the chain and its trace on the device), vb_, vb_device_ (the VB loop
               and its trace on the device), svi_schedule and svi_device_ (stochastic VI over windows of bins, on the device),
+              network_vb_device_ / network_svi_device_ (VB and SVI of a network process with a variational adjacency matrix, on
+              the device) and their host twin network_update_ / network_vb_targets,
               rand (host) and rand_device (nhp_disc_rand: the sample stays on the device)
 `data` is an N x T integer matrix (numpy row = node) as in the reference; arrays indexed theta[p, c, b].
 """
@@ -14,7 +16,7 @@ import time
 import weakref
 
 import numpy as np
-from scipy.special import digamma
+from scipy.special import digamma, gammaln
 
 from .continuous import BernoulliNetworkModel, DenseNetworkModel, DenseWeightModel  # noqa: F401
 from .core import _f64, _fmat, _ptr, default_context
@@ -402,20 +404,28 @@ def set_variational_params_(process, q):
     w.nuv = q[o + N * N:].reshape(N, N).T.copy()
 
 
-def _vb_device_run(process, d, nsteps, step):
-    """The device VB loop shared by vb_device_ and svi_device_: the variational parameters (kappav / nuv initialised as update_ does)
-    and the hyper-parameters go up once (nhp_disc_vb_set), the trace is open for nsteps slots, step(ctx, k) runs step k and returns
-    True to stop after it; the trace comes back in one read and the process holds the last state."""
+def _vb_device_run(process, d, nsteps, step, network=False):
+    """The device VB loop shared by vb_device_, svi_device_ and their network forms: the variational parameters (kappav / nuv
+    initialised as update_ does; for `network`, the state of network_variational_params) and the hyper-parameters go up once
+    (nhp_disc_vb_set, nhp_disc_vb_network_set), the trace is open for nsteps slots, step(ctx, k) runs step k and returns True to stop
+    after it; the trace comes back in one read and the process holds the last state."""
     ctx = process._ctx()
     b, w, imp = process.baseline, process.weights, process.impulses
-    if not hasattr(w, "kappav"):
-        w.kappav, w.nuv = np.ones_like(w.W), np.ones_like(w.W)
     N, B = d.N, imp.nbasis()
-    q = _f64(process.variational_params())
-    if q.size != 2 * N + N * N * (B + 2):
-        raise ValueError("variational parameter shapes do not match the data's number of nodes")
-    hy = np.array([b.alpha0, b.beta0, w.kappa, w.nu, imp.gamma], dtype=np.float64)
-    ctx.check(ctx.lib.nhp_disc_vb_set(ctx.h, N, B, process.dt, _ptr(hy), hy.size, _ptr(q)))
+    if network:
+        q = _f64(network_variational_params(process))
+        if q.size != _network_q_size(N, B):
+            raise ValueError("variational parameter shapes do not match the data's number of nodes")
+        hy = _network_hyper(process)
+        ctx.check(ctx.lib.nhp_disc_vb_network_set(ctx.h, N, B, process.dt, _ptr(hy), hy.size, _ptr(q)))
+    else:
+        if not hasattr(w, "kappav"):
+            w.kappav, w.nuv = np.ones_like(w.W), np.ones_like(w.W)
+        q = _f64(process.variational_params())
+        if q.size != 2 * N + N * N * (B + 2):
+            raise ValueError("variational parameter shapes do not match the data's number of nodes")
+        hy = np.array([b.alpha0, b.beta0, w.kappa, w.nu, imp.gamma], dtype=np.float64)
+        ctx.check(ctx.lib.nhp_disc_vb_set(ctx.h, N, B, process.dt, _ptr(hy), hy.size, _ptr(q)))
     ctx.check(ctx.lib.nhp_disc_vb_trace_begin(ctx.h, int(nsteps)))
     try:
         steps = 0
@@ -428,7 +438,7 @@ def _vb_device_run(process, d, nsteps, step):
         ctx.check(ctx.lib.nhp_disc_vb_trace_read(ctx.h, 0, steps, _ptr(out)))
     finally:
         ctx.check(ctx.lib.nhp_disc_vb_trace_free(ctx.h))
-    set_variational_params_(process, out[-1])
+    (set_network_variational_params_ if network else set_variational_params_)(process, out[-1])
     return list(out)
 
 
@@ -508,6 +518,191 @@ def svi_device_(process, data, nsteps, batch_bins, tau0=1.0, kappa=0.75, seed=0)
         return False
 
     return _vb_device_run(process, d, nsteps, step)
+
+
+# ------------------------------------------------------------------------------------------
+# VB and SVI of a network process.  W enters the intensity directly and has a Gamma mixture prior: W | A=1 ~ Gamma(kappa, nu) (the
+# slab: the weights model's kappa, nu), W | A=0 ~ Gamma(kappa0, nu0) (the spike, mean kappa0 / nu0), A[p,c] ~ Bernoulli(rho),
+# rho ~ Beta(alpha, beta) of the BernoulliNetworkModel.  A true spike W = 0 cannot be used: E[ln W] would be -inf wherever
+# q(A=1) < 1.  The factors: q(W | A=1) = Gamma(kappav, nuv), q(W | A=0) = Gamma(kappa0v, nu0v) (weights.kappa0v / nu0v),
+# q(A[p,c] = 1) = pv (network.pv), q(rho) = Beta(alphav, betav) (network.alphav / betav).
+# ------------------------------------------------------------------------------------------
+def _network_q_size(N, B):
+    return 2 * N + N * N * (B + 5) + 2
+
+
+def _spike(w):
+    return float(getattr(w, "kappa0", 0.1)), float(getattr(w, "nu0", 10.0))
+
+
+def _network_hyper(process):
+    """[alpha0, beta0, kappa, nu, gamma, kappa0, nu0, alpha_rho, beta_rho], the hyper-parameters of nhp_disc_vb_network_set."""
+    b, w, imp, net = process.baseline, process.weights, process.impulses, process.network
+    return np.array([b.alpha0, b.beta0, w.kappa, w.nu, imp.gamma, *_spike(w), net.alpha, net.beta], dtype=np.float64)
+
+
+def network_variational_params(process):
+    """The network VB state q = [alphav(N); betav(N); vec(gammav)(N*N*B); vec(kappav); vec(nuv); vec(kappa0v); vec(nu0v); vec(pv);
+    alpharhov; betarhov] (matrices column-major, [p + N c]): variational_params of the standard process followed by the spike,
+    the link probabilities and q(rho).  Missing factors start at kappav = nuv = 1 (as update_), kappa0v = kappa0, nu0v = nu0 (the
+    weights' spike hyper-parameters, default 0.1 and 10), pv = rho and q(rho) = Beta(alpha, beta).  adjacency_matrix, W and rho are
+    left as they are."""
+    b, w, imp, net = process.baseline, process.weights, process.impulses, process.network
+    N = process.ndims()
+    if not hasattr(w, "kappav"):
+        w.kappav, w.nuv = np.ones((N, N)), np.ones((N, N))
+    if not hasattr(w, "kappa0v"):
+        k0, n0 = _spike(w)
+        w.kappa0v, w.nu0v = np.full((N, N), k0), np.full((N, N), n0)
+    if not hasattr(net, "pv"):
+        net.pv = np.full((N, N), float(net.rho))
+    if not hasattr(net, "alphav"):
+        net.alphav, net.betav = float(net.alpha), float(net.beta)
+    f = lambda M: np.asarray(M, dtype=np.float64).T.ravel()
+    return np.concatenate([b.alphav, b.betav, imp.gammav.transpose(2, 1, 0).ravel(), f(w.kappav), f(w.nuv), f(w.kappa0v), f(w.nu0v), f(net.pv),
+                           [net.alphav, net.betav]])
+
+
+def set_network_variational_params_(process, q):
+    """Inverse of network_variational_params."""
+    b, w, imp, net = process.baseline, process.weights, process.impulses, process.network
+    N, B = process.ndims(), imp.nbasis()
+    q = np.asarray(q, dtype=np.float64).reshape(-1)
+    if q.size != _network_q_size(N, B):
+        raise ValueError(f"network variational parameter vector of {q.size} entries; N = {N}, B = {B} needs {_network_q_size(N, B)}")
+    NN, o = N * N, 2 * N + N * N * B
+    m = lambda k: q[o + k * NN:o + (k + 1) * NN].reshape(N, N).T.copy()  # [p + N c] -> [p, c]
+    b.alphav, b.betav = q[:N].copy(), q[N:2 * N].copy()
+    imp.gammav = q[2 * N:o].reshape(B, N, N).transpose(2, 1, 0).copy()
+    w.kappav, w.nuv, w.kappa0v, w.nu0v, net.pv = m(0), m(1), m(2), m(3), m(4)
+    net.alphav, net.betav = float(q[-2]), float(q[-1])
+
+
+def _network_blocks(q, N, B):
+    """Views of the blocks of a network state: alphav, betav, gammav[p, c, b], then kappav, nuv, kappa0v, nu0v, pv as [p, c]."""
+    NN, o = N * N, 2 * N + N * N * B
+    m = lambda k: q[o + k * NN:o + (k + 1) * NN].reshape(N, N).T
+    return q[:N], q[N:2 * N], q[2 * N:o].reshape(B, N, N).transpose(2, 1, 0), m(0), m(1), m(2), m(3), m(4)
+
+
+def network_expectations(q, N, B):
+    """The exp-expectations of a network state in the layouts of vb_statistics: e0[c] = exp(psi(alphav) - ln betav) and
+    E[p, c, b] = exp(psi(gammav) - psi(sum_b gammav) + E[ln W]) with the mixture E[ln W] = pv (psi(kappav) - ln nuv) +
+    (1 - pv) (psi(kappa0v) - ln nu0v)."""
+    q = np.asarray(q, dtype=np.float64)
+    av, bv, gv, kv, nv, k0v, n0v, pv = _network_blocks(q, N, B)
+    lw = pv * (digamma(kv) - np.log(nv)) + (1.0 - pv) * (digamma(k0v) - np.log(n0v))
+    return np.exp(digamma(av) - np.log(bv)), np.exp((digamma(gv) - digamma(gv.sum(axis=2, keepdims=True))) + lw[:, :, None])
+
+
+def _sigmoid(x):
+    with np.errstate(over="ignore", invalid="ignore"):
+        return np.where(x >= 0.0, 1.0 / (1.0 + np.exp(-x)), np.exp(x) / (1.0 + np.exp(x)))
+
+
+def network_vb_targets(q, stats, events, T, dt, hyper, s=1.0):
+    """The target q* of one network VB step from the state q and the statistics of a window scaled by s (s = 1 and the whole series
+    for VB): `stats` as vb_statistics returns them (alpha_sum[N], kappa_sum[p, c], gamma_sum[p, c, b]) for the expectations of q,
+    `events[p]` the events of node p in the window, `hyper` as _network_hyper.  With G = s kappa_sum and E = s events[p]:
+    alphav* = alpha0 + s alpha_sum, betav* = 1/beta0 + T dt, gammav* = gamma + s gamma_sum, kappav* = kappa + G, nuv* = nu + E,
+    kappa0v* = kappa0 + G, nu0v* = nu0 + E,
+      logit pv* = psi(alpharhov) - psi(betarhov) + [lgamma(kappav*) - kappav* ln nuv*] - [lgamma(kappa0v*) - kappa0v* ln nu0v*]
+                  + [kappa ln nu - lgamma(kappa)] - [kappa0 ln nu0 - lgamma(kappa0)],
+    and, with S = sum pv*, alpharhov* = alpha_rho + S, betarhov* = beta_rho + N^2 - S (N^2 counts links and is not scaled)."""
+    q = np.asarray(q, dtype=np.float64)
+    h = np.asarray(hyper, dtype=np.float64)
+    a = np.asarray(stats["alpha_sum"], dtype=np.float64)
+    N = a.size
+    NN = N * N
+    B = (q.size - 2 * N - 2) // NN - 5
+    if q.size != _network_q_size(N, B):
+        raise ValueError(f"network variational parameter vector of {q.size} entries does not fit N = {N}")
+    G = s * np.asarray(stats["kappa_sum"], dtype=np.float64).T.ravel()
+    E = s * np.tile(np.asarray(events, dtype=np.float64), N)  # events[p] at p + N c
+    k1, n1, k0, n0 = h[2] + G, h[3] + E, h[5] + G, h[6] + E
+    cprior = (h[2] * np.log(h[3]) - gammaln(h[2])) - (h[5] * np.log(h[6]) - gammaln(h[5]))
+    logit = (digamma(q[-2]) - digamma(q[-1])) + (gammaln(k1) - k1 * np.log(n1)) - (gammaln(k0) - k0 * np.log(n0)) + cprior
+    p = _sigmoid(logit)
+    S = float(np.sum(p))
+    gs = np.asarray(stats["gamma_sum"], dtype=np.float64).transpose(2, 1, 0).ravel()
+    return np.concatenate([h[0] + s * a, np.full(N, 1.0 / h[1] + T * dt), h[4] + s * gs, k1, n1, k0, n0, p, [h[7] + S, (h[8] + NN) - S]])
+
+
+def network_posterior_means(q, N, B):
+    """Posterior means of a network state: A = pv, W = pv kappav / nuv + (1 - pv) kappa0v / nu0v (both [p, c]), theta[p, c, b] =
+    gammav / sum_b gammav, lambda0 = alphav / betav and rho = alpharhov / (alpharhov + betarhov)."""
+    q = np.asarray(q, dtype=np.float64)
+    av, bv, gv, kv, nv, k0v, n0v, pv = _network_blocks(q, N, B)
+    return dict(A=pv.copy(), W=pv * kv / nv + (1.0 - pv) * k0v / n0v, theta=gv / gv.sum(axis=2, keepdims=True), lambda0=av / bv,
+                rho=float(q[-2] / (q[-2] + q[-1])))
+
+
+def _network_checks(process, name, kappa0, nu0):
+    if not isinstance(process, DiscreteNetworkHawkesProcess):
+        raise ValueError(f"{name}: needs a DiscreteNetworkHawkesProcess (vb_device_ / svi_device_ run a standard process)")
+    if not isinstance(process.network, BernoulliNetworkModel):
+        raise ValueError(f"{name}: network VB needs a BernoulliNetworkModel, got {type(process.network).__name__}")
+    for nm, v in (("kappa0", kappa0), ("nu0", nu0)):
+        if isinstance(v, (bool, np.bool_)) or not (float(v) > 0.0 and np.isfinite(float(v))):
+            raise ValueError(f"{name}: {nm} = {v!r} must be positive and finite")
+
+
+def network_update_(process, data, kappa0=0.1, nu0=10.0):
+    """The host twin of one network VB step (nhp_disc_vb_step on a network state): the expectations of network_expectations, the
+    statistics of vb_statistics (device), the events per node of the data and the targets of network_vb_targets with s = 1.  The
+    process holds the new state, which is returned."""
+    _network_checks(process, "network_update_", kappa0, nu0)
+    d = process._ready(data)
+    N, B = d.N, process.impulses.nbasis()
+    process.weights.kappa0, process.weights.nu0 = float(kappa0), float(nu0)
+    q = network_variational_params(process)
+    e0, E = network_expectations(q, N, B)
+    st = vb_statistics(process, d, e0, E)
+    qs = network_vb_targets(q, st, vb_row_sums(process, d), d.T, process.dt, _network_hyper(process), 1.0)
+    set_network_variational_params_(process, qs)
+    return qs
+
+
+def network_vb_device_(process, data, max_steps=100, rtol=None, kappa0=0.1, nu0=10.0):
+    """Mean-field VB of a discrete network process (BernoulliNetworkModel) with the loop and its trace on the device, shaped like
+    vb_device_: network_variational_params(process) and the hyper-parameters go up once (nhp_disc_vb_network_set), each step is one
+    nhp_disc_vb_step on the network state (the model and step are those of network_update_), the trace comes back in one read.  With
+    `rtol` it stops after the first step whose change (largest relative change of a positive entry, largest absolute change of a
+    link probability) is <= rtol.  Returns the list of state vectors, one per step; the process holds the last state.  A standard
+    process, another network model or a kappa0 / nu0 that is not positive and finite raise ValueError before any device call."""
+    _network_checks(process, "network_vb_device_", kappa0, nu0)
+    d = process._ready(data)
+    if max_steps < 1:
+        return []
+    process.weights.kappa0, process.weights.nu0 = float(kappa0), float(nu0)
+    change = ctypes.c_double()
+
+    def step(ctx, k):
+        ctx.check(ctx.lib.nhp_disc_vb_step(ctx.h, d.h, None if rtol is None else ctypes.byref(change)))
+        return rtol is not None and change.value <= rtol
+
+    return _vb_device_run(process, d, max_steps, step, network=True)
+
+
+def network_svi_device_(process, data, nsteps, batch_bins, tau0=1.0, kappa=0.75, seed=0, kappa0=0.1, nu0=10.0):
+    """Stochastic VI of a discrete network process with the loop and its trace on the device, shaped like svi_device_: step k is one
+    nhp_disc_svi_step on the network state over the window (t_begin[k], batch_bins) with step size step[k] of svi_schedule(T, nsteps,
+    batch_bins, tau0, kappa, seed).  Returns the list of state vectors, one per step; the process holds the last state.  Bad schedule
+    arguments and the refusals of network_vb_device_ raise ValueError before any device call."""
+    T = data.T if isinstance(data, DiscreteData) else np.shape(data)[1]
+    t_begin, steps = svi_schedule(T, nsteps, batch_bins, tau0, kappa, seed)
+    _network_checks(process, "network_svi_device_", kappa0, nu0)
+    d = process._ready(data)
+    if nsteps < 1:
+        return []
+    process.weights.kappa0, process.weights.nu0 = float(kappa0), float(nu0)
+    n = int(batch_bins)
+
+    def step(ctx, k):
+        ctx.check(ctx.lib.nhp_disc_svi_step(ctx.h, d.h, int(t_begin[k]), n, float(steps[k]), None))
+        return False
+
+    return _vb_device_run(process, d, nsteps, step, network=True)
 
 
 # ------------------------------------------------------------------------------------------
