@@ -71,8 +71,11 @@ int64_t nhp_events_count(const nhp_events *ev);
  * holds (nhp_cont_params_set), simulated on the device generation by generation (cluster representation: baseline events
  * baselines.jl:67-70, Poisson(W[p,c]) children per event and child node weights.jl:25-27, lags from the impulse response
  * impulses.jl:63-66, 196-202, truncated at `duration`), sorted by time and left device resident as an events handle -- no host
- * round trip for 1e8-event samples.  Philox keyed by `seed`; parity with the reference is distributional.  Fails when the
- * sample would exceed max_events.  nhp_events_download copies (events, nodes) of a handle to the host in Julia's conventions
+ * round trip for 1e8-event samples.  While LogGaussianCox curves are set (nhp_cont_baseline_grid), generation 0 of node k is the
+ * inhomogeneous Poisson process of rate lambda0_k(t), the curve the sweeps evaluate; the grid must then cover [0, duration]
+ * (x[0] <= 0 and x[n_grid-1] >= duration), NHP_ERR_INVALID otherwise, before anything is allocated.  Philox keyed by `seed`: the
+ * sample is a deterministic function of the parameters, the curves, `duration` and `seed`; parity with the reference is
+ * distributional.  Fails when the sample would exceed max_events.  nhp_events_download copies (events, nodes) of a handle to the host in Julia's conventions
  * (any pointer may be NULL). */
 int nhp_cont_rand(nhp_ctx *ctx, double duration, uint64_t seed, int64_t max_events, nhp_events **out);
 int nhp_events_download(nhp_ctx *ctx, nhp_events *ev, double *times, int64_t *nodes, double *duration);
@@ -92,7 +95,7 @@ int nhp_cont_params_set(nhp_ctx *ctx, int kind, int64_t K, const double *lambda0
  * event or query time outside [x[0], x[n_grid-1]] is an error (the reference throws a DomainError).  n_grid = 0 returns to the
  * homogeneous lambda0; nhp_cont_params_set also does (re-apply the curves after it).  The adjacency sampler and the structure
  * log-likelihood of a network process read lambda0_k(t_i) as well (the sampler returns NHP_ERR_NUMERIC, before changing anything,
- * when a curve is zero at an event of a column it sweeps); the analytic gradient takes a homogeneous baseline (NHP_ERR_UNSUPPORTED
+ * when a curve is zero at an event of a column it sweeps), and nhp_cont_rand draws the baseline events from the curves; the analytic gradient takes a homogeneous baseline (NHP_ERR_UNSUPPORTED
  * otherwise).  While the curves are set, the Exponential cut-off horizon measures the omitted tail against their smallest value. */
 int nhp_cont_baseline_grid(nhp_ctx *ctx, int64_t n_grid, const double *x, const double *values);
 /* The likelihood of the elliptical-slice update of the curves (baselines.jl:214-254: resample!(::LogGaussianCoxProcess) =

@@ -93,6 +93,7 @@ extern "C" int nhp_cont_baseline_grid(nhp_ctx *ctx, int64_t n_grid, const double
     for (int64_t e = 0; e < K * n_grid; e++) mn = std::min(mn, values[e]);
     ctx->baseline_integral = tot;
     ctx->bgrid_min = mn;
+    ctx->bgrid_lo = x[0]; ctx->bgrid_hi = x[n_grid - 1];
     ctx->lambda0_min = mn;  // the Exponential cut-off horizon measures the omitted tail against the smallest baseline rate
     return NHP_OK;
 }

@@ -4,7 +4,9 @@
 // homogeneous Poisson process (baselines.jl:67-70), and every event on node p spawns, on every child node c with
 // A[p,c] = 1, Poisson(W[p,c]) children (weights.jl:25-27) at lags drawn from the impulse response (impulses.jl:63-66,
 // 196-202); events beyond the duration are dropped.  Here the recursion becomes a breadth-first loop over generations:
-//   generation 0  n_k ~ Poisson(lambda0_k T) per node, times uniform on [0, T];
+//   generation 0  n_k ~ Poisson(lambda0_k T) per node, times uniform on [0, T]; with LogGaussianCox curves set
+//                 (nhp_cont_baseline_grid) an inhomogeneous Poisson process per node instead, drawn cell by cell of the grid
+//                 (Poisson count of the trapezoid area, times by the exact inverse CDF of the linear rate on the cell);
 //   generation g+1  every event of generation g draws its TOTAL number of children m ~ Poisson(sum_c A W[p,c]) and then each
 //                   child's node from Categorical(A W[p,:] / sum) -- by Poisson superposition / thinning exactly the law of
 //                   independent Poisson(W[p,c]) counts per child node -- and its lag from the (p, c) impulse response;
@@ -33,6 +35,44 @@ __global__ void k_rand_base_emit(int K, const long long *__restrict__ off, doubl
     RandStream r(seed, (uint64_t)e, 0u);
     t[e] = r.uniform() * T;
     c[e] = lo;
+}
+// Generation 0 of a LogGaussianCox baseline: an inhomogeneous Poisson process with the piecewise-linear rate of the sweeps
+// (cont_baseline.cu).  Cell i = (k, g), k = i / (G-1), is grid interval g of node k clipped to [0, T]; the rate is linear on it,
+// from a at its left end to b at its right end (the interpolation formula of grid_interp, interpolation.jl:31).
+__device__ __forceinline__ void rand_curve_cell(const double *__restrict__ x, const double *__restrict__ v, int G, long long i, double T, double *lo, double *hi,
+                                                double *a, double *b) {
+    const int k = (int)(i / (G - 1)), g = (int)(i - (long long)k * (G - 1));
+    const double x0 = x[g], x1 = x[g + 1], y0 = v[(int64_t)k * G + g], y1 = v[(int64_t)k * G + g + 1];
+    const double l = fmax(x0, 0.0), r = fmin(x1, T);
+    *lo = l; *hi = r;
+    *a = (y1 * (l - x0) + y0 * (x1 - l)) / (x1 - x0);
+    *b = (y1 * (r - x0) + y0 * (x1 - r)) / (x1 - x0);
+}
+// per cell: Poisson(trapezoid area of the clipped cell)
+__global__ void k_rand_curve_counts(long long ncell, int G, const double *__restrict__ x, const double *__restrict__ v, double T, uint64_t seed,
+                                    long long *__restrict__ counts) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= ncell) return;
+    double lo, hi, a, b;
+    rand_curve_cell(x, v, G, i, T, &lo, &hi, &a, &b);
+    RandStream r(seed, (uint64_t)i, 0x80000001u);
+    counts[i] = hi > lo ? r.poisson(0.5 * (a + b) * (hi - lo)) : 0;
+}
+// first event index of every cell -> (time, node): the inverse CDF of the linear density on the cell,
+//   s = h u (a + b) / (a + sqrt(a^2 + u (b^2 - a^2))),   exact for a = 0, b = 0 and a = b alike (a cell with a = b = 0 has no events)
+__global__ void k_rand_curve_emit(long long ncell, int G, const long long *__restrict__ off, const double *__restrict__ x, const double *__restrict__ v, double T,
+                                  uint64_t seed, double *__restrict__ t, int *__restrict__ c, long long n0) {
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n0) return;
+    long long lo = 0, hi = ncell;  // cell i with off[i] <= e < off[i+1]
+    while (hi - lo > 1) { const long long mid = (lo + hi) >> 1; if (off[mid] <= e) lo = mid; else hi = mid; }
+    double l, rt, a, b;
+    rand_curve_cell(x, v, G, lo, T, &l, &rt, &a, &b);
+    RandStream r(seed, (uint64_t)e, 0x80000002u);
+    const double u = r.uniform();
+    const double sd = (rt - l) * u * (a + b) / (a + sqrt(a * a + u * (b * b - a * a)));
+    t[e] = fmin(l + sd, rt);
+    c[e] = (int)(lo / (G - 1));
 }
 // number of children of every event of the current generation
 __global__ void k_rand_child_counts(const double *__restrict__ t, const int *__restrict__ c, long long g0, long long ng, const double *__restrict__ rowsum, double T,
@@ -95,6 +135,11 @@ extern "C" int nhp_cont_rand(nhp_ctx *ctx, double duration, uint64_t seed, int64
     NHP_CHECK(ctx, ctx->cont_set, NHP_ERR_STATE, "continuous parameters not set (call nhp_cont_params_set)");
     NHP_CHECK(ctx, duration > 0.0 && std::isfinite(duration), NHP_ERR_INVALID, "nhp_cont_rand: duration must be positive and finite");
     NHP_CHECK(ctx, max_events >= 1 && max_events < (int64_t)2147483000, NHP_ERR_INVALID, "nhp_cont_rand: max_events outside [1, 2^31)");
+    const bool curves = ctx->bgrid_n > 0;
+    NHP_CHECK(ctx, !curves || (ctx->bgrid_lo <= 0.0 && ctx->bgrid_hi >= duration), NHP_ERR_INVALID,
+              "nhp_cont_rand: the curves' grid [%g, %g] does not cover [0, duration = %g]", ctx->bgrid_lo, ctx->bgrid_hi, duration);
+    const int64_t ncell = curves ? ctx->K * (ctx->bgrid_n - 1) : 0;  // generation 0 with curves: one Poisson count per (node, grid interval)
+    NHP_CHECK(ctx, ncell < (int64_t)2147483000, NHP_ERR_INVALID, "nhp_cont_rand: K (n_grid - 1) = %lld cells exceed 2^31", (long long)ncell);
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     const int K = (int)ctx->K;
     const int64_t cap = max_events;
@@ -152,12 +197,23 @@ extern "C" int nhp_cont_rand(nhp_ctx *ctx, double duration, uint64_t seed, int64
         R_CUDA(cudaStreamSynchronize(s));
         return NHP_OK;
     };
-    k_rand_base_counts<<<(K + 127) / 128, 128, 0, s>>>(K, ctx->d_lambda0, duration, seed, d_cnt);
-    NHP_LAUNCHED(ctx);
     long long n0 = 0;
-    { int rc = scan_total(K, &n0); if (rc != NHP_OK) return rc; }
+    if (curves) {  // inhomogeneous: the curves of nhp_cont_baseline_grid, cell by cell
+        const int G = (int)ctx->bgrid_n;
+        R_CUDA(ensure_cnt(ncell));
+        k_rand_curve_counts<<<(unsigned)((ncell + 255) / 256), 256, 0, s>>>(ncell, G, ctx->d_bgrid_x, ctx->d_bgrid_v, duration, seed, d_cnt);
+        NHP_LAUNCHED(ctx);
+        { int rc = scan_total(ncell, &n0); if (rc != NHP_OK) return rc; }
+    } else {
+        k_rand_base_counts<<<(K + 127) / 128, 128, 0, s>>>(K, ctx->d_lambda0, duration, seed, d_cnt);
+        NHP_LAUNCHED(ctx);
+        { int rc = scan_total(K, &n0); if (rc != NHP_OK) return rc; }
+    }
     if (n0 > cap) return fin(nhp_fail(ctx, NHP_ERR_INVALID, "nhp_cont_rand: the sample needs more than max_events = %lld events (generation 0 alone has %lld)", (long long)cap, n0));
-    if (n0 > 0) {
+    if (n0 > 0 && curves) {
+        k_rand_curve_emit<<<(unsigned)((n0 + 255) / 256), 256, 0, s>>>(ncell, (int)ctx->bgrid_n, d_off, ctx->d_bgrid_x, ctx->d_bgrid_v, duration, seed, d_t, d_c, n0);
+        NHP_LAUNCHED(ctx);
+    } else if (n0 > 0) {
         k_rand_base_emit<<<(unsigned)((n0 + 255) / 256), 256, 0, s>>>(K, d_off, duration, seed, d_t, d_c, n0);
         NHP_LAUNCHED(ctx);
     }

@@ -164,6 +164,7 @@ struct nhp_ctx {
     int64_t bgrid_n = 0; uint64_t bgrid_version = 0;     // 0 points: homogeneous lambda0
     double baseline_integral = 0.0;                      // sum_k integrate(lambda0_k) over the grid (trapezoid)
     double bgrid_min = 0.0;                              // smallest curve value: lambda0_min while the grid is active
+    double bgrid_lo = 0.0, bgrid_hi = 0.0;               // x[0], x[bgrid_n-1] on the host (the simulator's coverage check)
     // GP prior of the log-curves, log lambda0_k = m + y_k, y_k ~ N(0, L L^T) (nhp_cont_baseline_prior; cont_slice.cu): [bprior_n^2] L
     double *d_bprior_L = nullptr; int64_t bprior_n = 0, bprior_cap = 0; double bprior_m = 0.0;  // 0 points: no prior
     void *d_slice = nullptr; size_t slice_cap = 0;       // work buffers of the elliptical-slice update

@@ -198,7 +198,7 @@ function rand(process::ContinuousHawkesProcess, duration::Float64)
     push_params!(process)
     K = ndims(process)
     Weff = process isa ContinuousNetworkHawkesProcess ? process.adjacency_matrix .* process.weights.W : process.weights.W
-    expected = sum(process.baseline.λ) * duration / max(0.05, 1 - min(0.95, maximum(sum(Weff, dims=2))))
+    expected = baseline_events(process.baseline, duration) / max(0.05, 1 - min(0.95, maximum(sum(Weff, dims=2))))
     h = Ref{Ptr{Cvoid}}(C_NULL)
     check(ccall((:nhp_cont_rand, LIB[]), Cint, (Ptr{Cvoid}, Float64, UInt64, Int64, Ref{Ptr{Cvoid}}),
         CTX[], duration, Base.rand(UInt64), ceil(Int64, 2expected + 10sqrt(expected) + 1000), h))
@@ -207,6 +207,21 @@ function rand(process::ContinuousHawkesProcess, duration::Float64)
     check(ccall((:nhp_events_download, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}), CTX[], h[], events, nodes, C_NULL))
     ccall((:nhp_events_free, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}), CTX[], h[])
     return events, nodes, duration
+end
+
+# expected number of baseline events on [0, duration]: a LogGaussianCoxProcess's curves integrated over the interval (the device draws
+# generation 0 from the curves; their grid must cover [0, duration])
+baseline_events(b::HomogeneousProcess, duration) = sum(b.λ) * duration
+function baseline_events(b::LogGaussianCoxProcess, duration)
+    s = 0.0
+    for y in b.λ, g in 1:length(b.x)-1
+        x0, x1 = b.x[g], b.x[g+1]
+        l, r = max(x0, 0.0), min(x1, duration)
+        r > l || continue
+        f(t) = (y[g+1] * (t - x0) + y[g] * (x1 - t)) / (x1 - x0)   # interpolation.jl:31
+        s += 0.5 * (f(l) + f(r)) * (r - l)
+    end
+    return s
 end
 
 # ---- parents.jl:1: the sweep and what it leaves behind ---------------------------------------------------------------------------

@@ -96,6 +96,28 @@ class LogGaussianCoxProcess:
     def integrated_intensity(self):
         return np.trapezoid(self.lam_grid, self.x, axis=1) if hasattr(np, "trapezoid") else np.trapz(self.lam_grid, self.x, axis=1)
 
+    def _clipped(self, duration):
+        """The grid clipped to [0, duration] (which it must cover) and the curves' values on it, exact for the piecewise-linear rate."""
+        if not (self.x[0] <= 0.0 and self.x[-1] >= duration):
+            raise ValueError(f"LogGaussianCoxProcess: the grid [{self.x[0]}, {self.x[-1]}] does not cover [0, {duration}]")
+        xs = np.concatenate([[0.0], self.x[(self.x > 0.0) & (self.x < duration)], [float(duration)]])
+        return xs, np.stack([np.interp(xs, self.x, y) for y in self.lam_grid])
+
+    def integrated_intensity_on(self, duration):
+        """Per node: the integral of the curve over [0, duration] (trapezoid on the clipped grid)."""
+        xs, ys = self._clipped(duration)
+        return np.sum(0.5 * (ys[:, 1:] + ys[:, :-1]) * np.diff(xs), axis=1)
+
+    def sample(self, node, duration, rng):
+        """The baseline events of `node` on [0, duration], sorted: Poisson(max * duration) uniform candidates, each kept with
+        probability lambda(t) / max, where max is the curve's maximum on [0, duration] (thinning, as the reference's rejection_sample)."""
+        xs, ys = self._clipped(duration)
+        top = float(np.max(ys[node]))
+        n = rng.poisson(top * duration)
+        ts = rng.uniform(0.0, duration, n)
+        keep = rng.random(n) * top < np.interp(ts, self.x, self.lam_grid[node])
+        return np.sort(ts[keep])
+
     def logprior(self):
         y = np.log(self.lam_grid) - self.m
         z = np.linalg.solve(self._chol, y.T)
@@ -813,10 +835,12 @@ def rand_device(process, duration, seed=0, max_events=None):
     """`rand(process, duration)` simulated on the GPU; returns device-resident data (`.download()` gives the host tuple)."""
     ctx = process._ctx()
     process._push(ctx)
-    if max_events is None:  # stationary mean (I - W^T)^-1 lambda0 T with head room
+    if max_events is None:  # stationary mean (I - W^T)^-1 lambda0 T with head room; curves: their integrals over [0, duration]
         Weff = process.weights.W if process.adjacency_matrix is None else process.adjacency_matrix * process.weights.W
         rad = float(np.max(np.sum(Weff, axis=1))) if Weff.size else 0.0
-        mean = float(np.sum(process.baseline.lam)) * duration / max(1.0 - min(rad, 0.95), 0.05)
+        b = process.baseline
+        base = float(np.sum(b.integrated_intensity_on(duration))) if isinstance(b, LogGaussianCoxProcess) else float(np.sum(b.lam)) * duration
+        mean = base / max(1.0 - min(rad, 0.95), 0.05)
         max_events = int(min(2.1e9, 2.0 * mean + 10.0 * np.sqrt(mean) + 1000))
     h = ctypes.c_void_p()
     ctx.check(ctx.lib.nhp_cont_rand(ctx.h, float(duration), int(seed), int(max_events), ctypes.byref(h)))
@@ -828,11 +852,17 @@ def rand(process, duration, rng=None):
     K = process.ndims()
     A = process.adjacency_matrix
     W = process.weights.W
+    lgcp = isinstance(process.baseline, LogGaussianCoxProcess)
+    if lgcp:
+        process.baseline._clipped(duration)  # ValueError before any draw when the grid does not cover [0, duration]
     per_node = [[] for _ in range(K)]
     stack = []
     for node in range(K):
-        n = rng.poisson(process.baseline.lam[node] * duration)  # baselines.jl:67-70
-        ts = np.sort(rng.uniform(0.0, duration, n))
+        if lgcp:
+            ts = process.baseline.sample(node, duration, rng)
+        else:
+            n = rng.poisson(process.baseline.lam[node] * duration)  # baselines.jl:67-70
+            ts = np.sort(rng.uniform(0.0, duration, n))
         per_node[node].extend(ts.tolist())
         stack.extend((t, node) for t in ts)
     while stack:
