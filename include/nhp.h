@@ -234,6 +234,47 @@ int nhp_cont_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity);
 int nhp_cont_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *rho, double *lambda0, double *W, double *A, double *p1, double *p2);
 int nhp_cont_trace_free(nhp_ctx *ctx);
 int nhp_cont_trace_read_curves(nhp_ctx *ctx, int64_t first, int64_t count, double *values);
+/* Mean-field VB of a continuous standard process with its state on the device (the reference's `vb!` is discrete only).  The model is
+ * the one of the Gibbs sweep: lambda0_k ~ Gamma(alpha0, beta0), W[p,c] ~ Gamma(kappa, nu), Exponential theta ~ Gamma(alpha, beta) or
+ * LogitNormal (mu, tau) ~ NormalGamma(mumu, kappamu, a0, b0) (all Gammas with rates), and the factorised posterior
+ *   q = [alphav(K); betav(K); kappav(K*K); nuv(K*K)], then Exponential atheta(K*K); btheta(K*K)  (2 K + 4 K*K doubles)
+ *                                                    or LogitNormal mv(K*K); lambdav(K*K); av(K*K); bv(K*K)  (2 K + 6 K*K doubles),
+ * K*K planes parent-major (X[p + K*c]): q(lambda0_k) = Gamma(alphav, betav), q(W) = Gamma(kappav, nuv), q(theta) = Gamma(atheta, btheta),
+ * q(mu, tau) = NormalGamma(mv, lambdav, av, bv).  _set takes the kind, K and dtmax of the current nhp_cont_params_set; hyper = [alpha0,
+ * beta0, kappa, nu, then alpha, beta | mumu, kappamu, a0, b0] (n_hyper 6 or 8, that of the kind), every entry finite and > 0 except
+ * mumu (finite); every entry of q finite and > 0 except mv (finite).  Otherwise NHP_ERR_INVALID (NHP_ERR_STATE without parameters)
+ * and the kept state is as it was.  _get copies q back.
+ * The E-step evaluates the parent probabilities at effective parameters, for which ln W_eff + ln h(dt) = E_q[ln W + ln h(dt)]:
+ *   lambda0_eff = exp(psi(alphav) - ln betav); Exponential theta_eff = atheta / btheta, W_eff = exp(psi(kappav) - ln nuv + psi(atheta)
+ *   - ln btheta) / theta_eff; LogitNormal mu_eff = mv, tau_eff = av / bv, W_eff = exp(psi(kappav) - ln nuv + (psi(av) - ln av) / 2
+ *   - 1 / (2 lambdav));
+ * with Z_i the total intensity at event i and u = W_eff h(t_i - t_j) / Z_i over the window of nhp_cont_resample_parents (dtmax for
+ * LogitNormal, the cut-off horizon of nhp_cont_horizon for Exponential, both at the effective parameters):
+ *   M0[k] = sum over the events of node k of lambda0_eff[k] / Z_i;  Mnm = sum u;  S1 = sum u (t_i - t_j) (Exponential) or sum u (y - mv)
+ *   with y = logit((t_i - t_j) / dtmax) (LogitNormal);  S2 = sum u (y - mv)^2 (LogitNormal; zeros for Exponential).
+ * nhp_cont_vb_stats runs the E-step only and returns those sums in the layouts of nhp_cont_suffstats (any output may be NULL); q does
+ * not change.  nhp_cont_vb_step then updates q in place: alphav = alpha0 + M0, betav = beta0 + T (T the duration of ev), kappav =
+ * kappa + Mnm, nuv = nu + Mn[p]; Exponential atheta = alpha + Mnm, btheta = beta + S1; LogitNormal, with n = Mnm, d = S1 / n (0 for
+ * n = 0), ybar = mv + d, S = max(S2 - n d^2, 0): lambdav = kappamu + n, mv = (kappamu mumu + n ybar) / lambdav, av = a0 + n / 2,
+ * bv = b0 + S / 2 + kappamu n (ybar - mumu)^2 / (2 lambdav) -- the textbook Normal-Gamma update, which keeps b0 where the Gibbs draw
+ * of nhp_cont_resample_params does not (quirk Q5).  A pair with n = 0 gets its prior.  change (may be NULL) = the largest of
+ * |new - old| / old over the positive entries and |new - old| over mv, the only value that crosses PCIe; then a push to the VB trace
+ * while it has room.  After either call the context's parameters are the posterior means of q (alphav / betav, kappav / nuv, atheta /
+ * btheta | mv, av / bv) with every table rebuilt, so nhp_cont_loglik, nhp_cont_intensity or nhp_cont_params_get see the fitted model;
+ * the parent assignment and gradient of earlier calls are invalidated.  Refused before anything changes: a network process (A set),
+ * LogGaussianCox curves set, a time shard (n_halo > 0) or a communicator of more than one rank (NHP_ERR_UNSUPPORTED); no parameters, no
+ * VB state, or a kind or K that changed since _set (NHP_ERR_STATE); an events handle of another K (NHP_ERR_INVALID); for _step, an
+ * open VB trace begun for another kind or K (NHP_ERR_STATE). */
+int nhp_cont_vb_set(nhp_ctx *ctx, const double *hyper, int n_hyper, const double *q);
+int nhp_cont_vb_get(nhp_ctx *ctx, double *q);
+int nhp_cont_vb_stats(nhp_ctx *ctx, nhp_events *ev, double *M0, double *Mnm, double *S1, double *S2);
+int nhp_cont_vb_step(nhp_ctx *ctx, nhp_events *ev, double *change);
+/* Device-side trace of the continuous VB state, independent of every other trace: one slot is q (laid out for the state at _begin);
+ * _read copies slots [first, first + count) one after the other. */
+int nhp_cont_vb_trace_begin(nhp_ctx *ctx, int64_t capacity);
+int nhp_cont_vb_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity);
+int nhp_cont_vb_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *q_out);
+int nhp_cont_vb_trace_free(nhp_ctx *ctx);
 
 /* ---- multi-GPU (one process and one context per GPU; NCCL over NVLink, loaded with dlopen) ---------------------
  * SURVEY.md section 8e.  Time shards (nhp_events_upload with n_halo / index_base) carry the log-likelihood, the parent

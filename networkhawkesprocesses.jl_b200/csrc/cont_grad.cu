@@ -19,6 +19,10 @@
 // are flushed to the K^2 planes once per child.  Pairs whose effective weight is structurally zero (a = 0) cost one
 // shared-memory read.  The result lives in the statistics buffers (dlambda0 -> M0 slot, dW -> Mnm, dp1 -> S1,
 // dp2 -> S2), so the multi-GPU reduction is the same two all-reduces as for the Gibbs statistics.
+//
+// The walk is a template over the per-pair terms it scatters: the gradient's (TERMS_GRAD), or the expected parent
+// statistics of mean-field VB (TERMS_VB, cont_vb.cu): with u = W h(dt) / lambda_i the probability that the pair is the
+// child's parent, (u, u dt) for Exponential and (u, u dz, u dz^2) for LogitNormal, dz = logit(dt / D) - mu.
 #include "cont_sweep.cuh"
 #include <algorithm>
 
@@ -45,16 +49,21 @@ template <int KIND> __device__ __forceinline__ GEntry make_entry(const GradArgs 
     return e;
 }
 
+enum { TERMS_GRAD = 0, TERMS_VB = 1 };
+
 // the three per-pair terms (already divided by lambda_i); returns false when the pair contributes nothing
-template <int KIND> __device__ __forceinline__ bool pair_terms(const GEntry &en, double dt, double D, double inv, const FastTables *ft, double &tw, double &t1,
-                                                              double &t2) {
+template <int KIND, int TERMS> __device__ __forceinline__ bool pair_terms(const GEntry &en, double dt, double D, double inv, const FastTables *ft, double &tw,
+                                                                         double &t1, double &t2) {
     if (en.c0 == 0.0) return false;
     if (KIND == NHP_EXPONENTIAL) {
         if (dt < 0.0) return false;
         const double x = -en.p1 * dt;
         const double ex = (__double2hiint(x) >= 0x40862800) ? exp(x) : fast_exp_c(x, ft);
         tw = en.c0 * ex * inv;
-        t1 = en.w * ex * fma(-en.p1, dt, 1.0) * inv;
+        if (TERMS == TERMS_VB) {  // u = W theta e^{-theta dt} / lambda_i, u dt
+            tw *= en.w;
+            t1 = tw * dt;
+        } else t1 = en.w * ex * fma(-en.p1, dt, 1.0) * inv;
         t2 = 0.0;
         return true;
     }
@@ -71,13 +80,19 @@ template <int KIND> __device__ __forceinline__ bool pair_terms(const GEntry &en,
     const double ex = fast_exp(-(0.5 * en.p2) * dz * dz, ft);
     const double ha = en.c0 * pj * ex * inv;  // a h / lambda_i
     const double v = en.w * ha;               // a W h / lambda_i
+    if (TERMS == TERMS_VB) {                  // u, u dz, u dz^2
+        tw = v;
+        t1 = v * dz;
+        t2 = t1 * dz;
+        return true;
+    }
     tw = ha;
     t1 = v * en.p2 * dz;
     t2 = v * (0.5 / en.p2 - 0.5 * dz * dz);
     return true;
 }
 
-template <int KIND> __global__ void __launch_bounds__(1024) k_child_grad(const GradArgs ga) {
+template <int KIND, int TERMS> __global__ void __launch_bounds__(1024) k_child_grad(const GradArgs ga) {
     const SweepArgs &a = ga.s;
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ FastTables s_ft;
@@ -127,7 +142,10 @@ template <int KIND> __global__ void __launch_bounds__(1024) k_child_grad(const G
             const int jlo = (int)a.jmin;
             const double lam = __ldg(ga.lam + (i - a.first));
             const double inv = 1.0 / lam;
-            if (lane == 0) { sum_log += log(lam); inv_sum += inv; }
+            if (lane == 0) {
+                if (TERMS == TERMS_GRAD) sum_log += log(lam);
+                inv_sum += inv;
+            }
             const int wraw = (int)__ldg(ga.wlen + (i - a.first));
             const int w = wraw < 65535 ? min(wraw, i - jlo) : i - jlo;  // known trip count: loads of several trips in flight
 #pragma unroll 2
@@ -137,7 +155,7 @@ template <int KIND> __global__ void __launch_bounds__(1024) k_child_grad(const G
                 if (wraw >= 65535 && !(tj > thr)) break;
                 const int p = __ldg(a.c + j);
                 double tw, t1, t2;
-                if (!pair_terms<KIND>(col[p], ti - tj, a.D, inv, ft, tw, t1, t2)) continue;
+                if (!pair_terms<KIND, TERMS>(col[p], ti - tj, a.D, inv, ft, tw, t1, t2)) continue;
                 if (ga.acc_smem) {
                     atomicAdd(acc + p, tw);
                     atomicAdd(acc + a.K + p, t1);
@@ -173,6 +191,51 @@ int nhp_cont_fill_args(nhp_ctx *ctx, nhp_events *ev, int recursive, SweepArgs &a
 int nhp_cont_run_event_intensity(nhp_ctx *ctx, nhp_events *ev, int recursive, double *d_out);     // cont_sweep.cu
 int nhp_cont_reduce_partials(nhp_ctx *ctx, nhp_events *ev, const double *partials, int grid, const double *rowsum);  // cont_sweep.cu
 
+// Sweep 2 of the gradient and of the VB statistics: the child-major scatter of the per-pair terms (`terms`: TERMS_GRAD | TERMS_VB)
+// of the context's parameters, given lam[n_own] = lambda_i of sweep 1, added into the zeroed planes g_l0[K] (sum of 1 / lambda_i per
+// child node), g_w, g_p1, g_p2 [K*K].  a: nhp_cont_fill_args of this call; its `partials` receive the per-CTA log-sums (TERMS_GRAD).
+// *grid_out = CTAs launched (0: no work items).
+int nhp_cont_child_scatter(nhp_ctx *ctx, nhp_events *ev, SweepArgs &a, const double *lam, int terms, double *g_l0, double *g_w, double *g_p1,
+                           double *g_p2, int *grid_out) {
+    const int64_t K = ctx->K;
+    cudaStream_t s = ctx->stream;
+    *grid_out = 0;
+    NHP_TRY(nhp_events_build_node_index(ctx, ev));
+    NHP_CUDA(ctx, fast_tables_upload(s));
+    GradArgs ga;
+    ga.s = a; ga.order = ev->d_order; ga.node_ptr = ev->d_node_ptr; ga.item_node = ev->d_item_node; ga.item_e0 = ev->d_item_e0; ga.nitems = ev->n_items;
+    ga.W = ctx->d_W; ga.A = ctx->has_A ? ctx->d_A : nullptr; ga.p1 = ctx->d_p1; ga.p2 = ctx->d_p2; ga.lam = lam;
+    ga.g_l0 = g_l0; ga.g_w = g_w; ga.g_p1 = g_p1; ga.g_p2 = g_p2; ga.wlen = ev->d_wlen;
+    const int np = ctx->kind == NHP_LOGITNORMAL ? 3 : 2;
+    const size_t lim = (size_t)ctx->smem_optin - 8192;
+    size_t smem = (size_t)K * (sizeof(GEntry) + np * sizeof(double));
+    ga.acc_smem = smem <= lim;
+    { const char *eg = getenv("NHP_GRAD_SMEM"); if (eg && atoi(eg) == 0) ga.acc_smem = 0; }  // A/B: accumulate with global RED.ADD.F64 instead
+    if (!ga.acc_smem) smem = (size_t)K * sizeof(GEntry);
+    NHP_CHECK(ctx, smem <= lim, NHP_ERR_INVALID, "%s: K=%lld needs %zu bytes of shared memory per CTA (limit %zu)",
+              terms == TERMS_VB ? "nhp_cont_vb" : "nhp_cont_loglik_grad", (long long)K, smem, lim);
+    NHP_TRY(nhp_partials(ctx, 2 * (int64_t)ctx->sm_count * 32, &a.partials));
+    ga.s.partials = a.partials;
+    auto launch = [&](auto kernel) -> int {
+        NHP_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 1024)));
+        NHP_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        int per_sm = 1;
+        const int fit = (int)std::max<size_t>(1, lim / std::max<size_t>(smem, 1));
+        const int block = fit >= 8 ? 256 : (fit >= 4 ? 512 : 1024);  // big columns leave room for few CTAs per SM: give them more warps
+        NHP_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, block, smem));
+        const int grid = (int)std::min<int64_t>(ev->n_items, (int64_t)ctx->sm_count * std::max(per_sm, 1));
+        kernel<<<grid, block, smem, s>>>(ga);
+        NHP_LAUNCHED(ctx);
+        NHP_CUDA(ctx, cudaGetLastError());
+        *grid_out = grid;
+        return NHP_OK;
+    };
+    if (ev->n_items == 0) return NHP_OK;
+    const bool ln = ctx->kind == NHP_LOGITNORMAL;
+    if (terms == TERMS_VB) return ln ? launch(k_child_grad<NHP_LOGITNORMAL, TERMS_VB>) : launch(k_child_grad<NHP_EXPONENTIAL, TERMS_VB>);
+    return ln ? launch(k_child_grad<NHP_LOGITNORMAL, TERMS_GRAD>) : launch(k_child_grad<NHP_EXPONENTIAL, TERMS_GRAD>);
+}
+
 extern "C" int nhp_cont_loglik_grad_dev(nhp_ctx *ctx, nhp_events *ev, int recursive) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -197,39 +260,9 @@ extern "C" int nhp_cont_loglik_grad_dev(nhp_ctx *ctx, nhp_events *ev, int recurs
         NHP_TRY(nhp_scratch(ctx, (size_t)own * sizeof(double), &scratch));
         NHP_TRY(nhp_cont_run_event_intensity(ctx, ev, recursive, (double *)scratch));
         // sweep 2: child-major scatter of the per-pair terms
-        NHP_TRY(nhp_events_build_node_index(ctx, ev));
-        NHP_CUDA(ctx, fast_tables_upload(s));
-        GradArgs ga;
-        ga.s = a; ga.order = ev->d_order; ga.node_ptr = ev->d_node_ptr; ga.item_node = ev->d_item_node; ga.item_e0 = ev->d_item_e0; ga.nitems = ev->n_items;
-        ga.W = ctx->d_W; ga.A = ctx->has_A ? ctx->d_A : nullptr; ga.p1 = ctx->d_p1; ga.p2 = ctx->d_p2; ga.lam = (const double *)scratch;
-        ga.g_l0 = g_l0; ga.g_w = g_w; ga.g_p1 = g_p1; ga.g_p2 = g_p2; ga.wlen = ev->d_wlen;
-        const int np = ctx->kind == NHP_LOGITNORMAL ? 3 : 2;
-        const size_t lim = (size_t)ctx->smem_optin - 8192;
-        size_t smem = (size_t)K * (sizeof(GEntry) + np * sizeof(double));
-        ga.acc_smem = smem <= lim;
-        { const char *eg = getenv("NHP_GRAD_SMEM"); if (eg && atoi(eg) == 0) ga.acc_smem = 0; }  // A/B: accumulate with global RED.ADD.F64 instead
-        if (!ga.acc_smem) smem = (size_t)K * sizeof(GEntry);
-        NHP_CHECK(ctx, smem <= lim, NHP_ERR_INVALID, "nhp_cont_loglik_grad: K=%lld needs %zu bytes of shared memory per CTA (limit %zu)", (long long)K, smem, lim);
-        NHP_TRY(nhp_partials(ctx, 2 * (int64_t)ctx->sm_count * 32, &ga.s.partials));
         int grid = 0;
-        auto launch = [&](auto kernel) -> int {
-            NHP_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 1024)));
-            NHP_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-            int per_sm = 1;
-            const int fit = (int)std::max<size_t>(1, lim / std::max<size_t>(smem, 1));
-            const int block = fit >= 8 ? 256 : (fit >= 4 ? 512 : 1024);  // big columns leave room for few CTAs per SM: give them more warps
-            NHP_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, block, smem));
-            grid = (int)std::min<int64_t>(ev->n_items, (int64_t)ctx->sm_count * std::max(per_sm, 1));
-            kernel<<<grid, block, smem, s>>>(ga);
-            NHP_LAUNCHED(ctx);
-            NHP_CUDA(ctx, cudaGetLastError());
-            return NHP_OK;
-        };
-        if (ev->n_items > 0) {
-            if (ctx->kind == NHP_LOGITNORMAL) NHP_TRY(launch(k_child_grad<NHP_LOGITNORMAL>));
-            else NHP_TRY(launch(k_child_grad<NHP_EXPONENTIAL>));
-            NHP_TRY(nhp_cont_reduce_partials(ctx, ev, ga.s.partials, grid, a.rowsum));
-        }
+        NHP_TRY(nhp_cont_child_scatter(ctx, ev, a, (const double *)scratch, TERMS_GRAD, g_l0, g_w, g_p1, g_p2, &grid));
+        if (grid > 0) NHP_TRY(nhp_cont_reduce_partials(ctx, ev, a.partials, grid, a.rowsum));
     }
     const double T_first = (ev->flags & 1) ? ev->duration : 0.0;
     k_grad_finish<<<(unsigned)((K * K + 255) / 256), 256, 0, s>>>((int)K, ev->d_Mn, ctx->has_A ? ctx->d_A : nullptr, rec && ctx->has_A ? 1 : 0, T_first, g_l0, g_w);

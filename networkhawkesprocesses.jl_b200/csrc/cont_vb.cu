@@ -1,0 +1,308 @@
+// cont_vb.cu -- mean-field VB of a continuous standard Hawkes process on the device (the reference has no `vb!` for continuous
+// processes; this is the model of the Gibbs sweep, SURVEY section 10, with a factorised posterior).
+//
+// Priors (the hyper-parameters of nhp_cont_resample_params): lambda0_k ~ Gamma(alpha0, beta0), W[p,c] ~ Gamma(kappa, nu), Exponential
+// theta ~ Gamma(alpha, beta), LogitNormal (mu, tau) ~ NormalGamma(mumu, kappamu, a0, b0); all rates.  The state q kept with the context:
+//   q = [alphav(K); betav(K); kappav(K^2); nuv(K^2); atheta(K^2); btheta(K^2)]                      Exponential
+//   q = [alphav(K); betav(K); kappav(K^2); nuv(K^2); mv(K^2); lambdav(K^2); av(K^2); bv(K^2)]        LogitNormal
+// K^2 planes parent-major, X[p + K c].
+//
+// E-step.  Under q the responsibilities of the augmented likelihood are those of the parent sweep at *effective* parameters, because
+// E_q[ln W + ln h(dt)] = ln W_eff + ln h(dt; theta_eff) for every lag dt:
+//   lambda0_eff = exp(psi(alphav) - ln betav),  lW = psi(kappav) - ln nuv
+//   Exponential:  theta_eff = atheta / btheta,  W_eff = exp(lW + psi(atheta) - ln btheta) / theta_eff      (E ln h = E ln theta - theta_eff dt)
+//   LogitNormal:  mu_eff = mv, tau_eff = av / bv,  W_eff = exp(lW + (psi(av) - ln av) / 2 - 1 / (2 lambdav))
+//                                                              (E[tau (y - mu)^2] = tau_eff (y - mv)^2 + 1 / lambdav)
+// k_cvb_expect writes them into the context's parameters and nhp_cont_params_refresh rebuilds the tables (and the Exponential cut-off
+// horizon) from them.  Sweep 1 (the ordinary intensity sweep) gives Z_i = lambda_i at those parameters; sweep 2 is the gradient's
+// child-major scatter (cont_grad.cu, TERMS_VB) of u = W_eff h(dt) / Z_i: Mnm = sum u, S1 = sum u dt | sum u (y - mv), S2 = sum u (y - mv)^2
+// (LogitNormal; y = logit(dt / dtmax)), and per child node sum 1 / Z_i, which times lambda0_eff is M0.  The LogitNormal sums are
+// shifted about the current mv, so one sweep gives the centred second moment: S = S2 - S1^2 / Mnm.
+//
+// M-step (k_cvb_update, in place): alphav = alpha0 + M0, betav = beta0 + T, kappav = kappa + Mnm, nuv = nu + Mn[p],
+//   Exponential  atheta = alpha + Mnm, btheta = beta + S1
+//   LogitNormal  n = Mnm, d = S1 / n (0 for n = 0), ybar = mv + d, S = max(S2 - n d^2, 0):
+//                lambdav = kappamu + n, mv = (kappamu mumu + n ybar) / lambdav, av = a0 + n / 2,
+//                bv = b0 + S / 2 + kappamu n (ybar - mumu)^2 / (2 lambdav)
+// (the textbook Normal-Gamma update; it keeps b0 where the Gibbs draw replaces it, quirk Q5).  A pair with n = 0 gets its prior.  The same
+// kernel then writes the posterior means (alphav / betav, kappav / nuv, atheta / btheta | mv, av / bv) into the context's parameters,
+// so a later log-likelihood, intensity or nhp_cont_params_get sees the fitted model.
+#include "cont_sweep.cuh"
+#include <algorithm>
+#include <cmath>
+
+static size_t cvb_q_doubles(int kind, int64_t K) { return (size_t)(2 * K) + (size_t)(K * K) * (kind == NHP_LOGITNORMAL ? 6 : 4); }
+
+// one thread per (p, c), e = p + K c (threads e < K also write lambda0_eff[e]): the effective parameters above
+__global__ void __launch_bounds__(256) k_cvb_expect(const double *__restrict__ q, int K, int kind, double *__restrict__ lambda0, double *__restrict__ W,
+                                                    double *__restrict__ p1, double *__restrict__ p2) {
+    const int64_t KK = (int64_t)K * K;
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= KK) return;
+    const double *kv = q + 2 * K, *nv = kv + KK, *x1 = nv + KK, *x2 = x1 + KK;
+    if (e < K) lambda0[e] = exp(nhp_digamma(q[e]) - log(q[K + e]));
+    const double lw = nhp_digamma(kv[e]) - log(nv[e]);
+    if (kind == NHP_EXPONENTIAL) {
+        const double a = x1[e], b = x2[e], th = a / b;
+        W[e] = exp(lw + (nhp_digamma(a) - log(b))) / th;
+        p1[e] = th;
+    } else {
+        const double *x3 = x2 + KK, *x4 = x3 + KK;
+        const double a = x3[e];
+        W[e] = exp(lw + 0.5 * (nhp_digamma(a) - log(a)) - 0.5 / x2[e]);
+        p1[e] = x1[e];
+        p2[e] = a / x4[e];
+    }
+}
+
+__device__ __forceinline__ double cvb_rel(double nw, double old) { return fabs(nw - old) / old; }
+
+struct CvbArgs {
+    int K, kind, update;      // update = 0: M0 and the posterior means of the unchanged q only (nhp_cont_vb_stats)
+    double T;                 // duration of the data
+    double h[8];              // hyper-parameters as cv_hyper
+    double *q;
+    double *M0;               // [K] in: sum of 1 / Z_i per node; out: M0 = lambda0_eff * that
+    const double *Mn, *Mnm, *S1, *S2;
+    double *lambda0, *W, *p1, *p2;  // in: the effective parameters (lambda0 read by threads e < K); out: the posterior means
+    unsigned long long *change;     // max relative change (|new - old| for mv), as the bits of a non-negative double
+};
+
+// one thread per (p, c) (+ alphav, betav and M0 for e < K): the M-step above in place, then the posterior means; change as k_vb_update
+// (an integer atomicMax per warp: the bit order of non-negative doubles is their numeric order)
+__global__ void __launch_bounds__(256) k_cvb_update(const CvbArgs a) {
+    const int K = a.K;
+    const int64_t KK = (int64_t)K * K;
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    double mx = 0.0;
+    if (e < KK) {
+        double *q = a.q, *kv = q + 2 * K, *nv = kv + KK, *x1 = nv + KK, *x2 = x1 + KK, *x3 = x2 + KK, *x4 = x3 + KK;
+        const bool ln = a.kind == NHP_LOGITNORMAL;
+        if (e < K) {
+            const double m0 = a.lambda0[e] * a.M0[e];
+            a.M0[e] = m0;
+            if (a.update) {
+                const double an = a.h[0] + m0, bn = a.h[1] + a.T;
+                mx = fmax(cvb_rel(an, q[e]), cvb_rel(bn, q[K + e]));
+                q[e] = an;
+                q[K + e] = bn;
+            }
+            a.lambda0[e] = q[e] / q[K + e];
+        }
+        if (a.update) {
+            const double n = a.Mnm[e];
+            const double kn = a.h[2] + n, nn = a.h[3] + a.Mn[e % K];
+            mx = fmax(mx, fmax(cvb_rel(kn, kv[e]), cvb_rel(nn, nv[e])));
+            kv[e] = kn;
+            nv[e] = nn;
+            if (!ln) {
+                const double an = a.h[4] + n, bn = a.h[5] + a.S1[e];
+                mx = fmax(mx, fmax(cvb_rel(an, x1[e]), cvb_rel(bn, x2[e])));
+                x1[e] = an;
+                x2[e] = bn;
+            } else {
+                const double mumu = a.h[4], kmu = a.h[5];
+                const double d = n > 0.0 ? a.S1[e] / n : 0.0;
+                const double ybar = x1[e] + d, S = fmax(a.S2[e] - n * d * d, 0.0);
+                const double lv = kmu + n, mv = (kmu * mumu + n * ybar) / lv, av = a.h[6] + 0.5 * n;
+                const double dm = ybar - mumu;
+                const double bv = a.h[7] + 0.5 * S + kmu * n * dm * dm / (2.0 * lv);
+                mx = fmax(mx, fabs(mv - x1[e]));
+                mx = fmax(mx, fmax(cvb_rel(lv, x2[e]), fmax(cvb_rel(av, x3[e]), cvb_rel(bv, x4[e]))));
+                x1[e] = mv; x2[e] = lv; x3[e] = av; x4[e] = bv;
+            }
+        }
+        a.W[e] = kv[e] / nv[e];
+        if (!ln) a.p1[e] = x1[e] / x2[e];
+        else { a.p1[e] = x1[e]; a.p2[e] = x3[e] / x4[e]; }
+    }
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
+    if ((threadIdx.x & 31) == 0 && mx > 0.0) atomicMax(a.change, (unsigned long long)__double_as_longlong(mx));
+}
+
+int nhp_cont_params_refresh(nhp_ctx *ctx);  // cont_conjugate.cu
+int nhp_cont_fill_args(nhp_ctx *ctx, nhp_events *ev, int recursive, SweepArgs &a);            // cont_sweep.cu
+int nhp_cont_run_event_intensity(nhp_ctx *ctx, nhp_events *ev, int recursive, double *d_out);  // cont_sweep.cu
+int nhp_cont_child_scatter(nhp_ctx *ctx, nhp_events *ev, SweepArgs &a, const double *lam, int terms, double *g_l0, double *g_w, double *g_p1,
+                           double *g_p2, int *grid_out);  // cont_grad.cu
+constexpr int CVB_TERMS = 1;                              // TERMS_VB of cont_grad.cu
+
+extern "C" int nhp_cont_vb_set(nhp_ctx *ctx, const double *hyper, int n_hyper, const double *q) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    NHP_CHECK(ctx, ctx->cont_set, NHP_ERR_STATE, "nhp_cont_vb_set: continuous parameters not set (kind, K and dtmax come from nhp_cont_params_set)");
+    NHP_CHECK(ctx, hyper != nullptr && q != nullptr, NHP_ERR_INVALID, "nhp_cont_vb_set: NULL argument");
+    const int kind = ctx->kind;
+    const int64_t K = ctx->K, KK = K * K;
+    const int want = kind == NHP_LOGITNORMAL ? 8 : 6;
+    NHP_CHECK(ctx, n_hyper == want, NHP_ERR_INVALID, "nhp_cont_vb_set: expected %d hyper-parameters, got %d", want, n_hyper);
+    for (int i = 0; i < n_hyper; i++) {
+        const bool mumu = kind == NHP_LOGITNORMAL && i == 4;  // the prior mean of mu may have any sign
+        NHP_CHECK(ctx, std::isfinite(hyper[i]) && (mumu || hyper[i] > 0.0), NHP_ERR_INVALID, "nhp_cont_vb_set: hyper-parameter %d must be %s", i,
+                  mumu ? "finite" : "positive and finite");
+    }
+    const size_t n = cvb_q_doubles(kind, K);
+    const size_t mv_lo = (size_t)(2 * K + 2 * KK), mv_hi = kind == NHP_LOGITNORMAL ? mv_lo + (size_t)KK : mv_lo;
+    for (size_t i = 0; i < n; i++) {
+        if (i >= mv_lo && i < mv_hi)
+            NHP_CHECK(ctx, std::isfinite(q[i]), NHP_ERR_INVALID, "nhp_cont_vb_set: q[%zu] = %g (mv) is not finite", i, q[i]);
+        else
+            NHP_CHECK(ctx, q[i] > 0.0 && std::isfinite(q[i]), NHP_ERR_INVALID, "nhp_cont_vb_set: q[%zu] = %g is not positive and finite", i, q[i]);
+    }
+    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (ctx->cv_cap < n + 1) {
+        NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        cudaFree(ctx->cv_q); ctx->cv_q = nullptr; ctx->cv_cap = 0; ctx->cv_set = false;
+        NHP_CUDA(ctx, cudaMalloc(&ctx->cv_q, (n + 1) * sizeof(double)));
+        ctx->cv_cap = n + 1;
+    }
+    NHP_CUDA(ctx, cudaMemcpyAsync(ctx->cv_q, q, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the caller may reuse q after return
+    ctx->cv_kind = kind; ctx->cv_K = K;
+    for (int i = 0; i < 8; i++) ctx->cv_hyper[i] = i < n_hyper ? hyper[i] : 0.0;
+    ctx->cv_set = true;
+    return NHP_OK;
+}
+
+extern "C" int nhp_cont_vb_get(nhp_ctx *ctx, double *q) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    NHP_CHECK(ctx, ctx->cv_set, NHP_ERR_STATE, "nhp_cont_vb_get: no VB state (call nhp_cont_vb_set)");
+    NHP_CHECK(ctx, q != nullptr, NHP_ERR_INVALID, "nhp_cont_vb_get: NULL argument");
+    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
+    NHP_CUDA(ctx, cudaMemcpyAsync(q, ctx->cv_q, cvb_q_doubles(ctx->cv_kind, ctx->cv_K) * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return NHP_OK;
+}
+
+// The E-step (and with `update` the M-step) on ev; every refusal comes before anything changes.  The statistics stay in the
+// statistics buffers: M0, Mn, Mnm, S1 in phase 0, S2 in phase 1.
+static int cvb_run(nhp_ctx *ctx, nhp_events *ev, const char *fn, bool update) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    NHP_CHECK(ctx, ev != nullptr, NHP_ERR_INVALID, "%s: events handle is NULL", fn);
+    NHP_CHECK(ctx, ctx->cont_set, NHP_ERR_STATE, "%s: continuous parameters not set (call nhp_cont_params_set)", fn);
+    NHP_CHECK(ctx, !ctx->has_A, NHP_ERR_UNSUPPORTED, "%s runs a standard process (the parameters have an adjacency matrix)", fn);
+    NHP_CHECK(ctx, ctx->bgrid_n == 0, NHP_ERR_UNSUPPORTED, "%s takes a homogeneous baseline (LogGaussianCox curves are set)", fn);
+    NHP_CHECK(ctx, ev->n_halo == 0 && ev->index_base == 0, NHP_ERR_UNSUPPORTED, "%s works on unsharded events", fn);
+    NHP_CHECK(ctx, !(ctx->comm && ctx->nranks > 1), NHP_ERR_UNSUPPORTED, "%s runs on one GPU (the context has a communicator of %d ranks)", fn, ctx->nranks);
+    NHP_CHECK(ctx, ctx->cv_set, NHP_ERR_STATE, "%s: no VB state (call nhp_cont_vb_set)", fn);
+    NHP_CHECK(ctx, ctx->cv_kind == ctx->kind && ctx->cv_K == ctx->K, NHP_ERR_STATE,
+              "%s: the VB state was set for kind %d, K=%lld; the parameters now have kind %d, K=%lld", fn, ctx->cv_kind, (long long)ctx->cv_K, ctx->kind,
+              (long long)ctx->K);
+    NHP_CHECK(ctx, ev->K == ctx->K, NHP_ERR_INVALID, "%s: events were uploaded with K=%lld but the VB state has K=%lld", fn, (long long)ev->K, (long long)ctx->K);
+    NHP_CHECK(ctx, !update || ctx->cv_trace_cap == 0 || (ctx->cv_trace_K == ctx->K && ctx->cv_trace_kind == ctx->kind), NHP_ERR_STATE,
+              "%s: the open VB trace was begun for kind %d, K=%lld", fn, ctx->cv_trace_kind, (long long)ctx->cv_trace_K);
+    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
+    const int64_t K = ctx->K, KK = K * K, own = ev->n;
+    const size_t nq = cvb_q_doubles(ctx->kind, K);
+    const StatsLayout sl{K};
+    const unsigned blocks = (unsigned)((KK + 255) / 256);
+    cudaStream_t s = ctx->stream;
+    // effective parameters -> the context's parameters and tables
+    k_cvb_expect<<<blocks, 256, 0, s>>>(ctx->cv_q, (int)K, ctx->kind, ctx->d_lambda0, ctx->d_W, ctx->d_p1, ctx->d_p2);
+    NHP_LAUNCHED(ctx);
+    NHP_CUDA(ctx, cudaGetLastError());
+    ctx->cont_set = false;
+    ctx->parents_valid = false;
+    ctx->sweep_ll_valid = false;
+    ctx->grad_valid = false;
+    NHP_TRY(nhp_cont_params_refresh(ctx));
+    ctx->cont_set = true;
+    double *st = ctx->d_stats0;
+    NHP_CUDA(ctx, cudaMemsetAsync(st, 0, (size_t)sl.total() * sizeof(double), s));
+    NHP_CUDA(ctx, cudaMemcpyAsync(st + sl.off_Mn(), ev->d_Mn, (size_t)K * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    NHP_CUDA(ctx, cudaMemsetAsync(ctx->d_stats1, 0, (size_t)KK * sizeof(double), s));
+    double *d_change = ctx->cv_q + nq;
+    NHP_CUDA(ctx, cudaMemsetAsync(d_change, 0, sizeof(double), s));
+    if (own > 0) {
+        SweepArgs a;
+        NHP_TRY(nhp_cont_fill_args(ctx, ev, 0, a));
+        void *scratch;  // sweep 1: Z_i (nothing else uses the scratch area until the call returns)
+        NHP_TRY(nhp_scratch(ctx, (size_t)own * sizeof(double), &scratch));
+        NHP_TRY(nhp_cont_run_event_intensity(ctx, ev, 0, (double *)scratch));
+        int grid = 0;   // sweep 2: the expected statistics
+        NHP_TRY(nhp_cont_child_scatter(ctx, ev, a, (const double *)scratch, CVB_TERMS, st + sl.off_M0(), st + sl.off_Mnm(), st + sl.off_S1(), ctx->d_stats1, &grid));
+    }
+    CvbArgs ca;
+    ca.K = (int)K; ca.kind = ctx->kind; ca.update = update ? 1 : 0; ca.T = ev->duration;
+    for (int i = 0; i < 8; i++) ca.h[i] = ctx->cv_hyper[i];
+    ca.q = ctx->cv_q; ca.M0 = st + sl.off_M0(); ca.Mn = st + sl.off_Mn(); ca.Mnm = st + sl.off_Mnm(); ca.S1 = st + sl.off_S1(); ca.S2 = ctx->d_stats1;
+    ca.lambda0 = ctx->d_lambda0; ca.W = ctx->d_W; ca.p1 = ctx->d_p1; ca.p2 = ctx->d_p2; ca.change = (unsigned long long *)d_change;
+    k_cvb_update<<<blocks, 256, 0, s>>>(ca);
+    NHP_LAUNCHED(ctx);
+    NHP_CUDA(ctx, cudaGetLastError());
+    // the posterior means are the context's parameters from here on
+    ctx->cont_set = false;
+    NHP_TRY(nhp_cont_params_refresh(ctx));
+    ctx->cont_set = true;
+    if (update && ctx->cv_trace_cap > 0 && ctx->cv_trace_len < ctx->cv_trace_cap) {  // the state of this step stays on the device
+        NHP_CUDA(ctx, cudaMemcpyAsync(ctx->cv_trace + (size_t)ctx->cv_trace_len * nq, ctx->cv_q, nq * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        ctx->cv_trace_len++;
+    }
+    return NHP_OK;
+}
+
+extern "C" int nhp_cont_vb_stats(nhp_ctx *ctx, nhp_events *ev, double *M0, double *Mnm, double *S1, double *S2) {
+    NHP_TRY(cvb_run(ctx, ev, "nhp_cont_vb_stats", false));
+    const int64_t K = ctx->K, KK = K * K;
+    const StatsLayout sl{K};
+    cudaStream_t s = ctx->stream;
+    if (M0) NHP_CUDA(ctx, cudaMemcpyAsync(M0, ctx->d_stats0 + sl.off_M0(), (size_t)K * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (Mnm) NHP_CUDA(ctx, cudaMemcpyAsync(Mnm, ctx->d_stats0 + sl.off_Mnm(), (size_t)KK * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (S1) NHP_CUDA(ctx, cudaMemcpyAsync(S1, ctx->d_stats0 + sl.off_S1(), (size_t)KK * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (S2) NHP_CUDA(ctx, cudaMemcpyAsync(S2, ctx->d_stats1, (size_t)KK * sizeof(double), cudaMemcpyDeviceToHost, s));
+    NHP_CUDA(ctx, cudaStreamSynchronize(s));
+    return NHP_OK;
+}
+
+extern "C" int nhp_cont_vb_step(nhp_ctx *ctx, nhp_events *ev, double *change) {
+    NHP_TRY(nhp_timer_begin(ctx));
+    NHP_TRY(cvb_run(ctx, ev, "nhp_cont_vb_step", true));
+    if (change) NHP_CUDA(ctx, cudaMemcpyAsync(change, ctx->cv_q + cvb_q_doubles(ctx->kind, ctx->K), sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    NHP_TRY(nhp_timer_end(ctx));
+    return NHP_OK;
+}
+
+extern "C" int nhp_cont_vb_trace_free(nhp_ctx *ctx) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    cudaSetDevice(ctx->device);
+    cudaStreamSynchronize(ctx->stream);
+    cudaFree(ctx->cv_trace);
+    ctx->cv_trace = nullptr; ctx->cv_trace_cap = ctx->cv_trace_len = 0;
+    return NHP_OK;
+}
+
+extern "C" int nhp_cont_vb_trace_begin(nhp_ctx *ctx, int64_t capacity) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    NHP_CHECK(ctx, ctx->cv_set, NHP_ERR_STATE, "nhp_cont_vb_trace_begin: no VB state (the slot size follows it; call nhp_cont_vb_set)");
+    NHP_CHECK(ctx, capacity >= 1, NHP_ERR_INVALID, "nhp_cont_vb_trace_begin: capacity must be positive");
+    NHP_TRY(nhp_cont_vb_trace_free(ctx));
+    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t n = cvb_q_doubles(ctx->cv_kind, ctx->cv_K);
+    if (cudaMalloc(&ctx->cv_trace, (size_t)capacity * n * sizeof(double)) != cudaSuccess) {
+        cudaGetLastError();
+        ctx->cv_trace = nullptr;
+        return nhp_fail(ctx, NHP_ERR_CUDA, "nhp_cont_vb_trace_begin: cannot allocate %lld slots of %.2f MB", (long long)capacity, 1e-6 * (double)(n * 8));
+    }
+    ctx->cv_trace_cap = capacity; ctx->cv_trace_len = 0; ctx->cv_trace_K = ctx->cv_K; ctx->cv_trace_kind = ctx->cv_kind;
+    return NHP_OK;
+}
+
+extern "C" int nhp_cont_vb_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity) {
+    if (!ctx) return NHP_ERR_INVALID;
+    if (count) *count = ctx->cv_trace_len;
+    if (capacity) *capacity = ctx->cv_trace_cap;
+    return NHP_OK;
+}
+
+extern "C" int nhp_cont_vb_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *q_out) {
+    NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
+    NHP_CHECK(ctx, first >= 0 && count >= 0 && first + count <= ctx->cv_trace_len, NHP_ERR_INVALID, "nhp_cont_vb_trace_read: slots [%lld, %lld) outside the %lld stored",
+              (long long)first, (long long)(first + count), (long long)ctx->cv_trace_len);
+    if (count == 0) return NHP_OK;
+    NHP_CHECK(ctx, q_out != nullptr, NHP_ERR_INVALID, "nhp_cont_vb_trace_read: NULL argument");
+    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t n = cvb_q_doubles(ctx->cv_trace_kind, ctx->cv_trace_K);
+    NHP_CUDA(ctx, cudaMemcpyAsync(q_out, ctx->cv_trace + (size_t)first * n, (size_t)count * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return NHP_OK;
+}

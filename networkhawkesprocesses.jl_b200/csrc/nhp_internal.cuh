@@ -244,6 +244,15 @@ struct nhp_ctx {
     double *dv_q = nullptr; size_t dv_cap = 0;  // doubles allocated
     double *dv_trace = nullptr;                 // [dv_trace_cap] slots of q for (dv_trace_N, dv_trace_B, dv_trace_network)
     int64_t dv_trace_cap = 0, dv_trace_len = 0, dv_trace_N = 0, dv_trace_B = 0; bool dv_trace_network = false;
+
+    // ---- continuous mean-field VB (cont_vb.cu): q = [alphav(K); betav(K); kappav(K^2); nuv(K^2)], then Exponential atheta(K^2);
+    // btheta(K^2) | LogitNormal mv(K^2); lambdav(K^2); av(K^2); bv(K^2); the kind and K of the parameters at nhp_cont_vb_set
+    bool cv_set = false;
+    int cv_kind = 0; int64_t cv_K = 0;
+    double cv_hyper[8] = {0};                   // alpha0, beta0, kappa, nu, then alpha, beta | mumu, kappamu, a0, b0
+    double *cv_q = nullptr; size_t cv_cap = 0;  // doubles allocated: the state and one change slot behind it
+    double *cv_trace = nullptr;                 // [cv_trace_cap] slots of q for (cv_trace_kind, cv_trace_K)
+    int64_t cv_trace_cap = 0, cv_trace_len = 0, cv_trace_K = 0; int cv_trace_kind = 0;
 };
 
 // launch bookkeeping

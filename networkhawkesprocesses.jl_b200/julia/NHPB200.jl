@@ -439,6 +439,41 @@ function mcmc_on_device!(process::ContinuousHawkesProcess, data; nsteps=1000, ba
     return NetworkHawkesProcesses.MarkovChainMonteCarlo(samples, time() - start)
 end
 
+# Mean-field VB of a continuous standard process (the reference's `vb!` is discrete only) with the loop and its trace on the device.
+# The state starts at the priors, q = [αv; βv; vec(κv); vec(νv); vec(aθ); vec(bθ)] (Exponential) or [...; vec(mv); vec(λv); vec(av);
+# vec(bv)] (LogitNormal), and goes up once with the hyper-parameters of the Gibbs draws (nhp_cont_vb_set); every step is one
+# nhp_cont_vb_step (expected parent statistics from two sweeps at the effective parameters, then the conjugate update in place; it
+# appends the new state to the VB trace), one read at the end.  With `rtol`, the loop stops after the first step whose change (largest
+# relative change of a positive entry, absolute change of mv) is <= rtol.  Returns the trace, one state per step; the process holds
+# the posterior means of the last one.  Julia is not installed where this package is built, so this stub has not been run.
+function vb_on_device!(process::ContinuousStandardHawkesProcess, data; max_steps=100, rtol=nothing)
+    process.baseline isa HomogeneousProcess || throw(ArgumentError("vb_on_device!: VB takes a HomogeneousProcess baseline"))
+    ev = device_events(process, data)
+    push_params!(process)
+    b, w, imp = process.baseline, process.weights, process.impulses
+    K = ndims(process); ln = imp isa LogitNormalImpulseResponse
+    fill2(x) = fill(Float64(x), K * K)
+    q = ln ? [fill(Float64(b.α0), K); fill(Float64(b.β0), K); fill2(w.κ); fill2(w.ν); fill2(imp.μμ); fill2(imp.κμ); fill2(imp.α0); fill2(imp.β0)] :
+             [fill(Float64(b.α0), K); fill(Float64(b.β0), K); fill2(w.κ); fill2(w.ν); fill2(imp.α); fill2(imp.β)]
+    hyper = gibbs_hyper(b, w, imp)
+    check(ccall((:nhp_cont_vb_set, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Float64}, Cint, Ptr{Float64}), CTX[], hyper, length(hyper), q))
+    check(ccall((:nhp_cont_vb_trace_begin, LIB[]), Cint, (Ptr{Cvoid}, Int64), CTX[], max_steps))
+    change = Ref{Float64}(0.0)
+    steps = 0
+    for step in 1:max_steps
+        check(ccall((:nhp_cont_vb_step, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}), CTX[], ev.h, change))
+        steps = step
+        rtol !== nothing && change[] <= rtol && break
+    end
+    Q = Matrix{Float64}(undef, length(q), steps)
+    check(ccall((:nhp_cont_vb_trace_read, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}), CTX[], 0, steps, Q))
+    check(ccall((:nhp_cont_vb_trace_free, LIB[]), Cint, (Ptr{Cvoid},), CTX[]))
+    last = Q[:, steps]; P(j) = reshape(last[2K+(j-1)*K*K+1:2K+j*K*K], K, K)   # the planes are column-major X[p, c] already
+    b.λ = last[1:K] ./ last[K+1:2K]; w.W = P(1) ./ P(2)
+    if ln; imp.μ = P(3); imp.τ = P(5) ./ P(6) else imp.θ = P(3) ./ P(4) end
+    return [Q[:, k] for k in 1:steps]
+end
+
 # ================================================== discrete path ===============================================================
 function device_counts(data::AbstractMatrix)
     cached(COUNT_CACHE, data) do

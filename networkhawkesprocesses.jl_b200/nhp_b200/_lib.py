@@ -88,6 +88,14 @@ PROTOTYPES = {
     "nhp_cont_resample_params": (c_int, [c_void_p, c_void_p, c_uint64, c_uint64, c_double, c_void_p, c_int, c_int]),
     "nhp_cont_params_get": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "nhp_cont_loglik_dev": (c_int, [c_void_p, c_void_p, c_int]),
+    "nhp_cont_vb_set": (c_int, [c_void_p, c_void_p, c_int, c_void_p]),
+    "nhp_cont_vb_get": (c_int, [c_void_p, c_void_p]),
+    "nhp_cont_vb_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "nhp_cont_vb_step": (c_int, [c_void_p, c_void_p, c_double_p]),
+    "nhp_cont_vb_trace_begin": (c_int, [c_void_p, c_int64]),
+    "nhp_cont_vb_trace_count": (c_int, [c_void_p, POINTER(c_int64), POINTER(c_int64)]),
+    "nhp_cont_vb_trace_read": (c_int, [c_void_p, c_int64, c_int64, c_void_p]),
+    "nhp_cont_vb_trace_free": (c_int, [c_void_p]),
     "nhp_disc_upload": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, POINTER(c_void_p)]),
     "nhp_disc_free": (c_int, [c_void_p, c_void_p]),
     "nhp_disc_rand": (c_int, [c_void_p, c_int64, c_int64, c_uint64, c_int64, POINTER(c_void_p)]),

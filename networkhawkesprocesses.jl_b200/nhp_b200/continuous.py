@@ -8,7 +8,8 @@ Same names, argument meaning and error behaviour as the reference:
   processes   ContinuousStandardHawkesProcess (continuous.jl:108-112),
               ContinuousNetworkHawkesProcess (continuous.jl:315-321)
   functions   loglikelihood, intensity, resample_parents, sufficient_statistics, resample_ ("resample!"),
-              resample_adjacency_matrix_, mcmc_ ("mcmc!"), mle_ ("mle!"), rand, params / params_
+              resample_adjacency_matrix_, mcmc_ ("mcmc!"), mle_ ("mle!"), rand, params / params_; vb_device_ (mean-field VB
+              of a standard process on the device, which the reference does not have for continuous processes)
 Matrices are numpy arrays indexed X[parent, child] like the Julia ones; nodes are 1-based.
 Everything that touches the event history runs in libnhp on the GPU; the conjugate draws
 (O(K^2) host math) stay here, as they stay in Julia.
@@ -745,6 +746,123 @@ def mcmc_device_(process, data, nsteps=1000, seed=0, baseline_on_device=False):
                 parts = [l0[k]] + imp + [W[k]]
             samples.append(np.concatenate(parts))
         return MarkovChainMonteCarlo(samples, time.time() - t0)
+    finally:
+        if tmp:
+            d.free()
+
+
+# ------------------------------------------------------------------------------------------
+# mean-field VB of a standard process (the reference's vb! is discrete only); the state q lives on the device
+# ------------------------------------------------------------------------------------------
+def _vb_checks(process, name):
+    """ValueError, before any device call, for what the device VB does not run."""
+    if not isinstance(process, ContinuousStandardHawkesProcess):
+        raise ValueError(f"{name}: VB runs a ContinuousStandardHawkesProcess (a network process has no variational adjacency matrix here)")
+    if isinstance(process.baseline, LogGaussianCoxProcess):
+        raise ValueError(f"{name}: VB takes a HomogeneousProcess baseline (LogGaussianCox curves have no variational factor)")
+
+
+def vb_size(process):
+    """Doubles in the variational state q: 2 K + 4 K^2 (Exponential) or 2 K + 6 K^2 (LogitNormal)."""
+    K = process.ndims()
+    return 2 * K + (4 if process.impulses.kind == NHP_EXPONENTIAL else 6) * K * K
+
+
+def prior_variational_params(process):
+    """The default start of VB: q set to the priors.  q = [alphav(K); betav(K); kappav; nuv; then atheta; btheta (Exponential) |
+    mv; lambdav; av; bv (LogitNormal)], each K^2 plane flat as X[p + K c] (the layout of nhp_cont_vb_set)."""
+    _vb_checks(process, "prior_variational_params")
+    K = process.ndims()
+    b, w, imp = process.baseline, process.weights, process.impulses
+    planes = [w.kappa, w.nu] + ([imp.alpha, imp.beta] if imp.kind == NHP_EXPONENTIAL else [imp.mumu, imp.kappamu, imp.alpha0, imp.beta0])
+    return np.concatenate([np.full(K, b.alpha0), np.full(K, b.beta0)] + [np.full(K * K, float(x)) for x in planes])
+
+
+def posterior_means(process, q):
+    """Posterior means of the state q: dict(lambda0 = alphav / betav, W = kappav / nuv, p1 = atheta / btheta | mv, p2 = None | av / bv),
+    matrices [parent, child] -- what the device holds as parameters after a VB call."""
+    K = process.ndims()
+    q = _f64(q).reshape(-1)
+    if q.size != vb_size(process):
+        raise ValueError(f"variational state of {q.size} entries; this process needs {vb_size(process)}")
+    KK = K * K
+    pl = [q[2 * K + j * KK:2 * K + (j + 1) * KK].reshape(K, K).T for j in range((q.size - 2 * K) // KK)]  # [p + K c] -> [p, c]
+    out = dict(lambda0=q[:K] / q[K:2 * K], W=pl[0] / pl[1])
+    if process.impulses.kind == NHP_EXPONENTIAL:
+        out.update(p1=pl[2] / pl[3], p2=None)
+    else:
+        out.update(p1=pl[2].copy(), p2=pl[4] / pl[5])
+    return out
+
+
+def _vb_set(ctx, process, q):
+    q = _f64(q).reshape(-1)
+    if q.size != vb_size(process):
+        raise ValueError(f"variational state of {q.size} entries; this process needs {vb_size(process)}")
+    hy = _hyper(process)
+    process._push(ctx)  # kind, K and dtmax of the state come from the device's parameters
+    ctx.check(ctx.lib.nhp_cont_vb_set(ctx.h, _ptr(hy), hy.size, _ptr(q)))
+    return q
+
+
+def vb_statistics(process, data, q):
+    """The E-step of VB from state q (nhp_cont_vb_stats): the expected Gibbs statistics dict(M0, Mnm, S1, S2), matrices [parent, child].
+    Mnm is the expected parent count, S1 the expected sum of lags (Exponential) or of y - mv with y = logit(lag / dtmax) (LogitNormal),
+    S2 the expected sum of (y - mv)^2 (LogitNormal; zeros for Exponential), M0 the expected baseline count per node.  The host objects
+    do not change; the device's parameters become the posterior means of q."""
+    _vb_checks(process, "vb_statistics")
+    ctx = process._ctx()
+    d, tmp = process._data(data)
+    try:
+        K = process.ndims()
+        _vb_set(ctx, process, q)
+        M0, Mnm, S1, S2 = np.empty(K), np.empty(K * K), np.empty(K * K), np.empty(K * K)
+        ctx.check(ctx.lib.nhp_cont_vb_stats(ctx.h, d.h, _ptr(M0), _ptr(Mnm), _ptr(S1), _ptr(S2)))
+        f = lambda v: v.reshape(K, K).T.copy()
+        return dict(M0=M0, Mnm=f(Mnm), S1=f(S1), S2=f(S2))
+    finally:
+        if tmp:
+            d.free()
+
+
+def vb_device_(process, data, max_steps=100, rtol=None, q0=None, trace=True):
+    """Mean-field VB of a ContinuousStandardHawkesProcess with the loop and the state on the device.  The state q0 (default
+    prior_variational_params) and the hyper-parameters go up once (nhp_cont_vb_set); each step is one nhp_cont_vb_step: the expected
+    parent statistics from two sweeps over the events at the effective parameters, then the conjugate update of q in place.  Without
+    `rtol` it runs max_steps steps; with it, it stops after the first step whose change (the largest |new - old| / old over the positive
+    entries, |new - old| over mv) is <= rtol.  Returns the list of states q, one per step (`trace=True`: they are kept in a device-side
+    trace and come back in one read), or a list holding only the last state (`trace=False`: no trace is kept, which matters at large K:
+    one state of K = 5000 is 800 MB).  The process then holds the posterior means of the last state (and the device does too)."""
+    _vb_checks(process, "vb_device_")
+    if max_steps < 1:
+        return []
+    ctx = process._ctx()
+    d, tmp = process._data(data)
+    try:
+        q = _vb_set(ctx, process, prior_variational_params(process) if q0 is None else q0)
+        change = ctypes.c_double()
+        if trace:
+            ctx.check(ctx.lib.nhp_cont_vb_trace_begin(ctx.h, int(max_steps)))
+        try:
+            steps = 0
+            for _ in range(max_steps):
+                ctx.check(ctx.lib.nhp_cont_vb_step(ctx.h, d.h, ctypes.byref(change)))
+                steps += 1
+                if rtol is not None and change.value <= rtol:
+                    break
+            if trace:
+                out = np.empty((steps, q.size))
+                ctx.check(ctx.lib.nhp_cont_vb_trace_read(ctx.h, 0, steps, _ptr(out)))
+                states = list(out)
+            else:
+                last = np.empty(q.size)
+                ctx.check(ctx.lib.nhp_cont_vb_get(ctx.h, _ptr(last)))
+                states = [last]
+        finally:
+            if trace:
+                ctx.check(ctx.lib.nhp_cont_vb_trace_free(ctx.h))
+        pull_params_(process, ctx)
+        return states
     finally:
         if tmp:
             d.free()
