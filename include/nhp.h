@@ -269,8 +269,31 @@ int nhp_cont_vb_set(nhp_ctx *ctx, const double *hyper, int n_hyper, const double
 int nhp_cont_vb_get(nhp_ctx *ctx, double *q);
 int nhp_cont_vb_stats(nhp_ctx *ctx, nhp_events *ev, double *M0, double *Mnm, double *S1, double *S2);
 int nhp_cont_vb_step(nhp_ctx *ctx, nhp_events *ev, double *change);
-/* Device-side trace of the continuous VB state, independent of every other trace: one slot is q (laid out for the state at _begin);
- * _read copies slots [first, first + count) one after the other. */
+/* Mean-field VB of a continuous network process with a BernoulliNetworkModel, the model of the discrete network VB
+ * (nhp_disc_vb_network_set): A[p,c] ~ Bernoulli(rho), rho ~ Beta(alpha_rho, beta_rho), W | A=1 ~ Gamma(kappa, nu) (the slab), W | A=0 ~
+ * Gamma(kappa0, nu0) (the spike), W entering the intensity directly; lambda0, theta | (mu, tau) with the priors of nhp_cont_vb_set.
+ * The state extends the standard layout: q = [standard q; kappa0v(K*K); nu0v(K*K); pv(K*K); alpharhov; betarhov] (2 K + 7 K*K + 2
+ * doubles for Exponential, 2 K + 9 K*K + 2 for LogitNormal), pv[p + K*c] = q(A[p,c] = 1); hyper = [hyper of nhp_cont_vb_set; kappa0,
+ * nu0, alpha_rho, beta_rho] (10 or 12 entries).  _network_set validates (every hyper-parameter finite and > 0 except mumu; every entry
+ * of q finite and > 0 except mv (finite) and pv (in [0, 1]); otherwise NHP_ERR_INVALID, NHP_ERR_STATE without parameters, and the kept
+ * state is as it was) and keeps a state of network kind; nhp_cont_vb_set keeps a standard one, and the later call decides the kind.
+ * nhp_cont_vb_get, _stats, _step and the VB trace serve both kinds.  On a network state the E-step is the standard one with
+ * lW = pv (psi(kappav) - ln nuv) + (1 - pv) (psi(kappa0v) - ln nu0v) in place of psi(kappav) - ln nuv; no link has a zero effective
+ * weight, so it sweeps the process as a standard one (no adjacency mask, and the events handle's cached pair structure is neither used
+ * nor dropped).  The step's update is the standard one plus, with G = Mnm[p,c] and E = Mn[p], kappa0v = kappa0 + G, nu0v = nu0 + E,
+ *   logit pv = psi(alpharhov) - psi(betarhov) + [lgamma(kappav) - kappav ln nuv] - [lgamma(kappa0v) - kappa0v ln nu0v]
+ *              + [kappa ln nu - lgamma(kappa)] - [kappa0 ln nu0 - lgamma(kappa0)]
+ * (the new kappav, nuv, kappa0v, nu0v; the old q(rho)) and, with S = sum of pv in a fixed order (the same state and statistics give the
+ * same bits), alpharhov = alpha_rho + S, betarhov = beta_rho + K*K - S.  change also covers |new - old| over pv.  After either call
+ * the context holds lambda0 = alphav / betav, W = kappav / nuv (the slab mean), A = [pv > 1/2], p1 and p2 as for the standard state,
+ * and the rho of nhp_cont_network_set = alpharhov / (alpharhov + betarhov), so nhp_cont_loglik, nhp_cont_params_get and a following
+ * nhp_cont_gibbs_sweep see a network process at the VB point estimate.  Refused before anything changes, for a network state:
+ * parameters without an adjacency matrix, a kind or K changed since _set, or an open VB trace begun for the other kind of state
+ * (NHP_ERR_STATE); LogGaussianCox curves, a time shard or more than one rank (NHP_ERR_UNSUPPORTED); events of another K
+ * (NHP_ERR_INVALID).  A standard state still refuses a network process (NHP_ERR_UNSUPPORTED). */
+int nhp_cont_vb_network_set(nhp_ctx *ctx, const double *hyper, int n_hyper, const double *q);
+/* Device-side trace of the continuous VB state, independent of every other trace: one slot is q (laid out for the state at _begin,
+ * standard or network); _read copies slots [first, first + count) one after the other. */
 int nhp_cont_vb_trace_begin(nhp_ctx *ctx, int64_t capacity);
 int nhp_cont_vb_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity);
 int nhp_cont_vb_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *q_out);

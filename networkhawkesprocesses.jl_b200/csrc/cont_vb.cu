@@ -27,21 +27,47 @@
 // (the textbook Normal-Gamma update; it keeps b0 where the Gibbs draw replaces it, quirk Q5).  A pair with n = 0 gets its prior.  The same
 // kernel then writes the posterior means (alphav / betav, kappav / nuv, atheta / btheta | mv, av / bv) into the context's parameters,
 // so a later log-likelihood, intensity or nhp_cont_params_get sees the fitted model.
+//
+// A network state (nhp_cont_vb_network_set) fits the Gamma mixture of the discrete network VB (disc_vb.cu): A[p,c] ~ Bernoulli(rho),
+// rho ~ Beta(alpha_rho, beta_rho), W | A=1 ~ Gamma(kappa, nu) (the slab), W | A=0 ~ Gamma(kappa0, nu0) (the spike), with
+//   q = [standard layout; kappa0v(K^2); nu0v(K^2); pv(K^2); alpharhov; betarhov],  pv[p + K c] = q(A[p,c] = 1).
+// The E-step is the standard one with the mixture lW = pv (psi(kappav) - ln nuv) + (1 - pv) (psi(kappa0v) - ln nu0v): no link has a zero
+// effective weight, so the sweeps run the process as a standard one (no adjacency mask, no cached pair structure).  The M-step is the
+// standard one plus kappa0v = kappa0 + Mnm, nu0v = nu0 + Mn[p] and
+//   logit pv = psi(alpharhov) - psi(betarhov) + [lgamma(kappav) - kappav ln nuv] - [lgamma(kappa0v) - kappa0v ln nu0v] + cprior
+// (new kappav, nuv, kappa0v, nu0v; the old q(rho); cprior = [kappa ln nu - lgamma(kappa)] - [kappa0 ln nu0 - lgamma(kappa0)]), and
+// k_vbn_finish (vb_network.cuh, shared with the discrete step) adds the per-block sums of pv in a fixed order into q(rho).  The context
+// then holds the slab means kappav / nuv as W, A = [pv > 1/2] and rho = alpharhov / (alpharhov + betarhov).
 #include "cont_sweep.cuh"
+#include "vb_network.cuh"
 #include <algorithm>
 #include <cmath>
 
 static size_t cvb_q_doubles(int kind, int64_t K) { return (size_t)(2 * K) + (size_t)(K * K) * (kind == NHP_LOGITNORMAL ? 6 : 4); }
+// the network state: the standard layout, then kappa0v(K^2); nu0v(K^2); pv(K^2); alpharhov; betarhov
+static size_t cvb_state_doubles(int kind, int64_t K, bool network) { return cvb_q_doubles(kind, K) + (network ? (size_t)(3 * K * K) + 2 : 0); }
+// what the state's buffer holds behind q: the change slot, and for a network state lrho and the per-block sums of pv
+static size_t cvb_alloc_doubles(int kind, int64_t K, bool network) {
+    return cvb_state_doubles(kind, K, network) + 1 + (network ? 1 + (size_t)((K * K + 255) / 256) : 0);
+}
 
-// one thread per (p, c), e = p + K c (threads e < K also write lambda0_eff[e]): the effective parameters above
+// one thread per (p, c), e = p + K c (threads e < K also write lambda0_eff[e]): the effective parameters above; NET: lW is the mixture's
+// and thread 0 writes lrho = psi(alpharhov) - psi(betarhov), the prior log-odds of a link
+template <bool NET>
 __global__ void __launch_bounds__(256) k_cvb_expect(const double *__restrict__ q, int K, int kind, double *__restrict__ lambda0, double *__restrict__ W,
-                                                    double *__restrict__ p1, double *__restrict__ p2) {
+                                                    double *__restrict__ p1, double *__restrict__ p2, double *__restrict__ lrho) {
     const int64_t KK = (int64_t)K * K;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= KK) return;
     const double *kv = q + 2 * K, *nv = kv + KK, *x1 = nv + KK, *x2 = x1 + KK;
     if (e < K) lambda0[e] = exp(nhp_digamma(q[e]) - log(q[K + e]));
-    const double lw = nhp_digamma(kv[e]) - log(nv[e]);
+    double lw = nhp_digamma(kv[e]) - log(nv[e]);
+    if constexpr (NET) {
+        const double *k0v = kv + KK * (kind == NHP_LOGITNORMAL ? 6 : 4), *n0v = k0v + KK, *pv = n0v + KK;
+        if (e == 0) *lrho = nhp_digamma(pv[KK]) - nhp_digamma(pv[KK + 1]);
+        const double p = pv[e];
+        lw = p * lw + (1.0 - p) * (nhp_digamma(k0v[e]) - log(n0v[e]));
+    }
     if (kind == NHP_EXPONENTIAL) {
         const double a = x1[e], b = x2[e], th = a / b;
         W[e] = exp(lw + (nhp_digamma(a) - log(b))) / th;
@@ -55,8 +81,6 @@ __global__ void __launch_bounds__(256) k_cvb_expect(const double *__restrict__ q
     }
 }
 
-__device__ __forceinline__ double cvb_rel(double nw, double old) { return fabs(nw - old) / old; }
-
 struct CvbArgs {
     int K, kind, update;      // update = 0: M0 and the posterior means of the unchanged q only (nhp_cont_vb_stats)
     double T;                 // duration of the data
@@ -66,15 +90,23 @@ struct CvbArgs {
     const double *Mn, *Mnm, *S1, *S2;
     double *lambda0, *W, *p1, *p2;  // in: the effective parameters (lambda0 read by threads e < K); out: the posterior means
     unsigned long long *change;     // max relative change (|new - old| for mv), as the bits of a non-negative double
+    // network state only (behind the standard fields, which keep their offsets)
+    double kappa0, nu0, cprior;     // the spike's hyper-parameters and the prior part of logit pv
+    const double *lrho;             // psi(alpharhov) - psi(betarhov) of the old q(rho)
+    double *A;                      // out: [pv > 1/2], the context's adjacency matrix
+    double *psum;                   // out: [gridDim.x] sums of the new pv per block (fixed order)
 };
 
 // one thread per (p, c) (+ alphav, betav and M0 for e < K): the M-step above in place, then the posterior means; change as k_vb_update
-// (an integer atomicMax per warp: the bit order of non-negative doubles is their numeric order)
+// (an integer atomicMax per warp: the bit order of non-negative doubles is their numeric order).  NET: also the spike, pv and A, and
+// the block sums of pv as k_vbn_update (a fixed shuffle tree, then the warps in order)
+template <bool NET>
 __global__ void __launch_bounds__(256) k_cvb_update(const CvbArgs a) {
     const int K = a.K;
     const int64_t KK = (int64_t)K * K;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     double mx = 0.0;
+    double pt = 0.0;  // NET: the new pv of this link
     if (e < KK) {
         double *q = a.q, *kv = q + 2 * K, *nv = kv + KK, *x1 = nv + KK, *x2 = x1 + KK, *x3 = x2 + KK, *x4 = x3 + KK;
         const bool ln = a.kind == NHP_LOGITNORMAL;
@@ -83,7 +115,7 @@ __global__ void __launch_bounds__(256) k_cvb_update(const CvbArgs a) {
             a.M0[e] = m0;
             if (a.update) {
                 const double an = a.h[0] + m0, bn = a.h[1] + a.T;
-                mx = fmax(cvb_rel(an, q[e]), cvb_rel(bn, q[K + e]));
+                mx = fmax(rel_change(an, q[e]), rel_change(bn, q[K + e]));
                 q[e] = an;
                 q[K + e] = bn;
             }
@@ -92,12 +124,20 @@ __global__ void __launch_bounds__(256) k_cvb_update(const CvbArgs a) {
         if (a.update) {
             const double n = a.Mnm[e];
             const double kn = a.h[2] + n, nn = a.h[3] + a.Mn[e % K];
-            mx = fmax(mx, fmax(cvb_rel(kn, kv[e]), cvb_rel(nn, nv[e])));
+            mx = fmax(mx, fmax(rel_change(kn, kv[e]), rel_change(nn, nv[e])));
             kv[e] = kn;
             nv[e] = nn;
+            if constexpr (NET) {
+                double *k0v = kv + KK * (ln ? 6 : 4), *n0v = k0v + KK, *pv = n0v + KK;
+                const double k0 = a.kappa0 + n, n0 = a.nu0 + a.Mn[e % K];
+                const double pn = stable_sigmoid(*a.lrho + (lgamma(kn) - kn * log(nn)) - (lgamma(k0) - k0 * log(n0)) + a.cprior);
+                mx = fmax(mx, fmax(rel_change(k0, k0v[e]), rel_change(n0, n0v[e])));
+                mx = fmax(mx, fabs(pn - pv[e]));
+                k0v[e] = k0; n0v[e] = n0; pv[e] = pn;
+            }
             if (!ln) {
                 const double an = a.h[4] + n, bn = a.h[5] + a.S1[e];
-                mx = fmax(mx, fmax(cvb_rel(an, x1[e]), cvb_rel(bn, x2[e])));
+                mx = fmax(mx, fmax(rel_change(an, x1[e]), rel_change(bn, x2[e])));
                 x1[e] = an;
                 x2[e] = bn;
             } else {
@@ -108,17 +148,40 @@ __global__ void __launch_bounds__(256) k_cvb_update(const CvbArgs a) {
                 const double dm = ybar - mumu;
                 const double bv = a.h[7] + 0.5 * S + kmu * n * dm * dm / (2.0 * lv);
                 mx = fmax(mx, fabs(mv - x1[e]));
-                mx = fmax(mx, fmax(cvb_rel(lv, x2[e]), fmax(cvb_rel(av, x3[e]), cvb_rel(bv, x4[e]))));
+                mx = fmax(mx, fmax(rel_change(lv, x2[e]), fmax(rel_change(av, x3[e]), rel_change(bv, x4[e]))));
                 x1[e] = mv; x2[e] = lv; x3[e] = av; x4[e] = bv;
             }
         }
         a.W[e] = kv[e] / nv[e];
         if (!ln) a.p1[e] = x1[e] / x2[e];
         else { a.p1[e] = x1[e]; a.p2[e] = x3[e] / x4[e]; }
+        if constexpr (NET) {
+            pt = kv[KK * (ln ? 8 : 6) + e];  // pv
+            a.A[e] = pt > 0.5 ? 1.0 : 0.0;
+        }
     }
+    if constexpr (!NET) {
 #pragma unroll
-    for (int d = 16; d >= 1; d >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
-    if ((threadIdx.x & 31) == 0 && mx > 0.0) atomicMax(a.change, (unsigned long long)__double_as_longlong(mx));
+        for (int d = 16; d >= 1; d >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
+        if ((threadIdx.x & 31) == 0 && mx > 0.0) atomicMax(a.change, (unsigned long long)__double_as_longlong(mx));
+    } else {
+        __shared__ double warp_sum[8];
+#pragma unroll
+        for (int d = 16; d >= 1; d >>= 1) {
+            mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
+            pt += __shfl_xor_sync(0xffffffffu, pt, d);
+        }
+        if ((threadIdx.x & 31) == 0) {
+            if (mx > 0.0) atomicMax(a.change, (unsigned long long)__double_as_longlong(mx));
+            warp_sum[threadIdx.x >> 5] = pt;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double t = 0.0;
+            for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += warp_sum[w];
+            a.psum[blockIdx.x] = t;
+        }
+    }
 }
 
 int nhp_cont_params_refresh(nhp_ctx *ctx);  // cont_conjugate.cu
@@ -128,40 +191,56 @@ int nhp_cont_child_scatter(nhp_ctx *ctx, nhp_events *ev, SweepArgs &a, const dou
                            double *g_p2, int *grid_out);  // cont_grad.cu
 constexpr int CVB_TERMS = 1;                              // TERMS_VB of cont_grad.cu
 
-extern "C" int nhp_cont_vb_set(nhp_ctx *ctx, const double *hyper, int n_hyper, const double *q) {
+// the two set calls: every hyper-parameter positive and finite except mumu (finite); every entry of q positive and finite except mv
+// (finite) and, for a network state, pv (in [0, 1]); refused before anything changes
+static int cvb_set_state(nhp_ctx *ctx, const char *fn, bool network, const double *hyper, int n_hyper, const double *q) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, ctx->cont_set, NHP_ERR_STATE, "nhp_cont_vb_set: continuous parameters not set (kind, K and dtmax come from nhp_cont_params_set)");
-    NHP_CHECK(ctx, hyper != nullptr && q != nullptr, NHP_ERR_INVALID, "nhp_cont_vb_set: NULL argument");
+    NHP_CHECK(ctx, ctx->cont_set, NHP_ERR_STATE, "%s: continuous parameters not set (kind, K and dtmax come from nhp_cont_params_set)", fn);
+    NHP_CHECK(ctx, hyper != nullptr && q != nullptr, NHP_ERR_INVALID, "%s: NULL argument", fn);
     const int kind = ctx->kind;
     const int64_t K = ctx->K, KK = K * K;
-    const int want = kind == NHP_LOGITNORMAL ? 8 : 6;
-    NHP_CHECK(ctx, n_hyper == want, NHP_ERR_INVALID, "nhp_cont_vb_set: expected %d hyper-parameters, got %d", want, n_hyper);
+    const int nstd = kind == NHP_LOGITNORMAL ? 8 : 6, want = nstd + (network ? 4 : 0);
+    NHP_CHECK(ctx, n_hyper == want, NHP_ERR_INVALID, "%s: expected %d hyper-parameters, got %d", fn, want, n_hyper);
     for (int i = 0; i < n_hyper; i++) {
         const bool mumu = kind == NHP_LOGITNORMAL && i == 4;  // the prior mean of mu may have any sign
-        NHP_CHECK(ctx, std::isfinite(hyper[i]) && (mumu || hyper[i] > 0.0), NHP_ERR_INVALID, "nhp_cont_vb_set: hyper-parameter %d must be %s", i,
+        NHP_CHECK(ctx, std::isfinite(hyper[i]) && (mumu || hyper[i] > 0.0), NHP_ERR_INVALID, "%s: hyper-parameter %d must be %s", fn, i,
                   mumu ? "finite" : "positive and finite");
     }
-    const size_t n = cvb_q_doubles(kind, K);
+    const size_t n = cvb_state_doubles(kind, K, network);
     const size_t mv_lo = (size_t)(2 * K + 2 * KK), mv_hi = kind == NHP_LOGITNORMAL ? mv_lo + (size_t)KK : mv_lo;
+    const size_t p_lo = network ? cvb_q_doubles(kind, K) + (size_t)(2 * KK) : n, p_hi = network ? p_lo + (size_t)KK : n;
     for (size_t i = 0; i < n; i++) {
         if (i >= mv_lo && i < mv_hi)
-            NHP_CHECK(ctx, std::isfinite(q[i]), NHP_ERR_INVALID, "nhp_cont_vb_set: q[%zu] = %g (mv) is not finite", i, q[i]);
+            NHP_CHECK(ctx, std::isfinite(q[i]), NHP_ERR_INVALID, "%s: q[%zu] = %g (mv) is not finite", fn, i, q[i]);
+        else if (i >= p_lo && i < p_hi)
+            NHP_CHECK(ctx, q[i] >= 0.0 && q[i] <= 1.0, NHP_ERR_INVALID, "%s: q[%zu] = %g is a link probability outside [0, 1]", fn, i, q[i]);
         else
-            NHP_CHECK(ctx, q[i] > 0.0 && std::isfinite(q[i]), NHP_ERR_INVALID, "nhp_cont_vb_set: q[%zu] = %g is not positive and finite", i, q[i]);
+            NHP_CHECK(ctx, q[i] > 0.0 && std::isfinite(q[i]), NHP_ERR_INVALID, "%s: q[%zu] = %g is not positive and finite", fn, i, q[i]);
     }
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    if (ctx->cv_cap < n + 1) {
+    const size_t cap = cvb_alloc_doubles(kind, K, network);
+    if (ctx->cv_cap < cap) {
         NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         cudaFree(ctx->cv_q); ctx->cv_q = nullptr; ctx->cv_cap = 0; ctx->cv_set = false;
-        NHP_CUDA(ctx, cudaMalloc(&ctx->cv_q, (n + 1) * sizeof(double)));
-        ctx->cv_cap = n + 1;
+        NHP_CUDA(ctx, cudaMalloc(&ctx->cv_q, cap * sizeof(double)));
+        ctx->cv_cap = cap;
     }
     NHP_CUDA(ctx, cudaMemcpyAsync(ctx->cv_q, q, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the caller may reuse q after return
-    ctx->cv_kind = kind; ctx->cv_K = K;
-    for (int i = 0; i < 8; i++) ctx->cv_hyper[i] = i < n_hyper ? hyper[i] : 0.0;
+    ctx->cv_kind = kind; ctx->cv_K = K; ctx->cv_network = network;
+    for (int i = 0; i < 12; i++) ctx->cv_hyper[i] = 0.0;  // [standard hyper-parameters, zero-padded to 8; kappa0, nu0, alpha_rho, beta_rho]
+    for (int i = 0; i < nstd; i++) ctx->cv_hyper[i] = hyper[i];
+    for (int i = nstd; i < n_hyper; i++) ctx->cv_hyper[8 + i - nstd] = hyper[i];
     ctx->cv_set = true;
     return NHP_OK;
+}
+
+extern "C" int nhp_cont_vb_set(nhp_ctx *ctx, const double *hyper, int n_hyper, const double *q) {
+    return cvb_set_state(ctx, "nhp_cont_vb_set", false, hyper, n_hyper, q);
+}
+
+extern "C" int nhp_cont_vb_network_set(nhp_ctx *ctx, const double *hyper, int n_hyper, const double *q) {
+    return cvb_set_state(ctx, "nhp_cont_vb_network_set", true, hyper, n_hyper, q);
 }
 
 extern "C" int nhp_cont_vb_get(nhp_ctx *ctx, double *q) {
@@ -169,18 +248,23 @@ extern "C" int nhp_cont_vb_get(nhp_ctx *ctx, double *q) {
     NHP_CHECK(ctx, ctx->cv_set, NHP_ERR_STATE, "nhp_cont_vb_get: no VB state (call nhp_cont_vb_set)");
     NHP_CHECK(ctx, q != nullptr, NHP_ERR_INVALID, "nhp_cont_vb_get: NULL argument");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    NHP_CUDA(ctx, cudaMemcpyAsync(q, ctx->cv_q, cvb_q_doubles(ctx->cv_kind, ctx->cv_K) * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    NHP_CUDA(ctx, cudaMemcpyAsync(q, ctx->cv_q, cvb_state_doubles(ctx->cv_kind, ctx->cv_K, ctx->cv_network) * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return NHP_OK;
 }
 
 // The E-step (and with `update` the M-step) on ev; every refusal comes before anything changes.  The statistics stay in the
-// statistics buffers: M0, Mn, Mnm, S1 in phase 0, S2 in phase 1.
+// statistics buffers: M0, Mn, Mnm, S1 in phase 0, S2 in phase 1.  A network state runs the sweeps with has_A cleared (a standard
+// process at the effective parameters), then sets it again with A = [pv > 1/2].
 static int cvb_run(nhp_ctx *ctx, nhp_events *ev, const char *fn, bool update) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
     NHP_CHECK(ctx, ev != nullptr, NHP_ERR_INVALID, "%s: events handle is NULL", fn);
     NHP_CHECK(ctx, ctx->cont_set, NHP_ERR_STATE, "%s: continuous parameters not set (call nhp_cont_params_set)", fn);
-    NHP_CHECK(ctx, !ctx->has_A, NHP_ERR_UNSUPPORTED, "%s runs a standard process (the parameters have an adjacency matrix)", fn);
+    const bool net = ctx->cv_set && ctx->cv_network;
+    if (net)
+        NHP_CHECK(ctx, ctx->has_A, NHP_ERR_STATE, "%s: the VB state is a network state but the parameters have no adjacency matrix", fn);
+    else
+        NHP_CHECK(ctx, !ctx->has_A, NHP_ERR_UNSUPPORTED, "%s runs a standard process (the parameters have an adjacency matrix)", fn);
     NHP_CHECK(ctx, ctx->bgrid_n == 0, NHP_ERR_UNSUPPORTED, "%s takes a homogeneous baseline (LogGaussianCox curves are set)", fn);
     NHP_CHECK(ctx, ev->n_halo == 0 && ev->index_base == 0, NHP_ERR_UNSUPPORTED, "%s works on unsharded events", fn);
     NHP_CHECK(ctx, !(ctx->comm && ctx->nranks > 1), NHP_ERR_UNSUPPORTED, "%s runs on one GPU (the context has a communicator of %d ranks)", fn, ctx->nranks);
@@ -191,15 +275,27 @@ static int cvb_run(nhp_ctx *ctx, nhp_events *ev, const char *fn, bool update) {
     NHP_CHECK(ctx, ev->K == ctx->K, NHP_ERR_INVALID, "%s: events were uploaded with K=%lld but the VB state has K=%lld", fn, (long long)ev->K, (long long)ctx->K);
     NHP_CHECK(ctx, !update || ctx->cv_trace_cap == 0 || (ctx->cv_trace_K == ctx->K && ctx->cv_trace_kind == ctx->kind), NHP_ERR_STATE,
               "%s: the open VB trace was begun for kind %d, K=%lld", fn, ctx->cv_trace_kind, (long long)ctx->cv_trace_K);
+    NHP_CHECK(ctx, !update || ctx->cv_trace_cap == 0 || ctx->cv_trace_network == net, NHP_ERR_STATE, "%s: the open VB trace was begun for a %s state",
+              fn, ctx->cv_trace_network ? "network" : "standard");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     const int64_t K = ctx->K, KK = K * K, own = ev->n;
-    const size_t nq = cvb_q_doubles(ctx->kind, K);
+    const size_t nq = cvb_state_doubles(ctx->kind, K, net);
     const StatsLayout sl{K};
     const unsigned blocks = (unsigned)((KK + 255) / 256);
     cudaStream_t s = ctx->stream;
+    double *d_change = ctx->cv_q + nq, *d_lrho = d_change + 1, *d_psum = d_lrho + 1;  // d_lrho, d_psum: network state only
     // effective parameters -> the context's parameters and tables
-    k_cvb_expect<<<blocks, 256, 0, s>>>(ctx->cv_q, (int)K, ctx->kind, ctx->d_lambda0, ctx->d_W, ctx->d_p1, ctx->d_p2);
+    if (net) {
+        k_cvb_expect<true><<<blocks, 256, 0, s>>>(ctx->cv_q, (int)K, ctx->kind, ctx->d_lambda0, ctx->d_W, ctx->d_p1, ctx->d_p2, d_lrho);
+        ctx->has_A = false;  // the E-step is that of a standard process: no mask, no pair structure (d_A keeps its values until the M-step)
+    } else {
+        k_cvb_expect<false><<<blocks, 256, 0, s>>>(ctx->cv_q, (int)K, ctx->kind, ctx->d_lambda0, ctx->d_W, ctx->d_p1, ctx->d_p2, nullptr);
+    }
     NHP_LAUNCHED(ctx);
+    struct RestoreA {  // a network process again on every way out of this call
+        nhp_ctx *c; bool on;
+        ~RestoreA() { if (on) c->has_A = true; }
+    } restore{ctx, net};
     NHP_CUDA(ctx, cudaGetLastError());
     ctx->cont_set = false;
     ctx->parents_valid = false;
@@ -211,7 +307,6 @@ static int cvb_run(nhp_ctx *ctx, nhp_events *ev, const char *fn, bool update) {
     NHP_CUDA(ctx, cudaMemsetAsync(st, 0, (size_t)sl.total() * sizeof(double), s));
     NHP_CUDA(ctx, cudaMemcpyAsync(st + sl.off_Mn(), ev->d_Mn, (size_t)K * sizeof(double), cudaMemcpyDeviceToDevice, s));
     NHP_CUDA(ctx, cudaMemsetAsync(ctx->d_stats1, 0, (size_t)KK * sizeof(double), s));
-    double *d_change = ctx->cv_q + nq;
     NHP_CUDA(ctx, cudaMemsetAsync(d_change, 0, sizeof(double), s));
     if (own > 0) {
         SweepArgs a;
@@ -227,13 +322,31 @@ static int cvb_run(nhp_ctx *ctx, nhp_events *ev, const char *fn, bool update) {
     for (int i = 0; i < 8; i++) ca.h[i] = ctx->cv_hyper[i];
     ca.q = ctx->cv_q; ca.M0 = st + sl.off_M0(); ca.Mn = st + sl.off_Mn(); ca.Mnm = st + sl.off_Mnm(); ca.S1 = st + sl.off_S1(); ca.S2 = ctx->d_stats1;
     ca.lambda0 = ctx->d_lambda0; ca.W = ctx->d_W; ca.p1 = ctx->d_p1; ca.p2 = ctx->d_p2; ca.change = (unsigned long long *)d_change;
-    k_cvb_update<<<blocks, 256, 0, s>>>(ca);
-    NHP_LAUNCHED(ctx);
+    double rho_q[2] = {0.0, 0.0};  // network state: q(rho) after the step
+    if (net) {
+        const double *hn = ctx->cv_hyper + 8, kappa = ctx->cv_hyper[2], nu = ctx->cv_hyper[3];
+        ca.kappa0 = hn[0]; ca.nu0 = hn[1];
+        ca.cprior = (kappa * std::log(nu) - std::lgamma(kappa)) - (hn[0] * std::log(hn[1]) - std::lgamma(hn[0]));
+        ca.lrho = d_lrho; ca.A = ctx->d_A; ca.psum = d_psum;
+        k_cvb_update<true><<<blocks, 256, 0, s>>>(ca);
+        NHP_LAUNCHED(ctx);
+        if (update) {
+            k_vbn_finish<<<1, 256, 0, s>>>(ctx->cv_q + nq - 2, d_psum, (int)blocks, hn[2], hn[3], (double)KK, 1.0, (unsigned long long *)d_change);
+            NHP_LAUNCHED(ctx);
+        }
+        NHP_CUDA(ctx, cudaMemcpyAsync(rho_q, ctx->cv_q + nq - 2, sizeof(rho_q), cudaMemcpyDeviceToHost, s));  // read after the refresh's synchronisation
+    } else {
+        ca.kappa0 = ca.nu0 = ca.cprior = 0.0; ca.lrho = nullptr; ca.A = nullptr; ca.psum = nullptr;
+        k_cvb_update<false><<<blocks, 256, 0, s>>>(ca);
+        NHP_LAUNCHED(ctx);
+    }
     NHP_CUDA(ctx, cudaGetLastError());
-    // the posterior means are the context's parameters from here on
+    // the posterior means are the context's parameters from here on (a network state: with A = [pv > 1/2])
+    if (net) ctx->has_A = true;
     ctx->cont_set = false;
     NHP_TRY(nhp_cont_params_refresh(ctx));
     ctx->cont_set = true;
+    if (net) ctx->rho = rho_q[0] / (rho_q[0] + rho_q[1]);
     if (update && ctx->cv_trace_cap > 0 && ctx->cv_trace_len < ctx->cv_trace_cap) {  // the state of this step stays on the device
         NHP_CUDA(ctx, cudaMemcpyAsync(ctx->cv_trace + (size_t)ctx->cv_trace_len * nq, ctx->cv_q, nq * sizeof(double), cudaMemcpyDeviceToDevice, s));
         ctx->cv_trace_len++;
@@ -257,7 +370,9 @@ extern "C" int nhp_cont_vb_stats(nhp_ctx *ctx, nhp_events *ev, double *M0, doubl
 extern "C" int nhp_cont_vb_step(nhp_ctx *ctx, nhp_events *ev, double *change) {
     NHP_TRY(nhp_timer_begin(ctx));
     NHP_TRY(cvb_run(ctx, ev, "nhp_cont_vb_step", true));
-    if (change) NHP_CUDA(ctx, cudaMemcpyAsync(change, ctx->cv_q + cvb_q_doubles(ctx->kind, ctx->K), sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    if (change)
+        NHP_CUDA(ctx, cudaMemcpyAsync(change, ctx->cv_q + cvb_state_doubles(ctx->kind, ctx->K, ctx->cv_network), sizeof(double), cudaMemcpyDeviceToHost,
+                                      ctx->stream));
     NHP_TRY(nhp_timer_end(ctx));
     return NHP_OK;
 }
@@ -277,13 +392,14 @@ extern "C" int nhp_cont_vb_trace_begin(nhp_ctx *ctx, int64_t capacity) {
     NHP_CHECK(ctx, capacity >= 1, NHP_ERR_INVALID, "nhp_cont_vb_trace_begin: capacity must be positive");
     NHP_TRY(nhp_cont_vb_trace_free(ctx));
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = cvb_q_doubles(ctx->cv_kind, ctx->cv_K);
+    const size_t n = cvb_state_doubles(ctx->cv_kind, ctx->cv_K, ctx->cv_network);
     if (cudaMalloc(&ctx->cv_trace, (size_t)capacity * n * sizeof(double)) != cudaSuccess) {
         cudaGetLastError();
         ctx->cv_trace = nullptr;
         return nhp_fail(ctx, NHP_ERR_CUDA, "nhp_cont_vb_trace_begin: cannot allocate %lld slots of %.2f MB", (long long)capacity, 1e-6 * (double)(n * 8));
     }
     ctx->cv_trace_cap = capacity; ctx->cv_trace_len = 0; ctx->cv_trace_K = ctx->cv_K; ctx->cv_trace_kind = ctx->cv_kind;
+    ctx->cv_trace_network = ctx->cv_network;
     return NHP_OK;
 }
 
@@ -301,7 +417,7 @@ extern "C" int nhp_cont_vb_trace_read(nhp_ctx *ctx, int64_t first, int64_t count
     if (count == 0) return NHP_OK;
     NHP_CHECK(ctx, q_out != nullptr, NHP_ERR_INVALID, "nhp_cont_vb_trace_read: NULL argument");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = cvb_q_doubles(ctx->cv_trace_kind, ctx->cv_trace_K);
+    const size_t n = cvb_state_doubles(ctx->cv_trace_kind, ctx->cv_trace_K, ctx->cv_trace_network);
     NHP_CUDA(ctx, cudaMemcpyAsync(q_out, ctx->cv_trace + (size_t)first * n, (size_t)count * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return NHP_OK;

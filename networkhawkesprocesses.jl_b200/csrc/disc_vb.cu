@@ -15,7 +15,7 @@
 // nu0v), q(A=1) = pv, q(rho) = Beta(alpharhov, betarhov) appended to q.  The step reuses nhp_disc_vb_reduce as it is: k_vbn_expect
 // adds the mixture E[ln W] to the expectations, k_vbn_update writes the per-link targets and block sums of the new q(A=1), and
 // k_vbn_finish adds those sums in a fixed order into q(rho).
-#include "nhp_internal.cuh"
+#include "vb_network.cuh"  // rel_change, blend, stable_sigmoid, k_vbn_finish
 #include <algorithm>
 #include <cmath>
 
@@ -40,10 +40,6 @@ __global__ void __launch_bounds__(256) k_vb_expect(const double *__restrict__ q,
     double *out = ET + e * B;  // c*N*B + p*B = (p + N c) * B
     for (int b = 0; b < B; b++) out[b] = exp((nhp_digamma(gv[e + NN * b]) - psiS) + lw);
 }
-
-__device__ __forceinline__ double rel_change(double nw, double old) { return fabs(nw - old) / old; }
-
-__device__ __forceinline__ double blend(double old, double target, double step) { return (1.0 - step) * old + step * target; }
 
 // in place, one thread per (p, c) (+ alphav, betav for e < N), the targets
 //   gammav* = gamma + s g,  kappav* = kappa + s sum_b g (b = 0 .. B-1, as k_vb_finish),  nuv* = nu + s events[p],
@@ -104,13 +100,6 @@ __global__ void __launch_bounds__(256) k_vbn_expect(const double *__restrict__ q
     for (int b = 0; b < B; b++) out[b] = exp((nhp_digamma(gv[e + NN * b]) - psiS) + lw);
 }
 
-// 1 / (1 + exp(-x)) without overflow for either sign of x
-__device__ __forceinline__ double stable_sigmoid(double x) {
-    if (x >= 0.0) return 1.0 / (1.0 + exp(-x));
-    const double z = exp(x);
-    return z / (1.0 + z);
-}
-
 // the network state in place, one thread per link (+ alphav, betav for e < N); with ks = sum_b g (b = 0 .. B-1) and E = events[p]
 //   gammav* = gamma + s g,  kappav* = kappa + s ks,  nuv* = nu + s E,  kappa0v* = kappa0 + s ks,  nu0v* = nu0 + s E,
 //   alphav* = alpha0 + s alpha_sum,  betav* = betav_new,
@@ -169,29 +158,6 @@ __global__ void __launch_bounds__(256) k_vbn_update(double *__restrict__ q, cons
         double t = 0.0;
         for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += warp_sum[w];
         psum[blockIdx.x] = t;
-    }
-}
-
-// one block of 256: S = sum of the nblocks partial sums in a fixed order, then alpharhov* = alpha_rho + S, betarhov* = beta_rho + N^2 - S
-// (N^2 counts links, not data: never scaled), blended, their relative change folded into change
-__global__ void __launch_bounds__(256) k_vbn_finish(double *__restrict__ rho, const double *__restrict__ psum, int nblocks, double alpha_rho,
-                                                    double beta_rho, double links, double step, unsigned long long *__restrict__ change) {
-    __shared__ double sh[256];
-    double a = 0.0;
-    for (int i = threadIdx.x; i < nblocks; i += 256) a += psum[i];
-    sh[threadIdx.x] = a;
-    __syncthreads();
-    for (int w = 128; w > 0; w >>= 1) {
-        if ((int)threadIdx.x < w) sh[threadIdx.x] += sh[threadIdx.x + w];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) {
-        const double S = sh[0];
-        const double an = blend(rho[0], alpha_rho + S, step), bn = blend(rho[1], (beta_rho + links) - S, step);
-        const double mx = fmax(rel_change(an, rho[0]), rel_change(bn, rho[1]));
-        rho[0] = an;
-        rho[1] = bn;
-        if (mx > 0.0) atomicMax(change, (unsigned long long)__double_as_longlong(mx));
     }
 }
 

@@ -246,13 +246,14 @@ struct nhp_ctx {
     int64_t dv_trace_cap = 0, dv_trace_len = 0, dv_trace_N = 0, dv_trace_B = 0; bool dv_trace_network = false;
 
     // ---- continuous mean-field VB (cont_vb.cu): q = [alphav(K); betav(K); kappav(K^2); nuv(K^2)], then Exponential atheta(K^2);
-    // btheta(K^2) | LogitNormal mv(K^2); lambdav(K^2); av(K^2); bv(K^2); the kind and K of the parameters at nhp_cont_vb_set
-    bool cv_set = false;
+    // btheta(K^2) | LogitNormal mv(K^2); lambdav(K^2); av(K^2); bv(K^2); the kind and K of the parameters at nhp_cont_vb_set; a network
+    // state (cv_network) appends [kappa0v(K^2); nu0v(K^2); pv(K^2); alpharhov; betarhov]
+    bool cv_set = false, cv_network = false;
     int cv_kind = 0; int64_t cv_K = 0;
-    double cv_hyper[8] = {0};                   // alpha0, beta0, kappa, nu, then alpha, beta | mumu, kappamu, a0, b0
-    double *cv_q = nullptr; size_t cv_cap = 0;  // doubles allocated: the state and one change slot behind it
-    double *cv_trace = nullptr;                 // [cv_trace_cap] slots of q for (cv_trace_kind, cv_trace_K)
-    int64_t cv_trace_cap = 0, cv_trace_len = 0, cv_trace_K = 0; int cv_trace_kind = 0;
+    double cv_hyper[12] = {0};                  // alpha0, beta0, kappa, nu, then alpha, beta, 0, 0 | mumu, kappamu, a0, b0; then kappa0, nu0, alpha_rho, beta_rho (network)
+    double *cv_q = nullptr; size_t cv_cap = 0;  // doubles allocated: the state, one change slot behind it, and for a network state lrho and the block sums of pv
+    double *cv_trace = nullptr;                 // [cv_trace_cap] slots of q for (cv_trace_kind, cv_trace_K, cv_trace_network)
+    int64_t cv_trace_cap = 0, cv_trace_len = 0, cv_trace_K = 0; int cv_trace_kind = 0; bool cv_trace_network = false;
 };
 
 // launch bookkeeping

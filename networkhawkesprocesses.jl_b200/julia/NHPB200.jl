@@ -474,6 +474,46 @@ function vb_on_device!(process::ContinuousStandardHawkesProcess, data; max_steps
     return [Q[:, k] for k in 1:steps]
 end
 
+# Mean-field VB of a continuous network process with a BernoulliNetworkModel: the Gamma mixture of the discrete network VB (slab
+# Gamma(κ, ν) of the weights model, spike Gamma(κ0, ν0), A ~ Bernoulli(ρ), ρ ~ Beta(α, β)).  The state is the standard one at its priors
+# followed by vec(κ0v) = κ0, vec(ν0v) = ν0, vec(pv) = 1 (every link on) and q(ρ) = Beta(α, β) (nhp_cont_vb_network_set); every step
+# is one nhp_cont_vb_step on it.  Returns the trace, one state per step; the process holds the device's point estimate: λ, the slab
+# means of W, A = [pv > 1/2], the impulse's means, and ρ = αρv / (αρv + βρv).  Julia is not installed where this package is built, so
+# this stub has not been run.
+function vb_on_device!(process::ContinuousNetworkHawkesProcess, data; max_steps=100, rtol=nothing, κ0=0.1, ν0=10.0)
+    process.baseline isa HomogeneousProcess || throw(ArgumentError("vb_on_device!: VB takes a HomogeneousProcess baseline"))
+    process.network isa BernoulliNetworkModel || throw(ArgumentError("vb_on_device!: network VB needs a BernoulliNetworkModel"))
+    (κ0 > 0 && isfinite(κ0) && ν0 > 0 && isfinite(ν0)) || throw(ArgumentError("vb_on_device!: κ0 and ν0 must be positive and finite"))
+    ev = device_events(process, data)
+    push_params!(process)
+    b, w, imp, net = process.baseline, process.weights, process.impulses, process.network
+    K = ndims(process); ln = imp isa LogitNormalImpulseResponse
+    fill2(x) = fill(Float64(x), K * K)
+    q = [fill(Float64(b.α0), K); fill(Float64(b.β0), K); fill2(w.κ); fill2(w.ν);
+         (ln ? [fill2(imp.μμ); fill2(imp.κμ); fill2(imp.α0); fill2(imp.β0)] : [fill2(imp.α); fill2(imp.β)]);
+         fill2(κ0); fill2(ν0); fill2(1.0); Float64(net.α); Float64(net.β)]
+    hyper = [gibbs_hyper(b, w, imp); Float64(κ0); Float64(ν0); Float64(net.α); Float64(net.β)]
+    check(ccall((:nhp_cont_vb_network_set, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Float64}, Cint, Ptr{Float64}), CTX[], hyper, length(hyper), q))
+    check(ccall((:nhp_cont_vb_trace_begin, LIB[]), Cint, (Ptr{Cvoid}, Int64), CTX[], max_steps))
+    change = Ref{Float64}(0.0)
+    steps = 0
+    for step in 1:max_steps
+        check(ccall((:nhp_cont_vb_step, LIB[]), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}), CTX[], ev.h, change))
+        steps = step
+        rtol !== nothing && change[] <= rtol && break
+    end
+    Q = Matrix{Float64}(undef, length(q), steps)
+    check(ccall((:nhp_cont_vb_trace_read, LIB[]), Cint, (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}), CTX[], 0, steps, Q))
+    check(ccall((:nhp_cont_vb_trace_free, LIB[]), Cint, (Ptr{Cvoid},), CTX[]))
+    last = Q[:, steps]; P(j) = reshape(last[2K+(j-1)*K*K+1:2K+j*K*K], K, K)   # the planes are column-major X[p, c] already
+    np = ln ? 6 : 4
+    b.λ = last[1:K] ./ last[K+1:2K]; w.W = P(1) ./ P(2)
+    if ln; imp.μ = P(3); imp.τ = P(5) ./ P(6) else imp.θ = P(3) ./ P(4) end
+    process.adjacency_matrix .= P(np + 3) .> 0.5
+    net.ρ = last[end-1] / (last[end-1] + last[end])
+    return [Q[:, k] for k in 1:steps]
+end
+
 # ================================================== discrete path ===============================================================
 function device_counts(data::AbstractMatrix)
     cached(COUNT_CACHE, data) do

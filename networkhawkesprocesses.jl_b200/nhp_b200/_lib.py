@@ -90,6 +90,7 @@ PROTOTYPES = {
     "nhp_cont_loglik_dev": (c_int, [c_void_p, c_void_p, c_int]),
     "nhp_cont_vb_set": (c_int, [c_void_p, c_void_p, c_int, c_void_p]),
     "nhp_cont_vb_get": (c_int, [c_void_p, c_void_p]),
+    "nhp_cont_vb_network_set": (c_int, [c_void_p, c_void_p, c_int, c_void_p]),
     "nhp_cont_vb_stats": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "nhp_cont_vb_step": (c_int, [c_void_p, c_void_p, c_double_p]),
     "nhp_cont_vb_trace_begin": (c_int, [c_void_p, c_int64]),

@@ -9,7 +9,8 @@ Same names, argument meaning and error behaviour as the reference:
               ContinuousNetworkHawkesProcess (continuous.jl:315-321)
   functions   loglikelihood, intensity, resample_parents, sufficient_statistics, resample_ ("resample!"),
               resample_adjacency_matrix_, mcmc_ ("mcmc!"), mle_ ("mle!"), rand, params / params_; vb_device_ (mean-field VB
-              of a standard process on the device, which the reference does not have for continuous processes)
+              of a standard process on the device, which the reference does not have for continuous processes) and
+              network_vb_device_ (the same for a network process, with a variational adjacency matrix)
 Matrices are numpy arrays indexed X[parent, child] like the Julia ones; nodes are 1-based.
 Everything that touches the event history runs in libnhp on the GPU; the conjugate draws
 (O(K^2) host math) stay here, as they stay in Julia.
@@ -840,28 +841,159 @@ def vb_device_(process, data, max_steps=100, rtol=None, q0=None, trace=True):
     d, tmp = process._data(data)
     try:
         q = _vb_set(ctx, process, prior_variational_params(process) if q0 is None else q0)
-        change = ctypes.c_double()
-        if trace:
-            ctx.check(ctx.lib.nhp_cont_vb_trace_begin(ctx.h, int(max_steps)))
-        try:
-            steps = 0
-            for _ in range(max_steps):
-                ctx.check(ctx.lib.nhp_cont_vb_step(ctx.h, d.h, ctypes.byref(change)))
-                steps += 1
-                if rtol is not None and change.value <= rtol:
-                    break
-            if trace:
-                out = np.empty((steps, q.size))
-                ctx.check(ctx.lib.nhp_cont_vb_trace_read(ctx.h, 0, steps, _ptr(out)))
-                states = list(out)
-            else:
-                last = np.empty(q.size)
-                ctx.check(ctx.lib.nhp_cont_vb_get(ctx.h, _ptr(last)))
-                states = [last]
-        finally:
-            if trace:
-                ctx.check(ctx.lib.nhp_cont_vb_trace_free(ctx.h))
+        states = _vb_device_loop(ctx, d, q.size, max_steps, rtol, trace)
         pull_params_(process, ctx)
+        return states
+    finally:
+        if tmp:
+            d.free()
+
+
+def _vb_device_loop(ctx, d, size, max_steps, rtol, trace):
+    """The step loop of vb_device_ and network_vb_device_ on the state the context keeps (`size` doubles): the states of the steps from
+    the device-side trace, or the last state alone."""
+    change = ctypes.c_double()
+    if trace:
+        ctx.check(ctx.lib.nhp_cont_vb_trace_begin(ctx.h, int(max_steps)))
+    try:
+        steps = 0
+        for _ in range(max_steps):
+            ctx.check(ctx.lib.nhp_cont_vb_step(ctx.h, d.h, ctypes.byref(change)))
+            steps += 1
+            if rtol is not None and change.value <= rtol:
+                break
+        if trace:
+            out = np.empty((steps, size))
+            ctx.check(ctx.lib.nhp_cont_vb_trace_read(ctx.h, 0, steps, _ptr(out)))
+            return list(out)
+        last = np.empty(size)
+        ctx.check(ctx.lib.nhp_cont_vb_get(ctx.h, _ptr(last)))
+        return [last]
+    finally:
+        if trace:
+            ctx.check(ctx.lib.nhp_cont_vb_trace_free(ctx.h))
+
+
+# ------------------------------------------------------------------------------------------
+# mean-field VB of a network process (BernoulliNetworkModel), the model of the discrete network VB: A[p,c] ~ Bernoulli(rho),
+# rho ~ Beta(alpha, beta) of the network model, W | A=1 ~ Gamma(kappa, nu) (the slab: the weights model's prior), W | A=0 ~
+# Gamma(kappa0, nu0) (the spike), W entering the intensity directly; lambda0 and the impulse as for vb_device_.  The state is the
+# standard one followed by kappa0v; nu0v; pv; alpharhov; betarhov, with pv[p + K c] = q(A[p,c] = 1).
+# ------------------------------------------------------------------------------------------
+def _network_vb_checks(process, name, kappa0=0.1, nu0=10.0):
+    """ValueError, before any device call, for what the device network VB does not run."""
+    if not isinstance(process, ContinuousNetworkHawkesProcess):
+        raise ValueError(f"{name}: network VB runs a ContinuousNetworkHawkesProcess (vb_device_ runs a standard process)")
+    if not isinstance(process.network, BernoulliNetworkModel):
+        raise ValueError(f"{name}: network VB needs a BernoulliNetworkModel, got {type(process.network).__name__}")
+    if isinstance(process.baseline, LogGaussianCoxProcess):
+        raise ValueError(f"{name}: VB takes a HomogeneousProcess baseline (LogGaussianCox curves have no variational factor)")
+    for nm, v in (("kappa0", kappa0), ("nu0", nu0)):
+        if isinstance(v, (bool, np.bool_)) or not (float(v) > 0.0 and np.isfinite(float(v))):
+            raise ValueError(f"{name}: {nm} = {v!r} must be positive and finite")
+
+
+def network_vb_size(process):
+    """Doubles in the network VB state: 2 K + 7 K^2 + 2 (Exponential) or 2 K + 9 K^2 + 2 (LogitNormal)."""
+    K = process.ndims()
+    return 2 * K + (7 if process.impulses.kind == NHP_EXPONENTIAL else 9) * K * K + 2
+
+
+def network_hyper(process, kappa0=0.1, nu0=10.0):
+    """The hyper-parameters of nhp_cont_vb_network_set: those of nhp_cont_vb_set, then kappa0, nu0 and the network model's alpha, beta."""
+    _network_vb_checks(process, "network_hyper", kappa0, nu0)
+    return np.concatenate([_hyper(process), [float(kappa0), float(nu0), process.network.alpha, process.network.beta]])
+
+
+def network_prior_variational_params(process, pv=1.0, kappa0=0.1, nu0=10.0):
+    """The default start of network VB: the standard factors at their priors (prior_variational_params), kappa0v = kappa0, nu0v = nu0,
+    every link probability pv (default 1: every link on) and q(rho) = Beta(alpha, beta) of the network model."""
+    _network_vb_checks(process, "network_prior_variational_params", kappa0, nu0)
+    pv = float(pv)
+    if not 0.0 <= pv <= 1.0:
+        raise ValueError(f"network_prior_variational_params: pv = {pv!r} is not a probability")
+    K = process.ndims()
+    b, w, imp = process.baseline, process.weights, process.impulses
+    planes = [w.kappa, w.nu] + ([imp.alpha, imp.beta] if imp.kind == NHP_EXPONENTIAL else [imp.mumu, imp.kappamu, imp.alpha0, imp.beta0])
+    planes += [kappa0, nu0, pv]
+    return np.concatenate([np.full(K, b.alpha0), np.full(K, b.beta0)] + [np.full(K * K, float(x)) for x in planes] +
+                          [[process.network.alpha, process.network.beta]])
+
+
+def network_posterior_means(process, q):
+    """Posterior means of a network state: dict(A = pv, W = pv kappav / nuv + (1 - pv) kappa0v / nu0v (the mixture mean), W_slab =
+    kappav / nuv, lambda0, p1, p2 as posterior_means, rho = alpharhov / (alpharhov + betarhov)), matrices [parent, child].  The device
+    holds W_slab as W and [A > 1/2] as the adjacency matrix after a network VB call."""
+    K = process.ndims()
+    q = _f64(q).reshape(-1)
+    if q.size != network_vb_size(process):
+        raise ValueError(f"network variational state of {q.size} entries; this process needs {network_vb_size(process)}")
+    KK, n = K * K, vb_size(process)
+    pl = [q[n + j * KK:n + (j + 1) * KK].reshape(K, K).T for j in range(3)]  # kappa0v, nu0v, pv as [p, c]
+    kv, nv = q[2 * K:2 * K + KK].reshape(K, K).T, q[2 * K + KK:2 * K + 2 * KK].reshape(K, K).T
+    out = dict(lambda0=q[:K] / q[K:2 * K], A=pl[2].copy(), W=pl[2] * kv / nv + (1.0 - pl[2]) * pl[0] / pl[1], W_slab=kv / nv,
+               rho=float(q[-2] / (q[-2] + q[-1])))
+    pl = [q[2 * K + j * KK:2 * K + (j + 1) * KK].reshape(K, K).T for j in range(2, (n - 2 * K) // KK)]
+    if process.impulses.kind == NHP_EXPONENTIAL:
+        out.update(p1=pl[0] / pl[1], p2=None)
+    else:
+        out.update(p1=pl[0].copy(), p2=pl[2] / pl[3])
+    return out
+
+
+def _network_vb_set(ctx, process, q, kappa0, nu0):
+    q = _f64(q).reshape(-1)
+    if q.size != network_vb_size(process):
+        raise ValueError(f"network variational state of {q.size} entries; this process needs {network_vb_size(process)}")
+    hy = network_hyper(process, kappa0, nu0)
+    process._push(ctx)  # kind, K and dtmax of the state come from the device's parameters; the adjacency matrix makes it a network process
+    ctx.check(ctx.lib.nhp_cont_vb_network_set(ctx.h, _ptr(hy), hy.size, _ptr(q)))
+    return q
+
+
+def network_vb_statistics(process, data, q):
+    """The E-step of network VB from state q (nhp_cont_vb_stats on a network state): dict(M0, Mnm, S1, S2) as vb_statistics, with the
+    effective weights of the mixture.  The host objects do not change; the device then holds the point estimate of q (the slab means
+    as W, A = [pv > 1/2], rho)."""
+    _network_vb_checks(process, "network_vb_statistics")
+    q = _f64(q).reshape(-1)
+    if q.size != network_vb_size(process):
+        raise ValueError(f"network variational state of {q.size} entries; this process needs {network_vb_size(process)}")
+    ctx = process._ctx()
+    d, tmp = process._data(data)
+    try:
+        K = process.ndims()
+        _network_vb_set(ctx, process, q, 0.1, 10.0)  # the spike's hyper-parameters do not enter the E-step
+        M0, Mnm, S1, S2 = np.empty(K), np.empty(K * K), np.empty(K * K), np.empty(K * K)
+        ctx.check(ctx.lib.nhp_cont_vb_stats(ctx.h, d.h, _ptr(M0), _ptr(Mnm), _ptr(S1), _ptr(S2)))
+        f = lambda v: v.reshape(K, K).T.copy()
+        return dict(M0=M0, Mnm=f(Mnm), S1=f(S1), S2=f(S2))
+    finally:
+        if tmp:
+            d.free()
+
+
+def network_vb_device_(process, data, max_steps=100, rtol=None, q0=None, trace=True, kappa0=0.1, nu0=10.0):
+    """Mean-field VB of a ContinuousNetworkHawkesProcess with a BernoulliNetworkModel, shaped like vb_device_: the state q0 (default
+    network_prior_variational_params, every link on) and network_hyper go up once (nhp_cont_vb_network_set); each step is one
+    nhp_cont_vb_step on the network state.  Returns the states as vb_device_ does.  The process then holds the device's point estimate
+    (lambda0, the slab means of W, [pv > 1/2] as its adjacency matrix, the impulse's means), network.rho = alpharhov / (alpharhov +
+    betarhov) and network.pv, the link probabilities [parent, child].  A standard process, another network model, a LogGaussianCox
+    baseline, a kappa0 / nu0 that is not positive and finite, or a q0 of the wrong size raise ValueError before any device call."""
+    _network_vb_checks(process, "network_vb_device_", kappa0, nu0)
+    q = network_prior_variational_params(process, 1.0, kappa0, nu0) if q0 is None else _f64(q0).reshape(-1)
+    if q.size != network_vb_size(process):
+        raise ValueError(f"network_vb_device_: variational state of {q.size} entries; this process needs {network_vb_size(process)}")
+    if max_steps < 1:
+        return []
+    ctx = process._ctx()
+    d, tmp = process._data(data)
+    try:
+        _network_vb_set(ctx, process, q, kappa0, nu0)
+        states = _vb_device_loop(ctx, d, q.size, max_steps, rtol, trace)
+        pull_params_(process, ctx)
+        m = network_posterior_means(process, states[-1])
+        process.network.rho, process.network.pv = m["rho"], m["A"]
         return states
     finally:
         if tmp:
