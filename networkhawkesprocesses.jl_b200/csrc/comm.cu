@@ -265,7 +265,7 @@ extern "C" int nhp_cont_gibbs_sweep(nhp_ctx *ctx, nhp_events *ev_shard, nhp_even
         NHP_TRY(nhp_comm_allgather_adjacency(ctx));
         if (net_alpha > 0.0) NHP_TRY(nhp_cont_resample_network(ctx, seed, counter, net_alpha, net_beta, nullptr));
     }
-    if (ctx->trace_cap > 0 && ctx->trace_len < ctx->trace_cap) NHP_TRY(nhp_cont_trace_push(ctx));  // the sample of this sweep stays on the device
+    if (ctx->cont_trace.next()) NHP_TRY(nhp_cont_trace_push(ctx));  // the sample of this sweep stays on the device
     return NHP_OK;
 }
 
@@ -293,7 +293,7 @@ extern "C" int nhp_disc_gibbs_sweep(nhp_ctx *ctx, nhp_disc *dd, uint64_t seed, u
         NHP_TRY(nhp_disc_resample_adjacency_dev(ctx, dd, bern ? -1.0 : 1.0, seed, counter + (1ull << 40)));  // Bernoulli: the context's rho; else dense (1)
         if (bern) NHP_TRY(nhp_disc_draw_network(ctx, seed, counter, net_alpha, net_beta));
     }
-    if (ctx->dd_trace_cap > 0 && ctx->dd_trace_len < ctx->dd_trace_cap) NHP_TRY(nhp_disc_trace_push(ctx));  // the sample stays on the device
+    if (ctx->disc_trace.next()) NHP_TRY(nhp_disc_trace_push(ctx));  // the sample stays on the device
     return NHP_OK;
 }
 

@@ -2,7 +2,8 @@
 // processes; this is the model of the Gibbs sweep, SURVEY section 10, with a factorised posterior).
 //
 // Priors (the hyper-parameters of nhp_cont_resample_params): lambda0_k ~ Gamma(alpha0, beta0), W[p,c] ~ Gamma(kappa, nu), Exponential
-// theta ~ Gamma(alpha, beta), LogitNormal (mu, tau) ~ NormalGamma(mumu, kappamu, a0, b0); all rates.  The state q kept with the context:
+// theta ~ Gamma(alpha, beta), LogitNormal (mu, tau) ~ NormalGamma(mumu, kappamu, a0, b0); all rates.  The state q kept with the context
+//   (ctx->cvb, a VbState: vb_state.cu holds its upload, read-back and trace):
 //   q = [alphav(K); betav(K); kappav(K^2); nuv(K^2); atheta(K^2); btheta(K^2)]                      Exponential
 //   q = [alphav(K); betav(K); kappav(K^2); nuv(K^2); mv(K^2); lambdav(K^2); av(K^2); bv(K^2)]        LogitNormal
 // K^2 planes parent-major, X[p + K c].
@@ -84,7 +85,7 @@ __global__ void __launch_bounds__(256) k_cvb_expect(const double *__restrict__ q
 struct CvbArgs {
     int K, kind, update;      // update = 0: M0 and the posterior means of the unchanged q only (nhp_cont_vb_stats)
     double T;                 // duration of the data
-    double h[8];              // hyper-parameters as cv_hyper
+    double h[8];              // the standard hyper-parameters of the state (ctx->cvb.hyper)
     double *q;
     double *M0;               // [K] in: sum of 1 / Z_i per node; out: M0 = lambda0_eff * that
     const double *Mn, *Mnm, *S1, *S2;
@@ -97,9 +98,8 @@ struct CvbArgs {
     double *psum;                   // out: [gridDim.x] sums of the new pv per block (fixed order)
 };
 
-// one thread per (p, c) (+ alphav, betav and M0 for e < K): the M-step above in place, then the posterior means; change as k_vb_update
-// (an integer atomicMax per warp: the bit order of non-negative doubles is their numeric order).  NET: also the spike, pv and A, and
-// the block sums of pv as k_vbn_update (a fixed shuffle tree, then the warps in order)
+// one thread per (p, c) (+ alphav, betav and M0 for e < K): the M-step above in place, then the posterior means; change and, NET, the
+// block sums of pv by vb_block_reduce.  NET: also the spike, pv and A
 template <bool NET>
 __global__ void __launch_bounds__(256) k_cvb_update(const CvbArgs a) {
     const int K = a.K;
@@ -160,28 +160,7 @@ __global__ void __launch_bounds__(256) k_cvb_update(const CvbArgs a) {
             a.A[e] = pt > 0.5 ? 1.0 : 0.0;
         }
     }
-    if constexpr (!NET) {
-#pragma unroll
-        for (int d = 16; d >= 1; d >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
-        if ((threadIdx.x & 31) == 0 && mx > 0.0) atomicMax(a.change, (unsigned long long)__double_as_longlong(mx));
-    } else {
-        __shared__ double warp_sum[8];
-#pragma unroll
-        for (int d = 16; d >= 1; d >>= 1) {
-            mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
-            pt += __shfl_xor_sync(0xffffffffu, pt, d);
-        }
-        if ((threadIdx.x & 31) == 0) {
-            if (mx > 0.0) atomicMax(a.change, (unsigned long long)__double_as_longlong(mx));
-            warp_sum[threadIdx.x >> 5] = pt;
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            double t = 0.0;
-            for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += warp_sum[w];
-            a.psum[blockIdx.x] = t;
-        }
-    }
+    vb_block_reduce<NET>(mx, pt, a.change, a.psum);
 }
 
 int nhp_cont_params_refresh(nhp_ctx *ctx);  // cont_conjugate.cu
@@ -192,7 +171,7 @@ int nhp_cont_child_scatter(nhp_ctx *ctx, nhp_events *ev, SweepArgs &a, const dou
 constexpr int CVB_TERMS = 1;                              // TERMS_VB of cont_grad.cu
 
 // the two set calls: every hyper-parameter positive and finite except mumu (finite); every entry of q positive and finite except mv
-// (finite) and, for a network state, pv (in [0, 1]); refused before anything changes
+// (finite) and, for a network state, pv (in [0, 1]); refused before anything changes.  The buffer also holds the work slots behind q
 static int cvb_set_state(nhp_ctx *ctx, const char *fn, bool network, const double *hyper, int n_hyper, const double *q) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
     NHP_CHECK(ctx, ctx->cont_set, NHP_ERR_STATE, "%s: continuous parameters not set (kind, K and dtmax come from nhp_cont_params_set)", fn);
@@ -209,29 +188,11 @@ static int cvb_set_state(nhp_ctx *ctx, const char *fn, bool network, const doubl
     const size_t n = cvb_state_doubles(kind, K, network);
     const size_t mv_lo = (size_t)(2 * K + 2 * KK), mv_hi = kind == NHP_LOGITNORMAL ? mv_lo + (size_t)KK : mv_lo;
     const size_t p_lo = network ? cvb_q_doubles(kind, K) + (size_t)(2 * KK) : n, p_hi = network ? p_lo + (size_t)KK : n;
-    for (size_t i = 0; i < n; i++) {
-        if (i >= mv_lo && i < mv_hi)
-            NHP_CHECK(ctx, std::isfinite(q[i]), NHP_ERR_INVALID, "%s: q[%zu] = %g (mv) is not finite", fn, i, q[i]);
-        else if (i >= p_lo && i < p_hi)
-            NHP_CHECK(ctx, q[i] >= 0.0 && q[i] <= 1.0, NHP_ERR_INVALID, "%s: q[%zu] = %g is a link probability outside [0, 1]", fn, i, q[i]);
-        else
-            NHP_CHECK(ctx, q[i] > 0.0 && std::isfinite(q[i]), NHP_ERR_INVALID, "%s: q[%zu] = %g is not positive and finite", fn, i, q[i]);
-    }
-    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t cap = cvb_alloc_doubles(kind, K, network);
-    if (ctx->cv_cap < cap) {
-        NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        cudaFree(ctx->cv_q); ctx->cv_q = nullptr; ctx->cv_cap = 0; ctx->cv_set = false;
-        NHP_CUDA(ctx, cudaMalloc(&ctx->cv_q, cap * sizeof(double)));
-        ctx->cv_cap = cap;
-    }
-    NHP_CUDA(ctx, cudaMemcpyAsync(ctx->cv_q, q, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the caller may reuse q after return
-    ctx->cv_kind = kind; ctx->cv_K = K; ctx->cv_network = network;
-    for (int i = 0; i < 12; i++) ctx->cv_hyper[i] = 0.0;  // [standard hyper-parameters, zero-padded to 8; kappa0, nu0, alpha_rho, beta_rho]
-    for (int i = 0; i < nstd; i++) ctx->cv_hyper[i] = hyper[i];
-    for (int i = nstd; i < n_hyper; i++) ctx->cv_hyper[8 + i - nstd] = hyper[i];
-    ctx->cv_set = true;
+    VbState &st = ctx->cvb;
+    NHP_TRY(nhp_vb_state_set(ctx, st, fn, q, n, cvb_alloc_doubles(kind, K, network), mv_lo, mv_hi, p_lo, p_hi, K, kind, network));
+    for (int i = 0; i < 12; i++) st.hyper[i] = 0.0;  // [standard hyper-parameters, zero-padded to 8; kappa0, nu0, alpha_rho, beta_rho]
+    for (int i = 0; i < nstd; i++) st.hyper[i] = hyper[i];
+    for (int i = nstd; i < n_hyper; i++) st.hyper[8 + i - nstd] = hyper[i];
     return NHP_OK;
 }
 
@@ -245,12 +206,7 @@ extern "C" int nhp_cont_vb_network_set(nhp_ctx *ctx, const double *hyper, int n_
 
 extern "C" int nhp_cont_vb_get(nhp_ctx *ctx, double *q) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, ctx->cv_set, NHP_ERR_STATE, "nhp_cont_vb_get: no VB state (call nhp_cont_vb_set)");
-    NHP_CHECK(ctx, q != nullptr, NHP_ERR_INVALID, "nhp_cont_vb_get: NULL argument");
-    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    NHP_CUDA(ctx, cudaMemcpyAsync(q, ctx->cv_q, cvb_state_doubles(ctx->cv_kind, ctx->cv_K, ctx->cv_network) * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return NHP_OK;
+    return nhp_vb_state_get(ctx, ctx->cvb, "nhp_cont_vb_get", "nhp_cont_vb_set", q);
 }
 
 // The E-step (and with `update` the M-step) on ev; every refusal comes before anything changes.  The statistics stay in the
@@ -260,7 +216,9 @@ static int cvb_run(nhp_ctx *ctx, nhp_events *ev, const char *fn, bool update) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
     NHP_CHECK(ctx, ev != nullptr, NHP_ERR_INVALID, "%s: events handle is NULL", fn);
     NHP_CHECK(ctx, ctx->cont_set, NHP_ERR_STATE, "%s: continuous parameters not set (call nhp_cont_params_set)", fn);
-    const bool net = ctx->cv_set && ctx->cv_network;
+    VbState &vb = ctx->cvb;
+    const DeviceTrace &tr = vb.trace;
+    const bool net = vb.set && vb.network;
     if (net)
         NHP_CHECK(ctx, ctx->has_A, NHP_ERR_STATE, "%s: the VB state is a network state but the parameters have no adjacency matrix", fn);
     else
@@ -268,28 +226,28 @@ static int cvb_run(nhp_ctx *ctx, nhp_events *ev, const char *fn, bool update) {
     NHP_CHECK(ctx, ctx->bgrid_n == 0, NHP_ERR_UNSUPPORTED, "%s takes a homogeneous baseline (LogGaussianCox curves are set)", fn);
     NHP_CHECK(ctx, ev->n_halo == 0 && ev->index_base == 0, NHP_ERR_UNSUPPORTED, "%s works on unsharded events", fn);
     NHP_CHECK(ctx, !(ctx->comm && ctx->nranks > 1), NHP_ERR_UNSUPPORTED, "%s runs on one GPU (the context has a communicator of %d ranks)", fn, ctx->nranks);
-    NHP_CHECK(ctx, ctx->cv_set, NHP_ERR_STATE, "%s: no VB state (call nhp_cont_vb_set)", fn);
-    NHP_CHECK(ctx, ctx->cv_kind == ctx->kind && ctx->cv_K == ctx->K, NHP_ERR_STATE,
-              "%s: the VB state was set for kind %d, K=%lld; the parameters now have kind %d, K=%lld", fn, ctx->cv_kind, (long long)ctx->cv_K, ctx->kind,
+    NHP_CHECK(ctx, vb.set, NHP_ERR_STATE, "%s: no VB state (call nhp_cont_vb_set)", fn);
+    NHP_CHECK(ctx, vb.b == ctx->kind && vb.n == ctx->K, NHP_ERR_STATE,
+              "%s: the VB state was set for kind %d, K=%lld; the parameters now have kind %d, K=%lld", fn, (int)vb.b, (long long)vb.n, ctx->kind,
               (long long)ctx->K);
     NHP_CHECK(ctx, ev->K == ctx->K, NHP_ERR_INVALID, "%s: events were uploaded with K=%lld but the VB state has K=%lld", fn, (long long)ev->K, (long long)ctx->K);
-    NHP_CHECK(ctx, !update || ctx->cv_trace_cap == 0 || (ctx->cv_trace_K == ctx->K && ctx->cv_trace_kind == ctx->kind), NHP_ERR_STATE,
-              "%s: the open VB trace was begun for kind %d, K=%lld", fn, ctx->cv_trace_kind, (long long)ctx->cv_trace_K);
-    NHP_CHECK(ctx, !update || ctx->cv_trace_cap == 0 || ctx->cv_trace_network == net, NHP_ERR_STATE, "%s: the open VB trace was begun for a %s state",
-              fn, ctx->cv_trace_network ? "network" : "standard");
+    NHP_CHECK(ctx, !update || tr.cap == 0 || (tr.shape.n == ctx->K && tr.shape.b == ctx->kind), NHP_ERR_STATE,
+              "%s: the open VB trace was begun for kind %d, K=%lld", fn, (int)tr.shape.b, (long long)tr.shape.n);
+    NHP_CHECK(ctx, !update || tr.cap == 0 || tr.shape.a == net, NHP_ERR_STATE, "%s: the open VB trace was begun for a %s state",
+              fn, tr.shape.a ? "network" : "standard");
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     const int64_t K = ctx->K, KK = K * K, own = ev->n;
-    const size_t nq = cvb_state_doubles(ctx->kind, K, net);
+    const size_t nq = vb.doubles;
     const StatsLayout sl{K};
     const unsigned blocks = (unsigned)((KK + 255) / 256);
     cudaStream_t s = ctx->stream;
-    double *d_change = ctx->cv_q + nq, *d_lrho = d_change + 1, *d_psum = d_lrho + 1;  // d_lrho, d_psum: network state only
+    double *d_change = vb.q + nq, *d_lrho = d_change + 1, *d_psum = d_lrho + 1;  // d_lrho, d_psum: network state only
     // effective parameters -> the context's parameters and tables
     if (net) {
-        k_cvb_expect<true><<<blocks, 256, 0, s>>>(ctx->cv_q, (int)K, ctx->kind, ctx->d_lambda0, ctx->d_W, ctx->d_p1, ctx->d_p2, d_lrho);
+        k_cvb_expect<true><<<blocks, 256, 0, s>>>(vb.q, (int)K, ctx->kind, ctx->d_lambda0, ctx->d_W, ctx->d_p1, ctx->d_p2, d_lrho);
         ctx->has_A = false;  // the E-step is that of a standard process: no mask, no pair structure (d_A keeps its values until the M-step)
     } else {
-        k_cvb_expect<false><<<blocks, 256, 0, s>>>(ctx->cv_q, (int)K, ctx->kind, ctx->d_lambda0, ctx->d_W, ctx->d_p1, ctx->d_p2, nullptr);
+        k_cvb_expect<false><<<blocks, 256, 0, s>>>(vb.q, (int)K, ctx->kind, ctx->d_lambda0, ctx->d_W, ctx->d_p1, ctx->d_p2, nullptr);
     }
     NHP_LAUNCHED(ctx);
     struct RestoreA {  // a network process again on every way out of this call
@@ -319,22 +277,22 @@ static int cvb_run(nhp_ctx *ctx, nhp_events *ev, const char *fn, bool update) {
     }
     CvbArgs ca;
     ca.K = (int)K; ca.kind = ctx->kind; ca.update = update ? 1 : 0; ca.T = ev->duration;
-    for (int i = 0; i < 8; i++) ca.h[i] = ctx->cv_hyper[i];
-    ca.q = ctx->cv_q; ca.M0 = st + sl.off_M0(); ca.Mn = st + sl.off_Mn(); ca.Mnm = st + sl.off_Mnm(); ca.S1 = st + sl.off_S1(); ca.S2 = ctx->d_stats1;
+    for (int i = 0; i < 8; i++) ca.h[i] = vb.hyper[i];
+    ca.q = vb.q; ca.M0 = st + sl.off_M0(); ca.Mn = st + sl.off_Mn(); ca.Mnm = st + sl.off_Mnm(); ca.S1 = st + sl.off_S1(); ca.S2 = ctx->d_stats1;
     ca.lambda0 = ctx->d_lambda0; ca.W = ctx->d_W; ca.p1 = ctx->d_p1; ca.p2 = ctx->d_p2; ca.change = (unsigned long long *)d_change;
     double rho_q[2] = {0.0, 0.0};  // network state: q(rho) after the step
     if (net) {
-        const double *hn = ctx->cv_hyper + 8, kappa = ctx->cv_hyper[2], nu = ctx->cv_hyper[3];
+        const double *hn = vb.hyper + 8, kappa = vb.hyper[2], nu = vb.hyper[3];
         ca.kappa0 = hn[0]; ca.nu0 = hn[1];
         ca.cprior = (kappa * std::log(nu) - std::lgamma(kappa)) - (hn[0] * std::log(hn[1]) - std::lgamma(hn[0]));
         ca.lrho = d_lrho; ca.A = ctx->d_A; ca.psum = d_psum;
         k_cvb_update<true><<<blocks, 256, 0, s>>>(ca);
         NHP_LAUNCHED(ctx);
         if (update) {
-            k_vbn_finish<<<1, 256, 0, s>>>(ctx->cv_q + nq - 2, d_psum, (int)blocks, hn[2], hn[3], (double)KK, 1.0, (unsigned long long *)d_change);
+            k_vbn_finish<<<1, 256, 0, s>>>(vb.q + nq - 2, d_psum, (int)blocks, hn[2], hn[3], (double)KK, 1.0, (unsigned long long *)d_change);
             NHP_LAUNCHED(ctx);
         }
-        NHP_CUDA(ctx, cudaMemcpyAsync(rho_q, ctx->cv_q + nq - 2, sizeof(rho_q), cudaMemcpyDeviceToHost, s));  // read after the refresh's synchronisation
+        NHP_CUDA(ctx, cudaMemcpyAsync(rho_q, vb.q + nq - 2, sizeof(rho_q), cudaMemcpyDeviceToHost, s));  // read after the refresh's synchronisation
     } else {
         ca.kappa0 = ca.nu0 = ca.cprior = 0.0; ca.lrho = nullptr; ca.A = nullptr; ca.psum = nullptr;
         k_cvb_update<false><<<blocks, 256, 0, s>>>(ca);
@@ -347,10 +305,7 @@ static int cvb_run(nhp_ctx *ctx, nhp_events *ev, const char *fn, bool update) {
     NHP_TRY(nhp_cont_params_refresh(ctx));
     ctx->cont_set = true;
     if (net) ctx->rho = rho_q[0] / (rho_q[0] + rho_q[1]);
-    if (update && ctx->cv_trace_cap > 0 && ctx->cv_trace_len < ctx->cv_trace_cap) {  // the state of this step stays on the device
-        NHP_CUDA(ctx, cudaMemcpyAsync(ctx->cv_trace + (size_t)ctx->cv_trace_len * nq, ctx->cv_q, nq * sizeof(double), cudaMemcpyDeviceToDevice, s));
-        ctx->cv_trace_len++;
-    }
+    if (update) NHP_TRY(nhp_vb_trace_push(ctx, vb));  // the state of this step stays on the device
     return NHP_OK;
 }
 
@@ -371,54 +326,28 @@ extern "C" int nhp_cont_vb_step(nhp_ctx *ctx, nhp_events *ev, double *change) {
     NHP_TRY(nhp_timer_begin(ctx));
     NHP_TRY(cvb_run(ctx, ev, "nhp_cont_vb_step", true));
     if (change)
-        NHP_CUDA(ctx, cudaMemcpyAsync(change, ctx->cv_q + cvb_state_doubles(ctx->kind, ctx->K, ctx->cv_network), sizeof(double), cudaMemcpyDeviceToHost,
-                                      ctx->stream));
+        NHP_CUDA(ctx, cudaMemcpyAsync(change, ctx->cvb.q + ctx->cvb.doubles, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     NHP_TRY(nhp_timer_end(ctx));
     return NHP_OK;
 }
 
 extern "C" int nhp_cont_vb_trace_free(nhp_ctx *ctx) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    cudaSetDevice(ctx->device);
-    cudaStreamSynchronize(ctx->stream);
-    cudaFree(ctx->cv_trace);
-    ctx->cv_trace = nullptr; ctx->cv_trace_cap = ctx->cv_trace_len = 0;
+    nhp_trace_free(ctx, ctx->cvb.trace);
     return NHP_OK;
 }
 
 extern "C" int nhp_cont_vb_trace_begin(nhp_ctx *ctx, int64_t capacity) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, ctx->cv_set, NHP_ERR_STATE, "nhp_cont_vb_trace_begin: no VB state (the slot size follows it; call nhp_cont_vb_set)");
-    NHP_CHECK(ctx, capacity >= 1, NHP_ERR_INVALID, "nhp_cont_vb_trace_begin: capacity must be positive");
-    NHP_TRY(nhp_cont_vb_trace_free(ctx));
-    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = cvb_state_doubles(ctx->cv_kind, ctx->cv_K, ctx->cv_network);
-    if (cudaMalloc(&ctx->cv_trace, (size_t)capacity * n * sizeof(double)) != cudaSuccess) {
-        cudaGetLastError();
-        ctx->cv_trace = nullptr;
-        return nhp_fail(ctx, NHP_ERR_CUDA, "nhp_cont_vb_trace_begin: cannot allocate %lld slots of %.2f MB", (long long)capacity, 1e-6 * (double)(n * 8));
-    }
-    ctx->cv_trace_cap = capacity; ctx->cv_trace_len = 0; ctx->cv_trace_K = ctx->cv_K; ctx->cv_trace_kind = ctx->cv_kind;
-    ctx->cv_trace_network = ctx->cv_network;
-    return NHP_OK;
+    return nhp_vb_trace_begin(ctx, ctx->cvb, "nhp_cont_vb_trace_begin", "nhp_cont_vb_set", capacity);
 }
 
 extern "C" int nhp_cont_vb_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity) {
     if (!ctx) return NHP_ERR_INVALID;
-    if (count) *count = ctx->cv_trace_len;
-    if (capacity) *capacity = ctx->cv_trace_cap;
-    return NHP_OK;
+    return nhp_trace_count(ctx->cvb.trace, count, capacity);
 }
 
 extern "C" int nhp_cont_vb_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *q_out) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, first >= 0 && count >= 0 && first + count <= ctx->cv_trace_len, NHP_ERR_INVALID, "nhp_cont_vb_trace_read: slots [%lld, %lld) outside the %lld stored",
-              (long long)first, (long long)(first + count), (long long)ctx->cv_trace_len);
-    if (count == 0) return NHP_OK;
-    NHP_CHECK(ctx, q_out != nullptr, NHP_ERR_INVALID, "nhp_cont_vb_trace_read: NULL argument");
-    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = cvb_state_doubles(ctx->cv_trace_kind, ctx->cv_trace_K, ctx->cv_trace_network);
-    NHP_CUDA(ctx, cudaMemcpyAsync(q_out, ctx->cv_trace + (size_t)first * n, (size_t)count * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return NHP_OK;
+    return nhp_vb_trace_read(ctx, ctx->cvb, "nhp_cont_vb_trace_read", first, count, q_out);
 }

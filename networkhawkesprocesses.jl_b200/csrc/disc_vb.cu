@@ -1,9 +1,10 @@
 // disc_vb.cu -- the discrete mean-field VB step on the device (`update!`, discrete.jl:369-375; `vb!`, inference.jl:153-181).
 //
-// The state q is the reference's variational_params vector (discrete.jl:204-209) kept with the context:
+// The state q is the reference's variational_params vector (discrete.jl:204-209) kept with the context (ctx->dvb, a VbState:
+// vb_state.cu holds its upload, read-back and trace):
 //   q = [alphav(N); betav(N); gammav(N^2 B); kappav(N^2); nuv(N^2)],  gammav[p + N(c + N b)], kappav[p + N c], nuv[p + N c].
-// One step: k_vb_expect turns q into the exp-expectations e0[c] and ET[c][p*B + b] (the statistics kernels' layout, so there is no
-// transpose), nhp_disc_vb_reduce runs the responsibilities and reductions of nhp_disc_vb_stats, k_vb_update writes the new q in place
+// One step: k_dvb_expect turns q into the exp-expectations e0[c] and ET[c][p*B + b] (the statistics kernels' layout, so there is no
+// transpose), nhp_disc_vb_reduce runs the responsibilities and reductions of nhp_disc_vb_stats, k_dvb_update writes the new q in place
 // and reduces the largest relative change.  Only that scalar crosses PCIe.
 //
 // Stochastic VI (Hoffman et al. 2013; the reference's `svi!` is an empty stub) runs the same step on a window of n of the T bins,
@@ -12,46 +13,64 @@
 //
 // A network state (nhp_disc_vb_network_set) fits the Gamma mixture W | A=1 ~ Gamma(kappa, nu), W | A=0 ~ Gamma(kappa0, nu0),
 // A ~ Bernoulli(rho), rho ~ Beta(alpha_rho, beta_rho) with the factors q(W | A=1) = Gamma(kappav, nuv), q(W | A=0) = Gamma(kappa0v,
-// nu0v), q(A=1) = pv, q(rho) = Beta(alpharhov, betarhov) appended to q.  The step reuses nhp_disc_vb_reduce as it is: k_vbn_expect
-// adds the mixture E[ln W] to the expectations, k_vbn_update writes the per-link targets and block sums of the new q(A=1), and
-// k_vbn_finish adds those sums in a fixed order into q(rho).
-#include "vb_network.cuh"  // rel_change, blend, stable_sigmoid, k_vbn_finish
+// nu0v), q(A=1) = pv, q(rho) = Beta(alpharhov, betarhov) appended to q.  The step reuses nhp_disc_vb_reduce as it is: the network
+// instantiations of the two kernels (NET = true) add the mixture E[ln W] to the expectations and write the per-link targets and block
+// sums of the new q(A=1), and k_vbn_finish adds those sums in a fixed order into q(rho).
+#include "vb_network.cuh"  // rel_change, blend, stable_sigmoid, vb_block_reduce, k_vbn_finish
 #include <algorithm>
 #include <cmath>
 
-static size_t vb_q_doubles(int64_t N, int64_t B) { return (size_t)(2 * N) + (size_t)(N * N) * (size_t)(B + 2); }
-// the network state: the standard layout, then kappa0v(N^2); nu0v(N^2); pv(N^2); alpharhov; betarhov
-static size_t vbn_q_doubles(int64_t N, int64_t B) { return (size_t)(2 * N) + (size_t)(N * N) * (size_t)(B + 5) + 2; }
-static size_t vb_state_doubles(int64_t N, int64_t B, bool network) { return network ? vbn_q_doubles(N, B) : vb_q_doubles(N, B); }
+// the standard layout; a network state appends kappa0v(N^2); nu0v(N^2); pv(N^2); alpharhov; betarhov
+static size_t vb_state_doubles(int64_t N, int64_t B, bool network) {
+    return (size_t)(2 * N) + (size_t)(N * N) * (size_t)(B + (network ? 5 : 2)) + (network ? 2 : 0);
+}
 
 // one thread per (p, c), e = p + N c: B + 2 digammas; threads e < N also write e0[e]
 //   e0[c]             = exp(psi(alphav[c]) - log betav[c])                                       baselines.jl:454-456
-//   ET[c][p*B + b]    = exp((psi(gammav[p,c,b]) - psi(sum_b gammav[p,c,:])) + (psi(kappav[p,c]) - log nuv[p,c]))
-//                                                                       impulses.jl:373-375 + weights.jl:95-97, summed as update_ does
-__global__ void __launch_bounds__(256) k_vb_expect(const double *__restrict__ q, int N, int B, double *__restrict__ e0, double *__restrict__ ET) {
+//   ET[c][p*B + b]    = exp((psi(gammav[p,c,b]) - psi(sum_b gammav[p,c,:])) + E[ln W[p,c]])
+//   E[ln W[p,c]]      = psi(kappav) - log nuv                                                    impulses.jl:373-375 + weights.jl:95-97,
+//                                                                                               summed as update_ does
+// NET: the mixture E[ln W[p,c]] = pv (psi(kappav) - log nuv) + (1 - pv) (psi(kappa0v) - log nu0v), and thread 0 writes
+// lrho = psi(alpharhov) - psi(betarhov), the prior log-odds of a link
+template <bool NET>
+__global__ void __launch_bounds__(256) k_dvb_expect(const double *__restrict__ q, int N, int B, double *__restrict__ e0, double *__restrict__ ET,
+                                                    double *__restrict__ lrho) {
     const int64_t NN = (int64_t)N * N;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= NN) return;
     const double *gv = q + 2 * N, *kv = gv + NN * B, *nv = kv + NN;
     if (e < N) e0[e] = exp(nhp_digamma(q[e]) - log(q[N + e]));
+    double lw = nhp_digamma(kv[e]) - log(nv[e]);
+    if constexpr (NET) {
+        const double *k0v = nv + NN, *n0v = k0v + NN, *pv = n0v + NN;
+        if (e == 0) *lrho = nhp_digamma(pv[NN]) - nhp_digamma(pv[NN + 1]);
+        const double p = pv[e];
+        lw = p * lw + (1.0 - p) * (nhp_digamma(k0v[e]) - log(n0v[e]));
+    }
     double S = 0.0;
     for (int b = 0; b < B; b++) S += gv[e + NN * b];
-    const double psiS = nhp_digamma(S), lw = nhp_digamma(kv[e]) - log(nv[e]);
+    const double psiS = nhp_digamma(S);
     double *out = ET + e * B;  // c*N*B + p*B = (p + N c) * B
     for (int b = 0; b < B; b++) out[b] = exp((nhp_digamma(gv[e + NN * b]) - psiS) + lw);
 }
 
-// in place, one thread per (p, c) (+ alphav, betav for e < N), the targets
-//   gammav* = gamma + s g,  kappav* = kappa + s sum_b g (b = 0 .. B-1, as k_vb_finish),  nuv* = nu + s events[p],
-//   alphav* = alpha0 + s alpha_sum,  betav* = betav_new (1/beta0 + T dt, computed on the host, unscaled)
-// blended as q = (1 - step) q + step q*;  change = max |new - old| / old over all of q (bit order of non-negative doubles is their
-// numeric order: an integer atomicMax per warp)
-__global__ void __launch_bounds__(256) k_vb_update(double *__restrict__ q, const double *__restrict__ gammaT, const double *__restrict__ alpha_sum,
-                                                   const double *__restrict__ events, int N, int B, double alpha0, double betav_new, double kappa,
-                                                   double nu, double gamma, double s, double step, unsigned long long *__restrict__ change) {
+// in place, one thread per (p, c) (+ alphav, betav for e < N); with ks = sum_b g (b = 0 .. B-1, as k_vb_finish) and E = events[p]
+//   gammav* = gamma + s g,  kappav* = kappa + s ks,  nuv* = nu + s E,  alphav* = alpha0 + s alpha_sum,
+//   betav* = betav_new (1/beta0 + T dt, computed on the host, unscaled)
+// blended as q = (1 - step) q + step q*;  change = max |new - old| / old over all of q (vb_block_reduce).
+// NET: also kappa0v* = kappa0 + s ks,  nu0v* = nu0 + s E,
+//   pv* = sigmoid(lrho + [lgamma(kappav*) - kappav* log nuv*] - [lgamma(kappa0v*) - kappa0v* log nu0v*] + cprior)
+// where cprior = [kappa log nu - lgamma(kappa)] - [kappa0 log nu0 - lgamma(kappa0)] (the brackets are the log marginal likelihoods of
+// the link's statistics under slab and spike); change takes |new - old| over pv, which may be exactly 0 or 1, and each block writes
+// the sum of its pv* to psum[blockIdx.x]
+template <bool NET>
+__global__ void __launch_bounds__(256) k_dvb_update(double *__restrict__ q, const double *__restrict__ gammaT, const double *__restrict__ alpha_sum,
+                                                    const double *__restrict__ events, const double *__restrict__ lrho, int N, int B, double alpha0,
+                                                    double betav_new, double kappa, double nu, double gamma, double kappa0, double nu0, double cprior,
+                                                    double s, double step, unsigned long long *__restrict__ change, double *__restrict__ psum) {
     const int64_t NN = (int64_t)N * N;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    double mx = 0.0;
+    double mx = 0.0, pt = 0.0;
     if (e < NN) {
         double *gv = q + 2 * N, *kv = gv + NN * B, *nv = kv + NN;
         const double *g = gammaT + e * B;
@@ -64,8 +83,18 @@ __global__ void __launch_bounds__(256) k_vb_update(double *__restrict__ q, const
             mx = fmax(mx, rel_change(nw, old));
             gv[e + NN * b] = nw;
         }
-        const double kn = blend(kv[e], kappa + s * ks, step), nn = blend(nv[e], nu + s * events[e % N], step);
+        const double ev = s * events[e % N], k1 = kappa + s * ks, n1 = nu + ev;
+        const double kn = blend(kv[e], k1, step), nn = blend(nv[e], n1, step);
         mx = fmax(mx, fmax(rel_change(kn, kv[e]), rel_change(nn, nv[e])));
+        if constexpr (NET) {
+            double *k0v = nv + NN, *n0v = k0v + NN, *pv = n0v + NN;
+            const double k0 = kappa0 + s * ks, n0 = nu0 + ev;
+            pt = stable_sigmoid(*lrho + (lgamma(k1) - k1 * log(n1)) - (lgamma(k0) - k0 * log(n0)) + cprior);
+            const double k0n = blend(k0v[e], k0, step), n0n = blend(n0v[e], n0, step), pn = blend(pv[e], pt, step);
+            mx = fmax(mx, fmax(rel_change(k0n, k0v[e]), rel_change(n0n, n0v[e])));
+            mx = fmax(mx, fabs(pn - pv[e]));
+            k0v[e] = k0n; n0v[e] = n0n; pv[e] = pn;
+        }
         kv[e] = kn;
         nv[e] = nn;
         if (e < N) {
@@ -75,94 +104,11 @@ __global__ void __launch_bounds__(256) k_vb_update(double *__restrict__ q, const
             q[N + e] = bn;
         }
     }
-#pragma unroll
-    for (int d = 16; d >= 1; d >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
-    if ((threadIdx.x & 31) == 0 && mx > 0.0) atomicMax(change, (unsigned long long)__double_as_longlong(mx));
-}
-
-// the network state, one thread per link e = p + N c: as k_vb_expect with the mixture
-//   E[ln W[p,c]] = pv (psi(kappav) - log nuv) + (1 - pv) (psi(kappa0v) - log nu0v)
-// in place of psi(kappav) - log nuv; thread 0 also writes lrho = psi(alpharhov) - psi(betarhov), the prior log-odds of a link
-__global__ void __launch_bounds__(256) k_vbn_expect(const double *__restrict__ q, int N, int B, double *__restrict__ e0, double *__restrict__ ET,
-                                                    double *__restrict__ lrho) {
-    const int64_t NN = (int64_t)N * N;
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= NN) return;
-    const double *gv = q + 2 * N, *kv = gv + NN * B, *nv = kv + NN, *k0v = nv + NN, *n0v = k0v + NN, *pv = n0v + NN;
-    if (e < N) e0[e] = exp(nhp_digamma(q[e]) - log(q[N + e]));
-    if (e == 0) *lrho = nhp_digamma(pv[NN]) - nhp_digamma(pv[NN + 1]);
-    const double p = pv[e];
-    const double lw = p * (nhp_digamma(kv[e]) - log(nv[e])) + (1.0 - p) * (nhp_digamma(k0v[e]) - log(n0v[e]));
-    double S = 0.0;
-    for (int b = 0; b < B; b++) S += gv[e + NN * b];
-    const double psiS = nhp_digamma(S);
-    double *out = ET + e * B;
-    for (int b = 0; b < B; b++) out[b] = exp((nhp_digamma(gv[e + NN * b]) - psiS) + lw);
-}
-
-// the network state in place, one thread per link (+ alphav, betav for e < N); with ks = sum_b g (b = 0 .. B-1) and E = events[p]
-//   gammav* = gamma + s g,  kappav* = kappa + s ks,  nuv* = nu + s E,  kappa0v* = kappa0 + s ks,  nu0v* = nu0 + s E,
-//   alphav* = alpha0 + s alpha_sum,  betav* = betav_new,
-//   pv* = sigmoid(lrho + [lgamma(kappav*) - kappav* log nuv*] - [lgamma(kappa0v*) - kappa0v* log nu0v*] + cprior)
-// where cprior = [kappa log nu - lgamma(kappa)] - [kappa0 log nu0 - lgamma(kappa0)] (the brackets are the log marginal likelihoods of
-// the link's statistics under slab and spike), blended as q = (1 - step) q + step q*.  Each block writes the sum of its pv* to
-// psum[blockIdx.x] (a fixed shuffle tree, then the warps in order); change = max of |new - old| / old over the positive entries and
-// |new - old| over pv, which may be exactly 0 or 1
-__global__ void __launch_bounds__(256) k_vbn_update(double *__restrict__ q, const double *__restrict__ gammaT, const double *__restrict__ alpha_sum,
-                                                    const double *__restrict__ events, const double *__restrict__ lrho, int N, int B, double alpha0,
-                                                    double betav_new, double kappa, double nu, double gamma, double kappa0, double nu0, double cprior,
-                                                    double s, double step, unsigned long long *__restrict__ change, double *__restrict__ psum) {
-    __shared__ double warp_sum[8];
-    const int64_t NN = (int64_t)N * N;
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    double mx = 0.0, pt = 0.0;
-    if (e < NN) {
-        double *gv = q + 2 * N, *kv = gv + NN * B, *nv = kv + NN, *k0v = nv + NN, *n0v = k0v + NN, *pv = n0v + NN;
-        const double *g = gammaT + e * B;
-        double ks = 0.0;
-#pragma unroll 1  // as k_vb_update
-        for (int b = 0; b < B; b++) {
-            const double gb = g[b];
-            ks += gb;
-            const double old = gv[e + NN * b], nw = blend(old, gamma + s * gb, step);
-            mx = fmax(mx, rel_change(nw, old));
-            gv[e + NN * b] = nw;
-        }
-        const double ev = s * events[e % N];
-        const double k1 = kappa + s * ks, n1 = nu + ev, k0 = kappa0 + s * ks, n0 = nu0 + ev;
-        pt = stable_sigmoid(*lrho + (lgamma(k1) - k1 * log(n1)) - (lgamma(k0) - k0 * log(n0)) + cprior);
-        const double kn = blend(kv[e], k1, step), nn = blend(nv[e], n1, step);
-        const double k0n = blend(k0v[e], k0, step), n0n = blend(n0v[e], n0, step), pn = blend(pv[e], pt, step);
-        mx = fmax(mx, fmax(rel_change(kn, kv[e]), rel_change(nn, nv[e])));
-        mx = fmax(mx, fmax(rel_change(k0n, k0v[e]), rel_change(n0n, n0v[e])));
-        mx = fmax(mx, fabs(pn - pv[e]));
-        kv[e] = kn; nv[e] = nn; k0v[e] = k0n; n0v[e] = n0n; pv[e] = pn;
-        if (e < N) {
-            const double an = blend(q[e], alpha0 + s * alpha_sum[e], step), bn = blend(q[N + e], betav_new, step);
-            mx = fmax(mx, fmax(rel_change(an, q[e]), rel_change(bn, q[N + e])));
-            q[e] = an;
-            q[N + e] = bn;
-        }
-    }
-#pragma unroll
-    for (int d = 16; d >= 1; d >>= 1) {
-        mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
-        pt += __shfl_xor_sync(0xffffffffu, pt, d);
-    }
-    if ((threadIdx.x & 31) == 0) {
-        if (mx > 0.0) atomicMax(change, (unsigned long long)__double_as_longlong(mx));
-        warp_sum[threadIdx.x >> 5] = pt;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double t = 0.0;
-        for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += warp_sum[w];
-        psum[blockIdx.x] = t;
-    }
+    vb_block_reduce<NET>(mx, pt, change, psum);
 }
 
 // the two set calls: every entry of hyper positive and finite; every entry of q positive and finite except, for a network state,
-// pv (finite, in [0, 1]); refused before anything changes
+// pv (in [0, 1]); refused before anything changes
 static int vb_set_state(nhp_ctx *ctx, const char *fn, bool network, int64_t N, int64_t B, double dt, const double *hyper, int n_hyper, const double *q) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
     NHP_CHECK(ctx, N >= 1 && N <= 32768 && B >= 1, NHP_ERR_INVALID, "%s: bad dimensions N=%lld B=%lld", fn, (long long)N, (long long)B);
@@ -174,24 +120,10 @@ static int vb_set_state(nhp_ctx *ctx, const char *fn, bool network, int64_t N, i
         NHP_CHECK(ctx, hyper[i] > 0.0 && std::isfinite(hyper[i]), NHP_ERR_INVALID, "%s: hyper-parameter %d must be positive and finite", fn, i);
     const size_t n = vb_state_doubles(N, B, network);
     const size_t p_lo = network ? (size_t)(2 * N) + (size_t)(N * N) * (size_t)(B + 4) : n, p_hi = network ? p_lo + (size_t)(N * N) : n;
-    for (size_t i = 0; i < n; i++) {
-        if (i >= p_lo && i < p_hi)
-            NHP_CHECK(ctx, q[i] >= 0.0 && q[i] <= 1.0, NHP_ERR_INVALID, "%s: q[%zu] = %g is a link probability outside [0, 1]", fn, i, q[i]);
-        else
-            NHP_CHECK(ctx, q[i] > 0.0 && std::isfinite(q[i]), NHP_ERR_INVALID, "%s: q[%zu] = %g is not positive and finite", fn, i, q[i]);
-    }
-    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    if (ctx->dv_cap < n) {
-        NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        cudaFree(ctx->dv_q); ctx->dv_q = nullptr; ctx->dv_cap = 0; ctx->dv_set = false;
-        NHP_CUDA(ctx, cudaMalloc(&ctx->dv_q, n * sizeof(double)));
-        ctx->dv_cap = n;
-    }
-    NHP_CUDA(ctx, cudaMemcpyAsync(ctx->dv_q, q, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the caller may reuse q after return
-    ctx->dv_N = N; ctx->dv_B = B; ctx->dv_dt = dt; ctx->dv_network = network;
-    for (int i = 0; i < n_hyper; i++) ctx->dv_hyper[i] = hyper[i];
-    ctx->dv_set = true;
+    VbState &st = ctx->dvb;
+    NHP_TRY(nhp_vb_state_set(ctx, st, fn, q, n, n, 0, 0, p_lo, p_hi, N, B, network));
+    st.dt = dt;
+    for (int i = 0; i < n_hyper; i++) st.hyper[i] = hyper[i];
     return NHP_OK;
 }
 
@@ -205,12 +137,7 @@ extern "C" int nhp_disc_vb_network_set(nhp_ctx *ctx, int64_t N, int64_t B, doubl
 
 extern "C" int nhp_disc_vb_get(nhp_ctx *ctx, double *q) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, ctx->dv_set, NHP_ERR_STATE, "nhp_disc_vb_get: no VB state (call nhp_disc_vb_set)");
-    NHP_CHECK(ctx, q != nullptr, NHP_ERR_INVALID, "nhp_disc_vb_get: NULL argument");
-    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    NHP_CUDA(ctx, cudaMemcpyAsync(q, ctx->dv_q, vb_state_doubles(ctx->dv_N, ctx->dv_B, ctx->dv_network) * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return NHP_OK;
+    return nhp_vb_state_get(ctx, ctx->dvb, "nhp_disc_vb_get", "nhp_disc_vb_set", q);
 }
 
 // One step over the window (t_begin + j) mod T, j < n_bins, blended with `step`; the refusals come before anything changes.  The window
@@ -220,22 +147,24 @@ static int vb_window_step(nhp_ctx *ctx, nhp_disc *dd, const char *fn, int64_t t_
     NHP_CHECK(ctx, dd != nullptr, NHP_ERR_INVALID, "%s: data handle is NULL", fn);
     NHP_CHECK(ctx, dd->t_halo == 0, NHP_ERR_UNSUPPORTED, "%s works on unsharded data", fn);
     NHP_CHECK(ctx, !(ctx->comm && ctx->nranks > 1), NHP_ERR_UNSUPPORTED, "%s runs on one GPU (the context has a communicator of %d ranks)", fn, ctx->nranks);
-    NHP_CHECK(ctx, ctx->dv_set, NHP_ERR_STATE, "%s: no VB state (call nhp_disc_vb_set)", fn);
+    VbState &st = ctx->dvb;
+    const DeviceTrace &tr = st.trace;
+    NHP_CHECK(ctx, st.set, NHP_ERR_STATE, "%s: no VB state (call nhp_disc_vb_set)", fn);
     NHP_CHECK(ctx, dd->d_conv != nullptr, NHP_ERR_STATE, "%s: call nhp_disc_convolve first", fn);
-    const int64_t N = ctx->dv_N, B = ctx->dv_B, NN = N * N, NB = N * B, T = dd->T;
+    const int64_t N = st.n, B = st.b, NN = N * N, NB = N * B, T = dd->T;
     NHP_CHECK(ctx, dd->N == N && dd->B == B, NHP_ERR_INVALID, "%s: the VB state has N=%lld B=%lld, the data N=%lld B=%lld", fn, (long long)N,
               (long long)B, (long long)dd->N, (long long)dd->B);
-    NHP_CHECK(ctx, ctx->dv_trace_cap == 0 || (ctx->dv_trace_N == N && ctx->dv_trace_B == B), NHP_ERR_STATE,
-              "%s: the open VB trace was begun for N=%lld B=%lld", fn, (long long)ctx->dv_trace_N, (long long)ctx->dv_trace_B);
-    NHP_CHECK(ctx, ctx->dv_trace_cap == 0 || ctx->dv_trace_network == ctx->dv_network, NHP_ERR_STATE, "%s: the open VB trace was begun for a %s state",
-              fn, ctx->dv_trace_network ? "network" : "standard");
+    NHP_CHECK(ctx, tr.cap == 0 || (tr.shape.n == N && tr.shape.b == B), NHP_ERR_STATE, "%s: the open VB trace was begun for N=%lld B=%lld", fn,
+              (long long)tr.shape.n, (long long)tr.shape.b);
+    NHP_CHECK(ctx, tr.cap == 0 || tr.shape.a == st.network, NHP_ERR_STATE, "%s: the open VB trace was begun for a %s state", fn,
+              tr.shape.a ? "network" : "standard");
     NHP_CHECK(ctx, t_begin >= 0 && t_begin < T && n_bins >= 1 && n_bins <= T, NHP_ERR_INVALID,
               "%s: window (t_begin=%lld, n_bins=%lld) outside 0 <= t_begin < T, 1 <= n_bins <= T (T=%lld)", fn, (long long)t_begin, (long long)n_bins, (long long)T);
     NHP_CHECK(ctx, step > 0.0 && step <= 1.0, NHP_ERR_INVALID, "%s: step=%g outside (0, 1]", fn, step);
     NHP_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
     void *scratch;
-    const bool net = ctx->dv_network;
+    const bool net = st.network;
     const unsigned blocks = (unsigned)((NN + 255) / 256);
     // layout: e0[N] | ET[N*NB] | gammaT[N*NB] | alpha_sum[N] | events[N] | change (the last four zeroed together), and for a network
     // state | lrho | psum[blocks]
@@ -245,9 +174,9 @@ static int vb_window_step(nhp_ctx *ctx, nhp_disc *dd, const char *fn, int64_t t_
     double *d_lrho = d_change + 1, *d_psum = d_lrho + 1;
     NHP_CUDA(ctx, cudaMemsetAsync(d_gT, 0, (size_t)(NB * N + 2 * N + 1) * sizeof(double), s));
     if (net)
-        k_vbn_expect<<<blocks, 256, 0, s>>>(ctx->dv_q, (int)N, (int)B, d_e0, d_ET, d_lrho);
+        k_dvb_expect<true><<<blocks, 256, 0, s>>>(st.q, (int)N, (int)B, d_e0, d_ET, d_lrho);
     else
-        k_vb_expect<<<blocks, 256, 0, s>>>(ctx->dv_q, (int)N, (int)B, d_e0, d_ET);
+        k_dvb_expect<false><<<blocks, 256, 0, s>>>(st.q, (int)N, (int)B, d_e0, d_ET, nullptr);
     NHP_LAUNCHED(ctx);
     // the window as at most two ranges [t_begin, end) and, when it wraps, [0, t_begin + n_bins - T)
     const int64_t end = std::min(t_begin + n_bins, T), wrap = t_begin + n_bins - end;
@@ -259,28 +188,23 @@ static int vb_window_step(nhp_ctx *ctx, nhp_disc *dd, const char *fn, int64_t t_
         NHP_TRY(nhp_disc_range_events(ctx, dd, 0, wrap, d_events));
         events = d_events;
     }
-    const double *h = ctx->dv_hyper;
-    const double betav = 1.0 / h[1] + (double)T * ctx->dv_dt;  // baselines.jl:450 as written (1 / beta0, not beta0)
+    const double *h = st.hyper;
+    const double betav = 1.0 / h[1] + (double)T * st.dt;  // baselines.jl:450 as written (1 / beta0, not beta0)
     const double scale = (double)T / (double)n_bins;
     if (net) {
         const double cprior = (h[2] * std::log(h[3]) - std::lgamma(h[2])) - (h[5] * std::log(h[6]) - std::lgamma(h[5]));
-        k_vbn_update<<<blocks, 256, 0, s>>>(ctx->dv_q, d_gT, d_alpha, events, d_lrho, (int)N, (int)B, h[0], betav, h[2], h[3], h[4], h[5], h[6],
-                                            cprior, scale, step, (unsigned long long *)d_change, d_psum);
+        k_dvb_update<true><<<blocks, 256, 0, s>>>(st.q, d_gT, d_alpha, events, d_lrho, (int)N, (int)B, h[0], betav, h[2], h[3], h[4], h[5], h[6],
+                                                  cprior, scale, step, (unsigned long long *)d_change, d_psum);
         NHP_LAUNCHED(ctx);
-        k_vbn_finish<<<1, 256, 0, s>>>(ctx->dv_q + vbn_q_doubles(N, B) - 2, d_psum, (int)blocks, h[7], h[8], (double)NN, step,
-                                       (unsigned long long *)d_change);
+        k_vbn_finish<<<1, 256, 0, s>>>(st.q + st.doubles - 2, d_psum, (int)blocks, h[7], h[8], (double)NN, step, (unsigned long long *)d_change);
         NHP_LAUNCHED(ctx);
     } else {
-        k_vb_update<<<blocks, 256, 0, s>>>(ctx->dv_q, d_gT, d_alpha, events, (int)N, (int)B, h[0], betav, h[2], h[3], h[4], scale, step,
-                                           (unsigned long long *)d_change);
+        k_dvb_update<false><<<blocks, 256, 0, s>>>(st.q, d_gT, d_alpha, events, nullptr, (int)N, (int)B, h[0], betav, h[2], h[3], h[4], 0.0, 0.0, 0.0,
+                                                   scale, step, (unsigned long long *)d_change, nullptr);
         NHP_LAUNCHED(ctx);
     }
     NHP_CUDA(ctx, cudaGetLastError());
-    if (ctx->dv_trace_cap > 0 && ctx->dv_trace_len < ctx->dv_trace_cap) {  // the state of this step stays on the device
-        const size_t n = vb_state_doubles(N, B, net);
-        NHP_CUDA(ctx, cudaMemcpyAsync(ctx->dv_trace + (size_t)ctx->dv_trace_len * n, ctx->dv_q, n * sizeof(double), cudaMemcpyDeviceToDevice, s));
-        ctx->dv_trace_len++;
-    }
+    NHP_TRY(nhp_vb_trace_push(ctx, st));  // the state of this step stays on the device
     if (change) {
         NHP_CUDA(ctx, cudaMemcpyAsync(change, d_change, sizeof(double), cudaMemcpyDeviceToHost, s));
         NHP_CUDA(ctx, cudaStreamSynchronize(s));
@@ -298,46 +222,21 @@ extern "C" int nhp_disc_svi_step(nhp_ctx *ctx, nhp_disc *dd, int64_t t_begin, in
 
 extern "C" int nhp_disc_vb_trace_free(nhp_ctx *ctx) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    cudaSetDevice(ctx->device);
-    cudaStreamSynchronize(ctx->stream);
-    cudaFree(ctx->dv_trace);
-    ctx->dv_trace = nullptr; ctx->dv_trace_cap = ctx->dv_trace_len = 0;
+    nhp_trace_free(ctx, ctx->dvb.trace);
     return NHP_OK;
 }
 
 extern "C" int nhp_disc_vb_trace_begin(nhp_ctx *ctx, int64_t capacity) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, ctx->dv_set, NHP_ERR_STATE, "nhp_disc_vb_trace_begin: no VB state (the slot size follows it; call nhp_disc_vb_set)");
-    NHP_CHECK(ctx, capacity >= 1, NHP_ERR_INVALID, "nhp_disc_vb_trace_begin: capacity must be positive");
-    NHP_TRY(nhp_disc_vb_trace_free(ctx));
-    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = vb_state_doubles(ctx->dv_N, ctx->dv_B, ctx->dv_network);
-    if (cudaMalloc(&ctx->dv_trace, (size_t)capacity * n * sizeof(double)) != cudaSuccess) {
-        cudaGetLastError();
-        ctx->dv_trace = nullptr;
-        return nhp_fail(ctx, NHP_ERR_CUDA, "nhp_disc_vb_trace_begin: cannot allocate %lld slots of %.2f MB", (long long)capacity, 1e-6 * (double)(n * 8));
-    }
-    ctx->dv_trace_cap = capacity; ctx->dv_trace_len = 0; ctx->dv_trace_N = ctx->dv_N; ctx->dv_trace_B = ctx->dv_B;
-    ctx->dv_trace_network = ctx->dv_network;
-    return NHP_OK;
+    return nhp_vb_trace_begin(ctx, ctx->dvb, "nhp_disc_vb_trace_begin", "nhp_disc_vb_set", capacity);
 }
 
 extern "C" int nhp_disc_vb_trace_count(const nhp_ctx *ctx, int64_t *count, int64_t *capacity) {
     if (!ctx) return NHP_ERR_INVALID;
-    if (count) *count = ctx->dv_trace_len;
-    if (capacity) *capacity = ctx->dv_trace_cap;
-    return NHP_OK;
+    return nhp_trace_count(ctx->dvb.trace, count, capacity);
 }
 
 extern "C" int nhp_disc_vb_trace_read(nhp_ctx *ctx, int64_t first, int64_t count, double *q_out) {
     NHP_CHECK(ctx, ctx != nullptr, NHP_ERR_INVALID, "ctx is NULL");
-    NHP_CHECK(ctx, first >= 0 && count >= 0 && first + count <= ctx->dv_trace_len, NHP_ERR_INVALID, "nhp_disc_vb_trace_read: slots [%lld, %lld) outside the %lld stored",
-              (long long)first, (long long)(first + count), (long long)ctx->dv_trace_len);
-    if (count == 0) return NHP_OK;
-    NHP_CHECK(ctx, q_out != nullptr, NHP_ERR_INVALID, "nhp_disc_vb_trace_read: NULL argument");
-    NHP_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = vb_state_doubles(ctx->dv_trace_N, ctx->dv_trace_B, ctx->dv_trace_network);
-    NHP_CUDA(ctx, cudaMemcpyAsync(q_out, ctx->dv_trace + (size_t)first * n, (size_t)count * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    NHP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return NHP_OK;
+    return nhp_vb_trace_read(ctx, ctx->dvb, "nhp_disc_vb_trace_read", first, count, q_out);
 }

@@ -78,12 +78,10 @@ extern "C" int nhp_destroy(nhp_ctx *ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     nhp_comm_destroy(ctx);
-    nhp_cont_trace_free(ctx);
-    nhp_disc_trace_free(ctx);
-    nhp_disc_vb_trace_free(ctx);
-    cudaFree(ctx->dv_q);
-    nhp_cont_vb_trace_free(ctx);
-    cudaFree(ctx->cv_q);
+    nhp_trace_free(ctx, ctx->cont_trace);
+    nhp_trace_free(ctx, ctx->disc_trace);
+    nhp_vb_state_free(ctx, ctx->dvb);
+    nhp_vb_state_free(ctx, ctx->cvb);
     nhp_big_flush(ctx);
     free_cont(ctx);
     cudaFree(ctx->d_partials); cudaFree(ctx->d_scratch); cudaFree(ctx->d_flag); cudaFree(ctx->d_winstat);

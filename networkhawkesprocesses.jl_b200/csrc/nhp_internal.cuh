@@ -132,6 +132,37 @@ struct nhp_disc {
     int64_t *d_scan = nullptr;  // exclusive scan of data in memory order (uniform index of each bin's first draw)
 };
 
+// the model shape a trace was begun for, compared whole: continuous Gibbs (K, kind, has_A, G), discrete Gibbs (N, B, has_A, 0),
+// VB (N | K, B | kind, network, 0)
+struct TraceShape {
+    int64_t n = 0, b = 0, a = 0, g = 0;
+    bool operator==(const TraceShape &o) const { return n == o.n && b == o.b && a == o.a && g == o.g; }
+};
+
+// a device-side trace (cont_trace.cu): cap slots, each of `doubles` doubles, `words` bit-packed adjacency words and `curve_doubles`
+// doubles of curves (the last two optional), filled by device-to-device copies on the context's stream and read back at the end
+struct DeviceTrace {
+    double *d = nullptr;
+    uint32_t *bits = nullptr;
+    double *curves = nullptr;
+    size_t doubles = 0, words = 0, curve_doubles = 0;  // per slot
+    int64_t cap = 0, len = 0;
+    TraceShape shape;
+    // the doubles of the next slot, or nullptr when the trace is closed or full
+    double *next() const { return len < cap ? d + (size_t)len * doubles : nullptr; }
+};
+
+// a mean-field VB state (vb_state.cu) of the discrete (disc_vb.cu) or the continuous (cont_vb.cu) model and its trace
+struct VbState {
+    bool set = false, network = false;
+    int64_t n = 0, b = 0;  // N and B (discrete), K and the impulse kind (continuous)
+    double dt = 1.0;
+    double hyper[12] = {0};
+    double *q = nullptr;
+    size_t doubles = 0, cap = 0;  // doubles of the state, doubles allocated
+    DeviceTrace trace;
+};
+
 struct nhp_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -184,10 +215,9 @@ struct nhp_ctx {
     unsigned long long *d_adj_stat = nullptr;  // [8] sweep diagnostics (steps, batches, flips, recomputed steps)
     double *d_save = nullptr;     // nhp_cont_params_save: [K + 4 K^2] copy of lambda0, W, A, p1, p2
     double rho = -1.0;            // link probability of the Bernoulli network kept with the context (nhp_cont_resample_network)
-    // device-side sample trace (cont_trace.cu): [trace_cap] slots of (rho, lambda0, W, p1 [, p2]) + bit-packed adjacency matrices
-    double *d_trace = nullptr; uint32_t *d_trace_bits = nullptr;
-    int64_t trace_cap = 0, trace_len = 0, trace_K = 0; int trace_kind = 0; bool trace_has_A = false;
-    double *d_trace_curves = nullptr; int64_t trace_G = 0;  // [trace_cap][K][trace_G] curves, for a trace begun with curves and a prior
+    // sample trace: slots of (rho, lambda0, W, p1 [, p2]) + bit-packed adjacency matrices, and the curves [K][G] for a trace begun
+    // with curves and a prior
+    DeviceTrace cont_trace;
     double sweep_info[8] = {0};   // last nhp_cont_gibbs_sweep: ms of the parent sweep, of (second pass + draws + tables), of the adjacency kernel, of the curves' slice update, its rounds
     double adj_info[8] = {0};     // last adjacency sweep: steps, batches, flips, recomputed steps, entries, chunks, kernel ms, build ms
 
@@ -232,28 +262,20 @@ struct nhp_ctx {
     double *dd_counts = nullptr;  // [N * (1 + N B)] counts of the last discrete Gibbs parent sweep (counts[c + N k]), kept for the device-side draws
     size_t dd_counts_cap = 0; int64_t dd_counts_N = 0, dd_counts_B = 0;
     int64_t dd_maxNA = 0;
-    // discrete sample trace (cont_trace.cu): [dd_trace_cap] slots of (rho, lambda0, W, theta) + bit-packed adjacency matrices
-    double *dd_trace = nullptr; uint32_t *dd_trace_bits = nullptr;
-    int64_t dd_trace_cap = 0, dd_trace_len = 0, dd_trace_N = 0, dd_trace_B = 0; bool dd_trace_has_A = false;
+    // discrete sample trace: slots of (rho, lambda0, W, theta) + bit-packed adjacency matrices
+    DeviceTrace disc_trace;
 
-    // ---- discrete mean-field VB (disc_vb.cu): q = [alphav(N); betav(N); gammav(N^2 B); kappav(N^2); nuv(N^2)] and its trace; a
-    // network state (dv_network) appends [kappa0v(N^2); nu0v(N^2); pv(N^2); alpharhov; betarhov]
-    bool dv_set = false, dv_network = false;
-    int64_t dv_N = 0, dv_B = 0;
-    double dv_dt = 1.0, dv_hyper[9] = {0};  // alpha0, beta0, kappa, nu, gamma (+ kappa0, nu0, alpha_rho, beta_rho for a network state)
-    double *dv_q = nullptr; size_t dv_cap = 0;  // doubles allocated
-    double *dv_trace = nullptr;                 // [dv_trace_cap] slots of q for (dv_trace_N, dv_trace_B, dv_trace_network)
-    int64_t dv_trace_cap = 0, dv_trace_len = 0, dv_trace_N = 0, dv_trace_B = 0; bool dv_trace_network = false;
+    // ---- discrete mean-field VB (disc_vb.cu): q = [alphav(N); betav(N); gammav(N^2 B); kappav(N^2); nuv(N^2)]; a network state
+    // appends [kappa0v(N^2); nu0v(N^2); pv(N^2); alpharhov; betarhov].  hyper: alpha0, beta0, kappa, nu, gamma (+ kappa0, nu0,
+    // alpha_rho, beta_rho for a network state)
+    VbState dvb;
 
     // ---- continuous mean-field VB (cont_vb.cu): q = [alphav(K); betav(K); kappav(K^2); nuv(K^2)], then Exponential atheta(K^2);
     // btheta(K^2) | LogitNormal mv(K^2); lambdav(K^2); av(K^2); bv(K^2); the kind and K of the parameters at nhp_cont_vb_set; a network
-    // state (cv_network) appends [kappa0v(K^2); nu0v(K^2); pv(K^2); alpharhov; betarhov]
-    bool cv_set = false, cv_network = false;
-    int cv_kind = 0; int64_t cv_K = 0;
-    double cv_hyper[12] = {0};                  // alpha0, beta0, kappa, nu, then alpha, beta, 0, 0 | mumu, kappamu, a0, b0; then kappa0, nu0, alpha_rho, beta_rho (network)
-    double *cv_q = nullptr; size_t cv_cap = 0;  // doubles allocated: the state, one change slot behind it, and for a network state lrho and the block sums of pv
-    double *cv_trace = nullptr;                 // [cv_trace_cap] slots of q for (cv_trace_kind, cv_trace_K, cv_trace_network)
-    int64_t cv_trace_cap = 0, cv_trace_len = 0, cv_trace_K = 0; int cv_trace_kind = 0; bool cv_trace_network = false;
+    // state appends [kappa0v(K^2); nu0v(K^2); pv(K^2); alpharhov; betarhov].  hyper: alpha0, beta0, kappa, nu, then alpha, beta, 0, 0 |
+    // mumu, kappamu, a0, b0; then kappa0, nu0, alpha_rho, beta_rho (network).  Allocated behind q: one change slot, and for a network
+    // state lrho and the block sums of pv
+    VbState cvb;
 };
 
 // launch bookkeeping
@@ -263,6 +285,27 @@ int nhp_scratch(nhp_ctx *ctx, size_t bytes, void **out);
 int nhp_partials(nhp_ctx *ctx, int64_t count, double **out);
 int nhp_timer_begin(nhp_ctx *ctx);
 int nhp_timer_end(nhp_ctx *ctx);  // synchronises the stream and stores last_ms
+
+// device traces (cont_trace.cu).  begin: refuses capacity < 1, frees the trace, allocates capacity slots for shape (a failed
+// allocation leaves it closed); free: synchronises the stream, releases the buffers and closes the trace
+int nhp_trace_begin(nhp_ctx *ctx, DeviceTrace &tr, const char *fn, int64_t capacity, size_t doubles, size_t words, size_t curve_doubles,
+                    TraceShape shape);
+void nhp_trace_free(nhp_ctx *ctx, DeviceTrace &tr);
+int nhp_trace_count(const DeviceTrace &tr, int64_t *count, int64_t *capacity);
+int nhp_trace_check_range(nhp_ctx *ctx, const DeviceTrace &tr, const char *fn, int64_t first, int64_t count);  // slots [first, first + count) stored
+// doubles [off, off + n) of slots [first, first + count) to the host, one slot after the other (nothing for out == NULL); stream-ordered
+int nhp_trace_read_field(nhp_ctx *ctx, const DeviceTrace &tr, int64_t first, int64_t count, size_t off, size_t n, double *out);
+
+// VB states (vb_state.cu).  set: every entry of q positive and finite, except [fin_lo, fin_hi) (finite) and [p_lo, p_hi) (a link
+// probability in [0, 1]); refused before anything changes.  Then the buffer grows to alloc doubles, q is uploaded (synchronised: the
+// caller may reuse q) and the state takes the shape (n, b, network); the caller adds dt and the hyper-parameters
+int nhp_vb_state_set(nhp_ctx *ctx, VbState &st, const char *fn, const double *q, size_t doubles, size_t alloc, size_t fin_lo, size_t fin_hi,
+                     size_t p_lo, size_t p_hi, int64_t n, int64_t b, bool network);
+int nhp_vb_state_get(nhp_ctx *ctx, const VbState &st, const char *fn, const char *set_fn, double *q);
+void nhp_vb_state_free(nhp_ctx *ctx, VbState &st);
+int nhp_vb_trace_begin(nhp_ctx *ctx, VbState &st, const char *fn, const char *set_fn, int64_t capacity);  // slots of the state's q
+int nhp_vb_trace_push(nhp_ctx *ctx, VbState &st);  // the state into the next slot of an open trace that is not full; stream-ordered
+int nhp_vb_trace_read(nhp_ctx *ctx, const VbState &st, const char *fn, int64_t first, int64_t count, double *q_out);
 
 // ---------------------------------------------------------------------------------------
 // device helpers

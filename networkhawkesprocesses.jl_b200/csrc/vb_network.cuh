@@ -1,6 +1,6 @@
 // vb_network.cuh -- pieces of the mean-field VB steps shared by the discrete (disc_vb.cu) and continuous (cont_vb.cu) paths: the
-// relative change and blend of an entry of q, the link probability's sigmoid, and the fixed-order reduction of the link probabilities
-// into q(rho) of a network state.
+// relative change and blend of an entry of q, the link probability's sigmoid, the end-of-kernel reduction of the update kernels, and
+// the fixed-order reduction of the link probabilities into q(rho) of a network state.
 #pragma once
 #include "nhp_internal.cuh"
 
@@ -13,6 +13,31 @@ __device__ __forceinline__ double stable_sigmoid(double x) {
     if (x >= 0.0) return 1.0 / (1.0 + exp(-x));
     const double z = exp(x);
     return z / (1.0 + z);
+}
+
+// the end of an update kernel of 256-thread blocks: the block's largest mx into *change (an integer atomicMax per warp: the bit order
+// of non-negative doubles is their numeric order); NET: also the block's sum of pt into psum[blockIdx.x] (a fixed shuffle tree, then
+// the warps in order), so the same inputs give the same bits
+template <bool NET>
+__device__ __forceinline__ void vb_block_reduce(double mx, double pt, unsigned long long *change, double *psum) {
+    __shared__ double warp_sum[8];
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) {
+        mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, d));
+        if constexpr (NET) pt += __shfl_xor_sync(0xffffffffu, pt, d);
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (mx > 0.0) atomicMax(change, (unsigned long long)__double_as_longlong(mx));
+        if constexpr (NET) warp_sum[threadIdx.x >> 5] = pt;
+    }
+    if constexpr (NET) {
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double t = 0.0;
+            for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += warp_sum[w];
+            psum[blockIdx.x] = t;
+        }
+    }
 }
 
 // one block of 256: S = sum of the nblocks partial sums in a fixed order, then alpharhov* = alpha_rho + S, betarhov* = beta_rho + N^2 - S
